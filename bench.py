@@ -2,8 +2,13 @@
 """
 bench.py — natgrad_step datapoints/s of the B200 t-SVGP path (BASELINE.json metric), one JSON line on rank 0.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
+
+`--dump-outputs DIR` writes the sites the last timed step left behind (what a caller of natgrad_step reads back: lambda_1 [M, L],
+lambda_2_sqrt [L, M, M]) as DIR/<name>.npy in float64, at most 64 MB in all; an array that does not fit is written as a fixed,
+seeded sample of its rows (see dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared
+array for array.
 
 Workload: BASELINE.json's metric is quoted "at 1/2/4/8 B200", which is configs[2] (cfg3: N=10M, M=2048, D=16, Matern-5/2, minibatch 1M
 "sharded over 1/2/4/8 B200"); configs[1] (cfg2) is pinned to one B200 and holds 0.15 ms of FP64 work per step, so it measures launch
@@ -79,7 +84,34 @@ def parse():
     ap.add_argument("--keep-cache", action="store_true", help="do not invalidate the kernel-matrix factors every step")
     ap.add_argument("--opt", action="append", default=[], help="library option name=value (tsvgp_set_option), repeatable")
     ap.add_argument("--no-balance", action="store_true", help="several GPUs: equal row shares and both preparation chains on every rank")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the sites of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times bounded samples, not the whole step")
+    return args
+
+
+DUMP_BYTES = 63_900_000   # array data of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float64, DUMP_BYTES in all.  Smallest first, each array may take an even share of
+    what is left; one larger than its share is viewed as rows of its last axis, and the rows
+    sorted(np.random.default_rng(0).choice(n_rows, k, replace=False)) are written, k as many as fit in the share."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].nbytes)
+    left = DUMP_BYTES
+    for i, (name, a) in enumerate(items):
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            rows = a.reshape(-1, a.shape[-1])
+            k = share // rows[0].nbytes
+            a = rows[np.sort(np.random.default_rng(0).choice(rows.shape[0], k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
 
 
 # ---- clocks -------------------------------------------------------------------------------------------------------------
@@ -465,6 +497,8 @@ def main():
 
     # ---------- value: device-resident inputs ----------
     res = timed_steps(model, rk, mbs_dev, cfg["lr"], Nb, args.warmup, args.steps, invalidate)
+    if args.dump_outputs and rank == 0:   # the dense phase is replicated: every rank holds the same sites
+        dump_outputs(args.dump_outputs, {"lambda_1": model.lambda_1, "lambda_2_sqrt": model.lambda_2_sqrt})
     ms_per_step, value, launches, phase, clocks = res["ms_per_step"], res["value"], res["launches"], res["phase"], res["clocks"]
     step_resident = res["step"]
     route = model.timings()
