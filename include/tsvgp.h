@@ -86,6 +86,7 @@ TSVGP_API int tsvgp_set_option(tsvgp_ctx* ctx, const char* name, double value); 
  * "async_issue" (1 = at M <= 1024 a helper host thread enqueues the Kuu + jitter I factorisation chain on the side stream while
  *          the calling thread enqueues the posterior chain; 0 = one thread enqueues both),
  * "mc_seed" (Softmax: key of the Monte-Carlo generator; resets the draw counter),
+ * "sample_seed" (tsvgp_predict_f_samples: key of its own generator; resets its own draw counter — never touches "mc_seed"'s),
  * "speculate" (1 = automatic route: when this context's last conditioning estimate chose the fused route, run the
  *          Kuu + jitter I chain UNDERNEATH the streaming pass instead of in front of it, read the probe after the pass and
  *          repeat the pass with the right route if the estimate crossed the threshold; 0 = always probe before the pass),
@@ -156,6 +157,18 @@ TSVGP_API int tsvgp_elbo_grad(tsvgp_ctx* ctx, double scale, double* elbo, double
                               double* d_Z, double* d_lik);
 /* base_SVGP.predict_f, full_cov = False (tsvgp.py:97-114): mean_out, var_out [N, L]                                     */
 TSVGP_API int tsvgp_predict_f(tsvgp_ctx* ctx, const double* Xnew, int64_t N, int D, const double* mean_X, double* mean_out, double* var_out);
+/* base_SVGP.predict_f, full_cov = True (tsvgp.py:97-114 -> GPflow conditional): mean_out [N, L], cov_out [L, N, N] with
+ * Sigma_l = k(X, X) - V_l^T V_l, V_l = T_l^T Kuf (DESIGN 13).  Only the diagonal of Sigma_l is checked for positivity
+ * (TSVGP_ERR_NONPOSITIVE_VARIANCE).  Not collective.  Not built for the whitened sibling (TSVGP_ERR_INVALID).  The N x N
+ * buffers must fit in free device memory, else TSVGP_ERR_INVALID (message: bytes needed) before anything is allocated.     */
+TSVGP_API int tsvgp_predict_f_full_cov(tsvgp_ctx* ctx, const double* Xnew, int64_t N, int D, const double* mean_X,
+                                       double* mean_out, double* cov_out);
+/* GPModel.predict_f_samples: samples_out [S, N, L].  full_cov = 1: mean + chol(Sigma_l + 1e-6 I) eps (a failed Cholesky is
+ * TSVGP_ERR_NOT_POSITIVE_DEFINITE, tsvgp_last_info() = 1-based query point); 0: mean + sqrt(var) eps (also for the whitened
+ * sibling).  eps [S, N, L] (HOST or DEVICE) or NULL = Philox draws keyed by option "sample_seed", a new draw per call.
+ * Not collective; the sites and cached factors are left unchanged.                                                       */
+TSVGP_API int tsvgp_predict_f_samples(tsvgp_ctx* ctx, const double* Xnew, int64_t N, int D, const double* mean_X, int S,
+                                      int full_cov, const double* eps, double* samples_out);
 /* t_SVGP_white.predict_f_extra_data (tsvgp_white.py:134-158; whitened sibling only): predictions at Xnew after conditioning the
  * current sites on the RESIDENT minibatch (the "extra data") without changing them; jitter is the reference's argument
  * (default gpflow default_jitter = 1e-6; its test passes 0).  mean_out, var_out [N, L].                                   */

@@ -69,6 +69,9 @@ _SIGNATURES = {
     "tsvgp_prior_kl": (C.c_int, [C.c_void_p, _dp]),
     "tsvgp_elbo_grad": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp, C.c_void_p, C.c_void_p, _dp]),
     "tsvgp_predict_f": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tsvgp_predict_f_full_cov": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "tsvgp_predict_f_samples": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                          C.c_void_p]),
     "tsvgp_predict_f_extra_data": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p]),
     "tsvgp_posterior": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "tsvgp_comm_unique_id": (C.c_int, [C.c_void_p]),

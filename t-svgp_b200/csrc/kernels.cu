@@ -444,6 +444,72 @@ int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s) {
     return count_launch();
 }
 
+// ---- posterior samples ------------------------------------------------------------------------------------------------------
+// eps(2 sp, n, l) and eps(2 sp + 1, n, l): one Philox block gives both draws of a sample pair
+__device__ __forceinline__ void sample_pair(const SampleArgs& a, long n, int sp, int l, double& z0, double& z1) {
+    const int s0 = 2 * sp;
+    if (a.eps) {
+        z0 = a.eps[((long)s0 * a.N + n) * a.L + l];
+        z1 = s0 + 1 < a.S ? a.eps[((long)(s0 + 1) * a.N + n) * a.L + l] : 0.0;
+    } else {
+        normal_pair(a.seed, a.draw, (unsigned long long)n, (unsigned)sp, (unsigned)l, z0, z1);
+    }
+}
+
+__global__ void __launch_bounds__(256) sample_normals_kernel(SampleArgs a, int l, double* __restrict__ E, long ld, long Np) {
+    const long half = ld >> 1;
+    const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= Np * half) return;
+    const long n = t / half;
+    const int sp = (int)(t - n * half);
+    double z0 = 0.0, z1 = 0.0;
+    if (n < a.N && 2 * sp < a.S) {
+        sample_pair(a, n, sp, l, z0, z1);
+        if (2 * sp + 1 >= a.S) z1 = 0.0;
+    }
+    *reinterpret_cast<double2*>(E + n * ld + 2 * sp) = make_double2(z0, z1);
+}
+int sample_normals_launch(const SampleArgs& a, int l, double* E, long ld, long Np, cudaStream_t s) {
+    if (ld & 1) return -1;
+    const long threads = Np * (ld >> 1);
+    sample_normals_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(a, l, E, ld, Np);
+    return count_launch();
+}
+
+__global__ void __launch_bounds__(256) add_mean_samples_kernel(const double* __restrict__ mean, const double* __restrict__ F, long ldf,
+                                                               long N, int S, int L, int l, double* __restrict__ out) {
+    const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;   // sample index fastest: coalesced reads of F's rows
+    if (t >= N * S) return;
+    const long n = t / S;
+    const int smp = (int)(t - n * S);
+    out[((long)smp * N + n) * L + l] = mean[n] + F[n * ldf + smp];
+}
+int add_mean_samples_launch(const double* mean, const double* F, long ldf, long N, int S, int L, int l, double* out, cudaStream_t s) {
+    add_mean_samples_kernel<<<(unsigned)((N * S + 255) / 256), 256, 0, s>>>(mean, F, ldf, N, S, L, l, out);
+    return count_launch();
+}
+
+__global__ void __launch_bounds__(256) diag_samples_kernel(SampleArgs a, const double* __restrict__ mean, const double* __restrict__ var,
+                                                           long ld, double* __restrict__ out) {
+    const int pairs = (a.S + 1) >> 1;
+    const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= a.N * pairs) return;
+    const long n = t / pairs;
+    const int sp = (int)(t - n * pairs);
+    for (int l = 0; l < a.L; ++l) {
+        double z0, z1;
+        sample_pair(a, n, sp, l, z0, z1);
+        const double mu = mean[(long)l * ld + n], sd = sqrt(var[(long)l * ld + n]);
+        out[((long)(2 * sp) * a.N + n) * a.L + l] = fma(sd, z0, mu);
+        if (2 * sp + 1 < a.S) out[((long)(2 * sp + 1) * a.N + n) * a.L + l] = fma(sd, z1, mu);
+    }
+}
+int diag_samples_launch(const SampleArgs& a, const double* mean, const double* var, long ld, double* out, cudaStream_t s) {
+    const long threads = a.N * ((a.S + 1) / 2);
+    diag_samples_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(a, mean, var, ld, out);
+    return count_launch();
+}
+
 __global__ void transpose_to_latent_major_kernel(const double* __restrict__ Y, long n, int L, double* __restrict__ Yt, long ld) {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;

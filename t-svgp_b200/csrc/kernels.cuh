@@ -70,6 +70,21 @@ int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s);
 int transpose_to_latent_major_launch(const double* Y, long n, int L, double* Yt, long ld, cudaStream_t s);
 int transpose_to_point_major_launch(const double* src, long ld, long n, int L, double* dst, cudaStream_t s);
 
+// Posterior samples (tsvgp_predict_f_samples).  The standard normal eps(s, n, l) is the explicit eps [S][N][L] when given, else
+// Philox4x32-10 + Box-Muller keyed by (seed, draw, point n, sample pair s / 2, latent l) — its own key, never the Softmax one.
+struct SampleArgs {
+    const double* eps;
+    unsigned long long seed, draw;
+    long N;
+    int S, L;
+};
+// E[n][s] = eps(s, n, l) for n < N and s < S, zero elsewhere; E [Np][ld], ld even and >= S
+int sample_normals_launch(const SampleArgs& a, int l, double* E, long ld, long Np, cudaStream_t s);
+// out[s][n][l] = mean[n] + F[n][s]   (F [N][ldf]: the correlated draw of latent l)
+int add_mean_samples_launch(const double* mean, const double* F, long ldf, long N, int S, int L, int l, double* out, cudaStream_t s);
+// out[s][n][l] = mean[l][n] + sqrt(var[l][n]) eps(s, n, l)  (mean, var [L][ld])
+int diag_samples_launch(const SampleArgs& a, const double* mean, const double* var, long ld, double* out, cudaStream_t s);
+
 struct GHTable { double z[MAX_GH]; double w[MAX_GH]; };   // nodes sqrt(2) x_k and weights w_k / sqrt(pi), passed by value
 int point_stats_launch(const LikSpec& lik, const PointArgs& a, const GHTable& gh, cudaStream_t s);
 

@@ -145,6 +145,7 @@ struct tsvgp_ctx {
     double* mc_eps = nullptr;  // explicit Monte-Carlo draws [S][mc_eps_n][L] of the Softmax likelihood (tsvgp_set_mc_epsilon) or null
     long mc_eps_n = 0;
     unsigned long long mc_seed = 0x5eed5eedULL, mc_draw = 0;   // Philox key and per-call draw counter otherwise
+    unsigned long long sample_seed = 0x5a3b1e5eULL, sample_draw = 0;   // the same for predict_f_samples (option "sample_seed")
     // inducing points and M x M state
     int M = 0, Mp = 0, D = 0;
     Pool pm;
@@ -1576,6 +1577,7 @@ int tsvgp_set_option(tsvgp_ctx* c, const char* name, double value) {
         c->route_opt = (int)value; c->k9_valid = false; return TSVGP_OK;
     }
     if (!strcmp(name, "mc_seed")) { c->mc_seed = (unsigned long long)value; c->mc_draw = 0; return TSVGP_OK; }
+    if (!strcmp(name, "sample_seed")) { c->sample_seed = (unsigned long long)value; c->sample_draw = 0; return TSVGP_OK; }
     if (!strcmp(name, "speculate")) { c->speculate = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "k9_defer")) { c->k9_defer = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "early_slabs")) { c->early_slabs = value < 0 ? 0 : (int)value; return TSVGP_OK; }
@@ -2221,6 +2223,164 @@ int tsvgp_predict_f(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const do
     OK(check_info(c, info_h));
     if (tail[1] != 0.0) FAIL(TSVGP_ERR_NONPOSITIVE_VARIANCE, "predict_f: non-positive predictive variance");
     return TSVGP_OK;
+}
+
+// The N x N path (DESIGN 13): cov_out != null -> predict_f(full_cov = True), mean_out [N, L], cov_out [L, N, N]; otherwise
+// predict_f_samples, samples_out [S, N, L].  Per latent l, in one Np x Np buffer:
+//   Sigma = k(X, X) (identity on the padding) ;  V = T_l^T Kuf ;  Sigma -= V^T V (lower tiles)
+//   covariance: mirror, copy [0, N)^2 out ;  samples: chol(Sigma + 1e-6 I) E_l + mean
+// The moments come from predict_f's own pass, so the means are predict_f's bits and the marginal variances are checked there.
+static int predict_full(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const double* mean_X, double* mean_out, double* cov_out,
+                        int S, int full_cov, const double* eps, double* samples_out) {
+    OK(require_model(c, false));
+    if (D != c->D) FAIL(TSVGP_ERR_INVALID, "Xnew has D=%d but the inducing points have D=%d", D, c->D);
+    const bool want_cov = cov_out != nullptr;
+    if (c->white && full_cov)
+        FAIL(TSVGP_ERR_INVALID, "full_cov is not built for the whitened sibling: its conditional computes the diagonal only "
+                                "(tsvgp_white.py:122-132)");
+    CU(cudaSetDevice(c->dev));
+    c->collective_ok = false;   // like predict_f: one rank may call it alone, so every product below stays on this GPU
+    cudaStream_t s = c->s_main;
+    const int L = c->L, Mp = c->Mp;
+    const long Np = round_up(N, 128), Sp = want_cov ? 0 : round_up(S, 128);
+    const bool x_host = !is_device_ptr(Xnew), eps_host = eps && !is_device_ptr(eps);
+    const bool out_host = !want_cov && !is_device_ptr(samples_out);
+    {   // every temporary below, counted before the first allocation
+        size_t need = (size_t)D * Np + Np + 2 * (size_t)L * Np + (mean_X ? Np : 0) + (x_host ? (size_t)N * D : 0) + (size_t)N * L;
+        if (full_cov) need += (size_t)Np * D + 2 * (size_t)Mp * Np + (size_t)Np * Np;
+        if (full_cov && !want_cov) need += (size_t)Np * 128 + 2 * (size_t)Np * Sp + L;
+        if (eps_host) need += (size_t)S * N * L;
+        if (out_host) need += (size_t)S * N * L;
+        size_t free_b = 0, total_b = 0;
+        CU(cudaMemGetInfo(&free_b, &total_b));
+        if (need * sizeof(double) > free_b)
+            FAIL(TSVGP_ERR_INVALID, "%s at N = %lld needs %zu bytes of device memory, %zu are free",
+                 want_cov ? "predict_f(full_cov = True)" : "predict_f_samples", (long long)N, need * sizeof(double), free_b);
+    }
+    CU(cudaMemsetAsync(c->info, 0, sizeof(int) * N_INFO, s));
+    OK(ensure_posterior(c));
+    Pool tp;
+    struct Rel { Pool& p; cudaStream_t s; ~Rel() { cudaStreamSynchronize(s); p.release(); } } rel{tp, s};
+    double *xsT, *x2, *md, *vd, *moff = nullptr;
+    const double* xsrc = Xnew;
+    if (x_host) {
+        double* xd;
+        NEED(xd = tp.get((size_t)N * D));
+        CU(cudaMemcpyAsync(xd, Xnew, sizeof(double) * (size_t)N * D, cudaMemcpyHostToDevice, s));
+        xsrc = xd;
+    }
+    NEED(xsT = tp.get((size_t)D * Np)); NEED(x2 = tp.get(Np)); NEED(md = tp.get((size_t)L * Np)); NEED(vd = tp.get((size_t)L * Np));
+    if (mean_X) {
+        NEED(moff = tp.get(Np));
+        CU(cudaMemcpyAsync(moff, mean_X, sizeof(double) * N, cudaMemcpyDefault, s));
+    }
+    LA(scale_points_launch(xsrc, N, D, c->ls_dev, xsT, Np, x2, Np, s));
+    OK(stream_pass(c, xsT, Np, x2, N, nullptr, moff, MODE_PREDICT, md, vd, PASS_WHOLE, 0, Np));   // exactly predict_f's moments
+
+    SampleArgs sa;
+    sa.eps = eps; sa.seed = c->sample_seed; sa.draw = c->sample_draw; sa.N = N; sa.S = S; sa.L = L;
+    double* out_d = samples_out;
+    if (!want_cov) {
+        ++c->sample_draw;   // a new draw per call
+        if (eps_host) {
+            double* e;
+            NEED(e = tp.get((size_t)S * N * L));
+            CU(cudaMemcpyAsync(e, eps, sizeof(double) * (size_t)S * N * L, cudaMemcpyHostToDevice, s));
+            sa.eps = e;
+        }
+        if (out_host) NEED(out_d = tp.get((size_t)S * N * L));
+    }
+    int* chol_info = nullptr;   // [L]: failing pivot of chol(Sigma_l + 1e-6 I), 1-based = query point
+    if (!full_cov) {
+        LA(diag_samples_launch(sa, md, vd, Np, out_d, s));
+    } else {
+        double *xr, *kuf, *V, *Sig, *dinv = nullptr, *E = nullptr, *F = nullptr;
+        NEED(xr = tp.get((size_t)Np * D)); NEED(kuf = tp.get((size_t)Mp * Np)); NEED(V = tp.get((size_t)Mp * Np));
+        NEED(Sig = tp.get((size_t)Np * Np));
+        LA(unpack_rows_launch(xsT, Np, (int)Np, D, xr, s));   // the query points as the row operand of k(X, X)
+        LA(kuf_launch(c->kern_kind, c->kern_var, xsT, Np, x2, 0, N, (int)Np, c->Zs, c->z2, c->M, Mp, D, nullptr, kuf, Np, nullptr, 0, 0, s));
+        if (!want_cov) {
+            NEED(dinv = tp.get((size_t)Np * 128)); NEED(E = tp.get((size_t)Np * Sp)); NEED(F = tp.get((size_t)Np * Sp));
+            NEED(chol_info = (int*)tp.get(L));
+            CU(cudaMemsetAsync(dinv, 0, sizeof(double) * (size_t)Np * 128, s));   // contract of diag_potrf_inv_launch
+            CU(cudaMemsetAsync(chol_info, 0, sizeof(int) * L, s));
+        }
+        for (int l = 0; l < L; ++l) {
+            select_latent(c, l);
+            // Sigma = k(X, X), recomputed per latent instead of keeping a second N x N copy
+            LA(kuf_launch(c->kern_kind, c->kern_var, xsT, Np, x2, 0, N, (int)Np, xr, x2, (int)N, (int)Np, D, nullptr, Sig, Np, nullptr, 0, 1, s));
+            {   // V = T^T Kuf  (the variance product of the pass, stored)
+                GemmP p;
+                p.A = c->T; p.lda = Mp; p.a_kc = 0; p.a_tri = 2;
+                p.B = kuf; p.ldb = Np; p.b_kc = 0;
+                p.C = V; p.ldc = Np; p.m = Mp; p.n = (int)Np; p.k = Mp;
+                LA(mm_gemm(c, p, s));
+            }
+            {   // Sigma -= V^T V  (lower tiles; split-K over idle SMs when Np is small)
+                GemmP p;
+                p.A = V; p.lda = Np; p.a_kc = 0;
+                p.B = V; p.ldb = Np; p.b_kc = 0;
+                p.C = Sig; p.ldc = Np; p.m = p.n = (int)Np; p.k = Mp;
+                p.alpha = -1.0; p.beta = 1.0; p.lower_out = 1;
+                LA(mm_gemm(c, p, s));
+            }
+            if (want_cov) {
+                LA(mirror_lower_launch(Sig, Np, (int)Np, s));
+                CU(cudaMemcpy2DAsync(cov_out + (size_t)l * N * N, sizeof(double) * N, Sig, sizeof(double) * Np, sizeof(double) * N, N,
+                                     cudaMemcpyDefault, s));
+                continue;
+            }
+            // gpflow sample_mvn: chol(Sigma + default_jitter I) eps.  The padding block stays the identity (V's padding columns are 0)
+            LA(add_diag_launch(Sig, Np, (int)Np, GPFLOW_DEFAULT_JITTER, s));
+            LA(chol_lower(Sig, Np, (int)Np, dinv, chol_info + l, s, c->gws, c->gws_doubles, &c->la_main));
+            LA(sample_normals_launch(sa, l, E, Sp, Np, s));
+            GemmP p;   // F = C E
+            p.A = Sig; p.lda = Np; p.a_kc = 1; p.a_tri = 1;
+            p.B = E; p.ldb = Sp; p.b_kc = 0;
+            p.C = F; p.ldc = Sp; p.m = (int)Np; p.n = (int)Sp; p.k = (int)Np;
+            LA(mm_gemm(c, p, s));
+            LA(add_mean_samples_launch(md + (size_t)l * Np, F, Sp, N, S, L, l, out_d, s));
+        }
+        select_latent(c, 0);
+    }
+    if (want_cov) {
+        if (L == 1) {
+            CU(cudaMemcpyAsync(mean_out, md, sizeof(double) * N, cudaMemcpyDefault, s));
+        } else {   // [L][Np] on the device -> the reference's [N, L]
+            double* mt;
+            NEED(mt = tp.get((size_t)N * L));
+            LA(transpose_to_point_major_launch(md, Np, N, L, mt, s));
+            CU(cudaMemcpyAsync(mean_out, mt, sizeof(double) * N * L, cudaMemcpyDefault, s));
+        }
+    } else if (out_host) {
+        CU(cudaMemcpyAsync(samples_out, out_d, sizeof(double) * (size_t)S * N * L, cudaMemcpyDeviceToHost, s));
+    }
+    std::vector<int> chol_h(chol_info ? L : 0);
+    if (chol_info) CU(cudaMemcpyAsync(chol_h.data(), chol_info, sizeof(int) * L, cudaMemcpyDeviceToHost, s));
+    double tail[4];
+    int info_h[N_INFO];
+    OK(read_tails(c, tail, nullptr, info_h));   // synchronises
+    OK(check_info(c, info_h));
+    if (tail[1] != 0.0) FAIL(TSVGP_ERR_NONPOSITIVE_VARIANCE, "predict_f: non-positive predictive variance");
+    for (int l = 0; l < (int)chol_h.size(); ++l)
+        if (chol_h[l]) {
+            c->last_info = chol_h[l];
+            FAIL(TSVGP_ERR_NOT_POSITIVE_DEFINITE, "Cholesky of Sigma + 1e-6 I (latent %d) failed at query point %d", l, chol_h[l]);
+        }
+    return TSVGP_OK;
+}
+
+int tsvgp_predict_f_full_cov(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const double* mean_X, double* mean_out, double* cov_out) {
+    if (!c) return TSVGP_ERR_INVALID;
+    if (!Xnew || !mean_out || !cov_out || N < 1) FAIL(TSVGP_ERR_INVALID, "Xnew [N >= 1, D], mean_out [N, L], cov_out [L, N, N] are required");
+    return predict_full(c, Xnew, N, D, mean_X, mean_out, cov_out, 0, 1, nullptr, nullptr);
+}
+
+int tsvgp_predict_f_samples(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const double* mean_X, int S, int full_cov,
+                            const double* eps, double* samples_out) {
+    if (!c) return TSVGP_ERR_INVALID;
+    if (!Xnew || !samples_out || N < 1 || S < 1) FAIL(TSVGP_ERR_INVALID, "Xnew [N >= 1, D] and samples_out [S >= 1, N, L] are required");
+    return predict_full(c, Xnew, N, D, mean_X, nullptr, nullptr, S, full_cov != 0, eps, samples_out);
 }
 
 int tsvgp_predict_f_extra_data(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const double* mean_X, double jitter,

@@ -332,25 +332,60 @@ class t_SVGP:
         self._check(self._lib.tsvgp_prior_kl(self._ctx, C.byref(out)))
         return out.value
 
-    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
-        """tsvgp.py:97-114 -> (mean [N, 1], var [N, 1]); raises if any variance is <= 0 (:113)."""
-        if full_cov or full_output_cov:
-            raise NotImplementedError("full_cov / full_output_cov: never exercised on this path by the reference")
+    def _query(self, Xnew):
+        """Xnew [N, D] (host array or DLPack device tensor, aliased) -> (tensor, N, D, mean_function(Xnew) [N] or None)."""
         self._sync_objects()
         tx = as_tensor(Xnew, "Xnew", self)
         if len(tx.shape) != 2:
             raise _lib.InvalidArgumentError(_lib.ERR_INVALID, "Xnew must be [N, D]")
         N, D = tx.shape
-        L = self.num_latent_gps
-        if N == 0:   # an empty query returns empty moments, as the reference's conditional does
-            return np.empty((0, L)), np.empty((0, L))
         mean_x = None
         if self._mean_fn(np.zeros((1, D))) is not None:
             mean_x = self._mean_fn(np.asarray(Xnew, dtype=np.float64))
+        return tx, N, D, mean_x
+
+    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
+        """tsvgp.py:97-114 -> (mean [N, L], var [N, L]); raises if any variance is <= 0 (:113).
+        full_cov=True -> (mean [N, L], cov [L, N, N]), GPflow's layouts; only the diagonal of cov is checked for positivity."""
+        if full_output_cov:
+            raise NotImplementedError("full_output_cov: never exercised on this path by the reference")
+        tx, N, D, mean_x = self._query(Xnew)
+        L = self.num_latent_gps
+        mx = None if mean_x is None else mean_x.ctypes.data
+        if full_cov:
+            if N == 0:
+                return np.empty((0, L)), np.empty((L, 0, 0))
+            mean, cov = np.empty((N, L)), np.empty((L, N, N))
+            self._check(self._lib.tsvgp_predict_f_full_cov(self._ctx, tx.ptr, N, D, mx, mean.ctypes.data, cov.ctypes.data))
+            return mean, cov
+        if N == 0:   # an empty query returns empty moments, as the reference's conditional does
+            return np.empty((0, L)), np.empty((0, L))
         mean, var = np.empty((N, L)), np.empty((N, L))
-        self._check(self._lib.tsvgp_predict_f(self._ctx, tx.ptr, N, D, None if mean_x is None else mean_x.ctypes.data,
-                                              mean.ctypes.data, var.ctypes.data))
+        self._check(self._lib.tsvgp_predict_f(self._ctx, tx.ptr, N, D, mx, mean.ctypes.data, var.ctypes.data))
         return mean, var
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, *, epsilon=None):
+        """GPModel.predict_f_samples -> [S, N, L], or [N, L] when num_samples is None.
+        full_cov=True: mean + chol(cov_l + 1e-6 I) eps per latent (gpflow sample_mvn); False: mean + sqrt(var) eps.
+        `epsilon [S, N, L]` fixes the standard-normal draws (as `set_mc_epsilon` does for Softmax); otherwise they come from the
+        library's Philox generator, option "sample_seed", a new draw per call."""
+        if full_output_cov:
+            raise NotImplementedError("full_output_cov: never exercised on this path by the reference")
+        tx, N, D, mean_x = self._query(Xnew)
+        L = self.num_latent_gps
+        S = 1 if num_samples is None else int(num_samples)
+        if S < 1:
+            raise _lib.InvalidArgumentError(_lib.ERR_INVALID, "num_samples must be >= 1")
+        eps = None
+        if epsilon is not None:
+            eps = as_tensor(epsilon, "epsilon", self)
+            if tuple(eps.shape) != (S, N, L):
+                raise _lib.InvalidArgumentError(_lib.ERR_INVALID, f"epsilon must be [{S}, {N}, {L}], got {tuple(eps.shape)}")
+        out = np.empty((S, N, L))
+        if N > 0:
+            self._check(self._lib.tsvgp_predict_f_samples(self._ctx, tx.ptr, N, D, None if mean_x is None else mean_x.ctypes.data,
+                                                          S, int(bool(full_cov)), None if eps is None else eps.ptr, out.ctypes.data))
+        return out[0] if num_samples is None else out
 
     def set_mc_epsilon(self, epsilon):
         """Softmax likelihood: fix the Monte-Carlo draws to `epsilon [S, N, L]` (GPflow's `epsilon` argument of
@@ -374,7 +409,9 @@ class t_SVGP:
     def predict_y(self, Xnew, full_cov=False, full_output_cov=False):
         """GPModel.predict_y -> likelihood.predict_mean_and_var(f_mean, f_var)."""
         from math import erf
-        mu, var = self.predict_f(Xnew, full_cov, full_output_cov)
+        if full_cov or full_output_cov:   # as GPflow 2.2.1's likelihoods: only the marginals are propagated
+            raise NotImplementedError("predict_y with full_cov / full_output_cov")
+        mu, var = self.predict_f(Xnew)
         name = type(self.likelihood).__name__
         if name == "Gaussian":
             return mu, var + float(_value(self.likelihood.variance))
@@ -387,9 +424,11 @@ class t_SVGP:
     def predict_log_density(self, data, full_cov=False, full_output_cov=False):
         """GPModel.predict_log_density -> log int p(y | f) q(f) df per point, [N]."""
         from math import lgamma
+        if full_cov or full_output_cov:
+            raise NotImplementedError("predict_log_density with full_cov / full_output_cov")
         X, Y = data
         Y = np.asarray(Y, dtype=np.float64)
-        mu, var = self.predict_f(X, full_cov, full_output_cov)
+        mu, var = self.predict_f(X)
         name = type(self.likelihood).__name__
         if name == "Gaussian":
             v = var + float(_value(self.likelihood.variance))
@@ -483,6 +522,16 @@ class t_SVGP_white(t_SVGP):
 
     def elbo_and_grad(self, data=None, *, global_minibatch_size=None):
         raise NotImplementedError("elbo_and_grad for t_SVGP_white")
+
+    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
+        if full_cov:   # the reference's whitened conditional computes the diagonal only (tsvgp_white.py:122-132)
+            raise NotImplementedError("full_cov for t_SVGP_white")
+        return super().predict_f(Xnew, full_cov, full_output_cov)
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, *, epsilon=None):
+        if full_cov:
+            raise NotImplementedError("full_cov for t_SVGP_white: pass full_cov=False")
+        return super().predict_f_samples(Xnew, num_samples, False, full_output_cov, epsilon=epsilon)
 
     def natgrad_step(self, data=None, lr=0.1, jitter=1e-9, *, global_minibatch_size=None, return_elbo=False):
         """tsvgp_white.py:215-246.  The reference accepts `jitter` but never forwards it: compute_data_natural_params is called
