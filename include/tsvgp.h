@@ -47,7 +47,8 @@ enum {
 };
 
 enum { TSVGP_KERNEL_SE = 0, TSVGP_KERNEL_MATERN52 = 1 };                       /* gpflow.kernels.{SquaredExponential,Matern52} */
-enum { TSVGP_LIK_GAUSSIAN = 0, TSVGP_LIK_BERNOULLI_PROBIT = 1, TSVGP_LIK_STUDENT_T = 2, TSVGP_LIK_SOFTMAX = 3 }; /* gpflow.likelihoods.* */
+/* gpflow.likelihoods.*; TSVGP_LIK_HETEROSKEDASTIC: HeteroskedasticTFPConditional(distribution_class = Normal), see set_likelihood */
+enum { TSVGP_LIK_GAUSSIAN = 0, TSVGP_LIK_BERNOULLI_PROBIT = 1, TSVGP_LIK_STUDENT_T = 2, TSVGP_LIK_SOFTMAX = 3, TSVGP_LIK_HETEROSKEDASTIC = 4 };
 
 typedef struct tsvgp_ctx tsvgp_ctx;   /* opaque: owns one CUDA stream, device buffers, optional NCCL communicator */
 
@@ -99,11 +100,23 @@ TSVGP_API int tsvgp_set_option(tsvgp_ctx* ctx, const char* name, double value); 
  * pipeline; TSVGP_FUSED_SPLITK=1 the fused (last-CTA) split-K reduction; TSVGP_DEBUG_SYNC=1 synchronise after every launch. */
 
 /* ---- model objects read by the path (tsvgp.py:209,268-269; GPflow kernel / likelihood / inducing attributes) ------ */
-/* lengthscales: HOST pointer, n_ls = 1 (isotropic) or D (ARD)                                                          */
+/* lengthscales: HOST pointer, n_ls = 1 (isotropic) or D (ARD).  One kernel shared by every latent (returns a context in
+ * separate-kernel mode to shared mode).                                                                                */
 TSVGP_API int tsvgp_set_kernel(tsvgp_ctx* ctx, int kind, double variance, const double* lengthscales, int n_ls);
+/* One kernel PER LATENT (gpflow.kernels.SeparateIndependent with SharedIndependentInducingVariables): kinds, variances and
+ * n_ls have L = tsvgp_num_latent entries (HOST); lengthscales holds the latents' n_ls[l] (1 or D) entries back to back.
+ * Every latent then uses its own Kuu_l, Kuu_l + 1e-6 I, Kuu_l + jitter I and Kuf_l; the conditional, the KL and the site update
+ * of each latent keep their form with these matrices.  Validated as tsvgp_set_kernel.  tsvgp_set_num_latent with a different L
+ * drops the per-latent kernels (compute calls return TSVGP_ERR_STATE until the next set_kernels / set_kernel).  Not built:
+ * option "white" = 1 and tsvgp_elbo_grad (TSVGP_ERR_INVALID).  Memory per extra latent: 5 M x M matrices and a scaled copy of
+ * the resident X.                                                                                                      */
+TSVGP_API int tsvgp_set_kernels(tsvgp_ctx* ctx, const int* kinds, const double* variances, const double* lengthscales, const int* n_ls);
 /* Gaussian: p0 = variance.  StudentT: p0 = scale, p1 = df.  Bernoulli: inv_probit link with GPflow's 1e-3 jitter.
  * n_gh Gauss-Hermite points (<= 64; GPflow default 20); gh_x/gh_w (HOST, numpy.polynomial.hermite.hermgauss order)
- * may be NULL, in which case the library generates them.                                                               */
+ * may be NULL, in which case the library generates them.
+ * Heteroskedastic: log p(y | f) = Normal(loc = f_0, scale = T(f_1)).log_prob(y) over L = 2 latents (checked at the first compute
+ * call), p0 = 0: T = exp, 1: T = softplus; the expectation is the n_gh x n_gh Gauss-Hermite grid (GPflow NDiagGHQuadrature).
+ * Y [N, 1] like Softmax; tsvgp_elbo_grad and option "white" are not built for it.                                      */
 TSVGP_API int tsvgp_set_likelihood(tsvgp_ctx* ctx, int kind, double p0, double p1, int n_gh, const double* gh_x, const double* gh_w);
 /* Z [M, D] inducing inputs (inducing_variable.Z); mean_Z [M] = mean_function(Z) or NULL for the Zero mean function     */
 TSVGP_API int tsvgp_set_inducing(tsvgp_ctx* ctx, const double* Z, int M, int D, const double* mean_Z);

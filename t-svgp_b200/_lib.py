@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libtsvgp.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOT_PD, ERR_NONPOS_VAR, ERR_COMM, ERR_STATE = 0, -1, -2, -3, -4, -5, -6
 KERNEL_SE, KERNEL_MATERN52 = 0, 1
-LIK_GAUSSIAN, LIK_BERNOULLI_PROBIT, LIK_STUDENT_T, LIK_SOFTMAX = 0, 1, 2, 3
+LIK_GAUSSIAN, LIK_BERNOULLI_PROBIT, LIK_STUDENT_T, LIK_SOFTMAX, LIK_HETEROSKEDASTIC = 0, 1, 2, 3, 4
 ABI_VERSION = 1
 
 
@@ -53,6 +53,7 @@ _SIGNATURES = {
     "tsvgp_last_info": (C.c_int, [C.c_void_p]),
     "tsvgp_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_double]),
     "tsvgp_set_kernel": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, C.c_int]),
+    "tsvgp_set_kernels": (C.c_int, [C.c_void_p, C.c_void_p, _dp, _dp, C.c_void_p]),
     "tsvgp_set_likelihood": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_int, _dp, _dp]),
     "tsvgp_set_inducing": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "tsvgp_set_num_latent": (C.c_int, [C.c_void_p, C.c_int]),

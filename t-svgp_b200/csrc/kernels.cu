@@ -383,7 +383,7 @@ __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
             double m = 0.0, q = 0.0;
             for (int p = 0; p < a.n_mu_part; ++p) m += a.mu_part[l * a.mu_lat + (long)p * a.ldmu + c];
             for (int p = 0; p < a.n_q_part; ++p) q += a.q_part[l * a.q_lat + (long)p * a.ldq + c];
-            const double var = a.kdiag - q;
+            const double var = a.kdiag[l] - q;
             mu[l] = m + off;
             bad = bad || !(var > 0.0);
             sd[l] = sqrt(var);
@@ -441,6 +441,94 @@ __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
 int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s) {
     if (a.L < 2 || a.L > MAX_SOFTMAX_CLASSES || a.S < 1) return -1;
     softmax_stats_kernel<<<(a.ncols + 127) / 128, 128, 0, s>>>(a);
+    return count_launch();
+}
+
+// ---- heteroskedastic Normal (2-D Gauss-Hermite) ------------------------------------------------------------------------
+// The integrand of every sum below is a product of a function of f_0 and one of f_1, so each double sum over the n_gh x n_gh
+// grid is the product of two single sums (the same value up to rounding).  With r = y - f_0, s = T(f_1), D = T'(f_1) / s and
+// E0[.] = sum_i w_i (.)(f_0 = mu_0 + sd_0 z_i), E1[.] = sum_j w_j (.)(f_1 = mu_1 + sd_1 z_j):
+//   ve = -1/2 log(2 pi) E0[1] E1[1] - E0[1] E1[log s] - 1/2 E0[r^2] E1[s^-2]
+//   d log p / d f_0 = r s^-2                     ->  g_0 = E0[r] E1[s^-2] ;            h_0 = E0[r z] E1[s^-2] / (2 sd_0)
+//   d log p / d f_1 = D (r^2 s^-2 - 1)           ->  g_1 = E0[r^2] E1[D s^-2] - E0[1] E1[D]
+//                                                    h_1 = (E0[r^2] E1[D s^-2 z] - E0[1] E1[D z]) / (2 sd_1)
+// (the pattern of the one-latent quadratures: d / d v_l = sum w d log p / d f_l z_l / (2 sd_l)).
+__global__ void __launch_bounds__(256) heteroskedastic_stats_kernel(LikSpec lk, SoftmaxArgs a, GHTable gh) {
+    __shared__ double sred[8];
+    const int c = blockIdx.x * 256 + threadIdx.x;
+    double ve = 0.0;
+    if (c < a.ncols) {
+        const bool valid = c < a.n_valid;
+        double mu[2], var[2];
+        for (int l = 0; l < 2; ++l) {
+            double m = 0.0, q = 0.0;
+            for (int p = 0; p < a.n_mu_part; ++p) m += a.mu_part[l * a.mu_lat + (long)p * a.ldmu + c];
+            for (int p = 0; p < a.n_q_part; ++p) q += a.q_part[l * a.q_lat + (long)p * a.ldq + c];
+            mu[l] = m;
+            var[l] = a.kdiag[l] - q;
+            if (valid && a.mean_out) { a.mean_out[l * a.out_lat + c] = mu[l]; a.var_out[l * a.out_lat + c] = var[l]; }
+        }
+        const bool bad = !(var[0] > 0.0) || !(var[1] > 0.0);
+        if (valid && bad) atomicOr(a.flags, 1);
+        double g0 = 0.0, g1 = 0.0, h0 = -1e-8, h1 = -1e-8;
+        if (valid && a.y && !bad) {
+            const double y = a.y[c], sd0 = sqrt(var[0]), sd1 = sqrt(var[1]);
+            double s0 = 0.0, er = 0.0, er2 = 0.0, erz = 0.0;
+            double s1 = 0.0, elog = 0.0, eb = 0.0, edb = 0.0, edbz = 0.0, ed = 0.0, edz = 0.0;
+            for (int k = 0; k < lk.n_gh; ++k) {
+                const double w = gh.w[k], z = gh.z[k];
+                const double r = y - fma(sd0, z, mu[0]);
+                s0 += w;
+                er = fma(w, r, er);
+                er2 = fma(w, r * r, er2);
+                erz = fma(w, r * z, erz);
+                const double f1 = fma(sd1, z, mu[1]);
+                double logs, d;
+                if (lk.p0 == 0.0) {   // exp: log s = f_1, T' / T = 1
+                    logs = f1;
+                    d = 1.0;
+                } else {              // softplus(f) = log(1 + e^f), stable form; T' = sigmoid(f)
+                    const double e = exp(-fabs(f1));
+                    const double sp = fmax(f1, 0.0) + log1p(e);
+                    logs = log(sp);
+                    d = (f1 >= 0.0 ? 1.0 : e) / ((1.0 + e) * sp);
+                }
+                const double b = exp(-2.0 * logs);
+                s1 += w;
+                elog = fma(w, logs, elog);
+                eb = fma(w, b, eb);
+                edb = fma(w, d * b, edb);
+                edbz = fma(w, d * b * z, edbz);
+                ed = fma(w, d, ed);
+                edz = fma(w, d * z, edz);
+            }
+            ve = -0.91893853320467274178 * s0 * s1 - s0 * elog - 0.5 * er2 * eb;
+            g0 = er * eb;
+            h0 = fmin(erz * eb / (2.0 * sd0), -1e-8);
+            g1 = er2 * edb - s0 * ed;
+            h1 = fmin((er2 * edbz - s0 * edz) / (2.0 * sd1), -1e-8);
+        }
+        if (!(valid && a.y)) h0 = h1 = 0.0;
+        if (a.g) {
+            a.g[c] = valid ? g0 : 0.0; a.h[c] = valid ? h0 : 0.0;
+            a.g[a.gh_lat + c] = valid ? g1 : 0.0; a.h[a.gh_lat + c] = valid ? h1 : 0.0;
+        }
+        if (!valid) ve = 0.0;
+    }
+    if (a.ve_blocks) {
+        ve = warp_sum(ve);
+        if ((threadIdx.x & 31) == 0) sred[threadIdx.x >> 5] = ve;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double s = 0.0;
+            for (int w = 0; w < 8; ++w) s += sred[w];
+            a.ve_blocks[blockIdx.x] = s;
+        }
+    }
+}
+int heteroskedastic_stats_launch(const LikSpec& lik, const SoftmaxArgs& a, const GHTable& gh, cudaStream_t s) {
+    if (a.L != 2 || lik.n_gh < 1 || lik.n_gh > MAX_GH) return -1;
+    heteroskedastic_stats_kernel<<<(a.ncols + 255) / 256, 256, 0, s>>>(lik, a, gh);
     return count_launch();
 }
 

@@ -6,13 +6,13 @@
 namespace tsvgp {
 
 enum { KERN_SE = 0, KERN_MATERN52 = 1 };
-enum { LIK_GAUSSIAN = 0, LIK_BERNOULLI = 1, LIK_STUDENT_T = 2, LIK_SOFTMAX = 3 };
+enum { LIK_GAUSSIAN = 0, LIK_BERNOULLI = 1, LIK_STUDENT_T = 2, LIK_SOFTMAX = 3, LIK_HETEROSKEDASTIC = 4 };
 constexpr int MAX_SOFTMAX_CLASSES = 16;
 constexpr int MAX_GH = 64;
 
 struct LikSpec {
     int kind = LIK_GAUSSIAN;
-    double p0 = 1.0;   // Gaussian: variance ; StudentT: scale
+    double p0 = 1.0;   // Gaussian: variance ; StudentT: scale ; heteroskedastic: scale transform (0 = exp, 1 = softplus)
     double p1 = 3.0;   // StudentT: df
     double c0 = 0.0;   // StudentT: log-density constant
     int n_gh = 20;
@@ -28,6 +28,8 @@ int scale_points_launch(const double* X, long n, int D, const double* ls, double
 int kuf_launch(int kind, double variance, const double* XsT, long ldx, const double* x2, long n0, long n_valid, int ncols,
                const double* ZsT_rows /*Zs [Mp][D]*/, const double* z2, int M, int Mp, int D, const double* alpha, double* K,
                long ldk, double* mu_part, long ldmu, int pad_identity, cudaStream_t s, double* Kp = nullptr /* dk/dr2 slab */);
+
+struct GHTable { double z[MAX_GH]; double w[MAX_GH]; };   // nodes sqrt(2) x_k and weights w_k / sqrt(pi), passed by value
 
 struct PointArgs {
     const double* mu_part; int n_mu_part; long ldmu;   // partial means   [n_mu_part][ldmu]
@@ -49,13 +51,14 @@ struct PointArgs {
 //   ve = mean_s log softmax(f_s)[y],  f_s = mu + sqrt(var) * eps_s ;  g_l = d ve / d mu_l ;  h_l = min(d ve / d var_l, -1e-8)
 // as called at reference tsvgp.py:256-263 (docs/notebooks/mnist.py:117-122).  Per-latent inputs / outputs are `*_lat` apart.
 // eps: explicit standard-normal draws [S][n_total][L] (GPflow's layout) or null = Philox4x32-10 + Box-Muller keyed by (seed, draw).
+// The heteroskedastic likelihood takes the same arguments (S, eps, seed and draw unused).
 struct SoftmaxArgs {
     const double* mu_part; int n_mu_part; long ldmu, mu_lat;
     const double* q_part; int n_q_part; long ldq, q_lat;
     int L, S;
-    const double* y;            // class labels as doubles, chunk-local
+    const double* y;            // class labels as doubles (heteroskedastic: the observation), chunk-local
     const double* mean_off;
-    double kdiag;
+    double kdiag[MAX_SOFTMAX_CLASSES];   // k_l(x,x) = latent l's kernel variance
     long n_valid, n0, n_total;  // n0: global index of the chunk's first point (addresses eps / the random stream)
     int ncols;
     double* g; double* h; long gh_lat;
@@ -66,6 +69,11 @@ struct SoftmaxArgs {
     unsigned long long seed, draw;
 };
 int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s);
+// Heteroskedastic Normal likelihood over L = 2 latents (GPflow HeteroskedasticTFPConditional(Normal, scale_transform) with its
+// NDiagGHQuadrature(2, n_gh)): log p(y | f) = Normal(loc = f_0, scale = T(f_1)).log_prob(y), T = exp (lik.p0 = 0) or softplus (1),
+// integrated on the tensor-product grid f = mu + sqrt(v) (z_i, z_j), weights w_i w_j.  Per point: ve, g_l = d ve / d mu_l,
+// h_l = min(d ve / d v_l, -1e-8); mean_out / var_out get the marginals of q(f) (predict).  One ve slot per 256 points.
+int heteroskedastic_stats_launch(const LikSpec& lik, const SoftmaxArgs& a, const GHTable& gh, cudaStream_t s);
 // Y [n][L] row-major -> Yt [L][ld] ; and back for outputs: src [L][ld] -> dst [n][L]
 int transpose_to_latent_major_launch(const double* Y, long n, int L, double* Yt, long ld, cudaStream_t s);
 int transpose_to_point_major_launch(const double* src, long ld, long n, int L, double* dst, cudaStream_t s);
@@ -85,7 +93,6 @@ int add_mean_samples_launch(const double* mean, const double* F, long ldf, long 
 // out[s][n][l] = mean[l][n] + sqrt(var[l][n]) eps(s, n, l)  (mean, var [L][ld])
 int diag_samples_launch(const SampleArgs& a, const double* mean, const double* var, long ld, double* out, cudaStream_t s);
 
-struct GHTable { double z[MAX_GH]; double w[MAX_GH]; };   // nodes sqrt(2) x_k and weights w_k / sqrt(pi), passed by value
 int point_stats_launch(const LikSpec& lik, const PointArgs& a, const GHTable& gh, cudaStream_t s);
 
 // y[i] = alpha * sum_j A[i][j] x[j] + beta * y[i]      (row-major A [m][n], lda)

@@ -129,6 +129,23 @@ struct tsvgp_ctx {
     LikSpec lik;
     GHTable gh;
     bool lik_set = false;
+    // Separate kernels (tsvgp_set_kernels; gpflow SeparateIndependent): one kernel per latent.  Each latent owns its kernel-
+    // dependent state (lengthscales, scaled inducing inputs, K, K6, the K9 chain), and select_latent() points the working views
+    // (kern_kind, kern_var, ls_dev, ZsT, Zs, z2, K, K6, C9, C9inv, K9inv and the Kuf slabs) at latent l's copies, so every
+    // single-latent routine runs unchanged.  Latent 0 uses the shared mode's buffers (`base`), the others live in `pks`; the
+    // scaled resident data XsT/x2 hold L copies back to back.  In shared mode none of this is allocated or touched.
+    struct KernelState {
+        int kind = -1;
+        double var = 1.0;
+        std::vector<double> ls;
+        double *ls_dev = nullptr, *ZsT = nullptr, *Zs = nullptr, *z2 = nullptr, *K = nullptr, *K6 = nullptr, *C9 = nullptr,
+               *C9inv = nullptr, *K9inv = nullptr;
+    };
+    bool sep = false;
+    std::vector<KernelState> lk;   // [L] in separate mode
+    KernelState base;              // buffers of alloc_m_state
+    Pool pks;
+    int ks_Mp = 0;                 // Mp the per-latent buffers were allocated for (0: none)
 
     // Latent GPs sharing the kernel and the inducing inputs (num_latent_gps = L, reference tsvgp.py:276-281): one site pair, one set of
     // posterior factors and one statistics accumulator per latent, stored as [L] contiguous copies.  The per-latent pointers below
@@ -202,6 +219,8 @@ struct tsvgp_ctx {
     int chunk_route = 0;
     int slab_streams = 0;
     double *wslab[MAXS] = {};
+    double *slab_all[MAXS] = {};   // [slab_lat][Mp][nc]: one Kuf slab per latent in separate mode
+    int slab_lat = 1;
     double *slab[MAXS] = {}, *mu_part[MAXS] = {}, *q_part[MAXS] = {}, *q2_part[MAXS] = {}, *gbuf[MAXS] = {}, *hbuf[MAXS] = {};
     double* ve_blocks = nullptr;
     long ve_cap = 0;
@@ -259,6 +278,7 @@ namespace {
     } while (0)
 
 int all_reduce(tsvgp_ctx* c, double* buf, size_t count);
+int alloc_separate(tsvgp_ctx* c);
 int ensure_posterior_white(tsvgp_ctx* c);
 int posterior_one(tsvgp_ctx* c);
 int ensure_kl_terms_white(tsvgp_ctx* c);
@@ -279,9 +299,19 @@ bool is_device_ptr(const void* p) {
 }
 
 // ---- latent views ---------------------------------------------------------------------------------------------------
+void view_kernel_buffers(tsvgp_ctx* c, const tsvgp_ctx::KernelState& k) {
+    c->ls_dev = k.ls_dev; c->ZsT = k.ZsT; c->Zs = k.Zs; c->z2 = k.z2;
+    c->K = k.K; c->K6 = k.K6; c->C9 = k.C9; c->C9inv = k.C9inv; c->K9inv = k.K9inv;
+}
+
 void select_latent(tsvgp_ctx* c, int l) {
     const size_t mm = (size_t)c->Mp * c->Mp, mp = c->Mp;
     c->cur = l;
+    if (c->sep && c->ks_Mp == c->Mp) {
+        const tsvgp_ctx::KernelState& k = c->lk[l];
+        c->kern_kind = k.kind; c->kern_var = k.var;
+        view_kernel_buffers(c, k);
+    }
     c->lam1 = c->lam1_all + l * mp; c->L2 = c->L2_all + l * mm; c->T = c->T_all + l * mm;
     c->alpha = c->alpha_all + l * mp; c->mZ = c->mZ_all + l * mp; c->mq = c->mq_all + l * mp; c->scal = c->scal_all + (size_t)l * N_SCAL;
     for (int s = 0; s < MAXS; ++s) {
@@ -295,6 +325,7 @@ void select_latent(tsvgp_ctx* c, int l) {
             c->q_part[s] = c->q_part_all[s] + l * (size_t)(c->Mp / 128) * nc;
             c->gbuf[s] = c->gbuf_all[s] + l * nc;
             c->hbuf[s] = c->hbuf_all[s] + l * nc;
+            if (c->slab_lat > 1) c->slab[s] = c->slab_all[s] + l * (size_t)c->Mp * nc;
         }
         c->ve_blocks = c->ve_all + (size_t)l * c->ve_cap;
     }
@@ -330,10 +361,48 @@ int alloc_m_state(tsvgp_ctx* c, int M, int D) {
     NEED(c->tmp2 = p.get((size_t)((c->Mp / 128 + 1) / 2) * 128 * mp)); NEED(c->dinv2 = p.get((size_t)(c->Mp / 128) * 128 * 128));
     CU(cudaMemsetAsync(c->dinv2, 0, sizeof(double) * (size_t)(c->Mp / 128) * 128 * 128, c->s_main));
     CU(cudaStreamSynchronize(c->s_main));   // the side and helper streams use these buffers too
-    NEED(c->pv1 = p.get(mp)); NEED(c->pv2 = p.get(mp)); NEED(c->gwork2 = p.get((size_t)(c->Mp / 64 + 1) * mp)); NEED(c->scal2 = p.get(N_SCAL));
+    NEED(c->pv1 = p.get(mp)); NEED(c->pv2 = p.get(mp)); NEED(c->gwork2 = p.get((size_t)(c->Mp / 64 + 1) * mp)); NEED(c->scal2 = p.get(nl * N_SCAL));
     c->sites_set = c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = c->c6_valid = c->wpost_valid = c->wkl_valid = false;
     c->chunk = 0;   // slab workspace depends on Mp
+    c->base.ls_dev = c->ls_dev; c->base.ZsT = c->ZsT; c->base.Zs = c->Zs; c->base.z2 = c->z2;
+    c->base.K = c->K; c->base.K6 = c->K6; c->base.C9 = c->C9; c->base.C9inv = c->C9inv; c->base.K9inv = c->K9inv;
+    c->ks_Mp = 0;
+    if (c->sep) OK(alloc_separate(c));
     select_latent(c, 0);
+    return TSVGP_OK;
+}
+
+// the per-latent kernel buffers of separate mode: latent 0 takes the shared mode's, latents 1.. get their own
+int alloc_separate(tsvgp_ctx* c) {
+    CU(cudaDeviceSynchronize());
+    c->pks.release();
+    const size_t mm = (size_t)c->Mp * c->Mp, mp = c->Mp;
+    for (int l = 0; l < c->L; ++l) {
+        tsvgp_ctx::KernelState& k = c->lk[l];
+        if (l == 0) {
+            k.ls_dev = c->base.ls_dev; k.ZsT = c->base.ZsT; k.Zs = c->base.Zs; k.z2 = c->base.z2;
+            k.K = c->base.K; k.K6 = c->base.K6; k.C9 = c->base.C9; k.C9inv = c->base.C9inv; k.K9inv = c->base.K9inv;
+            continue;
+        }
+        Pool& p = c->pks;
+        NEED(k.ls_dev = p.get(c->D)); NEED(k.ZsT = p.get((size_t)c->D * mp)); NEED(k.Zs = p.get(mp * c->D)); NEED(k.z2 = p.get(mp));
+        NEED(k.K = p.get(mm)); NEED(k.K6 = p.get(mm)); NEED(k.C9 = p.get(mm)); NEED(k.C9inv = p.get(mm)); NEED(k.K9inv = p.get(mm));
+    }
+    c->ks_Mp = c->Mp;
+    c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = false;
+    return TSVGP_OK;
+}
+
+// back to one kernel shared by every latent (tsvgp_set_kernel, tsvgp_set_num_latent)
+int drop_separate(tsvgp_ctx* c) {
+    if (!c->sep) return TSVGP_OK;
+    CU(cudaDeviceSynchronize());
+    view_kernel_buffers(c, c->base);
+    c->sep = false;
+    c->lk.clear();
+    c->pks.release();
+    c->ks_Mp = 0;
+    c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = c->xs_valid = false;
     return TSVGP_OK;
 }
 
@@ -347,29 +416,43 @@ int default_sites(tsvgp_ctx* c) {   // tsvgp.py:174-180 : lambda_1 = 0, lambda_2
     return TSVGP_OK;
 }
 
-int upload_lengthscales(tsvgp_ctx* c) {
+int upload_lengthscales(tsvgp_ctx* c, const std::vector<double>& ls_host) {
     if (c->kern_kind < 0) FAIL(TSVGP_ERR_STATE, "kernel not set (tsvgp_set_kernel)");
     if (c->D <= 0) FAIL(TSVGP_ERR_STATE, "inducing points not set (tsvgp_set_inducing)");
-    if (c->ls_host.size() != 1 && (int)c->ls_host.size() != c->D)
-        FAIL(TSVGP_ERR_INVALID, "lengthscales has %zu entries, expected 1 or D=%d", c->ls_host.size(), c->D);
+    if (ls_host.size() != 1 && (int)ls_host.size() != c->D)
+        FAIL(TSVGP_ERR_INVALID, "lengthscales has %zu entries, expected 1 or D=%d", ls_host.size(), c->D);
     std::vector<double> ls(c->D);
-    for (int d = 0; d < c->D; ++d) ls[d] = c->ls_host.size() == 1 ? c->ls_host[0] : c->ls_host[d];
+    for (int d = 0; d < c->D; ++d) ls[d] = ls_host.size() == 1 ? ls_host[0] : ls_host[d];
     CU(cudaMemcpyAsync(c->ls_dev, ls.data(), sizeof(double) * c->D, cudaMemcpyHostToDevice, c->s_main));
     CU(cudaStreamSynchronize(c->s_main));   // `ls` is a stack temporary
     return TSVGP_OK;
 }
 
 // K = k(Z,Z) (identity on the padding block), K6 = K + default_jitter I            tsvgp.py:209-211, :268
-int ensure_kuu(tsvgp_ctx* c) {
-    if (c->kuu_valid) return TSVGP_OK;
-    if (c->M <= 0) FAIL(TSVGP_ERR_STATE, "inducing points not set (tsvgp_set_inducing)");
-    OK(upload_lengthscales(c));
+int kuu_one(tsvgp_ctx* c, const std::vector<double>& ls_host) {   // the selected latent's kernel (shared mode: the kernel)
+    OK(upload_lengthscales(c, ls_host));
     cudaStream_t s = c->s_main;
     LA(scale_points_launch(c->Zraw, c->M, c->D, c->ls_dev, c->ZsT, c->Mp, c->z2, c->Mp, s));
     LA(unpack_rows_launch(c->ZsT, c->Mp, c->Mp, c->D, c->Zs, s));
     LA(kuf_launch(c->kern_kind, c->kern_var, c->ZsT, c->Mp, c->z2, 0, c->M, c->Mp, c->Zs, c->z2, c->M, c->Mp, c->D, nullptr,
                   c->K, c->Mp, nullptr, 0, 1, s));
     LA(copy_add_diag_launch(c->K, c->K6, c->Mp, c->Mp, c->jit6, s));
+    return TSVGP_OK;
+}
+
+int ensure_kuu(tsvgp_ctx* c) {
+    if (c->kuu_valid) return TSVGP_OK;
+    if (c->M <= 0) FAIL(TSVGP_ERR_STATE, "inducing points not set (tsvgp_set_inducing)");
+    if (c->sep) {   // K_l, K6_l per latent
+        for (int l = 0; l < c->L; ++l) {
+            select_latent(c, l);
+            const int rc = kuu_one(c, c->lk[l].ls);
+            if (rc != TSVGP_OK) { select_latent(c, 0); return rc; }
+        }
+        select_latent(c, 0);
+    } else {
+        OK(kuu_one(c, c->ls_host));
+    }
     c->kuu_valid = true;
     c->post_valid = c->kl_valid = c->k9_valid = c->c6_valid = c->wpost_valid = c->wkl_valid = false;
     return TSVGP_OK;
@@ -620,7 +703,20 @@ int ensure_xs(tsvgp_ctx* c) {
     if (!c->X) FAIL(TSVGP_ERR_STATE, "no data resident (tsvgp_set_data)");
     OK(ensure_kuu(c));
     if (c->dataD != c->D) FAIL(TSVGP_ERR_INVALID, "X has D=%d but the inducing points have D=%d", c->dataD, c->D);
-    LA(scale_points_launch(c->X, c->N, c->D, c->ls_dev, c->XsT, c->n_pad, c->x2, c->n_pad, c->s_main));
+    if (c->sep) {   // one scaled copy per latent kernel, back to back: XsT [L][D][n_pad], x2 [L][n_pad]
+        const long need = (long)c->L * c->D * c->n_pad, need_n = (long)c->L * c->n_pad;
+        if (need > c->xs_cap || need_n > c->xs_cap_n) {
+            CU(cudaStreamSynchronize(c->s_main));
+            c->pxs.release();
+            c->xs_cap = need; c->xs_cap_n = need_n;
+            NEED(c->XsT = c->pxs.get((size_t)need)); NEED(c->x2 = c->pxs.get((size_t)need_n));
+        }
+        for (int l = 0; l < c->L; ++l)
+            LA(scale_points_launch(c->X, c->N, c->D, c->lk[l].ls_dev, c->XsT + (size_t)l * c->D * c->n_pad, c->n_pad,
+                                   c->x2 + (size_t)l * c->n_pad, c->n_pad, c->s_main));
+    } else {
+        LA(scale_points_launch(c->X, c->N, c->D, c->ls_dev, c->XsT, c->n_pad, c->x2, c->n_pad, c->s_main));
+    }
     c->xs_valid = true;
     return TSVGP_OK;
 }
@@ -654,8 +750,9 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const long ve_need = (nchunks + 1) * ((nc + 255) / 256);
     const bool need_w = c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT;
     const int want_streams = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
+    const int slab_lat = c->sep ? c->L : 1;
     if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || c->grad_ws) &&
-        c->slab_streams >= want_streams)
+        c->slab_streams >= want_streams && c->slab_lat == slab_lat)
         return TSVGP_OK;
     CU(cudaStreamSynchronize(c->s_main));
     c->pc.release();
@@ -664,7 +761,7 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const int ns = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     c->slab_streams = ns;
     for (int s = 0; s < ns; ++s) {
-        NEED(c->slab[s] = p.get((size_t)c->Mp * nc));
+        NEED(c->slab_all[s] = c->slab[s] = p.get((size_t)slab_lat * c->Mp * nc));
         if (need_w) NEED(c->wslab[s] = p.get((size_t)c->Mp * nc));
         NEED(c->mu_part_all[s] = p.get((size_t)c->L * (c->Mp / 64) * nc));
         NEED(c->q_part_all[s] = p.get((size_t)c->L * (c->Mp / 128) * nc));
@@ -706,6 +803,7 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
         c->grad_ws = true;
     }
     c->ve_cap = ve_need;
+    c->slab_lat = slab_lat;
     c->chunk = nc;
     c->chunk_Mp = c->Mp;
     select_latent(c, c->cur);   // the per-slab views of the selected latent
@@ -719,11 +817,14 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
 // b += Kuf g).
 enum { PASS_WHOLE = 0, PASS_EARLY = 1, PASS_REST = 2 };
 inline bool grad_spread_skip(const tsvgp_ctx*) { return false; }
+// the likelihood couples the latents (one point kernel over all of them, Y [N, 1]): Softmax, heteroskedastic Normal
+inline bool coupled(const tsvgp_ctx* c) { return c->lik.kind == LIK_SOFTMAX || c->lik.kind == LIK_HETEROSKEDASTIC; }
 // y / mean_out / var_out of latent l live at + l * y_stride / + l * out_stride (Y transposed to [L][n_pad]; outputs [L][n_pad_out]).
 // lat_only >= 0 restricts the per-latent work to that latent (the M-step gradient pass runs latent by latent).
+// Separate kernels: latent l's scaled coordinates are at XsT + l * xs_lat, x2 + l * x2_lat, and every latent builds its own slab.
 int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, long N, const double* y, const double* mean_off,
                 int mode, double* mean_out, double* var_out, int phase = PASS_WHOLE, long y_stride = 0, long out_stride = 0,
-                int lat_only = -1) {
+                int lat_only = -1, long xs_lat = 0, long x2_lat = 0) {
     const bool grad = mode == MODE_GRAD;
     const bool stats = mode == MODE_STATS || grad;
     if (phase != PASS_REST) OK(ensure_slabs(c, N, grad));
@@ -733,7 +834,8 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
     const bool prof = c->profile && mode == MODE_STATS && c->L == 1;
     const int l_lo = lat_only >= 0 ? lat_only : 0, l_hi = lat_only >= 0 ? lat_only + 1 : c->L;
     const bool multi = c->L > 1;
-    const bool joint = c->lik.kind == LIK_SOFTMAX;   // the likelihood couples the latents: one point kernel over all of them
+    const bool joint = coupled(c);
+    const bool sep = c->sep;
     size_t pev_used = 0;
     auto mark = [&](cudaStream_t st) -> int {   // profile mode: one event between consecutive kernels
         if (!prof) return 0;
@@ -803,7 +905,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
     const bool const_h_pass = c->lik.kind == LIK_GAUSSIAN && !grad;
     if (phase == PASS_EARLY) {
         const bool ok = mode == MODE_STATS && const_h_pass && c->route == ROUTE_FUSED && !c->white && !prof && c->ksplit <= 1 &&
-                        nchunks >= 2 * nstr && !multi;
+                        nchunks >= 2 * nstr && !multi && !c->sep;   // (separate kernels build every slab in the pass itself)
         const int ne = ok ? (c->early_slabs < nstr ? c->early_slabs : nstr) : 0;
         for (int ci = 0; ci < ne; ++ci) {
             const long n0 = ci * ncu;
@@ -834,14 +936,17 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         select_latent(c, l_lo);
         if (mark(s)) FAIL(TSVGP_ERR_CUDA, "profile event");
         // (a) covariance slab K[Mp x ncols] — ONE slab for all latents — and, for a single latent, the partial means
-        //     sum_i alpha_i K[i][n] in the same kernel
-        if (!early)
+        //     sum_i alpha_i K[i][n] in the same kernel (separate kernels: per latent, below)
+        if (!early && !sep)
             LA(kuf_launch(c->kern_kind, c->kern_var, XsT, ldx, x2, n0, N, ncols, c->Zs, c->z2, c->M, Mp, c->D, multi ? nullptr : c->alpha,
                           c->slab[b], nc, multi ? nullptr : c->mu_part[b], nc, 0, s, grad ? c->kpslab[b] : nullptr));
         mark(s);
         for (int l = l_lo; l < l_hi; ++l) {
             select_latent(c, l);
-            if (early || multi)   // the slab exists already: the same per-64-row partial means from a transposed mat-vec over it
+            if (sep)   // (a') latent l's kernel and scaled coordinates into latent l's slab, with its partial means
+                LA(kuf_launch(c->kern_kind, c->kern_var, XsT + l * xs_lat, ldx, x2 + l * x2_lat, n0, N, ncols, c->Zs, c->z2, c->M, Mp,
+                              c->D, c->alpha, c->slab[b], nc, c->mu_part[b], nc, 0, s, nullptr));
+            else if (early || multi)   // the slab exists already: the same per-64-row partial means from a transposed mat-vec over it
                 LA(gemv_t_part_launch(c->slab[b], nc, Mp, ncols, c->alpha, c->mu_part[b], nc, s));
             if (!c->white) {   // (b) |T^T k_n|^2 : upper-triangular T^T times the slab, reduced to column norms in the epilogue
                 GemmP p;
@@ -883,7 +988,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             }
             mark(s);
         }
-        if (joint) {   // (c) Softmax: Monte-Carlo expectation over all latents of a point at once
+        if (joint) {   // (c) Softmax / heteroskedastic: the expectation over all latents of a point at once
             select_latent(c, 0);
             SoftmaxArgs a;
             a.mu_part = c->mu_part[b]; a.n_mu_part = Mp / 64; a.ldmu = nc; a.mu_lat = (long)(Mp / 64) * nc;
@@ -891,7 +996,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             a.L = c->L; a.S = c->lik.n_gh;
             a.y = y ? y + n0 : nullptr;
             a.mean_off = mean_off ? mean_off + n0 : nullptr;
-            a.kdiag = c->kern_var;
+            for (int l = 0; l < c->L; ++l) a.kdiag[l] = sep ? c->lk[l].var : c->kern_var;
             a.n_valid = nvalid; a.ncols = ncols; a.n0 = n0; a.n_total = N;
             a.g = stats ? c->gbuf[b] : nullptr; a.h = stats ? c->hbuf[b] : nullptr; a.gh_lat = nc;
             a.mean_out = mean_out ? mean_out + n0 : nullptr; a.var_out = var_out ? var_out + n0 : nullptr; a.out_lat = out_stride;
@@ -899,29 +1004,37 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             a.flags = c->flags;
             a.eps = (c->mc_eps && c->mc_eps_n == N) ? c->mc_eps : nullptr;
             a.seed = c->mc_seed; a.draw = c->mc_draw;
-            LA(softmax_stats_launch(a, s));
+            if (c->lik.kind == LIK_HETEROSKEDASTIC) LA(heteroskedastic_stats_launch(c->lik, a, c->gh, s));
+            else LA(softmax_stats_launch(a, s));
         }
         if (stats) {
-            const double* stat_slab = c->slab[b];
-            if ((c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT) && !grad) {   // (c') whitened slab  C9^-1 K  (reference order: A = K9^-1 Kuf first, tsvgp.py:271)
-                GemmP p;
-                p.A = c->C9inv; p.lda = Mp; p.a_kc = 1; p.a_tri = 1;
-                p.B = c->slab[b]; p.ldb = nc; p.b_kc = 0;
-                p.C = c->wslab[b]; p.ldc = nc; p.m = Mp; p.n = ncols; p.k = Mp;
-                LA(gemm_launch(p, s));
-                stat_slab = c->wslab[b];
-                if (c->route == ROUTE_EXACT) {   // (c'') A = C9^-T (C9^-1 K) = K9^-1 Kuf itself, written over the covariance slab (no longer needed)
-                    GemmP q;
-                    q.A = c->C9inv; q.lda = Mp; q.a_kc = 0; q.a_tri = 2;
-                    q.B = c->wslab[b]; q.ldb = nc; q.b_kc = 0;
-                    q.C = c->slab[b]; q.ldc = nc; q.m = Mp; q.n = ncols; q.k = Mp;
-                    LA(gemm_launch(q, s));
-                    stat_slab = c->slab[b];
+            // (c') whitened slab  C9^-1 K  (reference order: A = K9^-1 Kuf first, tsvgp.py:271) of the selected latent
+            auto stat_slab_of = [&](const double*& out) -> int {
+                out = c->slab[b];
+                if ((c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT) && !grad) {
+                    GemmP p;
+                    p.A = c->C9inv; p.lda = Mp; p.a_kc = 1; p.a_tri = 1;
+                    p.B = c->slab[b]; p.ldb = nc; p.b_kc = 0;
+                    p.C = c->wslab[b]; p.ldc = nc; p.m = Mp; p.n = ncols; p.k = Mp;
+                    LA(gemm_launch(p, s));
+                    out = c->wslab[b];
+                    if (c->route == ROUTE_EXACT) {   // (c'') A = C9^-T (C9^-1 K) = K9^-1 Kuf itself, written over the covariance slab (no longer needed)
+                        GemmP q;
+                        q.A = c->C9inv; q.lda = Mp; q.a_kc = 0; q.a_tri = 2;
+                        q.B = c->wslab[b]; q.ldb = nc; q.b_kc = 0;
+                        q.C = c->slab[b]; q.ldc = nc; q.m = Mp; q.n = ncols; q.k = Mp;
+                        LA(gemm_launch(q, s));
+                        out = c->slab[b];
+                    }
                 }
-            }
+                return TSVGP_OK;
+            };
+            const double* stat_slab = nullptr;
+            if (!sep) OK(stat_slab_of(stat_slab));   // one slab (and one K9) for every latent
             mark(s);
             for (int l = l_lo; l < l_hi; ++l) {   // (d) B_l += K diag(h_l) K^T, lower tiles (already enqueued for an early slab)
                 select_latent(c, l);
+                if (sep) OK(stat_slab_of(stat_slab));   // latent l's slab and C9_l
                 bool fused_b = false;
                 if (!early) OK(syrk(b, stat_slab, ncols, const_h_pass, true, fused_b));
                 mark(s);
@@ -1002,9 +1115,9 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
 
 // the pass over the RESIDENT minibatch: Y is the transposed copy [L][n_pad] when the L latents have independent likelihood terms
 int data_pass(tsvgp_ctx* c, int mode, int phase = PASS_WHOLE, int lat_only = -1) {
-    const bool per_latent_y = c->L > 1 && c->lik.kind != LIK_SOFTMAX;
+    const bool per_latent_y = c->L > 1 && !coupled(c);
     return stream_pass(c, c->XsT, c->n_pad, c->x2, c->N, per_latent_y ? c->Yt : c->Y, c->meanX, mode, nullptr, nullptr, phase,
-                       per_latent_y ? c->n_pad : 0, 0, lat_only);
+                       per_latent_y ? c->n_pad : 0, 0, lat_only, c->sep ? (long)c->D * c->n_pad : 0, c->sep ? c->n_pad : 0);
 }
 
 int all_reduce(tsvgp_ctx* c, double* buf, size_t count) {
@@ -1089,25 +1202,22 @@ int start_k9_async(tsvgp_ctx* c, double jitter, SideIssue& side) {
     return TSVGP_OK;
 }
 
-int k9_chain(tsvgp_ctx* c, double jitter) {
+// One kernel's chain: K9 = K + jitter I = C9 C9^T, C9^-1, K9^-1 (when `with_inv`) and the conditioning probe into probe[N_SCAL].
+// The buffers are passed explicitly: with separate kernels the chains run on the side stream, possibly issued from the helper
+// thread, while the calling thread moves the latent views.
+int k9_chain_one(tsvgp_ctx* c, double jitter, const double* K, double* C9, double* C9inv, double* K9inv, double* probe, bool with_inv) {
     cudaStream_t s = c->s_side;
-    LA(copy_add_diag_launch(c->K, c->C9, c->Mp, c->Mp, jitter, s));
-    LA(chol_lower(c->C9, c->Mp, c->Mp, c->dinv2, c->info + INFO_K9, s, c->gws2, c->gws_doubles, &c->la_side));
-    LA(trtri_lower(c->C9, c->Mp, c->Mp, c->dinv2, c->C9inv, c->tmp2, s, c->gws2, c->gws_doubles));
-    c->k9inv_valid = false;
-    if (!dist_active(c)) {   // single rank / small M: form K9^-1 here, hidden behind the main stream's posterior preparation
+    LA(copy_add_diag_launch(K, C9, c->Mp, c->Mp, jitter, s));
+    LA(chol_lower(C9, c->Mp, c->Mp, c->dinv2, c->info + INFO_K9, s, c->gws2, c->gws_doubles, &c->la_side));
+    LA(trtri_lower(C9, c->Mp, c->Mp, c->dinv2, C9inv, c->tmp2, s, c->gws2, c->gws_doubles));
+    if (with_inv) {
         GemmP p;
-        p.A = c->C9inv; p.lda = c->Mp; p.a_kc = 0; p.a_tri = 2;
-        p.B = c->C9inv; p.ldb = c->Mp; p.b_kc = 0; p.b_tri = 2;
-        p.C = c->K9inv; p.ldc = c->Mp; p.m = p.n = p.k = c->Mp; p.lower_out = 1;
+        p.A = C9inv; p.lda = c->Mp; p.a_kc = 0; p.a_tri = 2;
+        p.B = C9inv; p.ldb = c->Mp; p.b_kc = 0; p.b_tri = 2;
+        p.C = K9inv; p.ldc = c->Mp; p.m = p.n = p.k = c->Mp; p.lower_out = 1;
         LA(mm_gemm(c, p, s));
-        LA(mirror_lower_launch(c->K9inv, c->Mp, c->Mp, s));
-        c->k9inv_valid = true;
+        LA(mirror_lower_launch(K9inv, c->Mp, c->Mp, s));
     }
-    c->k9_valid = true;
-    c->k9_jitter = jitter;
-    c->cond_est = 0.0;
-    c->k9_pending = true;
     if (c->route_opt == ROUTE_AUTO) {
         // conditioning probe: 8 power iterations each on K and on K9^-1 = C9^-T C9^-1; Rayleigh ratios of the last two
         // iterates give lambda_max(K) and 1/lambda_min(K9) (both from below)
@@ -1115,25 +1225,47 @@ int k9_chain(tsvgp_ctx* c, double jitter) {
         double *a = c->pv1, *b = c->pv2;
         LA(probe_vector_launch(a, c->M, n, s));
         for (int it = 0; it < 8; ++it) {
-            if (it == 7) LA(dot_launch(a, a, c->M, c->scal2 + SC_PK0, s));
-            LA(gemv_n_launch(c->K, n, c->M, c->M, a, 1.0, 0.0, b, s));
+            if (it == 7) LA(dot_launch(a, a, c->M, probe + SC_PK0, s));
+            LA(gemv_n_launch(K, n, c->M, c->M, a, 1.0, 0.0, b, s));
             double* t = a; a = b; b = t;
         }
-        LA(dot_launch(a, a, c->M, c->scal2 + SC_PK1, s));
+        LA(dot_launch(a, a, c->M, probe + SC_PK1, s));
         LA(probe_vector_launch(a, c->M, n, s));
         for (int it = 0; it < 8; ++it) {
-            if (it == 7) LA(dot_launch(a, a, n, c->scal2 + SC_PI0, s));
-            if (c->k9inv_valid) {   // K9^-1 itself is at hand (formed just above): one mat-vec per iteration instead of two
-                LA(gemv_n_launch(c->K9inv, n, n, n, a, 1.0, 0.0, b, s));
+            if (it == 7) LA(dot_launch(a, a, n, probe + SC_PI0, s));
+            if (with_inv) {   // K9^-1 itself is at hand (formed just above): one mat-vec per iteration instead of two
+                LA(gemv_n_launch(K9inv, n, n, n, a, 1.0, 0.0, b, s));
                 double* t = a; a = b; b = t;
             } else {
-                LA(gemv_n_launch(c->C9inv, n, n, n, a, 1.0, 0.0, b, s));
-                LA(gemv_t_launch(c->C9inv, n, n, n, b, a, c->gwork2, s));
+                LA(gemv_n_launch(C9inv, n, n, n, a, 1.0, 0.0, b, s));
+                LA(gemv_t_launch(C9inv, n, n, n, b, a, c->gwork2, s));
             }
         }
-        LA(dot_launch(a, a, n, c->scal2 + SC_PI1, s));
+        LA(dot_launch(a, a, n, probe + SC_PI1, s));
     }
-    CU(cudaEventRecord(c->ev_side, s));
+    return TSVGP_OK;
+}
+
+int k9_chain(tsvgp_ctx* c, double jitter) {
+    // single rank / small M: form K9^-1 in the chain, hidden behind the main stream's posterior preparation.  Separate kernels
+    // always do (dense_update_one forms a missing K9^-1 once per step, not once per latent); their chains run back to back,
+    // each with its own probe slots.
+    const bool with_inv = !dist_active(c) || c->sep;
+    c->k9inv_valid = false;
+    if (c->sep) {
+        for (int l = 0; l < c->L; ++l) {
+            const tsvgp_ctx::KernelState& k = c->lk[l];
+            OK(k9_chain_one(c, jitter, k.K, k.C9, k.C9inv, k.K9inv, c->scal2 + (size_t)l * N_SCAL, true));
+        }
+    } else {
+        OK(k9_chain_one(c, jitter, c->K, c->C9, c->C9inv, c->K9inv, c->scal2, with_inv));
+    }
+    c->k9inv_valid = with_inv;
+    c->k9_valid = true;
+    c->k9_jitter = jitter;
+    c->cond_est = 0.0;
+    c->k9_pending = true;
+    CU(cudaEventRecord(c->ev_side, c->s_side));
     return TSVGP_OK;
 }
 
@@ -1145,13 +1277,19 @@ int route_for(const tsvgp_ctx* c, double cond) {
 // joins the side stream, reads the conditioning probe (if one ran) and fixes the statistics route of this step
 int choose_route(tsvgp_ctx* c, double jitter) {
     if (c->k9_pending) {
-        if (c->route_opt == ROUTE_AUTO) {
-            double sc[N_SCAL];
-            CU(cudaMemcpyAsync(sc, c->scal2, sizeof sc, cudaMemcpyDeviceToHost, c->s_side));
+        if (c->route_opt == ROUTE_AUTO) {   // separate kernels: the pass takes the route of the worst-conditioned latent
+            const int nk = c->sep ? c->L : 1;
+            std::vector<double> scv((size_t)nk * N_SCAL);
+            CU(cudaMemcpyAsync(scv.data(), c->scal2, sizeof(double) * scv.size(), cudaMemcpyDeviceToHost, c->s_side));
             CU(cudaStreamSynchronize(c->s_side));
-            const double lmax = sqrt(sc[SC_PK1] / sc[SC_PK0]) + jitter, inv_lmin = sqrt(sc[SC_PI1] / sc[SC_PI0]);
-            c->cond_est = lmax * inv_lmin;
-            if (!(c->cond_est == c->cond_est)) c->cond_est = INFINITY;   // failed factorisation: the step will report it
+            c->cond_est = 0.0;
+            for (int l = 0; l < nk; ++l) {
+                const double* sc = scv.data() + (size_t)l * N_SCAL;
+                const double lmax = sqrt(sc[SC_PK1] / sc[SC_PK0]) + jitter, inv_lmin = sqrt(sc[SC_PI1] / sc[SC_PI0]);
+                double e = lmax * inv_lmin;
+                if (!(e == e)) e = INFINITY;   // failed factorisation: the step will report it
+                if (l == 0 || e > c->cond_est) c->cond_est = e;
+            }
             c->cond_hint = c->cond_est;
             c->cond_hint_valid = true;
         }
@@ -1536,6 +1674,7 @@ void tsvgp_destroy(tsvgp_ctx* c) {
     cudaDeviceSynchronize();
     if (c->comm) nccl_api().CommDestroy(c->comm);
     c->pm.release(); c->pd.release(); c->pc.release(); c->ps.release(); c->pxs.release(); c->pyt.release(); c->pmc.release();
+    c->pks.release();
     if (c->s_copy) cudaStreamDestroy(c->s_copy);
     if (c->ev_copy) cudaEventDestroy(c->ev_copy);
     for (int s = 0; s < MAXS; ++s) {
@@ -1608,6 +1747,10 @@ int tsvgp_set_num_latent(tsvgp_ctx* c, int L) {
     if (L == c->L) return TSVGP_OK;
     CU(cudaSetDevice(c->dev));
     CU(cudaDeviceSynchronize());
+    if (c->sep) {   // the per-latent kernels no longer match: compute calls wait for the next set_kernels / set_kernel
+        OK(drop_separate(c));
+        c->kern_kind = -1;
+    }
     c->L = L;
     c->k9_pending = false;
     if (c->M > 0) {   // re-allocate the per-latent state; the inducing inputs survive on the host side of the caller: re-upload needed
@@ -1640,12 +1783,21 @@ int tsvgp_set_mc_epsilon(tsvgp_ctx* c, const double* eps, int S, int64_t N, int 
 
 int tsvgp_num_latent(const tsvgp_ctx* c) { return c ? c->L : 0; }
 
-int tsvgp_set_kernel(tsvgp_ctx* c, int kind, double variance, const double* lengthscales, int n_ls) {
-    if (!c) return TSVGP_ERR_INVALID;
+static int check_kernel(tsvgp_ctx* c, int kind, double variance, const double* lengthscales, int n_ls) {
     if (kind != TSVGP_KERNEL_SE && kind != TSVGP_KERNEL_MATERN52) FAIL(TSVGP_ERR_INVALID, "unknown kernel kind %d", kind);
     if (!lengthscales || n_ls < 1 || !(variance > 0.0)) FAIL(TSVGP_ERR_INVALID, "kernel needs variance > 0 and >= 1 lengthscale");
     for (int i = 0; i < n_ls; ++i)
         if (!(lengthscales[i] > 0.0)) FAIL(TSVGP_ERR_INVALID, "lengthscales must be positive");
+    return TSVGP_OK;
+}
+
+int tsvgp_set_kernel(tsvgp_ctx* c, int kind, double variance, const double* lengthscales, int n_ls) {
+    if (!c) return TSVGP_ERR_INVALID;
+    OK(check_kernel(c, kind, variance, lengthscales, n_ls));
+    if (c->sep) {
+        CU(cudaSetDevice(c->dev));
+        OK(drop_separate(c));
+    }
     c->kern_kind = kind; c->kern_var = variance;
     c->ls_host.assign(lengthscales, lengthscales + n_ls);
     c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = c->c6_valid = c->wpost_valid = c->wkl_valid = false;
@@ -1653,16 +1805,47 @@ int tsvgp_set_kernel(tsvgp_ctx* c, int kind, double variance, const double* leng
     return TSVGP_OK;
 }
 
+int tsvgp_set_kernels(tsvgp_ctx* c, const int* kinds, const double* variances, const double* lengthscales, const int* n_ls) {
+    if (!c) return TSVGP_ERR_INVALID;
+    if (!kinds || !variances || !lengthscales || !n_ls) FAIL(TSVGP_ERR_INVALID, "kinds, variances, lengthscales and n_ls are required");
+    std::vector<tsvgp_ctx::KernelState> ks(c->L);
+    const double* ls = lengthscales;
+    for (int l = 0; l < c->L; ++l) {
+        OK(check_kernel(c, kinds[l], variances[l], ls, n_ls[l]));
+        ks[l].kind = kinds[l]; ks[l].var = variances[l];
+        ks[l].ls.assign(ls, ls + n_ls[l]);
+        ls += n_ls[l];
+    }
+    CU(cudaSetDevice(c->dev));
+    const bool fresh = !c->sep || (int)c->lk.size() != c->L;
+    if (fresh) {
+        CU(cudaDeviceSynchronize());
+        c->sep = true;
+        c->lk = std::move(ks);
+        c->ks_Mp = 0;
+        if (c->M > 0) OK(alloc_separate(c));
+    } else {   // same latents: keep the buffers, take the new parameters
+        for (int l = 0; l < c->L; ++l) { c->lk[l].kind = ks[l].kind; c->lk[l].var = ks[l].var; c->lk[l].ls = ks[l].ls; }
+    }
+    if (c->M > 0) select_latent(c, 0);
+    c->kern_kind = c->lk[0].kind; c->kern_var = c->lk[0].var;
+    c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = c->c6_valid = c->wpost_valid = c->wkl_valid = false;
+    c->xs_valid = false;
+    return TSVGP_OK;
+}
+
 int tsvgp_set_likelihood(tsvgp_ctx* c, int kind, double p0, double p1, int n_gh, const double* gh_x, const double* gh_w) {
     if (!c) return TSVGP_ERR_INVALID;
-    if (kind < TSVGP_LIK_GAUSSIAN || kind > TSVGP_LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "unknown likelihood kind %d", kind);
+    if (kind < TSVGP_LIK_GAUSSIAN || kind > TSVGP_LIK_HETEROSKEDASTIC) FAIL(TSVGP_ERR_INVALID, "unknown likelihood kind %d", kind);
+    if (kind == TSVGP_LIK_HETEROSKEDASTIC && p0 != 0.0 && p0 != 1.0)
+        FAIL(TSVGP_ERR_INVALID, "heteroskedastic: p0 selects the scale transform, 0 (exp) or 1 (softplus)");
     if (kind == TSVGP_LIK_SOFTMAX) {   // p0 = number of classes (= latent GPs), n_gh = Monte-Carlo points per data point
         if (p0 < 2 || p0 > MAX_SOFTMAX_CLASSES || n_gh < 1) FAIL(TSVGP_ERR_INVALID, "Softmax: 2..%d classes and >= 1 Monte-Carlo point", MAX_SOFTMAX_CLASSES);
         c->lik.kind = kind; c->lik.p0 = p0; c->lik.p1 = 0.0; c->lik.n_gh = n_gh;
         c->lik_set = true;
         return TSVGP_OK;
     }
-    if (kind != TSVGP_LIK_BERNOULLI_PROBIT && !(p0 > 0.0)) FAIL(TSVGP_ERR_INVALID, "likelihood variance / scale must be positive");
+    if (kind != TSVGP_LIK_BERNOULLI_PROBIT && kind != TSVGP_LIK_HETEROSKEDASTIC && !(p0 > 0.0)) FAIL(TSVGP_ERR_INVALID, "likelihood variance / scale must be positive");
     if (kind == TSVGP_LIK_STUDENT_T && !(p1 > 0.0)) FAIL(TSVGP_ERR_INVALID, "Student-t df must be positive");
     if (kind != TSVGP_LIK_GAUSSIAN && (n_gh < 1 || n_gh > MAX_GH)) FAIL(TSVGP_ERR_INVALID, "n_gh must be in [1, %d]", MAX_GH);
     c->lik.kind = kind; c->lik.p0 = p0; c->lik.p1 = p1; c->lik.n_gh = kind == TSVGP_LIK_GAUSSIAN ? 0 : n_gh;
@@ -1787,7 +1970,7 @@ int tsvgp_set_data(tsvgp_ctx* c, const double* X, const double* Y, int64_t N, in
     const long npad = round_up(N, 128);
     // Y is [N, L] for L latents with independent likelihood terms (tsvgp.py:256-259 sums over the latent axis), [N, 1] class labels
     // for the Softmax likelihood (set the likelihood before the data)
-    const int ycols = (c->L > 1 && c->lik.kind != LIK_SOFTMAX) ? c->L : 1;
+    const int ycols = (c->L > 1 && !coupled(c)) ? c->L : 1;
     if (npad > c->cap_n || (long)N * D > c->cap_x || ycols > c->cap_yc) {   // (re)allocate the owned staging and scaled-coordinate buffers
         CU(cudaStreamSynchronize(s));
         c->pd.release();
@@ -1825,7 +2008,7 @@ int tsvgp_set_data(tsvgp_ctx* c, const double* X, const double* Y, int64_t N, in
 
 int tsvgp_stage_data(tsvgp_ctx* c, const double* X, const double* Y, int64_t N, int D, const double* mean_X) {
     if (!c) return TSVGP_ERR_INVALID;
-    if (c->L > 1 && c->lik.kind != LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "stage_data with num_latent_gps > 1: use set_data");
+    if (c->L > 1 && !coupled(c)) FAIL(TSVGP_ERR_INVALID, "stage_data with num_latent_gps > 1: use set_data");
     if (!X || !Y || N < 1) FAIL(TSVGP_ERR_INVALID, "X [N >= 1, D] and Y [N] are required");
     if (c->D > 0 && D != c->D) FAIL(TSVGP_ERR_INVALID, "X has D=%d but the inducing points have D=%d", D, c->D);
     CU(cudaSetDevice(c->dev));
@@ -1881,7 +2064,12 @@ static int require_model(tsvgp_ctx* c, bool need_data) {
     if (c->lik.kind == LIK_SOFTMAX && (int)c->lik.p0 != c->L)
         FAIL(TSVGP_ERR_INVALID, "Softmax with %d classes needs num_latent_gps = %d (tsvgp_set_num_latent), not %d", (int)c->lik.p0, (int)c->lik.p0, c->L);
     if (c->white && c->lik.kind == LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "the whitened sibling model is not built for the Softmax likelihood");
-    if (need_data && c->y_cols != ((c->L > 1 && c->lik.kind != LIK_SOFTMAX) ? c->L : 1))
+    if (c->lik.kind == LIK_HETEROSKEDASTIC && c->L != 2)
+        FAIL(TSVGP_ERR_INVALID, "the heteroskedastic likelihood needs num_latent_gps = 2 (loc, scale), not %d", c->L);
+    if (c->white && c->lik.kind == LIK_HETEROSKEDASTIC)
+        FAIL(TSVGP_ERR_INVALID, "the whitened sibling model is not built for the heteroskedastic likelihood");
+    if (c->white && c->sep) FAIL(TSVGP_ERR_INVALID, "the whitened sibling model is not built for separate kernels per latent");
+    if (need_data && c->y_cols != ((c->L > 1 && !coupled(c)) ? c->L : 1))
         FAIL(TSVGP_ERR_STATE, "the resident Y has %d column(s): set the likelihood and num_latent_gps before the data", c->y_cols);
     return TSVGP_OK;
 }
@@ -2134,6 +2322,8 @@ int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance
     if (2 * c->D + 1 > 128) FAIL(TSVGP_ERR_INVALID, "elbo_grad supports D <= 63 (D = %d)", c->D);
     if (c->white) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not available for the whitened sibling model");
     if (c->lik.kind == LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not available for the Softmax likelihood");
+    if (c->lik.kind == LIK_HETEROSKEDASTIC) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for the heteroskedastic likelihood");
+    if (c->sep) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for separate kernels per latent");
     CU(cudaSetDevice(c->dev));
     c->collective_ok = true;
     cudaStream_t s = c->s_main;
@@ -2178,6 +2368,17 @@ int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance
     return TSVGP_OK;
 }
 
+// the query points scaled by the kernel's lengthscales; separate kernels: one copy per latent, xsT [L][D][ld], x2 [L][ld]
+static int scale_query(tsvgp_ctx* c, const double* X, long N, int D, double* xsT, long ld, double* x2) {
+    if (!c->sep) {
+        LA(scale_points_launch(X, N, D, c->ls_dev, xsT, ld, x2, ld, c->s_main));
+        return TSVGP_OK;
+    }
+    for (int l = 0; l < c->L; ++l)
+        LA(scale_points_launch(X, N, D, c->lk[l].ls_dev, xsT + (size_t)l * D * ld, ld, x2 + (size_t)l * ld, ld, c->s_main));
+    return TSVGP_OK;
+}
+
 int tsvgp_predict_f(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const double* mean_X, double* mean_out, double* var_out) {
     if (!c) return TSVGP_ERR_INVALID;
     if (!Xnew || !mean_out || !var_out || N < 1) FAIL(TSVGP_ERR_INVALID, "Xnew [N >= 1, D], mean_out [N], var_out [N] are required");
@@ -2198,14 +2399,15 @@ int tsvgp_predict_f(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, const do
         CU(cudaMemcpyAsync(xd, Xnew, sizeof(double) * (size_t)N * D, cudaMemcpyHostToDevice, s));
         xsrc = xd;
     }
-    const int L = c->L;
-    NEED(xsT = tp.get((size_t)D * npad)); NEED(x2 = tp.get(npad)); NEED(md = tp.get((size_t)L * npad)); NEED(vd = tp.get((size_t)L * npad));
+    const int L = c->L, nk = c->sep ? L : 1;
+    NEED(xsT = tp.get((size_t)nk * D * npad)); NEED(x2 = tp.get((size_t)nk * npad)); NEED(md = tp.get((size_t)L * npad)); NEED(vd = tp.get((size_t)L * npad));
     if (mean_X) {
         NEED(moff = tp.get(npad));
         CU(cudaMemcpyAsync(moff, mean_X, sizeof(double) * N, cudaMemcpyDefault, s));
     }
-    LA(scale_points_launch(xsrc, N, D, c->ls_dev, xsT, npad, x2, npad, s));
-    OK(stream_pass(c, xsT, npad, x2, N, nullptr, moff, MODE_PREDICT, md, vd, PASS_WHOLE, 0, npad));
+    OK(scale_query(c, xsrc, N, D, xsT, npad, x2));
+    OK(stream_pass(c, xsT, npad, x2, N, nullptr, moff, MODE_PREDICT, md, vd, PASS_WHOLE, 0, npad, -1, c->sep ? (long)D * npad : 0,
+                   c->sep ? npad : 0));
     double tail[4];
     int info_h[N_INFO];
     if (L == 1) {
@@ -2245,8 +2447,9 @@ static int predict_full(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, cons
     const long Np = round_up(N, 128), Sp = want_cov ? 0 : round_up(S, 128);
     const bool x_host = !is_device_ptr(Xnew), eps_host = eps && !is_device_ptr(eps);
     const bool out_host = !want_cov && !is_device_ptr(samples_out);
+    const int nk = c->sep ? L : 1;   // scaled copies of the query points (one per latent kernel)
     {   // every temporary below, counted before the first allocation
-        size_t need = (size_t)D * Np + Np + 2 * (size_t)L * Np + (mean_X ? Np : 0) + (x_host ? (size_t)N * D : 0) + (size_t)N * L;
+        size_t need = (size_t)nk * (D * Np + Np) + 2 * (size_t)L * Np + (mean_X ? Np : 0) + (x_host ? (size_t)N * D : 0) + (size_t)N * L;
         if (full_cov) need += (size_t)Np * D + 2 * (size_t)Mp * Np + (size_t)Np * Np;
         if (full_cov && !want_cov) need += (size_t)Np * 128 + 2 * (size_t)Np * Sp + L;
         if (eps_host) need += (size_t)S * N * L;
@@ -2269,13 +2472,14 @@ static int predict_full(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, cons
         CU(cudaMemcpyAsync(xd, Xnew, sizeof(double) * (size_t)N * D, cudaMemcpyHostToDevice, s));
         xsrc = xd;
     }
-    NEED(xsT = tp.get((size_t)D * Np)); NEED(x2 = tp.get(Np)); NEED(md = tp.get((size_t)L * Np)); NEED(vd = tp.get((size_t)L * Np));
+    NEED(xsT = tp.get((size_t)nk * D * Np)); NEED(x2 = tp.get((size_t)nk * Np)); NEED(md = tp.get((size_t)L * Np)); NEED(vd = tp.get((size_t)L * Np));
     if (mean_X) {
         NEED(moff = tp.get(Np));
         CU(cudaMemcpyAsync(moff, mean_X, sizeof(double) * N, cudaMemcpyDefault, s));
     }
-    LA(scale_points_launch(xsrc, N, D, c->ls_dev, xsT, Np, x2, Np, s));
-    OK(stream_pass(c, xsT, Np, x2, N, nullptr, moff, MODE_PREDICT, md, vd, PASS_WHOLE, 0, Np));   // exactly predict_f's moments
+    OK(scale_query(c, xsrc, N, D, xsT, Np, x2));
+    OK(stream_pass(c, xsT, Np, x2, N, nullptr, moff, MODE_PREDICT, md, vd, PASS_WHOLE, 0, Np, -1, c->sep ? (long)D * Np : 0,
+                   c->sep ? Np : 0));   // exactly predict_f's moments
 
     SampleArgs sa;
     sa.eps = eps; sa.seed = c->sample_seed; sa.draw = c->sample_draw; sa.N = N; sa.S = S; sa.L = L;
@@ -2297,8 +2501,12 @@ static int predict_full(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, cons
         double *xr, *kuf, *V, *Sig, *dinv = nullptr, *E = nullptr, *F = nullptr;
         NEED(xr = tp.get((size_t)Np * D)); NEED(kuf = tp.get((size_t)Mp * Np)); NEED(V = tp.get((size_t)Mp * Np));
         NEED(Sig = tp.get((size_t)Np * Np));
-        LA(unpack_rows_launch(xsT, Np, (int)Np, D, xr, s));   // the query points as the row operand of k(X, X)
-        LA(kuf_launch(c->kern_kind, c->kern_var, xsT, Np, x2, 0, N, (int)Np, c->Zs, c->z2, c->M, Mp, D, nullptr, kuf, Np, nullptr, 0, 0, s));
+        auto build_kuf = [&](const double* xs, const double* xx) -> int {   // the query points as the row operand of k(X, X); Kuf
+            LA(unpack_rows_launch(xs, Np, (int)Np, D, xr, s));
+            LA(kuf_launch(c->kern_kind, c->kern_var, xs, Np, xx, 0, N, (int)Np, c->Zs, c->z2, c->M, Mp, D, nullptr, kuf, Np, nullptr, 0, 0, s));
+            return TSVGP_OK;
+        };
+        if (!c->sep) OK(build_kuf(xsT, x2));   // one kernel: built once for every latent
         if (!want_cov) {
             NEED(dinv = tp.get((size_t)Np * 128)); NEED(E = tp.get((size_t)Np * Sp)); NEED(F = tp.get((size_t)Np * Sp));
             NEED(chol_info = (int*)tp.get(L));
@@ -2307,8 +2515,11 @@ static int predict_full(tsvgp_ctx* c, const double* Xnew, int64_t N, int D, cons
         }
         for (int l = 0; l < L; ++l) {
             select_latent(c, l);
+            const double* xs_l = xsT + (size_t)(c->sep ? l : 0) * D * Np;
+            const double* x2_l = x2 + (size_t)(c->sep ? l : 0) * Np;
+            if (c->sep) OK(build_kuf(xs_l, x2_l));   // latent l's kernel
             // Sigma = k(X, X), recomputed per latent instead of keeping a second N x N copy
-            LA(kuf_launch(c->kern_kind, c->kern_var, xsT, Np, x2, 0, N, (int)Np, xr, x2, (int)N, (int)Np, D, nullptr, Sig, Np, nullptr, 0, 1, s));
+            LA(kuf_launch(c->kern_kind, c->kern_var, xs_l, Np, x2_l, 0, N, (int)Np, xr, x2_l, (int)N, (int)Np, D, nullptr, Sig, Np, nullptr, 0, 1, s));
             {   // V = T^T Kuf  (the variance product of the pass, stored)
                 GemmP p;
                 p.A = c->T; p.lda = Mp; p.a_kc = 0; p.a_tri = 2;
@@ -2489,8 +2700,9 @@ int tsvgp_posterior(tsvgp_ctx* c, double* m, double* chol_S) {
             CU(cudaMemcpy2DAsync(chol_S + (size_t)l * c->M * c->M, sizeof(double) * c->M, c->X2, sizeof(double) * n, sizeof(double) * c->M, c->M,
                                  cudaMemcpyDefault, s));
         }
-    } else if (chol_S) {   // S_l = K6 - (K6 T_l)(K6 T_l)^T   (util.py:387-388), chol_S [L, M, M]
+    } else if (chol_S) {   // S_l = K6_l - (K6_l T_l)(K6_l T_l)^T   (util.py:387-388), chol_S [L, M, M]
         for (int l = 0; l < c->L; ++l) {
+            select_latent(c, l);
             GemmP p;
             p.A = c->K6; p.lda = n; p.a_kc = 1;
             p.B = c->T_all + (size_t)l * n * n; p.ldb = n; p.b_kc = 0; p.b_tri = 2;
@@ -2508,6 +2720,7 @@ int tsvgp_posterior(tsvgp_ctx* c, double* m, double* chol_S) {
             CU(cudaMemcpy2DAsync(chol_S + (size_t)l * c->M * c->M, sizeof(double) * c->M, c->X2, sizeof(double) * n, sizeof(double) * c->M, c->M,
                                  cudaMemcpyDefault, s));
         }
+        select_latent(c, 0);
     }
     int info_h[N_INFO];
     CU(cudaMemcpyAsync(info_h, c->info, sizeof info_h, cudaMemcpyDeviceToHost, s));

@@ -4,8 +4,10 @@ implements: `natgrad_step`, `elbo`, `predict_f` over `DenseSites (lambda_1, lamb
 
 The GPflow kernel, likelihood and inducing-variable objects are used unchanged: only the attributes the reference path
 reads are touched (duck-typed; `.numpy()` is honoured):
-    kernel      SquaredExponential / RBF / Matern52 : .variance, .lengthscales (scalar, [D] or [1, D])
+    kernel      SquaredExponential / RBF / Matern52 : .variance, .lengthscales (scalar, [D] or [1, D]);
+                SharedIndependent (.kernel, .output_dim) ; SeparateIndependent (.kernels, one per latent)
     likelihood  Gaussian (.variance) | Bernoulli (inv_probit link) | StudentT (.scale, .df)   [+ .num_gauss_hermite_points]
+                | Softmax | HeteroskedasticTFPConditional (distribution_class Normal, scale_transform Exp / Softplus)
     inducing    InducingPoints (.Z) or an ndarray [M, D]
     mean_function  None / Zero, or a callable evaluated on the host
 All arithmetic runs in libtsvgp.so on the GPU (float64); tensors cross through DLPack + ctypes.  There is no CPU fallback.
@@ -28,8 +30,18 @@ def _value(p):
     return np.asarray(p, dtype=np.float64)
 
 
-def _kernel_spec(kernel):
+def _kernel_spec(kernel, num_latent_gps=None):
+    """(kind, variance, lengthscales) of one kernel; a list of them, one per latent, for SeparateIndependent."""
     name = type(kernel).__name__
+    if name == "SharedIndependent":   # gpflow.kernels.SharedIndependent(kernel, output_dim): one kernel for every latent
+        if num_latent_gps is not None and int(kernel.output_dim) != int(num_latent_gps):
+            raise _lib.InvalidArgumentError(_lib.ERR_INVALID, f"SharedIndependent output_dim {kernel.output_dim} != num_latent_gps {num_latent_gps}")
+        return _kernel_spec(kernel.kernel)
+    if name == "SeparateIndependent":   # gpflow.kernels.SeparateIndependent(kernels): one kernel per latent
+        specs = [_kernel_spec(k) for k in kernel.kernels]
+        if num_latent_gps is not None and len(specs) != int(num_latent_gps):
+            raise _lib.InvalidArgumentError(_lib.ERR_INVALID, f"SeparateIndependent has {len(specs)} kernels, num_latent_gps is {num_latent_gps}")
+        return specs
     if name in ("SquaredExponential", "RBF"):
         kind = _lib.KERNEL_SE
     elif name == "Matern52":
@@ -57,7 +69,33 @@ def _likelihood_spec(lik):
         return _lib.LIK_STUDENT_T, float(_value(lik.scale)), float(_value(lik.df)), n_gh
     if name == "Softmax":   # gpflow.likelihoods.Softmax(num_classes): MonteCarloLikelihood, num_monte_carlo_points = 100
         return _lib.LIK_SOFTMAX, float(lik.num_classes), 0.0, int(getattr(lik, "num_monte_carlo_points", 100))
-    raise NotImplementedError(f"likelihood {name}: the B200 path implements Gaussian, Bernoulli (probit) and StudentT")
+    if name == "HeteroskedasticTFPConditional":   # 2 latents (loc, scale), NDiagGHQuadrature(2, n_gh)
+        dist = getattr(getattr(lik, "distribution_class", None), "__name__", None)
+        transform = type(getattr(lik, "scale_transform", None)).__name__
+        if dist != "Normal":
+            raise NotImplementedError(f"HeteroskedasticTFPConditional: distribution_class {dist}; the B200 path implements Normal")
+        if transform not in ("Exp", "Softplus"):
+            raise NotImplementedError(f"HeteroskedasticTFPConditional: scale_transform {transform}; the B200 path implements Exp and Softplus")
+        return _lib.LIK_HETEROSKEDASTIC, 0.0 if transform == "Exp" else 1.0, 0.0, _n_gh(lik)
+    raise NotImplementedError(f"likelihood {name}: the B200 path implements Gaussian, Bernoulli (probit), StudentT, Softmax and "
+                              "HeteroskedasticTFPConditional")
+
+
+def _n_gh(lik):
+    """Gauss-Hermite points per axis: likelihood.quadrature.n_gh, else num_gauss_hermite_points, else GPflow's default 20."""
+    q = getattr(lik, "quadrature", None)
+    if q is not None and hasattr(q, "n_gh"):
+        return int(q.n_gh)
+    return int(getattr(lik, "num_gauss_hermite_points", DEFAULT_N_GH))
+
+
+def _coupled(lik):
+    """The likelihood couples the latents of a point: Y is [N, 1] whatever num_latent_gps is."""
+    return type(lik).__name__ in ("Softmax", "HeteroskedasticTFPConditional")
+
+
+def _separate(kernel):
+    return type(kernel).__name__ == "SeparateIndependent"
 
 
 class DenseSites:
@@ -153,11 +191,23 @@ class t_SVGP:
         return np.ascontiguousarray(_value(mf(X)).reshape(X.shape[0], -1)[:, 0])
 
     def _sync_objects(self):
-        kind, var, ls = _kernel_spec(self.kernel)
-        key = (kind, var, ls.tobytes())
-        if key != self._kernel_key:
-            self._check(self._lib.tsvgp_set_kernel(self._ctx, kind, var, ls.ctypes.data_as(_lib._dp), ls.size))
-            self._kernel_key = key
+        spec = _kernel_spec(self.kernel, self.num_latent_gps)
+        if isinstance(spec, list):   # one kernel per latent: the key holds every latent's parameters
+            key = tuple((kind, var, ls.tobytes()) for kind, var, ls in spec)
+            if key != self._kernel_key:
+                kinds = np.array([k for k, _, _ in spec], dtype=np.int32)
+                var = np.array([v for _, v, _ in spec], dtype=np.float64)
+                ls = np.ascontiguousarray(np.concatenate([l for _, _, l in spec]), dtype=np.float64)
+                nls = np.array([l.size for _, _, l in spec], dtype=np.int32)
+                self._check(self._lib.tsvgp_set_kernels(self._ctx, kinds.ctypes.data, var.ctypes.data_as(_lib._dp),
+                                                        ls.ctypes.data_as(_lib._dp), nls.ctypes.data))
+                self._kernel_key = key
+        else:
+            kind, var, ls = spec
+            key = (kind, var, ls.tobytes())
+            if key != self._kernel_key:
+                self._check(self._lib.tsvgp_set_kernel(self._ctx, kind, var, ls.ctypes.data_as(_lib._dp), ls.size))
+                self._kernel_key = key
         lk = _likelihood_spec(self.likelihood)
         if lk != self._lik_key:
             gx = gw = None
@@ -235,7 +285,7 @@ class t_SVGP:
             raise _lib.InvalidArgumentError(_lib.ERR_INVALID, "X must be [N, D]")
         N, D = tx.shape
         ny = int(np.prod(ty.shape))
-        ycols = 1 if type(self.likelihood).__name__ == "Softmax" else self.num_latent_gps
+        ycols = 1 if _coupled(self.likelihood) else self.num_latent_gps
         if ny != N * ycols:
             raise _lib.InvalidArgumentError(_lib.ERR_INVALID, f"Y must be [N, {ycols}] with N = {N}, got {ty.shape}")
         mean_x = None
@@ -248,7 +298,7 @@ class t_SVGP:
         return N
 
     def stage_data(self, data):
-        if self.num_latent_gps > 1 and type(self.likelihood).__name__ != "Softmax":
+        if self.num_latent_gps > 1 and not _coupled(self.likelihood):
             raise NotImplementedError("stage_data with num_latent_gps > 1: use set_data")
         """Start copying the NEXT minibatch to the GPU on a copy stream while the current step computes (use pinned host
         arrays, `tsvgp_b200.pinned_empty`, for a truly asynchronous copy); `commit_staged()` makes it resident."""
@@ -306,17 +356,22 @@ class t_SVGP:
         -> (elbo, {"variance", "lengthscales" (shape of kernel.lengthscales), "Z" [M, D], "likelihood"}), gradients w.r.t. the
         constrained parameter values (chain your own positive transform); "likelihood" is d/d variance (Gaussian),
         d/d scale (StudentT) or None (Bernoulli)."""
+        if _separate(self.kernel):
+            raise NotImplementedError("elbo_and_grad with SeparateIndependent kernels")
+        if type(self.likelihood).__name__ == "HeteroskedasticTFPConditional":
+            raise NotImplementedError("elbo_and_grad with the heteroskedastic likelihood")
         self._sync_objects()
         if self._mean_fn(np.zeros((1, self._D))) is not None:
             raise NotImplementedError("elbo_and_grad with a non-zero mean_function")
         n = self._ingest(data)
-        kind, _, ls = _kernel_spec(self.kernel)
+        kernel = self.kernel.kernel if type(self.kernel).__name__ == "SharedIndependent" else self.kernel
+        kind, _, ls = _kernel_spec(kernel)
         e, dv, dl = C.c_double(), C.c_double(), C.c_double()
         dls, dZ = np.empty(ls.size), np.empty((self._M, self._D))
         self._check(self._lib.tsvgp_elbo_grad(self._ctx, self._scale(n, global_minibatch_size), C.byref(e), C.byref(dv),
                                               dls.ctypes.data, dZ.ctypes.data, C.byref(dl)))
         lik = _likelihood_spec(self.likelihood)[0]
-        return e.value, {"variance": dv.value, "lengthscales": dls.reshape(np.shape(_value(self.kernel.lengthscales)) or ()),
+        return e.value, {"variance": dv.value, "lengthscales": dls.reshape(np.shape(_value(kernel.lengthscales)) or ()),
                          "Z": dZ, "likelihood": None if lik == _lib.LIK_BERNOULLI_PROBIT else dl.value}
 
     def maximum_log_likelihood_objective(self, data=None):  # tsvgp.py:72-77
@@ -402,17 +457,32 @@ class t_SVGP:
     # 145,251).  O(N) host arithmetic on the GPU's predict_f output; GPflow 2.2.1 likelihood semantics [GPflow-recalled]:
     # Gaussian closed forms; Bernoulli(inv_probit) analytic mean; Student-t / generic via 20-point Gauss-Hermite. -------------
     def _gh(self):
-        n = int(getattr(self.likelihood, "num_gauss_hermite_points", DEFAULT_N_GH))
-        x, w = np.polynomial.hermite.hermgauss(n)
+        x, w = np.polynomial.hermite.hermgauss(_n_gh(self.likelihood))
         return x * np.sqrt(2.0), w / np.sqrt(np.pi)
+
+    def _hetero_grid(self, Xnew):
+        """HeteroskedasticTFPConditional: predict_f's marginals on the NDiagGHQuadrature grid -> (loc F0 [N, n, 1],
+        scale T(F1) [N, 1, n], log weights [1, n, n]) over the n x n nodes."""
+        mu, var = self.predict_f(Xnew)
+        z, w = self._gh()
+        F0 = (mu[:, 0:1] + np.sqrt(var[:, 0:1]) * z)[:, :, None]
+        F1 = (mu[:, 1:2] + np.sqrt(var[:, 1:2]) * z)[:, None, :]
+        scale = np.exp(F1) if type(self.likelihood.scale_transform).__name__ == "Exp" else np.logaddexp(0.0, F1)
+        return F0, scale, np.log(w)[None, :, None] + np.log(w)[None, None, :]
 
     def predict_y(self, Xnew, full_cov=False, full_output_cov=False):
         """GPModel.predict_y -> likelihood.predict_mean_and_var(f_mean, f_var)."""
         from math import erf
         if full_cov or full_output_cov:   # as GPflow 2.2.1's likelihoods: only the marginals are propagated
             raise NotImplementedError("predict_y with full_cov / full_output_cov")
-        mu, var = self.predict_f(Xnew)
         name = type(self.likelihood).__name__
+        if name == "HeteroskedasticTFPConditional":   # QuadratureLikelihood: E[loc], E[scale^2 + loc^2] - E[loc]^2  -> [N, 1]
+            F0, scale, logw = self._hetero_grid(Xnew)
+            W = np.exp(logw)
+            Ey = np.sum(W * F0, axis=(1, 2))
+            Ey2 = np.sum(W * (np.square(scale) + np.square(F0)), axis=(1, 2))
+            return Ey[:, None], (Ey2 - np.square(Ey))[:, None]
+        mu, var = self.predict_f(Xnew)
         if name == "Gaussian":
             return mu, var + float(_value(self.likelihood.variance))
         if name == "Bernoulli":
@@ -428,8 +498,14 @@ class t_SVGP:
             raise NotImplementedError("predict_log_density with full_cov / full_output_cov")
         X, Y = data
         Y = np.asarray(Y, dtype=np.float64)
-        mu, var = self.predict_f(X)
         name = type(self.likelihood).__name__
+        if name == "HeteroskedasticTFPConditional":   # log sum_ij w_i w_j Normal(F0_i, T(F1_j)).pdf(y)  -> [N]
+            from scipy.special import logsumexp
+            F0, scale, logw = self._hetero_grid(X)
+            y = Y.reshape(-1, 1, 1)
+            logp = -0.5 * np.log(2 * np.pi) - np.log(scale) - 0.5 * np.square((y - F0) / scale)
+            return logsumexp(logp + logw, axis=(1, 2))
+        mu, var = self.predict_f(X)
         if name == "Gaussian":
             v = var + float(_value(self.likelihood.variance))
             return np.sum(-0.5 * (np.log(2 * np.pi) + np.log(v) + np.square(Y - mu) / v), axis=-1)
@@ -503,8 +579,10 @@ class t_SVGP_white(t_SVGP):
             lambda_2 = np.asarray(lambda_2, dtype=np.float64)
             assert lambda_2.ndim == 3  # tsvgp_white.py:87
             num_latent_gps = lambda_2.shape[0]
-        if type(likelihood).__name__ == "Softmax":
-            raise NotImplementedError("t_SVGP_white with the Softmax likelihood")
+        if _coupled(likelihood):
+            raise NotImplementedError(f"t_SVGP_white with the {type(likelihood).__name__} likelihood")
+        if _separate(kernel):
+            raise NotImplementedError("t_SVGP_white with SeparateIndependent kernels")
         super().__init__(kernel, likelihood, inducing_variable, mean_function=mean_function, num_latent_gps=num_latent_gps,
                          num_data=num_data, device=device)
         self.name = "t_svgp_white"

@@ -20,6 +20,21 @@ class Matern52:
         self.lengthscales = np.asarray(lengthscales, dtype=np.float64)
 
 
+class SharedIndependent:
+    """gpflow.kernels.SharedIndependent(kernel, output_dim): one kernel for every latent GP."""
+
+    def __init__(self, kernel, output_dim):
+        self.kernel = kernel
+        self.output_dim = int(output_dim)
+
+
+class SeparateIndependent:
+    """gpflow.kernels.SeparateIndependent(kernels): one kernel per latent GP."""
+
+    def __init__(self, kernels):
+        self.kernels = list(kernels)
+
+
 class Gaussian:
     def __init__(self, variance=1.0):
         self.variance = float(variance)
@@ -41,6 +56,35 @@ class Softmax:
     def __init__(self, num_classes, num_monte_carlo_points=100):
         self.num_classes = int(num_classes)
         self.num_monte_carlo_points = int(num_monte_carlo_points)
+
+
+class Normal:
+    """tfp.distributions.Normal: only the class name is read."""
+
+
+class Exp:
+    """tfp.bijectors.Exp: only the class name is read."""
+
+
+class Softplus:
+    """tfp.bijectors.Softplus: only the class name is read."""
+
+
+class NDiagGHQuadrature:
+    def __init__(self, dim, n_gh):
+        self.dim = int(dim)
+        self.n_gh = int(n_gh)
+
+
+class HeteroskedasticTFPConditional:
+    """gpflow.likelihoods.HeteroskedasticTFPConditional(distribution_class, scale_transform): two latent GPs, loc and
+    scale = scale_transform(f_1); quadrature NDiagGHQuadrature(latent_dim, num_gauss_hermite_points)."""
+
+    def __init__(self, distribution_class=Normal, scale_transform=None, num_gauss_hermite_points=20):
+        self.distribution_class = distribution_class
+        self.scale_transform = Exp() if scale_transform is None else scale_transform
+        self.latent_dim = 2
+        self.quadrature = NDiagGHQuadrature(self.latent_dim, num_gauss_hermite_points)
 
 
 class InducingPoints:

@@ -31,8 +31,12 @@ class _Adam:
 
 
 def fit(model, data, n_iters=10, n_e_steps=8, n_m_steps=20, lr_natgrad=1.0, lr_adam=0.1, train_Z=False, callback=None):
-    """Run variational EM on `data = (X, Y)` (kept resident on the GPU).  Mutates model.kernel / model.likelihood
+    """Run variational EM on `data = (X, Y)` (kept resident on the GPU).  Mutates model.kernel (the wrapped kernel of a
+    SharedIndependent) / model.likelihood
     (and model.inducing_variable when train_Z) in place; returns the ELBO trace (one value per M-step evaluation)."""
+    if type(model.kernel).__name__ == "SeparateIndependent":
+        raise NotImplementedError("vem.fit with SeparateIndependent kernels: elbo_and_grad is not built for them")
+    kernel = model.kernel.kernel if type(model.kernel).__name__ == "SharedIndependent" else model.kernel   # the shared kernel
     model.set_data(data)
     adam = _Adam(lr_adam)
     lik_name = type(model.likelihood).__name__
@@ -45,11 +49,11 @@ def fit(model, data, n_iters=10, n_e_steps=8, n_m_steps=20, lr_natgrad=1.0, lr_a
             elbo, g = model.elbo_and_grad()
             trace.append(elbo)
             adam.t += 1
-            var = float(_value(model.kernel.variance))
-            ls = _value(model.kernel.lengthscales)
-            _assign(model.kernel, "variance", float(np.exp(adam.step("log_var", np.log(var), var * g["variance"]))))
+            var = float(_value(kernel.variance))
+            ls = _value(kernel.lengthscales)
+            _assign(kernel, "variance", float(np.exp(adam.step("log_var", np.log(var), var * g["variance"]))))
             new_ls = np.exp(adam.step("log_ls", np.log(ls), ls * np.reshape(g["lengthscales"], np.shape(ls))))
-            _assign(model.kernel, "lengthscales", new_ls if np.ndim(ls) else float(new_ls))
+            _assign(kernel, "lengthscales", new_ls if np.ndim(ls) else float(new_ls))
             if lik_attr is not None:
                 th = float(_value(getattr(model.likelihood, lik_attr)))
                 _assign(model.likelihood, lik_attr, float(np.exp(adam.step("log_lik", np.log(th), th * g["likelihood"]))))
