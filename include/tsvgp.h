@@ -132,7 +132,8 @@ TSVGP_API int tsvgp_num_latent(const tsvgp_ctx* ctx);
  * (= L) and n_gh = Monte-Carlo points per data point (GPflow: 100).  GPflow draws fresh standard normals [S, N, L] in every
  * call; here they come from a counter-based generator (Philox4x32-10 + Box-Muller, option "mc_seed", a new draw per call) or,
  * for reproducible comparisons, from an explicit array eps [S, N, L] (HOST or DEVICE; used whenever a pass runs over exactly
- * N points; NULL clears it).                                                                                                   */
+ * N points; NULL clears it).  tsvgp_elbo and tsvgp_elbo_grad each take one draw: elbo_grad at draw k sees the draws (and
+ * returns the ELBO) that tsvgp_elbo would at draw k.                                                                           */
 TSVGP_API int tsvgp_set_mc_epsilon(tsvgp_ctx* ctx, const double* eps, int S, int64_t N, int L);
 
 /* ---- DenseSites state (src/sites.py:43-80): lambda_1 [M, L], lambda_2_sqrt [L, M, M] lower triangular ------------- */
@@ -163,9 +164,12 @@ TSVGP_API int tsvgp_elbo(tsvgp_ctx* ctx, double scale, double* out);
 TSVGP_API int tsvgp_prior_kl(tsvgp_ctx* ctx, double* out);
 /* M-step: ELBO of the resident minibatch and its gradient w.r.t. the kernel variance, the lengthscales (n_ls entries, as
  * given to tsvgp_set_kernel), the inducing inputs Z [M, D] and the likelihood parameter (Gaussian: variance; StudentT:
- * scale; Bernoulli: 0), with the sites held fixed — what the reference obtains by TensorFlow autodiff through `elbo`
- * (tsvgp.py:79-95; callers docs/notebooks/mnist.py:161-163,188-189; pinned by tests/models/test_tsvgp.py:168-188).
- * Gradients are w.r.t. the constrained (natural) parameter values; Zero mean function; D <= 63.                         */
+ * scale; Bernoulli, Softmax: 0), with the sites held fixed — what the reference obtains by TensorFlow autodiff through
+ * `elbo` (tsvgp.py:79-95; callers docs/notebooks/mnist.py:161-163,188-189; pinned by tests/models/test_tsvgp.py:168-188).
+ * Gradients are w.r.t. the constrained (natural) parameter values; Zero mean function; any D; one kernel shared by the
+ * latents.  Softmax: the derivatives of the Monte-Carlo sum for the call's draws (one per call, see tsvgp_set_mc_epsilon),
+ * with h = d ve / d var unclipped; one pass over the data for all latents.  Not built for the heteroskedastic likelihood,
+ * separate kernels per latent or the whitened sibling (TSVGP_ERR_INVALID).                                               */
 TSVGP_API int tsvgp_elbo_grad(tsvgp_ctx* ctx, double scale, double* elbo, double* d_variance, double* d_lengthscales,
                               double* d_Z, double* d_lik);
 /* base_SVGP.predict_f, full_cov = False (tsvgp.py:97-114): mean_out, var_out [N, L]                                     */

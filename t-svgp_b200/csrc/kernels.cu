@@ -373,7 +373,7 @@ __device__ __forceinline__ void normal_pair(unsigned long long seed, unsigned lo
 __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
     __shared__ double sred[4];
     const int c = blockIdx.x * 128 + threadIdx.x;
-    double ve = 0.0;
+    double ve = 0.0, hsum = 0.0;
     if (c < a.ncols) {
         const bool valid = c < a.n_valid;
         double mu[MAX_SOFTMAX_CLASSES], sd[MAX_SOFTMAX_CLASSES], gm[MAX_SOFTMAX_CLASSES], gs[MAX_SOFTMAX_CLASSES];
@@ -421,12 +421,18 @@ __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
             }
             const double invS = 1.0 / (double)a.S;
             ve *= invS;
-            for (int l = 0; l < a.L; ++l) { gm[l] *= invS; gs[l] = fmin(gs[l] * invS / (2.0 * sd[l]), -1e-8); }
+            for (int l = 0; l < a.L; ++l) {
+                gm[l] *= invS;
+                gs[l] = gs[l] * invS / (2.0 * sd[l]);
+                if (a.clip) gs[l] = fmin(gs[l], -1e-8);
+            }
         } else {
-            for (int l = 0; l < a.L; ++l) gs[l] = (valid && a.y) ? -1e-8 : 0.0;
+            for (int l = 0; l < a.L; ++l) gs[l] = (valid && a.y && a.clip) ? -1e-8 : 0.0;
         }
         if (a.g)
             for (int l = 0; l < a.L; ++l) { a.g[l * a.gh_lat + c] = valid ? gm[l] : 0.0; a.h[l * a.gh_lat + c] = valid ? gs[l] : 0.0; }
+        if (a.aux_blocks && valid)
+            for (int l = 0; l < a.L; ++l) hsum += gs[l];
         if (!valid) ve = 0.0;
     }
     ve = warp_sum(ve);
@@ -436,6 +442,13 @@ __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
         const double s2 = (sred[0] + sred[1]) + (sred[2] + sred[3]);
         // ve_blocks holds one slot per 256 points (point_stats_kernel's layout): two 128-thread blocks share one
         atomicAdd(a.ve_blocks + (blockIdx.x >> 1), s2);
+    }
+    if (a.aux_blocks) {   // sum of h for the s sum_n h term of the kernel-variance gradient; same slots and order as ve_blocks
+        __syncthreads();
+        hsum = warp_sum(hsum);
+        if ((threadIdx.x & 31) == 0) sred[threadIdx.x >> 5] = hsum;
+        __syncthreads();
+        if (threadIdx.x == 0) atomicAdd(a.aux_blocks + 2 * (blockIdx.x >> 1), (sred[0] + sred[1]) + (sred[2] + sred[3]));
     }
 }
 int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s) {
@@ -1738,29 +1751,35 @@ int stats_tail_launch(const double* ve_blocks, long nblocks, const int* flags, c
 
 // ---- M-step gradient helpers ------------------------------------------------------------------------------------
 // E[i][c] = scale * (alpha[i] g[c] - 2 h[c] U[i][c]) * Kp[i][c]   in place on U   (dELBO/dKuf times dk/dr2)
+// ACC: added to E instead (the latents of a coupled likelihood share Kuf, so their dELBO/dKuf add up before the F product)
+template <bool ACC>
 __global__ void egrad_uf_kernel(double* __restrict__ U, const double* __restrict__ Kp, long ld, int Mp, int ncols,
-                                const double* __restrict__ alpha, const double* __restrict__ g, const double* __restrict__ h, double scale) {
+                                const double* __restrict__ alpha, const double* __restrict__ g, const double* __restrict__ h, double scale,
+                                double* __restrict__ E) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     const int i0 = blockIdx.y * 16;
     if (c >= ncols) return;
     const double gc = g[c], hc2 = 2.0 * h[c];
     for (int i = i0; i < i0 + 16 && i < Mp; ++i) {
         const long o = (long)i * ld + c;
-        U[o] = scale * (alpha[i] * gc - hc2 * U[o]) * Kp[o];
+        if (ACC) E[o] += scale * (alpha[i] * gc - hc2 * U[o]) * Kp[o];
+        else U[o] = scale * (alpha[i] * gc - hc2 * U[o]) * Kp[o];
     }
 }
 int egrad_uf_launch(double* U, const double* Kp, long ld, int Mp, int ncols, const double* alpha, const double* g, const double* h,
-                    double scale, cudaStream_t s) {
-    egrad_uf_kernel<<<dim3((ncols + 255) / 256, (Mp + 15) / 16), 256, 0, s>>>(U, Kp, ld, Mp, ncols, alpha, g, h, scale);
+                    double scale, cudaStream_t s, double* E) {
+    const dim3 grid((ncols + 255) / 256, (Mp + 15) / 16);
+    if (E) egrad_uf_kernel<true><<<grid, 256, 0, s>>>(U, Kp, ld, Mp, ncols, alpha, g, h, scale, E);
+    else egrad_uf_kernel<false><<<grid, 256, 0, s>>>(U, Kp, ld, Mp, ncols, alpha, g, h, scale, nullptr);
     return count_launch();
 }
-// Xa[c][j] (row-major [ncols][128]) = xs_j | 1 | xs_j^2 | 0 ... of point n0 + c (zero rows for c >= nvalid)
+// Xa[c][j] (row-major [ncols][W], W = aug_width(D)) = xs_j | 1 | xs_j^2 | 0 ... of point n0 + c (zero rows for c >= nvalid)
 __global__ void xaug_kernel(const double* __restrict__ XsT, long ldx, long n0, long nvalid, int ncols, int D, double* __restrict__ Xa,
-                            const double* __restrict__ origin) {
+                            const double* __restrict__ origin, int W) {
     __shared__ double tile[32][33];
-    // block: 32 points x 128 aug columns; transposes through shared memory so both sides stay coalesced
+    // block: 32 points x W aug columns, 32 at a time; transposes through shared memory so both sides stay coalesced
     const int c0 = blockIdx.x * 32, tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 256 threads = 8 rows of 32
-    for (int jb = 0; jb < 128; jb += 32) {
+    for (int jb = 0; jb < W; jb += 32) {
         for (int r = ty; r < 32; r += 8) {   // r = aug column within the 32-block, tx = point
             const int j = jb + r;
             const long c = c0 + tx;
@@ -1776,13 +1795,13 @@ __global__ void xaug_kernel(const double* __restrict__ XsT, long ldx, long n0, l
         }
         __syncthreads();
         for (int r = ty; r < 32; r += 8) {   // r = point, tx = aug column
-            if (c0 + r < ncols) Xa[(long)(c0 + r) * 128 + jb + tx] = tile[tx][r];
+            if (c0 + r < ncols) Xa[(long)(c0 + r) * W + jb + tx] = tile[tx][r];
         }
         __syncthreads();
     }
 }
 int xaug_launch(const double* XsT, long ldx, long n0, long nvalid, int ncols, int D, double* Xa, cudaStream_t s, const double* origin) {
-    xaug_kernel<<<(ncols + 31) / 32, 256, 0, s>>>(XsT, ldx, n0, nvalid, ncols, D, Xa, origin);
+    xaug_kernel<<<(ncols + 31) / 32, 256, 0, s>>>(XsT, ldx, n0, nvalid, ncols, D, Xa, origin, aug_width(D));
     return count_launch();
 }
 // Gamma[i][j] = scale (QBQ_ij - (qb_i a_j + qb_j a_i)/2) - (a_i a_j - (qm_i a_j + qm_j a_i) + QKQ_ij)/2   (dELBO/dKuu, symmetric)

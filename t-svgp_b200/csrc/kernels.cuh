@@ -50,6 +50,7 @@ struct PointArgs {
 // Softmax likelihood over L latents (gpflow.likelihoods.Softmax = MonteCarloLikelihood, S = num_monte_carlo_points): per point
 //   ve = mean_s log softmax(f_s)[y],  f_s = mu + sqrt(var) * eps_s ;  g_l = d ve / d mu_l ;  h_l = min(d ve / d var_l, -1e-8)
 // as called at reference tsvgp.py:256-263 (docs/notebooks/mnist.py:117-122).  Per-latent inputs / outputs are `*_lat` apart.
+// clip = 0 (M-step gradients) leaves h_l unclipped and, with aux_blocks, adds the sum of h over the block's points and latents.
 // eps: explicit standard-normal draws [S][n_total][L] (GPflow's layout) or null = Philox4x32-10 + Box-Muller keyed by (seed, draw).
 // The heteroskedastic likelihood takes the same arguments (S, eps, seed and draw unused).
 struct SoftmaxArgs {
@@ -67,6 +68,8 @@ struct SoftmaxArgs {
     int* flags;
     const double* eps;
     unsigned long long seed, draw;
+    int clip = 1;                   // clip h_l at -1e-8 (natgrad_step); the ELBO gradient does not (heteroskedastic: always clipped)
+    double* aux_blocks = nullptr;   // out (Softmax M-step): per 256 points [sum h over points and latents, 0], as PointArgs
 };
 int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s);
 // Heteroskedastic Normal likelihood over L = 2 latents (GPflow HeteroskedasticTFPConditional(Normal, scale_transform) with its
@@ -156,10 +159,12 @@ int vadd_inplace_launch(double* dst, const double* src, long n, cudaStream_t s);
 int sum_rows_into_launch(const double* src, int rows, int n, double* dst, cudaStream_t s);   // dst[j] += sum_r src[r][j]  (fixed order)
 int stats_tail_launch(const double* ve_blocks, long nblocks, const int* flags, const double* aux, double* out, cudaStream_t s);
 // M-step gradient helpers (see tsvgp_elbo_grad)
+// E = scale (alpha g^T - 2 U diag(h)) .* Kp, written over U (E = null) or added to E (a coupled likelihood's latents share one E)
 int egrad_uf_launch(double* U, const double* Kp, long ld, int Mp, int ncols, const double* alpha, const double* g, const double* h,
-                    double scale, cudaStream_t s);
-// Xa[c][0:128] = [xs - origin | 1 | (xs - origin)^2] of point n0 + c (origin [D] device vector or null)
+                    double scale, cudaStream_t s, double* E = nullptr);
+// Xa[c][0:W] = [xs - origin | 1 | (xs - origin)^2 | 0] of point n0 + c (origin [D] device vector or null); W = aug_width(D)
 int xaug_launch(const double* XsT, long ldx, long n0, long nvalid, int ncols, int D, double* Xa, cudaStream_t s, const double* origin = nullptr);
+inline int aug_width(int D) { return (2 * D + 1 + 127) / 128 * 128; }
 int gamma_uu_launch(const double* QBQ, const double* QKQ, const double* qb, const double* qm, const double* al, const double* Kp,
                     double* Gamma, double* E, long ld, int n, double scale, cudaStream_t s);
 

@@ -228,6 +228,8 @@ struct tsvgp_ctx {
     double* aux_blocks = nullptr;
     int fsplit = 1;
     bool grad_ws = false;
+    int grad_lat = 0;     // U slabs per slab stream in the gradient workspace: L for a coupled likelihood (one pass), else 1
+    int waug = 128;       // columns of the augmented blocks [xs | 1 | xs^2 | 0] (xaug, zaug, facc, fuu, fpart): aug_width(D)
     double* kpart[MAXS] = {};     // split-K partial tiles of the SYRK when M is so small that its tiles cannot fill the SMs
     double* bacc[MAXS] = {};      // fused b += Kuf g shared by the tiles of a tile row: [L][2 pieces][Mp/128 tile columns][Mp] private slots
     int ksplit = 1;
@@ -355,7 +357,8 @@ int alloc_m_state(tsvgp_ctx* c, int M, int D) {
     // (on the context's own stream: it is non-blocking, a legacy-stream memset would not be ordered with it)
     CU(cudaMemsetAsync(c->gws + c->gws_doubles - GEMM_WS_COUNTER_DOUBLES, 0, sizeof(double) * GEMM_WS_COUNTER_DOUBLES, c->s_main));    // tile counters
     CU(cudaMemsetAsync(c->gws2 + c->gws_doubles - GEMM_WS_COUNTER_DOUBLES, 0, sizeof(double) * GEMM_WS_COUNTER_DOUBLES, c->s_main));
-    NEED(c->zaug = p.get(mp * 128)); NEED(c->fuu = p.get(mp * 128)); NEED(c->origin = p.get(D));
+    c->waug = aug_width(D);
+    NEED(c->zaug = p.get(mp * c->waug)); NEED(c->fuu = p.get(mp * c->waug)); NEED(c->origin = p.get(D));
     NEED(c->C6 = p.get(mm)); NEED(c->C6inv = p.get(mm));
     c->c6_valid = c->wpost_valid = c->wkl_valid = false;
     NEED(c->tmp2 = p.get((size_t)((c->Mp / 128 + 1) / 2) * 128 * mp)); NEED(c->dinv2 = p.get((size_t)(c->Mp / 128) * 128 * 128));
@@ -742,8 +745,12 @@ long used_chunk(const tsvgp_ctx* c, long n_points, long nc, int nstr) {
     return ncu < nc ? ncu : nc;
 }
 
+// the likelihood couples the latents (one point kernel over all of them, Y [N, 1]): Softmax, heteroskedastic Normal
+inline bool coupled(const tsvgp_ctx* c) { return c->lik.kind == LIK_SOFTMAX || c->lik.kind == LIK_HETEROSKEDASTIC; }
+
 int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const long nc = pick_chunk(c);
+    const int u_lat = need_grad && coupled(c) ? c->L : 1;   // the gradient pass of a coupled likelihood keeps every latent's U
     const int nstr_used = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     const long ncu = used_chunk(c, n_points, nc, nstr_used);
     const long nchunks = (n_points + ncu - 1) / ncu;
@@ -751,7 +758,7 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const bool need_w = c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT;
     const int want_streams = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     const int slab_lat = c->sep ? c->L : 1;
-    if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || c->grad_ws) &&
+    if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || (c->grad_ws && c->grad_lat >= u_lat)) &&
         c->slab_streams >= want_streams && c->slab_lat == slab_lat)
         return TSVGP_OK;
     CU(cudaStreamSynchronize(c->s_main));
@@ -788,19 +795,30 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     NEED(c->ve_all = p.get((size_t)c->L * ve_need));
     for (int s = 0; s < ns; ++s) NEED(c->bacc[s] = p.get((size_t)c->L * 2 * (c->Mp / 128) * c->Mp));
     c->grad_ws = false;
+    c->grad_lat = 0;
     if (need_grad) {
         int sms = 148;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->dev);
         c->fsplit = sms / (c->Mp / 128);
         if (c->fsplit > (int)(nc / 256)) c->fsplit = (int)(nc / 256);
         if (c->fsplit < 1) c->fsplit = 1;
+        const size_t W = (size_t)c->waug;
+        if (u_lat > 1) {   // U of every latent survives until the joint point kernel has run: L Mp nc doubles per slab stream
+            const size_t need = ((size_t)(2 + u_lat) * c->Mp * nc + nc * W + (size_t)(c->fsplit + 1) * c->Mp * W) * ns + 2 * ve_need;
+            size_t free_b = 0, total_b = 0;
+            CU(cudaMemGetInfo(&free_b, &total_b));
+            if (need * sizeof(double) > free_b)
+                FAIL(TSVGP_ERR_INVALID, "elbo_grad with %d coupled latents at M = %d needs %zu bytes of device memory for its slab workspace, "
+                     "%zu are free (option \"chunk\" narrows the slabs)", c->L, c->M, need * sizeof(double), free_b);
+        }
         for (int s = 0; s < ns; ++s) {
             NEED(c->kpslab[s] = p.get((size_t)c->Mp * nc)); NEED(c->vslab[s] = p.get((size_t)c->Mp * nc));
-            NEED(c->uslab[s] = p.get((size_t)c->Mp * nc)); NEED(c->xaug[s] = p.get((size_t)nc * 128));
-            NEED(c->fpart[s] = p.get((size_t)c->fsplit * c->Mp * 128)); NEED(c->facc[s] = p.get((size_t)c->Mp * 128));
+            NEED(c->uslab[s] = p.get((size_t)u_lat * c->Mp * nc)); NEED(c->xaug[s] = p.get((size_t)nc * W));
+            NEED(c->fpart[s] = p.get((size_t)c->fsplit * c->Mp * W)); NEED(c->facc[s] = p.get((size_t)c->Mp * W));
         }
         NEED(c->aux_blocks = p.get(2 * ve_need));
         c->grad_ws = true;
+        c->grad_lat = u_lat;
     }
     c->ve_cap = ve_need;
     c->slab_lat = slab_lat;
@@ -817,8 +835,6 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
 // b += Kuf g).
 enum { PASS_WHOLE = 0, PASS_EARLY = 1, PASS_REST = 2 };
 inline bool grad_spread_skip(const tsvgp_ctx*) { return false; }
-// the likelihood couples the latents (one point kernel over all of them, Y [N, 1]): Softmax, heteroskedastic Normal
-inline bool coupled(const tsvgp_ctx* c) { return c->lik.kind == LIK_SOFTMAX || c->lik.kind == LIK_HETEROSKEDASTIC; }
 // y / mean_out / var_out of latent l live at + l * y_stride / + l * out_stride (Y transposed to [L][n_pad]; outputs [L][n_pad_out]).
 // lat_only >= 0 restricts the per-latent work to that latent (the M-step gradient pass runs latent by latent).
 // Separate kernels: latent l's scaled coordinates are at XsT + l * xs_lat, x2 + l * x2_lat, and every latent builds its own slab.
@@ -863,7 +879,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                 CU(cudaMemsetAsync(c->stats_all[s], 0, sizeof(double) * c->L * (mm + Mp + 4), c->s_pp[s]));
                 CU(cudaMemsetAsync(c->stats2_all[s], 0, sizeof(double) * c->L * (mm + Mp), c->s_pp[s]));
                 if (c->spread_b) CU(cudaMemsetAsync(c->bacc[s], 0, sizeof(double) * c->L * 2 * (Mp / 128) * Mp, c->s_pp[s]));
-                if (grad) CU(cudaMemsetAsync(c->facc[s], 0, sizeof(double) * (size_t)Mp * 128, c->s_pp[s]));
+                if (grad) CU(cudaMemsetAsync(c->facc[s], 0, sizeof(double) * (size_t)Mp * c->waug, c->s_pp[s]));
             }
         }
         c->n_early = 0;
@@ -956,6 +972,13 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                 p.epilogue = grad ? EPI_STORE_COLNORM : EPI_COLNORM; p.norm_out = c->q_part[b]; p.ldn = nc;
                 if (grad) { p.C = c->vslab[b]; p.ldc = nc; }   // the M-step also needs V = T^T K itself
                 LA(gemm_launch(p, s));
+                if (grad && joint) {   // U_l = T_l V_l now, into latent l's own U slab: V is overwritten by the next latent
+                    GemmP u;
+                    u.A = c->T; u.lda = Mp; u.a_kc = 1; u.a_tri = 1;
+                    u.B = c->vslab[b]; u.ldb = nc; u.b_kc = 0;
+                    u.C = c->uslab[b] + (size_t)l * Mp * nc; u.ldc = nc; u.m = Mp; u.n = ncols; u.k = Mp;
+                    LA(gemm_launch(u, s));
+                }
             } else {           // (b') whitened sibling: |LA^-1 k_n|^2 and |LR^-1 k_n|^2, two lower-triangular products (util.py:78-85).
                 // The first does not depend on the latent: it is formed once per slab, into the buffer shared by the latents
                 // (`q2_part`); the per-latent one goes to the latent's own `q_part`.
@@ -1004,6 +1027,8 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             a.flags = c->flags;
             a.eps = (c->mc_eps && c->mc_eps_n == N) ? c->mc_eps : nullptr;
             a.seed = c->mc_seed; a.draw = c->mc_draw;
+            a.clip = grad ? 0 : 1;   // the ELBO gradient takes h unclipped
+            a.aux_blocks = grad ? c->aux_blocks + 2 * ci * vstride : nullptr;
             if (c->lik.kind == LIK_HETEROSKEDASTIC) LA(heteroskedastic_stats_launch(c->lik, a, c->gh, s));
             else LA(softmax_stats_launch(a, s));
         }
@@ -1045,7 +1070,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         }
         if (grad) {
             select_latent(c, l_lo);
-            {   // U = T V = Q K  (lower-triangular T times the stored V)
+            if (!joint) {   // U = T V = Q K  (lower-triangular T times the stored V)
                 GemmP p;
                 p.A = c->T; p.lda = Mp; p.a_kc = 1; p.a_tri = 1;
                 p.B = c->vslab[b]; p.ldb = nc; p.b_kc = 0;
@@ -1054,14 +1079,20 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             }
             // E = scale (alpha g^T - 2 U diag(h)) .* dK/dr2   (in place), then F += E [xs | 1 | xs^2]
             LA(egrad_uf_launch(c->uslab[b], c->kpslab[b], nc, Mp, ncols, c->alpha, c->gbuf[b], c->hbuf[b], c->grad_scale, s));
+            for (int l = l_lo + 1; joint && l < l_hi; ++l) {   // coupled likelihood: the latents share Kuf, so E = sum_l E_l (over U_0)
+                select_latent(c, l);
+                LA(egrad_uf_launch(c->uslab[b] + (size_t)l * Mp * nc, c->kpslab[b], nc, Mp, ncols, c->alpha, c->gbuf[b], c->hbuf[b],
+                                   c->grad_scale, s, c->uslab[b]));
+            }
+            select_latent(c, l_lo);
             LA(xaug_launch(XsT, ldx, n0, nvalid, ncols, c->D, c->xaug[b], s, c->origin));
             GemmP p;
             p.A = c->uslab[b]; p.lda = nc; p.a_kc = 1;
-            p.B = c->xaug[b]; p.ldb = 128; p.b_kc = 0;
-            p.C = c->facc[b]; p.ldc = 128; p.m = Mp; p.n = 128; p.k = ncols; p.beta = 1.0;
+            p.B = c->xaug[b]; p.ldb = c->waug; p.b_kc = 0;
+            p.C = c->facc[b]; p.ldc = c->waug; p.m = Mp; p.n = c->waug; p.k = ncols; p.beta = 1.0;
             const int fs = c->fsplit < ncols / 256 ? c->fsplit : ncols / 256;
             if (fs > 1) {
-                p.ksplit = fs; p.part = c->fpart[b]; p.part_stride = (long)Mp * 128;
+                p.ksplit = fs; p.part = c->fpart[b]; p.part_stride = (long)Mp * c->waug;
                 LA(gemm_launch(p, s));
                 LA(splitk_reduce_launch(p, s));
             } else {
@@ -1098,7 +1129,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         const long cnt = (long)((l_hi - l_lo) * (mm + Mp + 4)), cnt2 = (long)((l_hi - l_lo) * (mm + Mp));
         select_latent(c, l_lo);
         for (int s = 1; s < nstr; ++s) LA(vadd_inplace_launch(c->stats[0], c->stats[s], cnt, sm));
-        for (int s = 1; s < nstr && grad; ++s) LA(vadd_inplace_launch(c->facc[0], c->facc[s], (long)Mp * 128, sm));
+        for (int s = 1; s < nstr && grad; ++s) LA(vadd_inplace_launch(c->facc[0], c->facc[s], (long)Mp * c->waug, sm));
         for (int l = l_lo; l < l_hi && c->balance; ++l) {
             select_latent(c, l);
             for (int s = 0; s < nstr; ++s) LA(vadd_inplace_launch(c->stats[0], c->stats2[s], (long)(mm + Mp), sm));
@@ -1107,7 +1138,9 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
     }
     for (int l = l_lo; l < l_hi; ++l) {
         select_latent(c, l);
-        LA(stats_tail_launch(c->ve_blocks, nchunks * vstride, c->flags, grad ? c->aux_blocks : nullptr, c->stats[0] + mm + Mp, sm));
+        // (a coupled likelihood's expectations and sum of h are all in latent 0's slots)
+        LA(stats_tail_launch(c->ve_blocks, nchunks * vstride, c->flags, grad && (!joint || l == 0) ? c->aux_blocks : nullptr,
+                             c->stats[0] + mm + Mp, sm));
     }
     select_latent(c, l_lo);
     return TSVGP_OK;
@@ -2229,18 +2262,16 @@ int tsvgp_prior_kl(tsvgp_ctx* c, double* out) {
     return TSVGP_OK;
 }
 
-// ELBO terms and gradients of ONE latent (the selected one): *elbo = scale * sum ve_l - KL_l; gradients written to HOST vectors
-static int elbo_grad_one(tsvgp_ctx* c, int lat, double scale, const std::vector<double>& origin, double* elbo, double* d_variance,
-                         std::vector<double>& dls_out, std::vector<double>& dZ, double* d_lik) {
+// The dense epilogue of the gradient of ONE latent, after the pass has accumulated its statistics: *elbo = scale * sum ve_l - KL_l
+// (a coupled likelihood: latent 0 carries the whole expectation and sum of h), the kernel-variance and likelihood terms, and
+// F_uu = E_uu [zs | 1 | zs^2] on the host.  Reuses X1 (the KL terms are recomputed on the next call).
+static int grad_epilogue(tsvgp_ctx* c, int lat, double scale, double* elbo, double* d_variance, double* d_lik, std::vector<double>& Fuu) {
     cudaStream_t s = c->s_main;
-    const int n = c->Mp, M = c->M, D = c->D;
+    const int n = c->Mp, M = c->M, D = c->D, W = c->waug;
     const long ld = n;
     const size_t mm = (size_t)n * n;
-    c->grad_scale = scale;
-    OK(data_pass(c, MODE_GRAD, PASS_WHOLE, lat));
     select_latent(c, lat);
     OK(all_reduce(c, c->stats[0], mm + n + 4));
-    OK(all_reduce(c, c->facc[0], (size_t)n * 128));
     double* B = c->stats[0];
     double* bvec = c->stats[0] + mm;
     LA(mirror_lower_launch(B, ld, n, s));
@@ -2275,18 +2306,14 @@ static int elbo_grad_one(tsvgp_ctx* c, int lat, double scale, const std::vector<
     {   // F_uu = E_uu [zs | 1 | zs^2]
         GemmP p;
         p.A = c->G2; p.lda = ld; p.a_kc = 1;
-        p.B = c->zaug; p.ldb = 128; p.b_kc = 0;
-        p.C = c->fuu; p.ldc = 128; p.m = n; p.n = 128; p.k = n;
+        p.B = c->zaug; p.ldb = W; p.b_kc = 0;
+        p.C = c->fuu; p.ldc = W; p.m = n; p.n = W; p.k = n;
         LA(mm_gemm(c, p, s));
     }
-    std::vector<double> Fuf((size_t)n * 128), Fuu((size_t)n * 128), Zs((size_t)n * D), ls(D);
-    dZ.assign((size_t)M * D, 0.0);
+    Fuu.resize((size_t)n * W);
     double tail[4], sc[N_SCAL];
     int info_h[N_INFO];
-    CU(cudaMemcpyAsync(Fuf.data(), c->facc[0], sizeof(double) * n * 128, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(Fuu.data(), c->fuu, sizeof(double) * n * 128, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(Zs.data(), c->Zs, sizeof(double) * n * D, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(ls.data(), c->ls_dev, sizeof(double) * D, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(Fuu.data(), c->fuu, sizeof(double) * n * W, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(tail, c->stats[0] + mm + n, sizeof tail, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(sc, c->scal, sizeof sc, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(info_h, c->info, sizeof info_h, cudaMemcpyDeviceToHost, s));
@@ -2297,31 +2324,83 @@ static int elbo_grad_one(tsvgp_ctx* c, int lat, double scale, const std::vector<
     *elbo = scale * tail[0] - 0.5 * (sc[SC_M_ALPHA] - sc[SC_TR_QK] + 2.0 * sc[SC_LOGDIAG_W]);
     *d_variance = (scale * (sc[SC_A_B] - 2.0 * sc[SC_TR_QB]) + sc[SC_G_K]) / c->kern_var + scale * tail[2];
     *d_lik = scale * tail[3];
-    // d r2 / d lengthscale_d = -2 delta_d^2 / l_d, d r2 / d z_id = 2 delta_d / l_d with delta = zs - xs (scaled coordinates);
-    // sums over points expanded through F = E [xs | 1 | xs^2]:  sum_n E delta = zs S1 - EX ; sum E delta^2 = zs^2 S1 - 2 zs EX + C2
-    std::vector<double> dls(D, 0.0);
+    return TSVGP_OK;
+}
+
+// Lengthscale and Z gradients from F_uf = E_uf [xs | 1 | xs^2] (summed over the points) and F_uu (host, row stride waug):
+// d r2 / d lengthscale_d = -2 delta_d^2 / l_d, d r2 / d z_id = 2 delta_d / l_d with delta = zs - xs (scaled coordinates);
+// sums over points expanded through F:  sum_n E delta = zs S1 - EX ; sum E delta^2 = zs^2 S1 - 2 zs EX + C2
+static int f_to_grads(tsvgp_ctx* c, const std::vector<double>& origin, const std::vector<double>& Fuf, const std::vector<double>& Fuu,
+                      std::vector<double>& dls, std::vector<double>& dZ) {
+    cudaStream_t s = c->s_main;
+    const int n = c->Mp, M = c->M, D = c->D, W = c->waug;
+    std::vector<double> Zs((size_t)n * D), ls(D);
+    CU(cudaMemcpyAsync(Zs.data(), c->Zs, sizeof(double) * n * D, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(ls.data(), c->ls_dev, sizeof(double) * D, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    dZ.assign((size_t)M * D, 0.0);
+    dls.assign(D, 0.0);
     for (int d = 0; d < D; ++d) {
         double acc = 0.0;
         for (int i = 0; i < M; ++i) {
             const double z = Zs[(size_t)i * D + d] - origin[d];   // F was accumulated in the same shifted coordinates
-            const double* fu = &Fuf[(size_t)i * 128];
-            const double* fz = &Fuu[(size_t)i * 128];
+            const double* fu = &Fuf[(size_t)i * W];
+            const double* fz = &Fuu[(size_t)i * W];
             acc += z * z * fu[D] - 2.0 * z * fu[d] + fu[D + 1 + d];
             acc += z * z * fz[D] - 2.0 * z * fz[d] + fz[D + 1 + d];
             dZ[(size_t)i * D + d] = (2.0 / ls[d]) * (z * fu[D] - fu[d]) + (4.0 / ls[d]) * (z * fz[D] - fz[d]);
         }
         dls[d] = -(2.0 / ls[d]) * acc;
     }
-    dls_out = dls;
     return TSVGP_OK;
+}
+
+// F_uf of the last gradient pass, all-reduced over the ranks, to the host
+static int read_fuf(tsvgp_ctx* c, std::vector<double>& Fuf) {
+    const size_t cnt = (size_t)c->Mp * c->waug;
+    OK(all_reduce(c, c->facc[0], cnt));
+    Fuf.resize(cnt);
+    CU(cudaMemcpyAsync(Fuf.data(), c->facc[0], sizeof(double) * cnt, cudaMemcpyDeviceToHost, c->s_main));
+    CU(cudaStreamSynchronize(c->s_main));
+    return TSVGP_OK;
+}
+
+// ELBO terms and gradients of ONE latent with independent likelihood terms: its own pass, then its epilogue
+static int elbo_grad_one(tsvgp_ctx* c, int lat, double scale, const std::vector<double>& origin, double* elbo, double* d_variance,
+                         std::vector<double>& dls, std::vector<double>& dZ, double* d_lik) {
+    c->grad_scale = scale;
+    OK(data_pass(c, MODE_GRAD, PASS_WHOLE, lat));
+    select_latent(c, lat);
+    std::vector<double> Fuf, Fuu;
+    OK(read_fuf(c, Fuf));
+    OK(grad_epilogue(c, lat, scale, elbo, d_variance, d_lik, Fuu));
+    return f_to_grads(c, origin, Fuf, Fuu, dls, dZ);
+}
+
+// A coupled likelihood (Softmax): ONE pass over all latents (the point kernel needs every latent's moments of the same points),
+// then the epilogue per latent.  Kuf is shared, so F_uf holds the sum over the latents already and the F_uu add up.
+static int elbo_grad_coupled(tsvgp_ctx* c, double scale, const std::vector<double>& origin, double* elbo, double* d_variance,
+                             std::vector<double>& dls, std::vector<double>& dZ, double* d_lik) {
+    c->grad_scale = scale;
+    OK(data_pass(c, MODE_GRAD));
+    std::vector<double> Fuf, Fuu, Fuu_sum;
+    OK(read_fuf(c, Fuf));
+    double e_sum = 0.0, dv_sum = 0.0, dl_sum = 0.0;
+    for (int l = 0; l < c->L; ++l) {
+        double e = 0.0, dv = 0.0, dl = 0.0;
+        OK(grad_epilogue(c, l, scale, &e, &dv, &dl, Fuu));
+        if (l == 0) Fuu_sum = Fuu;
+        else for (size_t i = 0; i < Fuu.size(); ++i) Fuu_sum[i] += Fuu[i];
+        e_sum += e; dv_sum += dv; dl_sum += dl;
+    }
+    *elbo = e_sum; *d_variance = dv_sum; *d_lik = dl_sum;
+    return f_to_grads(c, origin, Fuf, Fuu_sum, dls, dZ);
 }
 
 int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance, double* d_lengthscales, double* d_Z, double* d_lik) {
     if (!c || !elbo || !d_variance || !d_lengthscales || !d_Z || !d_lik) return TSVGP_ERR_INVALID;
     OK(require_model(c, true));
-    if (2 * c->D + 1 > 128) FAIL(TSVGP_ERR_INVALID, "elbo_grad supports D <= 63 (D = %d)", c->D);
     if (c->white) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not available for the whitened sibling model");
-    if (c->lik.kind == LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not available for the Softmax likelihood");
     if (c->lik.kind == LIK_HETEROSKEDASTIC) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for the heteroskedastic likelihood");
     if (c->sep) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for separate kernels per latent");
     CU(cudaSetDevice(c->dev));
@@ -2347,14 +2426,21 @@ int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance
     // q(u_l); tsvgp.py:65-95), and so is every gradient
     double e_sum = 0.0, dv_sum = 0.0, dl_sum = 0.0;
     std::vector<double> dls_sum(D, 0.0), dZ_sum((size_t)M * D, 0.0), dls, dZ;
-    for (int l = 0; l < c->L; ++l) {
-        double e = 0.0, dv = 0.0, dl = 0.0;
-        const int rc = elbo_grad_one(c, l, scale, origin, &e, &dv, dls, dZ, &dl);
+    if (coupled(c)) {
+        const int rc = elbo_grad_coupled(c, scale, origin, &e_sum, &dv_sum, dls_sum, dZ_sum, &dl_sum);
         select_latent(c, 0);
         if (rc != TSVGP_OK) return rc;
-        e_sum += e; dv_sum += dv; dl_sum += dl;
-        for (int d = 0; d < D; ++d) dls_sum[d] += dls[d];
-        for (size_t i = 0; i < dZ.size(); ++i) dZ_sum[i] += dZ[i];
+        ++c->mc_draw;   // one Monte-Carlo draw per call, as tsvgp_elbo: the ELBO returned here at draw k is elbo's at draw k
+    } else {
+        for (int l = 0; l < c->L; ++l) {
+            double e = 0.0, dv = 0.0, dl = 0.0;
+            const int rc = elbo_grad_one(c, l, scale, origin, &e, &dv, dls, dZ, &dl);
+            select_latent(c, 0);
+            if (rc != TSVGP_OK) return rc;
+            e_sum += e; dv_sum += dv; dl_sum += dl;
+            for (int d = 0; d < D; ++d) dls_sum[d] += dls[d];
+            for (size_t i = 0; i < dZ.size(); ++i) dZ_sum[i] += dZ[i];
+        }
     }
     *elbo = e_sum; *d_variance = dv_sum; *d_lik = dl_sum;
     if (c->ls_host.size() == 1) {

@@ -355,7 +355,8 @@ class t_SVGP:
         `elbo` / `training_loss_closure`; tsvgp.py:72-95, tests/models/test_tsvgp.py:168-188).
         -> (elbo, {"variance", "lengthscales" (shape of kernel.lengthscales), "Z" [M, D], "likelihood"}), gradients w.r.t. the
         constrained parameter values (chain your own positive transform); "likelihood" is d/d variance (Gaussian),
-        d/d scale (StudentT) or None (Bernoulli)."""
+        d/d scale (StudentT) or None (Bernoulli, Softmax).  Softmax: one Monte-Carlo draw per call, the one `elbo` would use
+        next (or the draws fixed by `set_mc_epsilon`)."""
         if _separate(self.kernel):
             raise NotImplementedError("elbo_and_grad with SeparateIndependent kernels")
         if type(self.likelihood).__name__ == "HeteroskedasticTFPConditional":
@@ -372,7 +373,7 @@ class t_SVGP:
                                               dls.ctypes.data, dZ.ctypes.data, C.byref(dl)))
         lik = _likelihood_spec(self.likelihood)[0]
         return e.value, {"variance": dv.value, "lengthscales": dls.reshape(np.shape(_value(kernel.lengthscales)) or ()),
-                         "Z": dZ, "likelihood": None if lik == _lib.LIK_BERNOULLI_PROBIT else dl.value}
+                         "Z": dZ, "likelihood": None if lik in (_lib.LIK_BERNOULLI_PROBIT, _lib.LIK_SOFTMAX) else dl.value}
 
     def maximum_log_likelihood_objective(self, data=None):  # tsvgp.py:72-77
         return self.elbo(data)
