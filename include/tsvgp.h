@@ -156,7 +156,10 @@ TSVGP_API int tsvgp_commit_staged(tsvgp_ctx* ctx);
 /* ---- the hot path ----------------------------------------------------------------------------------------------------- */
 /* t_SVGP.natgrad_step (tsvgp.py:234-304) on the resident data and sites.  scale = num_data / minibatch_size or 1
  * (tsvgp.py:286-291) with minibatch_size summed over ranks.  elbo_before (may be NULL) receives the ELBO of the
- * pre-update state on the same minibatch (a by-product of the same pass).                                              */
+ * pre-update state on the same minibatch (a by-product of the same pass).
+ * TSVGP_ERR_NONPOSITIVE_VARIANCE (sites unchanged): some v_n <= 0 or non-finite.  The Gaussian likelihood's update does not
+ * read v_n, so its step forms no per-point variance: it reports the error when a point of X or its predictive mean is not finite
+ * and, with elbo_before, when the sum of the variances taken from the statistics is not finite and positive.       */
 TSVGP_API int tsvgp_natgrad_step(tsvgp_ctx* ctx, double lr, double jitter, double scale, double* elbo_before);
 /* base_SVGP.elbo (tsvgp.py:79-95) on the resident data                                                                 */
 TSVGP_API int tsvgp_elbo(tsvgp_ctx* ctx, double scale, double* out);
@@ -213,8 +216,8 @@ TSVGP_API int tsvgp_get_timings(tsvgp_ctx* ctx, double* out, int n);
 TSVGP_API int tsvgp_sync(tsvgp_ctx* ctx);
 /* With option "profile" = 1 the streaming pass runs on one stream and brackets every kernel with CUDA events.  After a
  * natgrad_step, out[2*k] = summed duration (ms) and out[2*k+1] = launch count of kernel class k:
- *  0 Kuf slab, 1 variance product (triangular DMMA GEMM + column norms), 2 point statistics, 3 whitening GEMM,
- *  4 weighted SYRK (DMMA), 5 Kuf g                                                                                      */
+ *  0 Kuf slab, 1 variance product (triangular DMMA GEMM + column norms; not run by a Gaussian step: (0, 0)), 2 point
+ *  statistics, 3 whitening GEMM, 4 weighted SYRK (DMMA), 5 Kuf g                                                        */
 TSVGP_API int tsvgp_get_kernel_profile(tsvgp_ctx* ctx, double* out, int n);
 /* CUDA-event stopwatch on the context's stream (every call's work, host<->device copies included, is ordered on it)   */
 TSVGP_API int tsvgp_timer_start(tsvgp_ctx* ctx);

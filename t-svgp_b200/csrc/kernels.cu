@@ -267,7 +267,9 @@ __global__ void __launch_bounds__(256) point_stats_kernel(LikSpec lk, PointArgs 
         }
         const double mean = mu + (a.mean_off ? a.mean_off[c] : 0.0);
         const double var = a.kdiag - q;
-        if (valid && !(var > 0.0)) atomicOr(a.flags, 1);
+        // with x2 (the Gaussian natgrad_step, which forms no v_n): non-finite data raises the flag that keeps the step from
+        // committing (the covariance clamps a NaN distance to a finite k, so a NaN in X shows in x2, not in the mean)
+        if (valid && (!(var > 0.0) || (a.x2 && !(isfinite(mean) && isfinite(a.x2[c]))))) atomicOr(a.flags, 1);
         if (valid && a.mean_out) { a.mean_out[c] = mean; a.var_out[c] = var; }
         double gm = 0.0, gv = 0.0;
         if (valid && a.y) {
@@ -1746,6 +1748,17 @@ __global__ void __launch_bounds__(256) stats_tail_kernel(const double* ve_blocks
 }
 int stats_tail_launch(const double* ve_blocks, long nblocks, const int* flags, const double* aux, double* out, cudaStream_t s) {
     stats_tail_kernel<<<1, 256, 0, s>>>(ve_blocks, nblocks, flags, aux, out);
+    return count_launch();
+}
+// q = tr[0] * inv_c = sum_n |T^T k_n|^2 ;  out[0] += half_inv_s2 * q ;  out[1] = 1 unless sum_n v_n = sum_kdiag - q is finite and > 0
+__global__ void variance_term_kernel(const double* tr, double inv_c, double sum_kdiag, double half_inv_s2, double* out) {
+    const double q = tr[0] * inv_c;
+    const double v = sum_kdiag - q;
+    out[0] += half_inv_s2 * q;
+    if (!isfinite(v) || (sum_kdiag > 0.0 && !(v > 0.0))) out[1] = 1.0;   // (a rank without rows has sum_kdiag = q = 0)
+}
+int variance_term_launch(const double* tr, double inv_c, double sum_kdiag, double half_inv_s2, double* out, cudaStream_t s) {
+    variance_term_kernel<<<1, 1, 0, s>>>(tr, inv_c, sum_kdiag, half_inv_s2, out);
     return count_launch();
 }
 

@@ -33,7 +33,7 @@ struct GHTable { double z[MAX_GH]; double w[MAX_GH]; };   // nodes sqrt(2) x_k a
 
 struct PointArgs {
     const double* mu_part; int n_mu_part; long ldmu;   // partial means   [n_mu_part][ldmu]
-    const double* q_part; int n_q_part; long ldq;      // partial |T^T k|^2 [n_q_part][ldq]   (subtracted from k(x,x))
+    const double* q_part; int n_q_part; long ldq;      // partial |T^T k|^2 [n_q_part][ldq]   (subtracted from k(x,x); none: var = k(x,x))
     const double* q2_part = nullptr;                   // optional second set, same shape, ADDED (whitened sibling: + |LR^-1 k|^2)
     const double* y;            // [ncols] (chunk-local pointer) or null (predict)
     const double* mean_off;     // [ncols] mean_function(X) or null
@@ -45,7 +45,8 @@ struct PointArgs {
     double* ve_blocks;          // out: per-block sum of ve   [gridDim.x]
     double* aux_blocks = nullptr;   // out (M-step): per-block [sum h, sum d ve / d likelihood parameter]   [2 * gridDim.x]
     int clip = 1;               // clip d ve / d var at -1e-8 (natgrad_step, tsvgp.py:262-263); the ELBO gradient does not
-    int* flags;                 // flags[0] |= 1 if any var <= 0
+    int* flags;                 // flags[0] |= 1 if any var <= 0, or (x2 given) any mean or x2 is not finite
+    const double* x2 = nullptr; // [ncols] squared norms of the scaled points (chunk-local), or null
 };
 // Softmax likelihood over L latents (gpflow.likelihoods.Softmax = MonteCarloLikelihood, S = num_monte_carlo_points): per point
 //   ve = mean_s log softmax(f_s)[y],  f_s = mu + sqrt(var) * eps_s ;  g_l = d ve / d mu_l ;  h_l = min(d ve / d var_l, -1e-8)
@@ -158,6 +159,9 @@ int axpby_guarded_launch(double* P, const double* X, long ld, int M, double a, d
 int vadd_inplace_launch(double* dst, const double* src, long n, cudaStream_t s);
 int sum_rows_into_launch(const double* src, int rows, int n, double* dst, cudaStream_t s);   // dst[j] += sum_r src[r][j]  (fixed order)
 int stats_tail_launch(const double* ve_blocks, long nblocks, const int* flags, const double* aux, double* out, cudaStream_t s);
+// Gaussian natgrad_step, whose pass took var = k(x,x): with tr[0] = tr(P^T B P) and q = tr[0] * inv_c = sum_n |T^T k_n|^2,
+// out[0] (sum ve) += half_inv_s2 * q, and out[1] (the variance flag) = 1 unless sum_n v_n = sum_kdiag - q is finite and positive
+int variance_term_launch(const double* tr, double inv_c, double sum_kdiag, double half_inv_s2, double* out, cudaStream_t s);
 // M-step gradient helpers (see tsvgp_elbo_grad)
 // E = scale (alpha g^T - 2 U diag(h)) .* Kp, written over U (E = null) or added to E (a coupled likelihood's latents share one E)
 int egrad_uf_launch(double* U, const double* Kp, long ld, int Mp, int ncols, const double* alpha, const double* g, const double* h,

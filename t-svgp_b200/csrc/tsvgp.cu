@@ -7,6 +7,8 @@
 //   stream  : per slab of `chunk` points, on two alternating streams:
 //               Kuf slab + partial means  ->  |T^T k_n|^2 by a triangular DMMA product with a column-norm epilogue
 //               -> per-point likelihood statistics (g_n, h_n, ve_n)  ->  B += Kuf diag(h) Kfu (DMMA SYRK), b += Kuf g
+//             (Gaussian likelihood: g_n, h_n do not read v_n, so there is no |T^T k_n|^2; the ELBO takes sum_n |T^T k_n|^2 =
+//              tr(T^T B T) / h from the statistics instead, see variance_term_from_stats)
 //   reduce  : one all-reduce (NCCL) of [B | b | sum ve | flag] when the minibatch is sharded over ranks
 //   update  : G2 = K9^-1 B K9^-1, G1 = K9^-1 b, lambda_1, P = (1-lr) L2 L2^T - 2 lr s G2 + jitter I, L2 = -chol(P)
 // There is no CPU path: every entry point that computes needs a CUDA device.
@@ -64,7 +66,7 @@ enum { MODE_STATS = 0, MODE_ELBO = 1, MODE_PREDICT = 2, MODE_GRAD = 3 };   // MO
 enum { INFO_W = 0, INFO_K9 = 1, INFO_P = 2, INFO_S = 3, N_INFO = 4 };
 enum { EV_T0 = 0, EV_PREP, EV_STREAM, EV_REDUCE, EV_DENSE, N_EV };
 // device scalars
-enum { SC_LOGDIAG_W = 0, SC_M_ALPHA, SC_TR_QK, SC_PK0, SC_PK1, SC_PI0, SC_PI1, SC_G_K, SC_TR_QB, SC_A_B, N_SCAL = 12 };
+enum { SC_LOGDIAG_W = 0, SC_M_ALPHA, SC_TR_QK, SC_PK0, SC_PK1, SC_PI0, SC_PI1, SC_G_K, SC_TR_QB, SC_A_B, SC_TR_PBP, N_SCAL = 12 };
 enum { ROUTE_AUTO = 0, ROUTE_FUSED = 1, ROUTE_WHITENED = 2, ROUTE_EXACT = 3 };
 
 }  // namespace
@@ -919,6 +921,11 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         return TSVGP_OK;
     };
     const bool const_h_pass = c->lik.kind == LIK_GAUSSIAN && !grad;
+    // Gaussian natgrad_step: g_n and h_n do not read v_n, so neither do B, b and the new sites.  The variance product is skipped
+    // and the ELBO's variance term taken from B afterwards (variance_term_from_stats); the point kernel then sees var = k(x,x).
+    const bool skip_var = mode == MODE_STATS && const_h_pass && !c->white;
+    // ... and with one kernel every latent's B is the same matrix K diag(h) K^T: one SYRK (latent l_lo's), copied after the pass
+    const bool one_syrk = stats && const_h_pass && !sep && l_hi - l_lo > 1;
     if (phase == PASS_EARLY) {
         const bool ok = mode == MODE_STATS && const_h_pass && c->route == ROUTE_FUSED && !c->white && !prof && c->ksplit <= 1 &&
                         nchunks >= 2 * nstr && !multi && !c->sep;   // (separate kernels build every slab in the pass itself)
@@ -964,7 +971,9 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                               c->D, c->alpha, c->slab[b], nc, c->mu_part[b], nc, 0, s, nullptr));
             else if (early || multi)   // the slab exists already: the same per-64-row partial means from a transposed mat-vec over it
                 LA(gemv_t_part_launch(c->slab[b], nc, Mp, ncols, c->alpha, c->mu_part[b], nc, s));
-            if (!c->white) {   // (b) |T^T k_n|^2 : upper-triangular T^T times the slab, reduced to column norms in the epilogue
+            if (skip_var) {
+                // (b) not formed: the pass needs no v_n (see skip_var)
+            } else if (!c->white) {   // (b) |T^T k_n|^2 : upper-triangular T^T times the slab, reduced to column norms in the epilogue
                 GemmP p;
                 p.A = c->T; p.lda = Mp; p.a_kc = 0; p.a_tri = 2;
                 p.B = c->slab[b]; p.ldb = nc; p.b_kc = 0;
@@ -995,7 +1004,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             if (!joint) {   // (c) marginals -> likelihood expectations and gradients, latent by latent (independent likelihood terms)
                 PointArgs a;
                 a.mu_part = c->mu_part[b]; a.n_mu_part = Mp / 64; a.ldmu = nc;
-                a.q_part = c->white ? c->q2_part[b] : c->q_part[b]; a.n_q_part = Mp / 128; a.ldq = nc;   // subtracted: |LA^-1 k|^2 (white) / |T^T k|^2
+                a.q_part = c->white ? c->q2_part[b] : c->q_part[b]; a.n_q_part = skip_var ? 0 : Mp / 128; a.ldq = nc;   // subtracted: |LA^-1 k|^2 (white) / |T^T k|^2
                 a.q2_part = c->white ? c->q_part[b] : nullptr;                                           // added:      |LR_l^-1 k|^2 (white)
                 a.y = y ? y + l * y_stride + n0 : nullptr;
                 a.mean_off = mean_off ? mean_off + n0 : nullptr;
@@ -1007,6 +1016,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                 a.mean_out = mean_out ? mean_out + l * out_stride + n0 : nullptr; a.var_out = var_out ? var_out + l * out_stride + n0 : nullptr;
                 a.ve_blocks = c->ve_blocks + ci * vstride;
                 a.flags = c->flags;
+                a.x2 = skip_var ? x2 + l * x2_lat + n0 : nullptr;   // no v_n to catch non-finite data: check the points themselves
                 LA(point_stats_launch(c->lik, a, c->gh, s));
             }
             mark(s);
@@ -1061,7 +1071,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                 select_latent(c, l);
                 if (sep) OK(stat_slab_of(stat_slab));   // latent l's slab and C9_l
                 bool fused_b = false;
-                if (!early) OK(syrk(b, stat_slab, ncols, const_h_pass, true, fused_b));
+                if (!early && !(one_syrk && l > l_lo)) OK(syrk(b, stat_slab, ncols, const_h_pass, true, fused_b));
                 mark(s);
                 // (e) b += K g as its own kernel when the SYRK ran split-K or ahead of the posterior
                 if (!fused_b) LA(gemv_n_launch(stat_slab, nc, Mp, ncols, c->gbuf[b], 1.0, 1.0, c->stats[b] + (size_t)Mp * Mp, s));
@@ -1108,6 +1118,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             for (int k = 0; k < 6; ++k) {
                 float ms = 0;
                 cudaEventElapsedTime(&ms, c->pev[e + k], c->pev[e + k + 1]);
+                if (k == 1 && skip_var) continue;
                 if (k == 3 && c->route != ROUTE_WHITENED && c->route != ROUTE_EXACT) continue;
                 c->kprof[2 * k] += ms;
                 c->kprof[2 * k + 1] += 1.0;
@@ -1135,6 +1146,9 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             for (int s = 0; s < nstr; ++s) LA(vadd_inplace_launch(c->stats[0], c->stats2[s], (long)(mm + Mp), sm));
         }
         (void)cnt2;
+        for (int l = l_lo + 1; l < l_hi && one_syrk; ++l)
+            CU(cudaMemcpyAsync(c->stats_all[0] + l * (mm + Mp + 4), c->stats_all[0] + l_lo * (mm + Mp + 4), sizeof(double) * mm,
+                               cudaMemcpyDeviceToDevice, sm));
     }
     for (int l = l_lo; l < l_hi; ++l) {
         select_latent(c, l);
@@ -1477,6 +1491,7 @@ int exchange_k9(tsvgp_ctx* c, double jitter) {
     CU(cudaStreamWaitEvent(s, c->ev_mid, 0));
     OK(nccl_chk(c, api.GroupStart(), "ncclGroupStart"));
     int r = 0;
+    r |= api.Broadcast(c->C9, c->C9, mm, NCCL_FLOAT64, root, c->comm, s);   // (the ELBO of a Gaussian step on another route)
     r |= api.Broadcast(c->C9inv, c->C9inv, mm, NCCL_FLOAT64, root, c->comm, s);
     r |= api.Broadcast(c->K9inv, c->K9inv, mm, NCCL_FLOAT64, root, c->comm, s);
     r |= api.Broadcast(c->scal2, c->scal2, N_SCAL, NCCL_FLOAT64, root, c->comm, s);
@@ -1584,6 +1599,53 @@ int dense_update_one(tsvgp_ctx* c, double lr, double jitter, double scale, bool 
     // commit (skipped on the device if any variance was non-positive or a factorisation failed)
     LA(update_lambda1_launch(c->lam1, c->v2, c->v3, c->M, lr, scale, bad, c->info, s));
     LA(finalize_sites_launch(c->P, c->L2, ld, c->M, n, bad, c->info, s));
+    return TSVGP_OK;
+}
+
+// Gaussian natgrad_step: the pass took v_n = k(x,x) (stream_pass, skip_var), so its sum of ve lacks + 1/(2 s2) sum_n |T^T k_n|^2.
+// Every route's accumulator is B = c R^-1 (sum_n k_n k_n^T) R^-T, c the SYRK's constant weight, R = I (fused), C9 (whitened) or
+// K9 = C9 C9^T (exact); with P = R^T T
+//   sum_n |T^T k_n|^2 = tr(T^T (sum_n k_n k_n^T) T) = tr(P^T B P) / c          (one M^3 product per latent instead of M^2 per point)
+// The term is added to each latent's sum of ve, and the variance flag raised unless sum_n v_n is finite and positive.  Runs on this
+// rank's rows before the reduction, which then sums the corrected ve and the flags as before.
+int variance_term_from_stats(tsvgp_ctx* c) {
+    cudaStream_t s = c->s_main;
+    const int n = c->Mp;
+    const long ld = n;
+    const size_t mm = (size_t)n * n;
+    const double cst = fmin(-0.5 / c->lik.p0, -1e-8);   // the weight of stream_pass's constant-weight SYRK
+    for (int l = 0; l < c->L; ++l) {
+        select_latent(c, l);
+        double* B = c->stats[0];
+        LA(mirror_lower_launch(B, ld, n, s));   // (the pass accumulated lower tiles only)
+        const double* P = c->T;
+        if (c->route != ROUTE_FUSED) {   // X2 = C9^T T
+            GemmP p;
+            p.A = c->C9; p.lda = ld; p.a_kc = 0; p.a_tri = 2;
+            p.B = c->T; p.ldb = ld; p.b_kc = 0; p.b_tri = 2;
+            p.C = c->X2; p.ldc = ld; p.m = p.n = p.k = n;
+            LA(mm_gemm(c, p, s));
+            P = c->X2;
+            if (c->route == ROUTE_EXACT) {   // X1 = C9 X2 = K9 T
+                GemmP q;
+                q.A = c->C9; q.lda = ld; q.a_kc = 1; q.a_tri = 1;
+                q.B = c->X2; q.ldb = ld; q.b_kc = 0;
+                q.C = c->X1; q.ldc = ld; q.m = q.n = q.k = n;
+                LA(mm_gemm(c, q, s));
+                P = c->X1;
+            }
+        }
+        {   // G2 = B P  (G2 is formed again by the update)
+            GemmP p;
+            p.A = B; p.lda = ld; p.a_kc = 1;
+            p.B = P; p.ldb = ld; p.b_kc = 0; p.b_tri = P == c->T ? 2 : 0;
+            p.C = c->G2; p.ldc = ld; p.m = p.n = p.k = n;
+            LA(mm_gemm(c, p, s));
+        }
+        LA(matdot_launch(P, c->G2, ld, n, c->scal + SC_TR_PBP, c->red, s));
+        LA(variance_term_launch(c->scal + SC_TR_PBP, 1.0 / cst, (double)c->N * c->kern_var, 0.5 / c->lik.p0, B + mm + n, s));
+    }
+    select_latent(c, 0);
     return TSVGP_OK;
 }
 
@@ -2177,6 +2239,7 @@ int tsvgp_natgrad_step(tsvgp_ctx* c, double lr, double jitter, double scale, dou
                 OK(data_pass(c, MODE_STATS));
         }
     }
+    if (elbo_before && c->lik.kind == LIK_GAUSSIAN && !c->white) OK(variance_term_from_stats(c));
     CU(cudaEventRecord(c->ev[EV_STREAM], s));
     struct NvtxRange { NvtxRange(const char* n) { nvtxRangePushA(n); } ~NvtxRange() { nvtxRangePop(); } } nvtx_dense("tsvgp_dense");
     if (sharded_update_active(c)) {

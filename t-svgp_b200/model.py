@@ -334,7 +334,10 @@ class t_SVGP:
 
     # ---- the path ---------------------------------------------------------------------------------------------------
     def natgrad_step(self, data=None, lr=0.1, jitter=1e-9, *, global_minibatch_size=None, return_elbo=False):
-        """tsvgp.py:234-304.  Mutates lambda_1 / lambda_2_sqrt (on the device).  `data=None` reuses the resident data."""
+        """tsvgp.py:234-304.  Mutates lambda_1 / lambda_2_sqrt (on the device).  `data=None` reuses the resident data.
+        Raises NonPositiveVarianceError, sites unchanged, when a predictive variance of the minibatch is not positive.  The
+        Gaussian update does not read the variances and forms none per point: it raises when a point of X or its predictive mean is
+        not finite and, with return_elbo, when the sum of the variances (from the step's statistics) is not positive."""
         self._sync_objects()
         n = self._ingest(data)
         out = C.c_double()
