@@ -1,0 +1,351 @@
+// Exact fixed-point Gram product on the INT8 tensor cores (tcgen05.mma kind::i8, SASS UTCIMMA): see int8_gram.cuh and DESIGN §2.
+//   i8_residue_kernel : K (FP64 slab) -> A = rint(K 2^52 / v) -> 16 int8 residue planes, written as the shared-memory image the
+//                       MMA descriptors describe (128-row x 128-byte k-blocks of K-major core matrices, 128-byte swizzle)
+//   i8_gram_kernel    : persistent, warp-specialised: one producer thread streams k-blocks into a 4-stage mbarrier ring with
+//                       cp.async.bulk, one thread issues 128 x 256 x 32 MMAs into a double-buffered TMEM accumulator, four
+//                       epilogue warps reduce the int32 tiles modulo p_i into residue tiles.  Modulus-major schedule: the lower
+//                       128 x 256 blocks of modulus i, then i + 1 (one modulus's planes stay in L2 while its blocks run)
+//   i8_crt_kernel     : Garner's mixed-radix digits + Horner in 128-bit integers -> the exact integer -> one rounding -> C += alpha ...
+#include "int8_gram.cuh"
+#include "common.cuh"
+
+namespace tsvgp {
+
+namespace i8 {
+
+constexpr int KB_BYTES = 16384;                 // one 128-row x 128-byte k-block
+constexpr int BN = 256;                         // output block: two 128-tiles of one tile row
+constexpr int STAGES = 4;
+constexpr int STAGE_BYTES = KB_BYTES + BN * 128;
+constexpr int GEMM_SMEM = STAGES * STAGE_BYTES + 1024;
+constexpr int GEMM_THREADS = 192;               // warp 0 producer, warp 1 MMA issuer, warps 2..5 epilogue
+
+__host__ __device__ constexpr int modulus(int i) {
+    constexpr int p[I8_NMOD] = {256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193};
+    return p[i];
+}
+__host__ __device__ constexpr int inv_mod(int a, int m) {   // a^-1 mod m (a, m coprime)
+    int t = 0, nt = 1, r = m, nr = a % m;
+    while (nr) { const int q = r / nr, t2 = t - q * nt, r2 = r - q * nr; t = nt; nt = t2; r = nr; nr = r2; }
+    return t < 0 ? t + m : t;
+}
+__host__ __device__ constexpr unsigned __int128 prod_moduli() {
+    unsigned __int128 P = 1;
+    for (int i = 0; i < I8_NMOD; ++i) P *= (unsigned)modulus(i);
+    return P;
+}
+
+// byte offset of (row r, byte k) inside a k-block: 8-row x 128-byte swizzle atoms, 16-byte chunk c of row r at c ^ (r & 7)
+__device__ __forceinline__ uint32_t kblock_off(int r, int k) {
+    return (r >> 3) * 1024 + (r & 7) * 128 + ((((k >> 4) ^ (r & 7)) << 4) | (k & 15));
+}
+
+// lower blocks of one modulus: tile row i holds ceil((i + 1) / 2) blocks of two tiles (the last may reach one tile past the diagonal)
+__host__ __device__ inline int blocks_per_modulus(int nt) {
+    int n = 0;
+    for (int i = 0; i < nt; ++i) n += (i + 2) / 2;
+    return n;
+}
+__device__ __forceinline__ void block_coords(int blk, int& i, int& jp) {
+    i = 0;
+    while (blk >= (i + 2) / 2) { blk -= (i + 2) / 2; ++i; }
+    jp = blk;
+}
+
+// ---- tcgen05 -------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t saddr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// shared-memory matrix descriptor: start >> 4, stride between 8-row groups 1024 B, version 1 (bit 46), 128-byte swizzle (mode 2)
+__device__ __forceinline__ uint64_t sdesc(uint32_t a) {
+    return (uint64_t)((a >> 4) & 0x3FFF) | (uint64_t)(1024 >> 4) << 32 | 1ull << 46 | 2ull << 61;
+}
+// instruction descriptor: D s32, A and B signed 8-bit, both K-major, M = 128, N = BN
+constexpr uint32_t IDESC = 2u << 4 | 1u << 7 | 1u << 10 | (uint32_t)(BN >> 3) << 17 | (128u >> 4) << 24;
+__device__ __forceinline__ void mma_i8(uint32_t d, uint64_t a, uint64_t b, uint32_t acc) {
+    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(d), "l"(a), "l"(b),
+                 "r"(IDESC), "r"(acc));
+}
+__device__ __forceinline__ void mma_commit(uint64_t* bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(saddr(bar)) : "memory");
+}
+__device__ __forceinline__ void fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,"
+                 "%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n"
+                 "tcgen05.wait::ld.sync.aligned;\n"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
+                   "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
+                   "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
+                   "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+                 : "r"(taddr)
+                 : "memory");
+}
+
+// ---- residues --------------------------------------------------------------------------------------------------------------
+template <int M>
+__device__ __forceinline__ uint32_t residue4(const double* a) {   // symmetric residues of 4 grid integers mod p_M, packed
+    constexpr double p = modulus(M), ip = 1.0 / modulus(M);
+    constexpr double hi = (modulus(M) - 1) / 2, lo = -(modulus(M) / 2);   // [-128, 127] for 256, [-(p-1)/2, (p-1)/2] otherwise
+    uint32_t w = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const double q = rint(a[j] * ip);
+        double r = fma(-q, p, a[j]);   // exact: |A - q p| is a small integer
+        if (r > hi) r -= p;
+        else if (r < lo) r += p;
+        w |= (uint32_t)((int)r & 0xFF) << (8 * j);
+    }
+    return w;
+}
+template <int M>
+__device__ __forceinline__ void store_residues(const double* a, int8_t* dst, size_t pstride) {
+    if constexpr (M < I8_NMOD) {
+        uint4 w;
+        w.x = residue4<M>(a); w.y = residue4<M>(a + 4); w.z = residue4<M>(a + 8); w.w = residue4<M>(a + 12);
+        *reinterpret_cast<uint4*>(dst + M * pstride) = w;
+        store_residues<M + 1>(a, dst, pstride);
+    }
+}
+
+// block (kb, rb): one 128-row x 128-column k-block of every plane; a thread takes 16 consecutive columns of a row (one chunk)
+__global__ void __launch_bounds__(256) i8_residue_kernel(const double* __restrict__ K, long ldk, double scale, int8_t* __restrict__ planes,
+                                                         size_t pstride, int nrb) {
+    const int kb = blockIdx.x, rb = blockIdx.y;
+#pragma unroll 1
+    for (int it = 0; it < 4; ++it) {
+        const int c = threadIdx.x + 256 * it, row = c >> 3, kc = c & 7;
+        const double2* src = reinterpret_cast<const double2*>(K + (size_t)(rb * 128 + row) * ldk + kb * 128 + kc * 16);
+        double a[16];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const double2 v = __ldg(src + j);
+            a[2 * j] = v.x; a[2 * j + 1] = v.y;
+        }
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+            const double t = rint(a[j] * scale);
+            a[j] = fabs(t) < 9007199254740992.0 ? t : 0.0;   // off the grid (non-finite): 0; the point kernel flags such a step
+        }
+        store_residues<0>(a, planes + (size_t)(kb * nrb + rb) * KB_BYTES + kblock_off(row, kc * 16), pstride);
+    }
+}
+
+// ---- products --------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* __restrict__ planes, size_t pstride, int nrb, int nkb,
+                                                                  int nblk, uint8_t* __restrict__ tiles, size_t tstride) {
+    extern __shared__ uint8_t smem_raw[];
+    uint8_t* smem = smem_raw + ((1024 - (saddr(smem_raw) & 1023)) & 1023);   // swizzle atoms on 1 KB boundaries
+    __shared__ uint64_t full[STAGES], empty[STAGES], tfull[2], tempty[2];
+    __shared__ uint32_t tslot;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int units = I8_NMOD * nblk;
+    if (warp == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(saddr(&tslot)));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 4); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    fence_before();
+    __syncthreads();
+    fence_after();
+    const uint32_t tmem = tslot;
+
+    if (warp == 0) {
+        if (lane == 0) {   // producer
+            int k = 0;
+            for (int u = blockIdx.x; u < units; u += gridDim.x) {
+                const int m = u / nblk;
+                int i, jp;
+                block_coords(u - m * nblk, i, jp);
+                const int8_t* pa = planes + m * pstride + (size_t)i * KB_BYTES;
+                const int8_t* pb = planes + m * pstride + (size_t)(2 * jp) * KB_BYTES;
+                for (int kb = 0; kb < nkb; ++kb, ++k) {
+                    const int s = k % STAGES;
+                    if (k >= STAGES) mbar_wait(&empty[s], ((k / STAGES) - 1) & 1);
+                    uint8_t* st = smem + s * STAGE_BYTES;
+                    mbar_expect_tx(&full[s], STAGE_BYTES);
+                    tma_bulk_g2s(st, pa + (size_t)kb * nrb * KB_BYTES, KB_BYTES, &full[s]);
+                    tma_bulk_g2s(st + KB_BYTES, pb + (size_t)kb * nrb * KB_BYTES, BN * 128, &full[s]);
+                }
+            }
+        }
+    } else if (warp == 1) {
+        if (lane == 0) {   // MMA issuer
+            int k = 0, t = 0;
+            for (int u = blockIdx.x; u < units; u += gridDim.x, ++t) {
+                const int buf = t & 1;
+                if (t >= 2) mbar_wait(&tempty[buf], ((t >> 1) - 1) & 1);
+                fence_after();
+                const uint32_t d = tmem + buf * BN;
+                for (int kb = 0; kb < nkb; ++kb, ++k) {
+                    const int s = k % STAGES;
+                    mbar_wait(&full[s], (k / STAGES) & 1);
+                    fence_after();
+                    const uint32_t a = saddr(smem + s * STAGE_BYTES), b = a + KB_BYTES;
+#pragma unroll
+                    for (int kk = 0; kk < 4; ++kk) mma_i8(d, sdesc(a + 32 * kk), sdesc(b + 32 * kk), (kb | kk) != 0);
+                    mma_commit(&empty[s]);
+                }
+                mma_commit(&tfull[buf]);
+            }
+        }
+    } else {   // epilogue: TMEM lanes 32 (warp % 4) .. + 31 are rows of the block
+        const int row = (warp & 3) * 32 + lane;
+        const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+        int t = 0;
+        for (int u = blockIdx.x; u < units; u += gridDim.x, ++t) {
+            const int m = u / nblk;
+            int i, jp;
+            block_coords(u - m * nblk, i, jp);
+            const int buf = t & 1;
+            mbar_wait(&tfull[buf], (t >> 1) & 1);
+            __syncwarp();
+            fence_after();
+            int pm = 0;
+#pragma unroll
+            for (int q = 0; q < I8_NMOD; ++q) pm = m == q ? modulus(q) : pm;
+            const double ipm = 1.0 / pm;
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int j = 2 * jp + h;
+                if (j > i) break;
+                uint8_t* dst = tiles + m * tstride + ((size_t)(i * (i + 1) / 2 + j) * KB_BYTES) + row * 128;
+#pragma unroll 1
+                for (int c0 = 0; c0 < 128; c0 += 32) {
+                    uint32_t v[32];
+                    tmem_ld32(lane_base + buf * BN + h * 128 + c0, v);
+                    uint32_t w[8];
+#pragma unroll
+                    for (int e = 0; e < 32; ++e) {
+                        const int x = (int)v[e];
+                        int r = x - (int)floor((double)x * ipm) * pm;
+                        r = r < 0 ? r + pm : (r >= pm ? r - pm : r);
+                        if ((e & 3) == 0) w[e >> 2] = 0;
+                        w[e >> 2] |= (uint32_t)r << (8 * (e & 3));
+                    }
+                    uint4* d4 = reinterpret_cast<uint4*>(dst + c0);
+                    d4[0] = make_uint4(w[0], w[1], w[2], w[3]);
+                    d4[1] = make_uint4(w[4], w[5], w[6], w[7]);
+                }
+            }
+            fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&tempty[buf]);
+        }
+    }
+    fence_before();
+    __syncthreads();
+    fence_after();
+    if (warp == 1) {
+        __syncwarp();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem));
+    }
+}
+
+// ---- reconstruction ----------------------------------------------------------------------------------------------------------
+// Garner: digit I from residue r_I and the digits below it, every modulus a compile-time constant
+template <int I, int J>
+__host__ __device__ inline int garner_step(int t, const int* v) {
+    if constexpr (J == I) {
+        return t;
+    } else {
+        constexpr int p = modulus(I), inv = inv_mod(modulus(J) % modulus(I), modulus(I));
+        const int vj = v[J] >= p ? v[J] - p : v[J];   // v_J < p_J <= 256 < 2 p_I
+        return garner_step<I, J + 1>((t + p - vj) * inv % p, v);
+    }
+}
+template <int I>
+__host__ __device__ inline void garner(const int* r, int* v) {
+    if constexpr (I < I8_NMOD) {
+        v[I] = garner_step<I, 0>(r[I], v);
+        garner<I + 1>(r, v);
+    }
+}
+
+__host__ __device__ inline int clz64(uint64_t x) {
+#ifdef __CUDA_ARCH__
+    return __clzll((long long)x);
+#else
+    return __builtin_clzll(x);
+#endif
+}
+__host__ __device__ inline double u128_to_double(unsigned __int128 u) {   // correctly rounded (to nearest even)
+    const uint64_t hi = (uint64_t)(u >> 64), lo = (uint64_t)u;
+    if (hi == 0) return (double)lo;
+    const int sh = 64 - clz64(hi);                 // 1 .. 62: the value has 64 + sh significant bits
+    uint64_t m = (uint64_t)(u >> sh);              // top 64 bits; what is shifted out only matters as a sticky bit
+    if (lo & ((1ull << sh) - 1)) m |= 1;
+    return scalbn((double)m, sh);
+}
+
+__global__ void __launch_bounds__(256) i8_crt_kernel(const uint8_t* __restrict__ tiles, size_t tstride, double* __restrict__ C, long ldc,
+                                                     double scale) {
+    constexpr unsigned __int128 P = prod_moduli();
+    const int tile = blockIdx.x >> 4;
+    int ti = 0;
+    while ((ti + 1) * (ti + 2) / 2 <= tile) ++ti;
+    const int tj = tile - ti * (ti + 1) / 2;
+    const int e = (blockIdx.x & 15) * 1024 + threadIdx.x * 4, row = e >> 7, col = e & 127;
+    uint32_t w[I8_NMOD];
+#pragma unroll
+    for (int m = 0; m < I8_NMOD; ++m) w[m] = __ldg(reinterpret_cast<const uint32_t*>(tiles + m * tstride + (size_t)tile * KB_BYTES + e));
+    double out[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        int r[I8_NMOD], v[I8_NMOD];
+#pragma unroll
+        for (int m = 0; m < I8_NMOD; ++m) r[m] = (w[m] >> (8 * q)) & 0xFF;
+        garner<0>(r, v);
+        unsigned __int128 x = (unsigned)v[I8_NMOD - 1];
+#pragma unroll
+        for (int m = I8_NMOD - 2; m >= 0; --m) x = x * (unsigned)modulus(m) + (unsigned)v[m];
+        const bool neg = x > P / 2;   // symmetric range: the exact integer is x - P
+        const double d = u128_to_double(neg ? P - x : x);
+        out[q] = (neg ? -d : d) * scale;
+    }
+    double2* c = reinterpret_cast<double2*>(C + (size_t)(ti * 128 + row) * ldc + tj * 128 + col);
+    double2 a = c[0], b = c[1];
+    a.x += out[0]; a.y += out[1]; b.x += out[2]; b.y += out[3];
+    c[0] = a; c[1] = b;
+}
+
+}  // namespace i8
+
+using namespace i8;
+
+static int plane_row_blocks(int Mp) { return (Mp / 128 + 1) & ~1; }   // even: the last block of an odd tile row reads one past it
+
+size_t i8_plane_bytes(int Mp, long nc) { return (size_t)I8_NMOD * (nc / 128) * plane_row_blocks(Mp) * KB_BYTES; }
+size_t i8_tile_bytes(int Mp) {
+    const size_t nt = Mp / 128;
+    return (size_t)I8_NMOD * nt * (nt + 1) / 2 * KB_BYTES;
+}
+
+int i8_planes_init(int8_t* planes, int Mp, long nc_alloc, cudaStream_t s) {
+    return (int)cudaMemsetAsync(planes, 0, i8_plane_bytes(Mp, nc_alloc), s);
+}
+
+int i8_syrk_launch(const double* K, long ldk, int Mp, int ncols, double var, double alpha, int8_t* planes, long nc_alloc, uint8_t* tiles,
+                   double* C, long ldc, cudaStream_t s) {
+    if (ncols <= 0 || ncols % 128 || ncols > I8_MAX_COLS || ncols > nc_alloc || Mp % 128 || ldk % 2 || ldc % 2)
+        return (int)cudaErrorInvalidValue;
+    const int nt = Mp / 128, nrb = plane_row_blocks(Mp), nkb = ncols / 128;
+    const size_t pstride = (size_t)(nc_alloc / 128) * nrb * KB_BYTES;
+    const size_t tstride = (size_t)nt * (nt + 1) / 2 * KB_BYTES;
+    i8_residue_kernel<<<dim3(nkb, nt), 256, 0, s>>>(K, ldk, 4503599627370496.0 / var, planes, pstride, nrb);
+    if (int e = count_launch()) return e;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (cudaError_t e = cudaFuncSetAttribute(i8_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM)) return (int)e;
+    const int nblk = blocks_per_modulus(nt), units = I8_NMOD * nblk;
+    i8_gram_kernel<<<units < sms ? units : sms, GEMM_THREADS, GEMM_SMEM, s>>>(planes, pstride, nrb, nkb, nblk, tiles, tstride);
+    if (int e = count_launch()) return e;
+    i8_crt_kernel<<<(unsigned)(tstride / KB_BYTES) * 16, 256, 0, s>>>(tiles, tstride, C, ldc, alpha * var * var * 0x1p-104);
+    return count_launch();
+}
+
+}  // namespace tsvgp

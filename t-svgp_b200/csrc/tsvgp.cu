@@ -16,6 +16,7 @@
 #include "common.cuh"
 #include "dense.cuh"
 #include "gemm.cuh"
+#include "int8_gram.cuh"
 #include "kernels.cuh"
 #include "nccl_dyn.h"
 #include <nvtx3/nvToolsExt.h>   // header-only; ranges let ncu select the kernels of one phase (--nvtx --nvtx-include "tsvgp_stream/")
@@ -235,6 +236,11 @@ struct tsvgp_ctx {
     double* kpart[MAXS] = {};     // split-K partial tiles of the SYRK when M is so small that its tiles cannot fill the SMs
     double* bacc[MAXS] = {};      // fused b += Kuf g shared by the tiles of a tile row: [L][2 pieces][Mp/128 tile columns][Mp] private slots
     int ksplit = 1;
+    // Gaussian step, fused route: the constant-weight SYRK as an exact int8 Gram product (int8_gram.cuh) — per slab stream the
+    // 16 residue planes of the slab and the residues of the lower tiles; allocated for a Gaussian model (i8_alloc)
+    int8_t* i8_planes[MAXS] = {};
+    uint8_t* i8_tiles[MAXS] = {};
+    bool i8_alloc = false;
 
     // multi-GPU
     NcclComm comm = nullptr;
@@ -760,8 +766,9 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const bool need_w = c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT;
     const int want_streams = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     const int slab_lat = c->sep ? c->L : 1;
+    const bool want_i8 = c->lik.kind == LIK_GAUSSIAN && !c->white && nc <= I8_MAX_COLS;
     if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || (c->grad_ws && c->grad_lat >= u_lat)) &&
-        c->slab_streams >= want_streams && c->slab_lat == slab_lat)
+        c->slab_streams >= want_streams && c->slab_lat == slab_lat && c->i8_alloc == want_i8)
         return TSVGP_OK;
     CU(cudaStreamSynchronize(c->s_main));
     c->pc.release();
@@ -793,6 +800,13 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
             c->kpart[s] = nullptr;
             if (c->ksplit > 1) NEED(c->kpart[s] = p.get((size_t)c->ksplit * c->Mp * c->Mp));
         }
+    }
+    for (int s = 0; s < MAXS; ++s) { c->i8_planes[s] = nullptr; c->i8_tiles[s] = nullptr; }
+    c->i8_alloc = want_i8;
+    for (int s = 0; s < ns && want_i8 && c->ksplit <= 1; ++s) {   // (split-K products stay FP64)
+        NEED(c->i8_planes[s] = (int8_t*)p.get((i8_plane_bytes(c->Mp, nc) + 7) / 8));
+        NEED(c->i8_tiles[s] = (uint8_t*)p.get((i8_tile_bytes(c->Mp) + 7) / 8));
+        LA(i8_planes_init(c->i8_planes[s], c->Mp, nc, c->s_main));
     }
     NEED(c->ve_all = p.get((size_t)c->L * ve_need));
     for (int s = 0; s < ns; ++s) NEED(c->bacc[s] = p.get((size_t)c->L * 2 * (c->Mp / 128) * c->Mp));
@@ -901,6 +915,11 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         const int nt = Mp / 128;
         const int ks_here = c->ksplit < ncols / 128 ? c->ksplit : ncols / 128;
         fused_b = false;
+        if (const_h && c->route == ROUTE_FUSED && !c->white && ks_here <= 1 && c->i8_planes[b] && ncols <= I8_MAX_COLS) {
+            // the raw covariance slab, one weight: B += alpha K K^T exactly on the int8 tensor cores (b += K g by the caller's gemv)
+            LA(i8_syrk_launch(stat_slab, nc, Mp, ncols, c->kern_var, p.alpha, c->i8_planes[b], nc, c->i8_tiles[b], c->stats[b], Mp, s));
+            return TSVGP_OK;
+        }
         if (ks_here > 1) {
             p.ksplit = ks_here; p.part = c->kpart[b]; p.part_stride = (long)Mp * Mp;
             LA(gemm_launch(p, s));
