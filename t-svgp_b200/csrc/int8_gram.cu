@@ -304,11 +304,12 @@ __global__ void __launch_bounds__(256) i8_crt_kernel(const uint8_t* __restrict__
         for (int m = I8_NMOD - 2; m >= 0; --m) x = x * (unsigned)modulus(m) + (unsigned)v[m];
         const bool neg = x > P / 2;   // symmetric range: the exact integer is x - P
         const double d = u128_to_double(neg ? P - x : x);
-        out[q] = (neg ? -d : d) * scale;
+        out[q] = neg ? -d : d;
     }
+    // C + fl(B') scale with one rounding (fma), written out so that it does not rest on the compiler's contraction
     double2* c = reinterpret_cast<double2*>(C + (size_t)(ti * 128 + row) * ldc + tj * 128 + col);
     double2 a = c[0], b = c[1];
-    a.x += out[0]; a.y += out[1]; b.x += out[2]; b.y += out[3];
+    a.x = fma(out[0], scale, a.x); a.y = fma(out[1], scale, a.y); b.x = fma(out[2], scale, b.x); b.y = fma(out[3], scale, b.y);
     c[0] = a; c[1] = b;
 }
 

@@ -18,6 +18,10 @@ M = 1536
 # cond(K9) at M = 1536 on these points: 5.4e3, 1.3e3, 1.9e3
 KERNELS = [orc.Matern52(variance=1.3, lengthscales=3.0), orc.SquaredExponential(variance=0.6, lengthscales=2.0),
            orc.Matern52(variance=0.8, lengthscales=2.5)]
+# the smallest variance first: a kernel variance left over from an earlier latent would put this latent's entries off the grid
+# (above 2 v), where the residue kernel maps them to 0.  cond(K9) at M = 1536: 1.3e3, 5.4e3, 1.9e3
+KERNELS_SMALL_FIRST = [orc.SquaredExponential(variance=0.3, lengthscales=2.0), orc.Matern52(variance=1.3, lengthscales=3.0),
+                       orc.Matern52(variance=0.8, lengthscales=2.5)]
 
 
 def _case(L, N, M, D=16, seed=21, noise=0.1):
@@ -27,11 +31,11 @@ def _case(L, N, M, D=16, seed=21, noise=0.1):
     return X, F + 0.3 * rng.standard_normal((N, L)), X[:M].copy(), orc.Gaussian(variance=noise)
 
 
-def _pair(L=1, separate=False, streams=2, early=1, N=4600, chunk=1024):
+def _pair(L=1, separate=False, streams=2, early=1, N=4600, chunk=1024, M=M, kernels=KERNELS):
     import tsvgp_b200 as tb
     X, Y, Z, lik = _case(L, N=N, M=M)
     if separate:
-        kernel = so.SeparateIndependent(KERNELS[:L])   # Matern-5/2, SE, Matern-5/2
+        kernel = so.SeparateIndependent(kernels[:L])   # Matern-5/2, SE, Matern-5/2 by default
         ref = so.OracleSeparateTSVGP(kernel, lik, orc.InducingPoints(Z.copy()), num_latent_gps=L, num_data=4 * N)
     else:
         kernel = KERNELS[0]
@@ -51,10 +55,29 @@ def test_single_latent_matches_the_oracle(streams, early):
     dev.close()
 
 
-@pytest.mark.parametrize("separate", [False, True], ids=["L3_shared", "L3_separate_se_matern52"])
-def test_three_latents_match_the_oracle(separate):
-    dev, ref, data = _pair(L=3, separate=separate)
-    _elbo_and_sites_errors(dev, ref, data, steps=2)
+def _int8_products(fn):
+    """Run fn() and count the int8 products (i8_gram_kernel launches) it ran, from the CUDA kernels the profiler records."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+    return sum(1 for e in prof.events() if "i8_gram_kernel" in e.name)
+
+
+@pytest.mark.parametrize("separate,m,kernels", [(False, M, KERNELS), (True, M, KERNELS), (True, M, KERNELS_SMALL_FIRST),
+                                                (False, 1600, KERNELS), (False, 2048, KERNELS)],
+                         ids=["L3_shared", "L3_separate_se_matern52", "L3_separate_smallest_variance_first",
+                              "L3_shared_M1600_odd_tile_count", "L3_shared_M2048"])
+def test_three_latents_match_the_oracle(separate, m, kernels):
+    # M = 1600 pads to Mp = 1664: 13 tile rows (the planes' padding row block) and padding rows in the slab; M = 2048 is cfg3's
+    dev, ref, data = _pair(L=3, separate=separate, M=m, kernels=kernels)
+    Z = data[0][:m]
+    for k in (kernels if separate else kernels[:1]):   # the fused route, which takes the int8 product, needs cond(K9) < 1e4
+        ev = np.linalg.eigvalsh(k.K(Z))
+        assert ev[-1] / ev[0] < 1e4
+    n_i8 = _int8_products(lambda: _elbo_and_sites_errors(dev, ref, data, steps=2))
+    t = dev.timings()
+    assert t["route"] == 1
+    assert n_i8 == 2 * t["slabs"] * (3 if separate else 1)   # every SYRK of both steps: one per slab and latent (one if shared)
     dev.close()
 
 

@@ -11,73 +11,7 @@ import numpy as np
 import pytest
 import scipy.linalg as sla
 
-MODULI = [256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193]
-P = int(np.prod([int(p) for p in MODULI], dtype=object))
-GRID = 2.0 ** 52
-MAX_POINTS = 2 ** 17 - 128   # widest slab the int32 accumulation takes (a multiple of 128 below 2^17)
-
-
-def grid(K, v):
-    A = np.rint(np.asarray(K, dtype=np.float64) * (GRID / v))
-    A[~np.isfinite(A)] = 0.0
-    return A
-
-
-def residues(A):
-    """[16, rows, n] symmetric residues of the grid integers (what the int8 planes hold)."""
-    Ai = A.astype(np.int64)
-    out = []
-    for p in MODULI:
-        r = Ai % p
-        r = np.where(r > (p - 1) // 2, r - p, r)   # [-128, 127] for 256, [-(p-1)/2, (p-1)/2] for odd p
-        out.append(r.astype(np.int8))
-    return np.stack(out)
-
-
-def modular_gram(R):
-    """C_i mod p_i in [0, p_i) from the int32-exact products of the residue planes."""
-    out = []
-    for p, r in zip(MODULI, R):
-        c = r.astype(np.int64) @ r.astype(np.int64).T
-        assert np.abs(c).max(initial=0) < 2 ** 31   # the tensor cores accumulate in int32
-        out.append(c % p)
-    return out
-
-
-def crt(cs):
-    """Garner's mixed-radix digits, then Horner; the integer in the symmetric range (-P/2, P/2)."""
-    n = len(MODULI)
-    shape = cs[0].shape
-    out = np.empty(shape, dtype=object)
-    inv = [[pow(MODULI[j], -1, MODULI[i]) if j < i else 0 for j in range(n)] for i in range(n)]
-    for idx in np.ndindex(shape):
-        v = []
-        for i in range(n):
-            t = int(cs[i][idx])
-            for j in range(i):
-                t = (t - v[j]) * inv[i][j] % MODULI[i]
-            v.append(t)
-        x = 0
-        for i in reversed(range(n)):
-            x = x * MODULI[i] + v[i]
-        out[idx] = x - P if x > P // 2 else x
-    return out
-
-
-def exact_gram(A):
-    """The exact integer A A^T from 18-bit limbs (int64 products summed exactly), combined in Python integers."""
-    Ai = A.astype(np.int64)
-    limbs = [(Ai >> (18 * k)) & ((1 << 18) - 1) for k in range(3)]
-    out = np.zeros((A.shape[0], A.shape[0]), dtype=object)
-    for a in range(3):
-        for b in range(3):
-            out = out + (limbs[a] @ limbs[b].T).astype(object) * (1 << (18 * (a + b)))
-    return out
-
-
-def to_double(B_int, v, alpha=1.0):
-    return np.vectorize(lambda x: float(x))(B_int).astype(np.float64) * (alpha * v * v * 2.0 ** -104)
-
+from tests.int8_gram_ref import GRID, MAX_POINTS, MODULI, P, crt, exact_gram, grid, modular_gram, residues, to_double
 
 def emulated_gram(K, v, alpha=1.0):
     return to_double(crt(modular_gram(residues(grid(K, v)))), v, alpha)
