@@ -1,11 +1,13 @@
 // Exact fixed-point Gram product on the INT8 tensor cores (tcgen05.mma kind::i8, SASS UTCIMMA): see int8_gram.cuh and DESIGN §2.
-//   i8_residue_kernel : K (FP64 slab) -> A = rint(K 2^52 / v) -> 16 int8 residue planes, written as the shared-memory image the
-//                       MMA descriptors describe (128-row x 128-byte k-blocks of K-major core matrices, 128-byte swizzle)
+//   i8_residue_kernel : K (FP64 slab) -> A = rint(K 2^52 / v) -> 64-bit integer -> three 18-bit limbs -> 16 int8 residue planes
+//                       (integer arithmetic: one multiply-high per modulus), written as the shared-memory image the MMA descriptors
+//                       describe (128-row x 128-byte k-blocks of K-major core matrices, 128-byte swizzle)
 //   i8_gram_kernel    : persistent, warp-specialised: one producer thread streams k-blocks into a 4-stage mbarrier ring with
 //                       cp.async.bulk, one thread issues 128 x 256 x 32 MMAs into a double-buffered TMEM accumulator, four
 //                       epilogue warps reduce the int32 tiles modulo p_i into residue tiles.  Modulus-major schedule: the lower
 //                       128 x 256 blocks of modulus i, then i + 1 (one modulus's planes stay in L2 while its blocks run)
-//   i8_crt_kernel     : Garner's mixed-radix digits + Horner in 128-bit integers -> the exact integer -> one rounding -> C += alpha ...
+//   i8_crt_kernel     : Garner's mixed-radix digits (one reduction per digit) + Horner in 128-bit integers -> the exact integer ->
+//                       one rounding -> C += alpha ...
 #include "int8_gram.cuh"
 #include "common.cuh"
 
@@ -82,23 +84,49 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
 }
 
 // ---- residues --------------------------------------------------------------------------------------------------------------
-template <int M>
-__device__ __forceinline__ uint32_t residue4(const double* a) {   // symmetric residues of 4 grid integers mod p_M, packed
-    constexpr double p = modulus(M), ip = 1.0 / modulus(M);
-    constexpr double hi = (modulus(M) - 1) / 2, lo = -(modulus(M) / 2);   // [-128, 127] for 256, [-(p-1)/2, (p-1)/2] otherwise
-    uint32_t w = 0;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const double q = rint(a[j] * ip);
-        double r = fma(-q, p, a[j]);   // exact: |A - q p| is a small integer
-        if (r > hi) r -= p;
-        else if (r < lo) r += p;
-        w |= (uint32_t)((int)r & 0xFF) << (8 * j);
-    }
-    return w;
+// x mod p for x <= MOD_X_MAX by one multiply-high: q = floor(x m / 2^36) with m = ceil(2^36 / p) is floor(x / p) while x (m p - 2^36)
+// < 2^36 (the error x (m p - 2^36) / (p 2^36) stays below 1 / p); both callers' bounds are checked at compile time below
+constexpr uint32_t MOD_X_MAX = (1u << 28) - 1;
+__host__ __device__ constexpr uint32_t mod_magic(int p) { return (uint32_t)(((1ull << 36) + p - 1) / p); }
+__host__ __device__ constexpr bool mod_magic_exact(int i) {
+    return i == I8_NMOD || ((uint64_t)MOD_X_MAX * ((uint64_t)mod_magic(modulus(i)) * modulus(i) - (1ull << 36)) < (1ull << 36) &&
+                            mod_magic_exact(i + 1));
+}
+static_assert(mod_magic_exact(0), "mod_small: the multiply-high quotient is exact for x <= MOD_X_MAX");
+template <int P>
+__device__ __forceinline__ uint32_t mod_small(uint32_t x) {   // x mod P, x <= MOD_X_MAX
+    return x - (__umulhi(x, mod_magic(P)) >> 4) * P;
+}
+
+// The grid integer t (|t| < 2^53) enters as u = t + 2^53 in [1, 2^54), split into 18-bit limbs u = l2 2^36 + l1 2^18 + l0.  For an
+// odd modulus p with h = (p - 1) / 2,  x = l2 (2^36 mod p) + l1 (2^18 mod p) + l0 + ((h - 2^53) mod p)  is t + h (mod p) and below
+// 2^27, so  (x mod p) - h  is t's residue in the symmetric range [-h, h].  Modulus 256 is t's low byte (2^53 = 0 mod 256), the
+// two's complement of its residue in [-128, 127].
+struct Limbs { uint32_t l0, l1, l2; };
+__device__ __forceinline__ Limbs limbs_of(double t) {
+    const uint64_t u = (uint64_t)(__double2ll_rn(t) + (1ll << 53));
+    const uint32_t lo = (uint32_t)u, hi = (uint32_t)(u >> 32);
+    return {lo & 0x3FFFF, __funnelshift_r(lo, hi, 18) & 0x3FFFF, hi >> 4};
 }
 template <int M>
-__device__ __forceinline__ void store_residues(const double* a, int8_t* dst, size_t pstride) {
+__device__ __forceinline__ uint32_t residue_byte(const Limbs& a) {   // symmetric residue mod p_M; only the low byte counts
+    constexpr int p = modulus(M), h = (p - 1) / 2;
+    constexpr uint32_t c18 = (1u << 18) % p, c36 = (uint32_t)((1ull << 36) % p);
+    constexpr uint32_t off = (uint32_t)((h + p - (int)((1ull << 53) % p)) % p);
+    if constexpr (M == 0) {
+        return a.l0;
+    } else {
+        const uint32_t x = a.l2 * c36 + a.l1 * c18 + a.l0 + off;
+        return mod_small<p>(x) - h;
+    }
+}
+template <int M>
+__device__ __forceinline__ uint32_t residue4(const Limbs* a) {   // 4 residue bytes, packed
+    return __byte_perm(__byte_perm(residue_byte<M>(a[0]), residue_byte<M>(a[1]), 0x0040),
+                       __byte_perm(residue_byte<M>(a[2]), residue_byte<M>(a[3]), 0x0040), 0x5410);
+}
+template <int M>
+__device__ __forceinline__ void store_residues(const Limbs* a, int8_t* dst, size_t pstride) {
     if constexpr (M < I8_NMOD) {
         uint4 w;
         w.x = residue4<M>(a); w.y = residue4<M>(a + 4); w.z = residue4<M>(a + 8); w.w = residue4<M>(a + 12);
@@ -115,16 +143,17 @@ __global__ void __launch_bounds__(256) i8_residue_kernel(const double* __restric
     for (int it = 0; it < 4; ++it) {
         const int c = threadIdx.x + 256 * it, row = c >> 3, kc = c & 7;
         const double2* src = reinterpret_cast<const double2*>(K + (size_t)(rb * 128 + row) * ldk + kb * 128 + kc * 16);
-        double a[16];
+        double k[16];
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             const double2 v = __ldg(src + j);
-            a[2 * j] = v.x; a[2 * j + 1] = v.y;
+            k[2 * j] = v.x; k[2 * j + 1] = v.y;
         }
+        Limbs a[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
-            const double t = rint(a[j] * scale);
-            a[j] = fabs(t) < 9007199254740992.0 ? t : 0.0;   // off the grid (non-finite): 0; the point kernel flags such a step
+            const double t = rint(k[j] * scale);
+            a[j] = limbs_of(fabs(t) < 9007199254740992.0 ? t : 0.0);   // off the grid (non-finite): 0; the point kernel flags such a step
         }
         store_residues<0>(a, planes + (size_t)(kb * nrb + rb) * KB_BYTES + kblock_off(row, kc * 16), pstride);
     }
@@ -246,21 +275,37 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* 
 }
 
 // ---- reconstruction ----------------------------------------------------------------------------------------------------------
-// Garner: digit I from residue r_I and the digits below it, every modulus a compile-time constant
+// Garner's digits with one reduction each: x = sum_J v_J prod_{K<J} p_K with 0 <= v_J < p_J, so
+//   v_I = (r_I - sum_{J<I} v_J c_IJ) inv_I mod p_I = (r_I inv_I + sum_{J<I} v_J c'_IJ) mod p_I,
+// c_IJ = (prod_{K<J} p_K) mod p_I, inv_I = (prod_{K<I} p_K)^-1 mod p_I and c'_IJ = -c_IJ inv_I mod p_I, all compile-time constants.
+// The sum is below 16 * 255 * 255 < MOD_X_MAX: one exact reduction per digit.
+__host__ __device__ constexpr int prefix_mod(int J, int I) {   // (prod_{K<J} p_K) mod p_I
+    int c = 1;
+    for (int K = 0; K < J; ++K) c = c * modulus(K) % modulus(I);
+    return c;
+}
+__host__ __device__ constexpr int garner_inv(int I) { return inv_mod(prefix_mod(I, I), modulus(I)); }
+__host__ __device__ constexpr int garner_coef(int I, int J) {   // c'_IJ
+    return (modulus(I) - prefix_mod(J, I) * garner_inv(I) % modulus(I)) % modulus(I);
+}
 template <int I, int J>
-__host__ __device__ inline int garner_step(int t, const int* v) {
+__device__ __forceinline__ uint32_t garner_sum(uint32_t s, const uint32_t* v) {
     if constexpr (J == I) {
-        return t;
+        return s;
     } else {
-        constexpr int p = modulus(I), inv = inv_mod(modulus(J) % modulus(I), modulus(I));
-        const int vj = v[J] >= p ? v[J] - p : v[J];   // v_J < p_J <= 256 < 2 p_I
-        return garner_step<I, J + 1>((t + p - vj) * inv % p, v);
+        constexpr uint32_t c = garner_coef(I, J);
+        return garner_sum<I, J + 1>(s + v[J] * c, v);
     }
 }
 template <int I>
-__host__ __device__ inline void garner(const int* r, int* v) {
-    if constexpr (I < I8_NMOD) {
-        v[I] = garner_step<I, 0>(r[I], v);
+__device__ __forceinline__ void garner(const uint32_t* r, uint32_t* v) {
+    if constexpr (I == 0) {
+        v[0] = r[0];
+        garner<1>(r, v);
+    } else if constexpr (I < I8_NMOD) {
+        constexpr uint32_t inv = garner_inv(I);
+        const uint32_t s = garner_sum<I, 0>(r[I] * inv, v);
+        v[I] = mod_small<modulus(I)>(s);
         garner<I + 1>(r, v);
     }
 }
@@ -295,13 +340,13 @@ __global__ void __launch_bounds__(256) i8_crt_kernel(const uint8_t* __restrict__
     double out[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-        int r[I8_NMOD], v[I8_NMOD];
+        uint32_t r[I8_NMOD], v[I8_NMOD];
 #pragma unroll
         for (int m = 0; m < I8_NMOD; ++m) r[m] = (w[m] >> (8 * q)) & 0xFF;
         garner<0>(r, v);
-        unsigned __int128 x = (unsigned)v[I8_NMOD - 1];
+        unsigned __int128 x = v[I8_NMOD - 1];
 #pragma unroll
-        for (int m = I8_NMOD - 2; m >= 0; --m) x = x * (unsigned)modulus(m) + (unsigned)v[m];
+        for (int m = I8_NMOD - 2; m >= 0; --m) x = x * (unsigned)modulus(m) + v[m];
         const bool neg = x > P / 2;   // symmetric range: the exact integer is x - P
         const double d = u128_to_double(neg ? P - x : x);
         out[q] = neg ? -d : d;
