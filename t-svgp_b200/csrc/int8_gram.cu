@@ -2,10 +2,11 @@
 //   i8_residue_kernel : K (FP64 slab) -> A = rint(K 2^52 / v) -> 64-bit integer -> three 18-bit limbs -> 16 int8 residue planes
 //                       (integer arithmetic: one multiply-high per modulus), written as the shared-memory image the MMA descriptors
 //                       describe (128-row x 128-byte k-blocks of K-major core matrices, 128-byte swizzle)
-//   i8_gram_kernel    : persistent, warp-specialised: one producer thread streams k-blocks into a 4-stage mbarrier ring with
-//                       cp.async.bulk, one thread issues 128 x 256 x 32 MMAs into a double-buffered TMEM accumulator, four
-//                       epilogue warps reduce the int32 tiles modulo p_i into residue tiles.  Modulus-major schedule: the lower
-//                       128 x 256 blocks of modulus i, then i + 1 (one modulus's planes stay in L2 while its blocks run)
+//   i8_gram_kernel    : persistent CTA pairs, warp-specialised: in each CTA one producer thread streams k-blocks into a 6-stage
+//                       mbarrier ring with cp.async.bulk; the pair's leader issues 256 x 256 x 32 MMAs (cta_group::2) into a
+//                       double-buffered TMEM accumulator; four epilogue warps per CTA reduce the int32 tiles modulo p_i into
+//                       residue tiles.  Modulus-major schedule: the lower 256 x 256 blocks of modulus i, then i + 1 (one modulus's
+//                       planes stay in L2 while its blocks run)
 //   i8_crt_kernel     : Garner's mixed-radix digits (one reduction per digit) + Horner in 128-bit integers -> the exact integer ->
 //                       one rounding -> C += alpha ...
 #include "int8_gram.cuh"
@@ -16,11 +17,11 @@ namespace tsvgp {
 namespace i8 {
 
 constexpr int KB_BYTES = 16384;                 // one 128-row x 128-byte k-block
-constexpr int BN = 256;                         // output block: two 128-tiles of one tile row
-constexpr int STAGES = 4;
-constexpr int STAGE_BYTES = KB_BYTES + BN * 128;
+constexpr int BN = 256;                         // accumulator columns: two 128-tiles of one tile row per CTA
+constexpr int STAGES = 6;
+constexpr int STAGE_BYTES = 2 * KB_BYTES;       // one CTA's A and B row blocks of one k-block
 constexpr int GEMM_SMEM = STAGES * STAGE_BYTES + 1024;
-constexpr int GEMM_THREADS = 192;               // warp 0 producer, warp 1 MMA issuer, warps 2..5 epilogue
+constexpr int GEMM_THREADS = 192;               // warp 0 producer, warp 1 MMA issuer (rank 0) or stage forwarder (rank 1), warps 2..5 epilogue
 
 __host__ __device__ constexpr int modulus(int i) {
     constexpr int p[I8_NMOD] = {256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193};
@@ -42,16 +43,12 @@ __device__ __forceinline__ uint32_t kblock_off(int r, int k) {
     return (r >> 3) * 1024 + (r & 7) * 128 + ((((k >> 4) ^ (r & 7)) << 4) | (k & 15));
 }
 
-// lower blocks of one modulus: tile row i holds ceil((i + 1) / 2) blocks of two tiles (the last may reach one tile past the diagonal)
+// lower 128 x 256 blocks of one modulus: tile row i holds ceil((i + 1) / 2) blocks of two tiles.  The product kernel takes this count
+// (its `nblk`) for the tile count it names; it schedules 256 x 256 pair blocks
 __host__ __device__ inline int blocks_per_modulus(int nt) {
     int n = 0;
     for (int i = 0; i < nt; ++i) n += (i + 2) / 2;
     return n;
-}
-__device__ __forceinline__ void block_coords(int blk, int& i, int& jp) {
-    i = 0;
-    while (blk >= (i + 2) / 2) { blk -= (i + 2) / 2; ++i; }
-    jp = blk;
 }
 
 // ---- tcgen05 -------------------------------------------------------------------------------------------------------------
@@ -60,15 +57,8 @@ __device__ __forceinline__ uint32_t saddr(const void* p) { return (uint32_t)__cv
 __device__ __forceinline__ uint64_t sdesc(uint32_t a) {
     return (uint64_t)((a >> 4) & 0x3FFF) | (uint64_t)(1024 >> 4) << 32 | 1ull << 46 | 2ull << 61;
 }
-// instruction descriptor: D s32, A and B signed 8-bit, both K-major, M = 128, N = BN
-constexpr uint32_t IDESC = 2u << 4 | 1u << 7 | 1u << 10 | (uint32_t)(BN >> 3) << 17 | (128u >> 4) << 24;
-__device__ __forceinline__ void mma_i8(uint32_t d, uint64_t a, uint64_t b, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(d), "l"(a), "l"(b),
-                 "r"(IDESC), "r"(acc));
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(saddr(bar)) : "memory");
-}
+// instruction descriptor: D s32, A and B signed 8-bit, both K-major, M = 256 (a CTA pair), N = BN
+constexpr uint32_t IDESC = 2u << 4 | 1u << 7 | 1u << 10 | (uint32_t)(BN >> 3) << 17 | (256u >> 4) << 24;
 __device__ __forceinline__ void fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -160,51 +150,104 @@ __global__ void __launch_bounds__(256) i8_residue_kernel(const double* __restric
 }
 
 // ---- products --------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* __restrict__ planes, size_t pstride, int nrb, int nkb,
-                                                                  int nblk, uint8_t* __restrict__ tiles, size_t tstride) {
+// CTA pairs (cluster of 2): pair unit (m, I, J <= I) is the 256 x 256 block of pair row I and pair column J of modulus m.  CTA rank r
+// loads A = row block 2I + r and B = row block 2J + r (16 KB each per k-block, one copy when I == J); the leader (rank 0) issues
+// 256 x 256 x 32 MMAs (cta_group::2), which read A's 256 rows and B's 256 rows from both CTAs' shared memory and leave rank r's 128
+// rows, tiles (2I + r, 2J) and (2I + r, 2J + 1), in rank r's TMEM.  Stages are released to both producers by a multicast commit.
+// Rank 1's copies complete on its own `full` barrier (a bulk copy signals a barrier of the CTA it writes to); one thread of rank 1
+// forwards each completed stage to the leader's `full`, which therefore counts two arrivals.  Pairs depend on no other pair.
+__device__ __forceinline__ uint32_t cluster_rank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+__device__ __forceinline__ uint32_t leader_addr(const void* p) {   // the same shared-memory object in rank 0 of the cluster
+    uint32_t a;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(a) : "r"(saddr(p)));
+    return a;
+}
+// An arrival on a barrier of the other CTA.  Its default CTA-scope release is enough: what it orders is data the async proxy wrote
+// (a stage a bulk copy completed) or read (TMEM after tcgen05.wait::ld and a tcgen05 fence).  A cluster-scope release would put a
+// GPU-wide memory barrier in front of every forwarded stage: measured, that halves the product rate.
+__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
+    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
+}
+__device__ __forceinline__ void cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release;\nbarrier.cluster.wait.acquire;" ::: "memory");
+}
+__device__ __forceinline__ void mma_i8_pair(uint32_t d, uint64_t a, uint64_t b, uint32_t acc) {
+    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(d), "l"(a), "l"(b),
+                 "r"(IDESC), "r"(acc));
+}
+__device__ __forceinline__ void mma_commit_pair(uint64_t* bar) {   // arrive on `bar` in both CTAs once the MMAs issued so far are done
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(saddr(bar)),
+                 "h"((uint16_t)3) : "memory");
+}
+__device__ __forceinline__ void pair_coords(int u, int& I, int& J) {
+    I = 0;
+    while (u > I) { u -= I + 1; ++I; }
+    J = u;
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
+    i8_gram_kernel(const int8_t* __restrict__ planes, size_t pstride, int nrb, int nkb, int nblk, uint8_t* __restrict__ tiles, size_t tstride) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024 - (saddr(smem_raw) & 1023)) & 1023);   // swizzle atoms on 1 KB boundaries
     __shared__ uint64_t full[STAGES], empty[STAGES], tfull[2], tempty[2];
     __shared__ uint32_t tslot;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int units = I8_NMOD * nblk;
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(saddr(&tslot)));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    const uint32_t rank = cluster_rank();
+    int nt = 0;   // blocks_per_modulus is strictly increasing: nblk names the tile count
+    for (int n = 0; n < nblk; ++nt) n += (nt + 2) / 2;
+    const int per_mod = (nrb / 2) * (nrb / 2 + 1) / 2, units = I8_NMOD * per_mod;
+    const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;   // a 1-D grid of clusters of 2: ranks are blockIdx.x & 1
     if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 4); }
+        for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], rank == 0 ? 2 : 1); mbar_init(&empty[s], 1); }
+        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 8); }   // the epilogue warps of both CTAs
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    if (warp == 1) {   // one warp of each CTA: the same 512 columns in both
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(saddr(&tslot)));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
+    }
     fence_before();
-    __syncthreads();
+    cluster_sync();
     fence_after();
     const uint32_t tmem = tslot;
 
     if (warp == 0) {
-        if (lane == 0) {   // producer
+        if (lane == 0) {   // producer (both CTAs)
             int k = 0;
-            for (int u = blockIdx.x; u < units; u += gridDim.x) {
-                const int m = u / nblk;
-                int i, jp;
-                block_coords(u - m * nblk, i, jp);
-                const int8_t* pa = planes + m * pstride + (size_t)i * KB_BYTES;
-                const int8_t* pb = planes + m * pstride + (size_t)(2 * jp) * KB_BYTES;
+            for (int u = pair; u < units; u += npairs) {
+                const int m = u / per_mod;
+                int I, J;
+                pair_coords(u - m * per_mod, I, J);
+                const int8_t* pa = planes + m * pstride + (size_t)(2 * I + rank) * KB_BYTES;
+                const int8_t* pb = planes + m * pstride + (size_t)(2 * J + rank) * KB_BYTES;
                 for (int kb = 0; kb < nkb; ++kb, ++k) {
                     const int s = k % STAGES;
                     if (k >= STAGES) mbar_wait(&empty[s], ((k / STAGES) - 1) & 1);
                     uint8_t* st = smem + s * STAGE_BYTES;
-                    mbar_expect_tx(&full[s], STAGE_BYTES);
+                    mbar_expect_tx(&full[s], I == J ? KB_BYTES : 2 * KB_BYTES);
                     tma_bulk_g2s(st, pa + (size_t)kb * nrb * KB_BYTES, KB_BYTES, &full[s]);
-                    tma_bulk_g2s(st + KB_BYTES, pb + (size_t)kb * nrb * KB_BYTES, BN * 128, &full[s]);
+                    if (I != J) tma_bulk_g2s(st + KB_BYTES, pb + (size_t)kb * nrb * KB_BYTES, KB_BYTES, &full[s]);
                 }
             }
         }
     } else if (warp == 1) {
-        if (lane == 0) {   // MMA issuer
+        if (lane == 0 && rank != 0) {   // forwards rank 1's completed stages to the leader
+            int k = 0;
+            for (int u = pair; u < units; u += npairs)
+                for (int kb = 0; kb < nkb; ++kb, ++k) {
+                    const int s = k % STAGES;
+                    mbar_wait(&full[s], (k / STAGES) & 1);
+                    mbar_arrive_remote(leader_addr(&full[s]));
+                }
+        } else if (lane == 0) {   // MMA issuer (leader)
             int k = 0, t = 0;
-            for (int u = blockIdx.x; u < units; u += gridDim.x, ++t) {
+            for (int u = pair; u < units; u += npairs, ++t) {
+                int I, J;
+                pair_coords(u % per_mod, I, J);
                 const int buf = t & 1;
                 if (t >= 2) mbar_wait(&tempty[buf], ((t >> 1) - 1) & 1);
                 fence_after();
@@ -213,22 +256,23 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* 
                     const int s = k % STAGES;
                     mbar_wait(&full[s], (k / STAGES) & 1);
                     fence_after();
-                    const uint32_t a = saddr(smem + s * STAGE_BYTES), b = a + KB_BYTES;
+                    const uint32_t a = saddr(smem + s * STAGE_BYTES), b = I == J ? a : a + KB_BYTES;
 #pragma unroll
-                    for (int kk = 0; kk < 4; ++kk) mma_i8(d, sdesc(a + 32 * kk), sdesc(b + 32 * kk), (kb | kk) != 0);
-                    mma_commit(&empty[s]);
+                    for (int kk = 0; kk < 4; ++kk) mma_i8_pair(d, sdesc(a + 32 * kk), sdesc(b + 32 * kk), (kb | kk) != 0);
+                    mma_commit_pair(&empty[s]);
                 }
-                mma_commit(&tfull[buf]);
+                mma_commit_pair(&tfull[buf]);
             }
         }
-    } else {   // epilogue: TMEM lanes 32 (warp % 4) .. + 31 are rows of the block
+    } else {   // epilogue (both CTAs): TMEM lanes 32 (warp % 4) .. + 31 are rows of this CTA's row block
         const int row = (warp & 3) * 32 + lane;
         const uint32_t lane_base = tmem + ((uint32_t)((warp & 3) * 32) << 16);
         int t = 0;
-        for (int u = blockIdx.x; u < units; u += gridDim.x, ++t) {
-            const int m = u / nblk;
-            int i, jp;
-            block_coords(u - m * nblk, i, jp);
+        for (int u = pair; u < units; u += npairs, ++t) {
+            const int m = u / per_mod;
+            int I, J;
+            pair_coords(u - m * per_mod, I, J);
+            const int i = 2 * I + rank;   // tile row; i == nt is the padding block of an odd tile count
             const int buf = t & 1;
             mbar_wait(&tfull[buf], (t >> 1) & 1);
             __syncwarp();
@@ -239,8 +283,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* 
             const double ipm = 1.0 / pm;
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-                const int j = 2 * jp + h;
-                if (j > i) break;
+                const int j = 2 * J + h;
+                if (j > i || i >= nt) break;
                 uint8_t* dst = tiles + m * tstride + ((size_t)(i * (i + 1) / 2 + j) * KB_BYTES) + row * 128;
 #pragma unroll 1
                 for (int c0 = 0; c0 < 128; c0 += 32) {
@@ -262,15 +306,16 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) i8_gram_kernel(const int8_t* 
             }
             fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[buf]);
+            if (lane == 0) mbar_arrive_remote(leader_addr(&tempty[buf]));
         }
     }
+    __syncwarp();
     fence_before();
-    __syncthreads();
+    cluster_sync();   // every MMA has completed and no CTA of the pair still signals the other's barriers
     fence_after();
     if (warp == 1) {
         __syncwarp();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem));
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tmem));
     }
 }
 
@@ -374,6 +419,25 @@ int i8_planes_init(int8_t* planes, int Mp, long nc_alloc, cudaStream_t s) {
     return (int)cudaMemsetAsync(planes, 0, i8_plane_bytes(Mp, nc_alloc), s);
 }
 
+// CTAs of the product launch: two per cluster that can be resident at once (queried once per device and host thread), so that
+// every pair runs in the first wave, and at most two per pair unit
+static int i8_gram_grid(int nrb, int& grid) {
+    thread_local int cached_dev = -1, clusters = 0;
+    int dev = 0;
+    if (cudaError_t e = cudaGetDevice(&dev)) return (int)e;
+    if (dev != cached_dev) {
+        if (cudaError_t e = cudaFuncSetAttribute(i8_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM)) return (int)e;
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3(2); cfg.blockDim = dim3(GEMM_THREADS); cfg.dynamicSmemBytes = GEMM_SMEM;
+        if (cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, i8_gram_kernel, &cfg)) return (int)e;
+        if (clusters < 1) return (int)cudaErrorInvalidConfiguration;
+        cached_dev = dev;
+    }
+    const int pairs = I8_NMOD * (nrb / 2) * (nrb / 2 + 1) / 2;
+    grid = 2 * (pairs < clusters ? pairs : clusters);
+    return 0;
+}
+
 int i8_syrk_launch(const double* K, long ldk, int Mp, int ncols, double var, double alpha, int8_t* planes, long nc_alloc, uint8_t* tiles,
                    double* C, long ldc, cudaStream_t s) {
     if (ncols <= 0 || ncols % 128 || ncols > I8_MAX_COLS || ncols > nc_alloc || Mp % 128 || ldk % 2 || ldc % 2)
@@ -383,12 +447,9 @@ int i8_syrk_launch(const double* K, long ldk, int Mp, int ncols, double var, dou
     const size_t tstride = (size_t)nt * (nt + 1) / 2 * KB_BYTES;
     i8_residue_kernel<<<dim3(nkb, nt), 256, 0, s>>>(K, ldk, 4503599627370496.0 / var, planes, pstride, nrb);
     if (int e = count_launch()) return e;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaError_t e = cudaFuncSetAttribute(i8_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM)) return (int)e;
-    const int nblk = blocks_per_modulus(nt), units = I8_NMOD * nblk;
-    i8_gram_kernel<<<units < sms ? units : sms, GEMM_THREADS, GEMM_SMEM, s>>>(planes, pstride, nrb, nkb, nblk, tiles, tstride);
+    int grid = 0;
+    if (int e = i8_gram_grid(nrb, grid)) return e;
+    i8_gram_kernel<<<grid, GEMM_THREADS, GEMM_SMEM, s>>>(planes, pstride, nrb, nkb, blocks_per_modulus(nt), tiles, tstride);
     if (int e = count_launch()) return e;
     i8_crt_kernel<<<(unsigned)(tstride / KB_BYTES) * 16, 256, 0, s>>>(tiles, tstride, C, ldc, alpha * var * var * 0x1p-104);
     return count_launch();

@@ -3,6 +3,8 @@
 //   resident : operands stay in shared memory, one thread issues 128 x N x 32 MMAs back to back
 //   streamed : a 4-stage mbarrier ring fed by cp.async.bulk (one 128-row x 128-byte A k-block + one N-row B k-block per stage)
 //              from a 32 MB operand image laid out as the Gram product's residue planes ([k-block][128-row block][16 KB])
+//   pair     : the same stream into CTA pairs (clusters of 2): 256 x 256 x 32 MMAs (cta_group::2) issued by the leader, each CTA
+//              loading one 128-row A and one 128-row B k-block per stage (32 KB), 6 stages; as many pairs as can be resident
 // Both operand layouts are checked bit-exactly against the host first: K-major core matrices without swizzle, and 128-byte swizzle.
 // Tooling only (not part of the product library). Build: see tools/Makefile.
 #include <cstdint>
@@ -201,6 +203,90 @@ __global__ void __launch_bounds__(128, 1) k_stream(const int8_t* img, int nrb, i
     if (warp == 0) tmem_dealloc(tm, 2 * N);
 }
 
+// streamed CTA pairs: pair unit u has A = pair row u % (nrb / 2), B = pair row (u / (nrb / 2)) % (nrb / 2); rank r loads row 2I + r
+// of each.  Rank 1's copies complete on its own barrier and one thread forwards them to the leader's (as the Gram product does).
+template <int STAGES>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1) k_stream_pair(const int8_t* img, int nrb, int nkb, int units, int32_t* sink) {
+    extern __shared__ __align__(1024) uint8_t smem_raw[];
+    uint8_t* smem = smem_raw + ((1024 - (sa(smem_raw) & 1023)) & 1023);
+    __shared__ uint64_t full[STAGES], empty[STAGES], done;
+    __shared__ uint32_t tslot;
+    constexpr uint32_t SA = 16384, SS = 2 * SA;
+    constexpr uint32_t IDESC2 = 2u << 4 | 1u << 7 | 1u << 10 | (256u >> 3) << 17 | (256u >> 4) << 24;   // M = 256, N = 256
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint32_t rank;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    const int pr = nrb / 2, pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < STAGES; ++s) { mbar_init(&full[s], rank == 0 ? 2 : 1); mbar_init(&empty[s], 1); }
+        mbar_init(&done, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(sa(&tslot)));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;");
+    asm volatile("barrier.cluster.arrive.release;\nbarrier.cluster.wait.acquire;" ::: "memory");
+    asm volatile("tcgen05.fence::after_thread_sync;");
+    const uint32_t tm = tslot;
+    if (warp == 0 && lane == 0) {   // producer
+        int k = 0;
+        for (int u = pair; u < units; u += npairs) {
+            const int ra = 2 * (u % pr) + rank, rb = 2 * ((u / pr) % pr) + rank;
+            for (int kb = 0; kb < nkb; ++kb, ++k) {
+                const int s = k % STAGES;
+                if (k >= STAGES) mbar_wait(&empty[s], ((k / STAGES) - 1) & 1);
+                uint8_t* st = smem + s * SS;
+                mbar_expect_tx(&full[s], SS);
+                bulk_g2s(st, img + ((size_t)kb * nrb + ra) * 16384, SA, &full[s]);
+                bulk_g2s(st + SA, img + ((size_t)kb * nrb + rb) * 16384, SA, &full[s]);
+            }
+        }
+    } else if (warp == 1 && lane == 0 && rank != 0) {   // forward rank 1's stages to the leader
+        int k = 0;
+        for (int u = pair; u < units; u += npairs)
+            for (int kb = 0; kb < nkb; ++kb, ++k) {
+                const int s = k % STAGES;
+                mbar_wait(&full[s], (k / STAGES) & 1);
+                uint32_t ra;
+                asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(ra) : "r"(sa(&full[s])));
+                asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(ra) : "memory");
+            }
+    } else if (warp == 1 && lane == 0) {   // MMA issuer (leader)
+        int k = 0, t = 0;
+        for (int u = pair; u < units; u += npairs, ++t) {
+            for (int kb = 0; kb < nkb; ++kb, ++k) {
+                const int s = k % STAGES;
+                asm volatile("{\n.reg .pred P1;\nWC:\nmbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n@P1 bra DC;\n"
+                             "bra WC;\nDC:\n}\n" ::"r"(sa(&full[s])), "r"((k / STAGES) & 1) : "memory");
+                asm volatile("tcgen05.fence::after_thread_sync;");
+                const uint32_t a = sa(smem + s * SS), b = a + SA;
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk)
+                    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n}\n"
+                                 ::"r"(tm + (t & 1) * 256), "l"(sdesc(a + 32 * kk, 128, 1024, 2)), "l"(sdesc(b + 32 * kk, 128, 1024, 2)),
+                                 "r"(IDESC2), "r"((uint32_t)(kb > 0 || kk > 0)));
+                asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                             ::"r"(sa(&empty[s])), "h"((uint16_t)3) : "memory");
+            }
+        }
+        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                     ::"r"(sa(&done)), "h"((uint16_t)3) : "memory");
+    }
+    __syncwarp();
+    if (pair < units) mbar_wait(&done, 0);   // a pair without units issues no commit
+    __syncwarp();
+    asm volatile("tcgen05.fence::after_thread_sync;");
+    uint32_t v;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\ntcgen05.wait::ld.sync.aligned;" : "=r"(v) : "r"(tm + ((uint32_t)(warp * 32) << 16)));
+    if (v == 0x7fffffffu) sink[blockIdx.x] = v;
+    asm volatile("tcgen05.fence::before_thread_sync;");
+    asm volatile("barrier.cluster.arrive.release;\nbarrier.cluster.wait.acquire;" ::: "memory");
+    asm volatile("tcgen05.fence::after_thread_sync;");
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tm));
+}
+
 static float time_ms(cudaEvent_t a, cudaEvent_t b) { float ms; cudaEventElapsedTime(&ms, a, b); return ms; }
 
 static void smi(const char* tag) {
@@ -275,6 +361,27 @@ static double stream(int sms, const int8_t* img, int nrb, int nkb, int units, in
     return ops / ms * 1e-9;
 }
 
+template <int STAGES>
+static void stream_pair(const int8_t* img, int nrb, int nkb, int units, int32_t* sink, cudaEvent_t e0, cudaEvent_t e1, int reps) {
+    const int sm_bytes = STAGES * 32768 + 1024;
+    CK(cudaFuncSetAttribute(k_stream_pair<STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm_bytes));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = sm_bytes;
+    int clusters = 0;
+    CK(cudaOccupancyMaxActiveClusters(&clusters, k_stream_pair<STAGES>, &cfg));
+    const int grid = 2 * clusters;
+    k_stream_pair<STAGES><<<grid, 128, sm_bytes>>>(img, nrb, nkb, units, sink);
+    CK(cudaDeviceSynchronize());
+    cudaEventRecord(e0);
+    for (int r = 0; r < reps; ++r) k_stream_pair<STAGES><<<grid, 128, sm_bytes>>>(img, nrb, nkb, units, sink);
+    cudaEventRecord(e1); CK(cudaDeviceSynchronize());
+    const float ms = time_ms(e0, e1) / reps;
+    const double ops = 2.0 * units * 256.0 * 256 * 128.0 * nkb;
+    const double bytes = (double)units * nkb * 2 * 32768;
+    printf("streamed pairs 256x256 %d stages sw128, %d pair units x %d k-blocks, %d CTAs (%d resident clusters): %8.3f ms  %7.1f TOP/s  "
+           "(smem fill %.1f TB/s)\n", STAGES, units, nkb, grid, clusters, ms, ops / ms * 1e-9, bytes / ms * 1e-9);
+}
+
 int main() {
     cudaDeviceProp p; CK(cudaGetDeviceProperties(&p, 0));
     const int sms = p.multiProcessorCount;
@@ -296,6 +403,8 @@ int main() {
         stream<128, 6>(sms, img, nrb, nkb, 1152 * 2, sink, e0, e1, swz, 5);
         stream<256, 4>(sms, img, nrb, nkb, 1152, sink, e0, e1, swz, 5);
     }
+    // the same work in 576 pair units of 256 x 256
+    stream_pair<6>(img, nrb, nkb, 576, sink, e0, e1, 5);
     // sustained: ~2 s of the streamed 128 x 256 loop, clocks sampled while it runs
     {
         const int reps = 60;

@@ -1,6 +1,8 @@
 // Tooling: one slab of the Gaussian step's constant-weight SYRK  C += alpha K K^T  (lower tiles) as the exact int8 Gram product
 // (t-svgp_b200/csrc/int8_gram.cu) against the FP64 DMMA SYRK, and both against the exact integer product on the host for sampled
-// entries.  Random K in [0, v] with exact 0 and v entries; per-kernel times with CUDA events.
+// entries.  Random K in [0, v] with exact 0 and v entries; per-kernel times with CUDA events.  The products are timed twice, each
+// behind the residue kernel: (a) as the launcher runs them, (b) with pstride = 0, so that all 16 moduli read plane 0 (L2-resident
+// operands; the tiles it writes are not checked).  (a) - (b) is what reading the 16 freshly written planes costs.
 // Build: make -C tools i8_syrk_bench ; run: tools/i8_syrk_bench [Mp=2048] [ncols=16384]
 #include <cmath>
 #include <cstdio>
@@ -81,26 +83,38 @@ int main(int argc, char** argv) {
     // timing: the three kernels separately, then the FP64 SYRK
     const int nt = Mp / 128, nrb = (nt + 1) & ~1, nkb = ncols / 128, nblk = blocks_per_modulus(nt);
     const size_t pstride = (size_t)(nc / 128) * nrb * KB_BYTES, tstride = (size_t)nt * (nt + 1) / 2 * KB_BYTES;
-    cudaEvent_t ev[5];
+    int grid = 0;
+    CK((cudaError_t)i8_gram_grid(nrb, grid));
+    cudaEvent_t ev[7];
     for (auto& x : ev) cudaEventCreate(&x);
     const int reps = 10;
-    float t[4] = {0, 0, 0, 0};
+    float t[5] = {0, 0, 0, 0, 0};
     for (int r = 0; r < reps + 1; ++r) {
         cudaEventRecord(ev[0]);
         i8_residue_kernel<<<dim3(nkb, nt), 256>>>(K, nc, scale, planes, pstride, nrb);
         cudaEventRecord(ev[1]);
-        i8_gram_kernel<<<prop.multiProcessorCount, GEMM_THREADS, GEMM_SMEM>>>(planes, pstride, nrb, nkb, nblk, tiles, tstride);
+        i8_gram_kernel<<<grid, GEMM_THREADS, GEMM_SMEM>>>(planes, pstride, nrb, nkb, nblk, tiles, tstride);
         cudaEventRecord(ev[2]);
         i8_crt_kernel<<<(unsigned)(tstride / KB_BYTES) * 16, 256>>>(tiles, tstride, C8, Mp, alpha * v * v * 0x1p-104);
         cudaEventRecord(ev[3]);
         gemm_launch(p, 0);
         cudaEventRecord(ev[4]);
-        CK(cudaEventSynchronize(ev[4]));
-        if (r) for (int k = 0; k < 4; ++k) t[k] += ev_ms(ev[k], ev[k + 1]) / reps;
+        i8_residue_kernel<<<dim3(nkb, nt), 256>>>(K, nc, scale, planes, pstride, nrb);
+        cudaEventRecord(ev[5]);
+        i8_gram_kernel<<<grid, GEMM_THREADS, GEMM_SMEM>>>(planes, 0, nrb, nkb, nblk, tiles, tstride);
+        cudaEventRecord(ev[6]);
+        CK(cudaEventSynchronize(ev[6]));
+        if (r) {
+            for (int k = 0; k < 4; ++k) t[k] += ev_ms(ev[k], ev[k + 1]) / reps;
+            t[4] += ev_ms(ev[5], ev[6]) / reps;
+        }
     }
+    CK(cudaGetLastError());
     const double ops8 = 16.0 * nblk * 2.0 * 128 * 256 * ncols, flops64 = (double)nt * (nt + 1) / 2 * 2.0 * 128 * 128 * ncols;
     printf("i8_residue_kernel  %8.3f ms  (%.2f TB/s: slab read + planes written)\n", t[0], (8.0 * Mp * ncols + 16.0 * Mp * ncols) / t[0] * 1e-9);
-    printf("i8_gram_kernel     %8.3f ms  %.1f TOP/s int8 (%d units of 128x256x%d)\n", t[1], ops8 / t[1] * 1e-9, 16 * nblk, ncols);
+    printf("i8_gram_kernel     %8.3f ms  %.1f TOP/s int8 (%d blocks of 128x256x%d, %d CTAs in pairs)  (a) as launched\n", t[1],
+           ops8 / t[1] * 1e-9, 16 * nblk, ncols, grid);
+    printf("i8_gram_kernel     %8.3f ms  %.1f TOP/s int8  (b) pstride = 0: every modulus reads plane 0\n", t[4], ops8 / t[4] * 1e-9);
     printf("i8_crt_kernel      %8.3f ms\n", t[2]);
     printf("int8 total         %8.3f ms\n", t[0] + t[1] + t[2]);
     printf("FP64 DMMA SYRK     %8.3f ms  %.1f TFLOP/s\n", t[3], flops64 / t[3] * 1e-9);
