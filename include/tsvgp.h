@@ -46,7 +46,9 @@ enum {
     TSVGP_ERR_STATE = -6              /* called before the kernel / inducing points / data it needs were set             */
 };
 
-enum { TSVGP_KERNEL_SE = 0, TSVGP_KERNEL_MATERN52 = 1 };                       /* gpflow.kernels.{SquaredExponential,Matern52} */
+/* gpflow.kernels.{SquaredExponential,Matern52,Matern12,Matern32}; the Matern kernels take r = sqrt(max(r2, 1e-36)) as GPflow does.
+ * Matern12's derivative in r2 (tsvgp_elbo_grad) is the one autodiff takes through that clamp: 0 for r2 < 1e-36.            */
+enum { TSVGP_KERNEL_SE = 0, TSVGP_KERNEL_MATERN52 = 1, TSVGP_KERNEL_MATERN12 = 2, TSVGP_KERNEL_MATERN32 = 3 };
 /* gpflow.likelihoods.*; TSVGP_LIK_HETEROSKEDASTIC: HeteroskedasticTFPConditional(distribution_class = Normal), see set_likelihood */
 enum { TSVGP_LIK_GAUSSIAN = 0, TSVGP_LIK_BERNOULLI_PROBIT = 1, TSVGP_LIK_STUDENT_T = 2, TSVGP_LIK_SOFTMAX = 3, TSVGP_LIK_HETEROSKEDASTIC = 4 };
 

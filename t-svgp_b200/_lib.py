@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libtsvgp.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOT_PD, ERR_NONPOS_VAR, ERR_COMM, ERR_STATE = 0, -1, -2, -3, -4, -5, -6
-KERNEL_SE, KERNEL_MATERN52 = 0, 1
+KERNEL_SE, KERNEL_MATERN52, KERNEL_MATERN12, KERNEL_MATERN32 = 0, 1, 2, 3
 LIK_GAUSSIAN, LIK_BERNOULLI_PROBIT, LIK_STUDENT_T, LIK_SOFTMAX, LIK_HETEROSKEDASTIC = 0, 1, 2, 3, 4
 ABI_VERSION = 1
 

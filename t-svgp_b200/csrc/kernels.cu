@@ -10,6 +10,7 @@ namespace tsvgp {
 // Covariance tiles.  Restates GPflow 2.2.1 stationaries.py / utilities/ops.py::square_distance (SURVEY Appendix B):
 //   Xs = X / lengthscales ;  r2 = |xs|^2 + |zs|^2 - 2 xs.zs  (expansion form, not clipped for SE)
 //   SE: variance * exp(-r2/2) ;  Matern52: r = sqrt(max(r2,1e-36)), variance (1 + sqrt5 r + 5/3 r^2) exp(-sqrt5 r)
+//   Matern32: variance (1 + sqrt3 r) exp(-sqrt3 r) ;  Matern12: variance exp(-r)   (same r)
 // called by the reference at src/models/tsvgp.py:209,268,269 and inside gpflow.conditionals.conditional (:103).
 // =====================================================================================================================
 __global__ void scale_points_kernel(const double* __restrict__ X, long n, int D, const double* __restrict__ ls,
@@ -84,13 +85,28 @@ __device__ __forceinline__ double sqrt_pos(double m) {
     return fma(0.5 * y, e, r);
 }
 
-// k(r2) and, when asked, dk/d(r2)  (SE: -k/2 ; Matern-5/2: -(5/6) variance (1 + sqrt5 r) exp(-sqrt5 r))
+// k(r2) and, when asked, dk/d(r2)  (SE: -k/2 ; Matern-5/2: -(5/6) variance (1 + sqrt5 r) exp(-sqrt5 r) ;
+// Matern-3/2: -(3/2) variance exp(-sqrt3 r) ; Matern-1/2: -k / (2 r) for r2 >= 1e-36, else 0)
 template <int KIND, bool DERIV>
 __device__ __forceinline__ double cov_from_r2(double r2, double variance, double& dk) {
     if (KIND == KERN_SE) {
         const double k = variance * exp_nonpos(-0.5 * r2);
         if (DERIV) dk = -0.5 * k;
         return k;
+    } else if (KIND == KERN_MATERN12) {
+        // GPflow: variance exp(-r), r = sqrt(max(r2, 1e-36)).  The derivative is the one TensorFlow's autodiff takes through the
+        // clamp: 1 / (2 r) below it would put -5e17 variance into the M-step's E at a coincident point (r2 = 0 exactly when a
+        // point equals an inducing input: x2, z2 and x.z come from the same fma chain)
+        const double r = sqrt_pos(fmax(r2, 1e-36));
+        const double k = variance * exp_nonpos(-r);
+        if (DERIV) dk = r2 >= 1e-36 ? -0.5 * k / r : 0.0;
+        return k;
+    } else if (KIND == KERN_MATERN32) {
+        const double r = sqrt_pos(fmax(r2, 1e-36));
+        const double sqrt3 = 1.73205080756887729353;
+        const double e = variance * exp_nonpos(-sqrt3 * r);
+        if (DERIV) dk = -1.5 * e;
+        return fma(sqrt3, r, 1.0) * e;
     } else {
         const double r = sqrt_pos(fmax(r2, 1e-36));
         const double sqrt5 = 2.23606797749978969641;
@@ -221,6 +237,10 @@ int kuf_launch(int kind, double variance, const double* XsT, long ldx, const dou
     else if (kind == KERN_SE) kuf_kernel<KERN_SE, true><<<grid, 256, 0, s>>>(KUF_ARGS);
     else if (kind == KERN_MATERN52 && !Kp) kuf_kernel<KERN_MATERN52, false><<<grid, 256, 0, s>>>(KUF_ARGS);
     else if (kind == KERN_MATERN52) kuf_kernel<KERN_MATERN52, true><<<grid, 256, 0, s>>>(KUF_ARGS);
+    else if (kind == KERN_MATERN12 && !Kp) kuf_kernel<KERN_MATERN12, false><<<grid, 256, 0, s>>>(KUF_ARGS);
+    else if (kind == KERN_MATERN12) kuf_kernel<KERN_MATERN12, true><<<grid, 256, 0, s>>>(KUF_ARGS);
+    else if (kind == KERN_MATERN32 && !Kp) kuf_kernel<KERN_MATERN32, false><<<grid, 256, 0, s>>>(KUF_ARGS);
+    else if (kind == KERN_MATERN32) kuf_kernel<KERN_MATERN32, true><<<grid, 256, 0, s>>>(KUF_ARGS);
     else return -1;
 #undef KUF_ARGS
     return count_launch();

@@ -5,7 +5,7 @@
 
 namespace tsvgp {
 
-enum { KERN_SE = 0, KERN_MATERN52 = 1 };
+enum { KERN_SE = 0, KERN_MATERN52 = 1, KERN_MATERN12 = 2, KERN_MATERN32 = 3 };
 enum { LIK_GAUSSIAN = 0, LIK_BERNOULLI = 1, LIK_STUDENT_T = 2, LIK_SOFTMAX = 3, LIK_HETEROSKEDASTIC = 4 };
 constexpr int MAX_SOFTMAX_CLASSES = 16;
 constexpr int MAX_GH = 64;

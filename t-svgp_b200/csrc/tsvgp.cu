@@ -1898,7 +1898,8 @@ int tsvgp_set_mc_epsilon(tsvgp_ctx* c, const double* eps, int S, int64_t N, int 
 int tsvgp_num_latent(const tsvgp_ctx* c) { return c ? c->L : 0; }
 
 static int check_kernel(tsvgp_ctx* c, int kind, double variance, const double* lengthscales, int n_ls) {
-    if (kind != TSVGP_KERNEL_SE && kind != TSVGP_KERNEL_MATERN52) FAIL(TSVGP_ERR_INVALID, "unknown kernel kind %d", kind);
+    if (kind != TSVGP_KERNEL_SE && kind != TSVGP_KERNEL_MATERN52 && kind != TSVGP_KERNEL_MATERN12 && kind != TSVGP_KERNEL_MATERN32)
+        FAIL(TSVGP_ERR_INVALID, "unknown kernel kind %d", kind);
     if (!lengthscales || n_ls < 1 || !(variance > 0.0)) FAIL(TSVGP_ERR_INVALID, "kernel needs variance > 0 and >= 1 lengthscale");
     for (int i = 0; i < n_ls; ++i)
         if (!(lengthscales[i] > 0.0)) FAIL(TSVGP_ERR_INVALID, "lengthscales must be positive");

@@ -4,7 +4,7 @@ implements: `natgrad_step`, `elbo`, `predict_f` over `DenseSites (lambda_1, lamb
 
 The GPflow kernel, likelihood and inducing-variable objects are used unchanged: only the attributes the reference path
 reads are touched (duck-typed; `.numpy()` is honoured):
-    kernel      SquaredExponential / RBF / Matern52 : .variance, .lengthscales (scalar, [D] or [1, D]);
+    kernel      SquaredExponential / RBF / Matern12 / Matern32 / Matern52 : .variance, .lengthscales (scalar, [D] or [1, D]);
                 SharedIndependent (.kernel, .output_dim) ; SeparateIndependent (.kernels, one per latent)
     likelihood  Gaussian (.variance) | Bernoulli (inv_probit link) | StudentT (.scale, .df)   [+ .num_gauss_hermite_points]
                 | Softmax | HeteroskedasticTFPConditional (distribution_class Normal, scale_transform Exp / Softplus)
@@ -46,8 +46,12 @@ def _kernel_spec(kernel, num_latent_gps=None):
         kind = _lib.KERNEL_SE
     elif name == "Matern52":
         kind = _lib.KERNEL_MATERN52
+    elif name == "Matern32":
+        kind = _lib.KERNEL_MATERN32
+    elif name == "Matern12":
+        kind = _lib.KERNEL_MATERN12
     else:
-        raise NotImplementedError(f"kernel {name}: the B200 path implements SquaredExponential and Matern52")
+        raise NotImplementedError(f"kernel {name}: the B200 path implements SquaredExponential, Matern12, Matern32 and Matern52")
     active = getattr(kernel, "active_dims", None)
     if active is not None and not (isinstance(active, slice) and active == slice(None, None, None)):
         raise NotImplementedError("active_dims other than all dimensions")

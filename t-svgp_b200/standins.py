@@ -20,6 +20,18 @@ class Matern52:
         self.lengthscales = np.asarray(lengthscales, dtype=np.float64)
 
 
+class Matern12:
+    def __init__(self, variance=1.0, lengthscales=1.0):
+        self.variance = float(variance)
+        self.lengthscales = np.asarray(lengthscales, dtype=np.float64)
+
+
+class Matern32:
+    def __init__(self, variance=1.0, lengthscales=1.0):
+        self.variance = float(variance)
+        self.lengthscales = np.asarray(lengthscales, dtype=np.float64)
+
+
 class SharedIndependent:
     """gpflow.kernels.SharedIndependent(kernel, output_dim): one kernel for every latent GP."""
 
