@@ -173,8 +173,9 @@ TSVGP_API int tsvgp_prior_kl(tsvgp_ctx* ctx, double* out);
  * `elbo` (tsvgp.py:79-95; callers docs/notebooks/mnist.py:161-163,188-189; pinned by tests/models/test_tsvgp.py:168-188).
  * Gradients are w.r.t. the constrained (natural) parameter values; Zero mean function; any D; one kernel shared by the
  * latents.  Softmax: the derivatives of the Monte-Carlo sum for the call's draws (one per call, see tsvgp_set_mc_epsilon),
- * with h = d ve / d var unclipped; one pass over the data for all latents.  Not built for the heteroskedastic likelihood,
- * separate kernels per latent or the whitened sibling (TSVGP_ERR_INVALID).                                               */
+ * with h = d ve / d var unclipped; one pass over the data for all latents.  The whitened sibling (option "white") holds its
+ * own sites fixed, lambda_1 and the full Lambda_2, and runs one pass per latent like the plain model (DESIGN 10).  Collective
+ * with several ranks.  Not built for the heteroskedastic likelihood or separate kernels per latent (TSVGP_ERR_INVALID).    */
 TSVGP_API int tsvgp_elbo_grad(tsvgp_ctx* ctx, double scale, double* elbo, double* d_variance, double* d_lengthscales,
                               double* d_Z, double* d_lik);
 /* base_SVGP.predict_f, full_cov = False (tsvgp.py:97-114): mean_out, var_out [N, L]                                     */

@@ -541,6 +541,7 @@ int gemm_init() {
     e |= init_inst<false, false, false, EPI_STORE_COLNORM>();
     e |= init_inst<true, false, false, EPI_STORE>();
     e |= init_inst<true, false, false, EPI_COLNORM>();
+    e |= init_inst<true, false, false, EPI_STORE_COLNORM>();
     return e;
 }
 
@@ -622,6 +623,7 @@ int gemm_launch(const GemmP& p, cudaStream_t stream) {
     }
     if (p.a_kc && !p.b_kc) {
         if (p.epilogue == EPI_COLNORM) return p.ksplit == 1 && !p.C2 ? launch_inst<true, false, false, EPI_COLNORM>(p, stream) : -1;
+        if (p.epilogue == EPI_STORE_COLNORM) return p.ksplit == 1 && !p.C2 ? launch_inst<true, false, false, EPI_STORE_COLNORM>(p, stream) : -1;
         if (p.epilogue != EPI_STORE) return -1;
         return launch_inst<true, false, false, EPI_STORE>(p, stream);
     }

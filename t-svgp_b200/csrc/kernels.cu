@@ -1854,5 +1854,26 @@ int gamma_uu_launch(const double* QBQ, const double* QKQ, const double* qb, cons
     gamma_uu_kernel<<<EW_GRID(n), 0, s>>>(QBQ, QKQ, qb, qm, al, Kp, Gamma, E, ld, n, scale);
     return count_launch();
 }
+// The whitened sibling's dELBO/dKuu (DESIGN §10), symmetric; D = A^-1 B A^-1 - R^-1 B R^-1, W = R0^-1 A R0^-1, rb = R^-1 b,
+// al = R^-1 lambda_1, a0 = R0^-1 lambda_1, w = R0^-1 A a0:
+// Gamma[i][j] = scale (D_ij - (rb_i al_j + rb_j al_i)/2) - (2 R0inv_ij - Ainv_ij - W_ij + a0_i a0_j - (w_i a0_j + w_j a0_i))/2
+// E[i][j] = Gamma[i][j] * Kp[i][j] off the diagonal, 0 on it
+__global__ void gamma_uu_white_kernel(const double* D, const double* W, const double* R0inv, const double* Ainv, const double* rb,
+                                      const double* al, const double* a0, const double* w, const double* Kp, double* Gamma, double* E,
+                                      long ld, int n, double scale) {
+    EW_IJ;
+    const long o = (long)i * ld + j, t = (long)j * ld + i;
+    const double a0i = a0[i], a0j = a0[j];
+    const double gmm = scale * (0.5 * (D[o] + D[t]) - 0.5 * (rb[i] * al[j] + rb[j] * al[i])) -
+                       0.5 * (2.0 * R0inv[o] - Ainv[o] - 0.5 * (W[o] + W[t]) + a0i * a0j - (w[i] * a0j + w[j] * a0i));
+    Gamma[o] = gmm;
+    E[o] = i == j ? 0.0 : gmm * Kp[o];
+}
+int gamma_uu_white_launch(const double* D, const double* W, const double* R0inv, const double* Ainv, const double* rb, const double* al,
+                          const double* a0, const double* w, const double* Kp, double* Gamma, double* E, long ld, int n, double scale,
+                          cudaStream_t s) {
+    gamma_uu_white_kernel<<<EW_GRID(n), 0, s>>>(D, W, R0inv, Ainv, rb, al, a0, w, Kp, Gamma, E, ld, n, scale);
+    return count_launch();
+}
 
 }  // namespace tsvgp

@@ -171,5 +171,9 @@ int xaug_launch(const double* XsT, long ldx, long n0, long nvalid, int ncols, in
 inline int aug_width(int D) { return (2 * D + 1 + 127) / 128 * 128; }
 int gamma_uu_launch(const double* QBQ, const double* QKQ, const double* qb, const double* qm, const double* al, const double* Kp,
                     double* Gamma, double* E, long ld, int n, double scale, cudaStream_t s);
+// the whitened sibling's counterpart (tsvgp.cu, grad_epilogue_white): D = A^-1 B A^-1 - R^-1 B R^-1, W = R0^-1 A R0^-1
+int gamma_uu_white_launch(const double* D, const double* W, const double* R0inv, const double* Ainv, const double* rb, const double* al,
+                          const double* a0, const double* w, const double* Kp, double* Gamma, double* E, long ld, int n, double scale,
+                          cudaStream_t s);
 
 }  // namespace tsvgp

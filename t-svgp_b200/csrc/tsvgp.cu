@@ -67,7 +67,7 @@ enum { MODE_STATS = 0, MODE_ELBO = 1, MODE_PREDICT = 2, MODE_GRAD = 3 };   // MO
 enum { INFO_W = 0, INFO_K9 = 1, INFO_P = 2, INFO_S = 3, N_INFO = 4 };
 enum { EV_T0 = 0, EV_PREP, EV_STREAM, EV_REDUCE, EV_DENSE, N_EV };
 // device scalars
-enum { SC_LOGDIAG_W = 0, SC_M_ALPHA, SC_TR_QK, SC_PK0, SC_PK1, SC_PI0, SC_PI1, SC_G_K, SC_TR_QB, SC_A_B, SC_TR_PBP, N_SCAL = 12 };
+enum { SC_LOGDIAG_W = 0, SC_M_ALPHA, SC_TR_QK, SC_PK0, SC_PK1, SC_PI0, SC_PI1, SC_G_K, SC_TR_QB, SC_A_B, SC_TR_PBP, SC_TR_RB, N_SCAL = 12 };
 enum { ROUTE_AUTO = 0, ROUTE_FUSED = 1, ROUTE_WHITENED = 2, ROUTE_EXACT = 3 };
 
 }  // namespace
@@ -228,6 +228,7 @@ struct tsvgp_ctx {
     double* ve_blocks = nullptr;
     long ve_cap = 0;
     double *kpslab[MAXS] = {}, *vslab[MAXS] = {}, *uslab[MAXS] = {}, *xaug[MAXS] = {}, *fpart[MAXS] = {}, *facc[MAXS] = {};   // M-step gradient workspace
+    double* aslab[MAXS] = {};     // ... and the whitened sibling's LA^-1 K (latent-independent)
     double* aux_blocks = nullptr;
     int fsplit = 1;
     bool grad_ws = false;
@@ -767,12 +768,14 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const int want_streams = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     const int slab_lat = c->sep ? c->L : 1;
     const bool want_i8 = c->lik.kind == LIK_GAUSSIAN && !c->white && nc <= I8_MAX_COLS;
+    const bool need_a = need_grad && c->white;   // the whitened gradient pass keeps LA^-1 K beside LR^-1 K
     if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || (c->grad_ws && c->grad_lat >= u_lat)) &&
+        (!need_a || c->aslab[0]) &&
         c->slab_streams >= want_streams && c->slab_lat == slab_lat && c->i8_alloc == want_i8)
         return TSVGP_OK;
     CU(cudaStreamSynchronize(c->s_main));
     c->pc.release();
-    for (int s = 0; s < MAXS; ++s) c->wslab[s] = nullptr;
+    for (int s = 0; s < MAXS; ++s) c->wslab[s] = c->aslab[s] = nullptr;
     Pool& p = c->pc;
     const int ns = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     c->slab_streams = ns;
@@ -819,15 +822,22 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
         if (c->fsplit > (int)(nc / 256)) c->fsplit = (int)(nc / 256);
         if (c->fsplit < 1) c->fsplit = 1;
         const size_t W = (size_t)c->waug;
-        if (u_lat > 1) {   // U of every latent survives until the joint point kernel has run: L Mp nc doubles per slab stream
-            const size_t need = ((size_t)(2 + u_lat) * c->Mp * nc + nc * W + (size_t)(c->fsplit + 1) * c->Mp * W) * ns + 2 * ve_need;
+        // U of every latent survives until the joint point kernel has run: L Mp nc doubles per slab stream; the whitened sibling
+        // keeps one more Mp x nc slab per stream (LA^-1 K)
+        if (u_lat > 1 || need_a) {
+            const size_t need = ((size_t)(2 + u_lat + (need_a ? 1 : 0)) * c->Mp * nc + nc * W + (size_t)(c->fsplit + 1) * c->Mp * W) * ns + 2 * ve_need;
             size_t free_b = 0, total_b = 0;
             CU(cudaMemGetInfo(&free_b, &total_b));
-            if (need * sizeof(double) > free_b)
+            if (need * sizeof(double) > free_b) {
+                if (need_a)
+                    FAIL(TSVGP_ERR_INVALID, "elbo_grad of the whitened sibling at M = %d needs %zu bytes of device memory for its slab "
+                         "workspace, %zu are free (option \"chunk\" narrows the slabs)", c->M, need * sizeof(double), free_b);
                 FAIL(TSVGP_ERR_INVALID, "elbo_grad with %d coupled latents at M = %d needs %zu bytes of device memory for its slab workspace, "
                      "%zu are free (option \"chunk\" narrows the slabs)", c->L, c->M, need * sizeof(double), free_b);
+            }
         }
         for (int s = 0; s < ns; ++s) {
+            if (need_a) NEED(c->aslab[s] = p.get((size_t)c->Mp * nc));
             NEED(c->kpslab[s] = p.get((size_t)c->Mp * nc)); NEED(c->vslab[s] = p.get((size_t)c->Mp * nc));
             NEED(c->uslab[s] = p.get((size_t)u_lat * c->Mp * nc)); NEED(c->xaug[s] = p.get((size_t)nc * W));
             NEED(c->fpart[s] = p.get((size_t)c->fsplit * c->Mp * W)); NEED(c->facc[s] = p.get((size_t)c->Mp * W));
@@ -1009,13 +1019,15 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                 }
             } else {           // (b') whitened sibling: |LA^-1 k_n|^2 and |LR^-1 k_n|^2, two lower-triangular products (util.py:78-85).
                 // The first does not depend on the latent: it is formed once per slab, into the buffer shared by the latents
-                // (`q2_part`); the per-latent one goes to the latent's own `q_part`.
+                // (`q2_part`); the per-latent one goes to the latent's own `q_part`.  The M-step also keeps both products
+                // (LA^-1 K in `aslab`, LR^-1 K in `vslab`) for U = Q K below.
                 for (int which = l == l_lo ? 0 : 1; which < 2; ++which) {
                     GemmP p;
                     p.A = which == 0 ? c->C6inv : c->T; p.lda = Mp; p.a_kc = 1; p.a_tri = 1;
                     p.B = c->slab[b]; p.ldb = nc; p.b_kc = 0;
                     p.m = Mp; p.n = ncols; p.k = Mp;
-                    p.epilogue = EPI_COLNORM; p.norm_out = which == 0 ? c->q2_part[b] : c->q_part[b]; p.ldn = nc;
+                    p.epilogue = grad ? EPI_STORE_COLNORM : EPI_COLNORM; p.norm_out = which == 0 ? c->q2_part[b] : c->q_part[b]; p.ldn = nc;
+                    if (grad) { p.C = which == 0 ? c->aslab[b] : c->vslab[b]; p.ldc = nc; }
                     LA(gemm_launch(p, s));
                 }
             }
@@ -1099,7 +1111,16 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         }
         if (grad) {
             select_latent(c, l_lo);
-            if (!joint) {   // U = T V = Q K  (lower-triangular T times the stored V)
+            if (c->white) {   // U = Q K = LA^-T (LA^-1 K) - LR^-T (LR^-1 K)  (two upper-triangular products over the stored slabs)
+                for (int which = 0; which < 2; ++which) {
+                    GemmP p;
+                    p.A = which == 0 ? c->C6inv : c->T; p.lda = Mp; p.a_kc = 0; p.a_tri = 2;
+                    p.B = which == 0 ? c->aslab[b] : c->vslab[b]; p.ldb = nc; p.b_kc = 0;
+                    p.C = c->uslab[b]; p.ldc = nc; p.m = Mp; p.n = ncols; p.k = Mp;
+                    if (which == 1) { p.alpha = -1.0; p.beta = 1.0; }
+                    LA(gemm_launch(p, s));
+                }
+            } else if (!joint) {   // U = T V = Q K  (lower-triangular T times the stored V)
                 GemmP p;
                 p.A = c->T; p.lda = Mp; p.a_kc = 1; p.a_tri = 1;
                 p.B = c->vslab[b]; p.ldb = nc; p.b_kc = 0;
@@ -2410,6 +2431,89 @@ static int grad_epilogue(tsvgp_ctx* c, int lat, double scale, double* elbo, doub
     return TSVGP_OK;
 }
 
+// C = Linv^T Linv (symmetric, both triangles) of a lower-triangular Mp x Mp Linv, on the main stream: the inverse of the matrix
+// whose Cholesky factor Linv inverts
+static int gram_lower_t(tsvgp_ctx* c, const double* Linv, double* C) {
+    GemmP p;
+    p.A = Linv; p.lda = c->Mp; p.a_kc = 0; p.a_tri = 2;
+    p.B = Linv; p.ldb = c->Mp; p.b_kc = 0; p.b_tri = 2;
+    p.C = C; p.ldc = c->Mp; p.m = p.n = p.k = c->Mp; p.lower_out = 1;
+    LA(mm_gemm(c, p, c->s_main));
+    LA(mirror_lower_launch(C, c->Mp, c->Mp, c->s_main));
+    return TSVGP_OK;
+}
+
+// The whitened sibling's dense epilogue of ONE latent (DESIGN §10): A = K6, R = Lambda_2 + A + 1e-9 I (T = LR^-1, alpha = R^-1
+// lambda_1), R0 = Lambda_2 + A (the KL's matrix, factored again here: ensure_kl_terms_white keeps the last latent's factor only),
+//   Gamma_K = s [A^-1 B A^-1 - R^-1 B R^-1 - sym(R^-1 b alpha^T)]
+//             - 1/2 [2 R0^-1 - A^-1 - R0^-1 A R0^-1 + alpha0 alpha0^T - 2 sym(R0^-1 A alpha0 alpha0^T)],  alpha0 = R0^-1 lambda_1,
+// and <Q, B> = <A^-1, B> - <R^-1, B>.  P must hold A^-1 (formed once per call by tsvgp_elbo_grad).  Reuses Wm, Wf, V, X1, X2, G2.
+static int grad_epilogue_white(tsvgp_ctx* c, int lat, double scale, double* elbo, double* d_variance, double* d_lik, std::vector<double>& Fuu) {
+    cudaStream_t s = c->s_main;
+    const int n = c->Mp, M = c->M, D = c->D, W = c->waug;
+    const long ld = n;
+    const size_t mm = (size_t)n * n;
+    select_latent(c, lat);
+    OK(all_reduce(c, c->stats[0], mm + n + 4));
+    double* B = c->stats[0];
+    double* bvec = c->stats[0] + mm;
+    LA(mirror_lower_launch(B, ld, n, s));
+    auto full_gemm = [&](const double* A, const double* Bm, double* C, double alpha, double beta) {   // C = alpha A Bm + beta C
+        GemmP p;
+        p.A = A; p.lda = ld; p.a_kc = 1;
+        p.B = Bm; p.ldb = ld; p.b_kc = 0;
+        p.C = C; p.ldc = ld; p.m = p.n = p.k = n; p.alpha = alpha; p.beta = beta;
+        return mm_gemm(c, p, s);
+    };
+    const double* Ainv = c->P;
+    OK(gram_lower_t(c, c->T, c->Wm));                 // R^-1
+    LA(full_gemm(Ainv, B, c->X1, 1.0, 0.0));          // A^-1 B
+    LA(full_gemm(c->X1, Ainv, c->X2, 1.0, 0.0));      // A^-1 B A^-1
+    LA(full_gemm(c->Wm, B, c->G2, 1.0, 0.0));         // R^-1 B
+    LA(full_gemm(c->G2, c->Wm, c->X2, -1.0, 1.0));    // X2 = A^-1 B A^-1 - R^-1 B R^-1
+    LA(gemv_n_launch(c->Wm, ld, n, n, bvec, 1.0, 0.0, c->v1, s));   // R^-1 b
+    LA(matdot_launch(Ainv, B, ld, n, c->scal + SC_TR_QB, c->red, s));
+    LA(matdot_launch(c->Wm, B, ld, n, c->scal + SC_TR_RB, c->red, s));
+    LA(dot_launch(c->alpha, bvec, n, c->scal + SC_A_B, s));
+    // R0 = Lambda_2 + K6 -> Wf = LR0, V = LR0^-1, G2 = R0^-1
+    CU(cudaMemcpyAsync(c->Wf, c->K6, sizeof(double) * mm, cudaMemcpyDeviceToDevice, s));
+    LA(vadd_inplace_launch(c->Wf, c->L2, (long)mm, s));
+    LA(chol_lower(c->Wf, ld, n, c->dinv, c->info + INFO_P, s, c->gws, c->gws_doubles, &c->la_main));
+    LA(trtri_lower(c->Wf, ld, n, c->dinv, c->V, c->tmp, s, c->gws, c->gws_doubles));
+    OK(gram_lower_t(c, c->V, c->G2));
+    LA(full_gemm(c->G2, c->K6, c->X1, 1.0, 0.0));   // R0^-1 A
+    LA(full_gemm(c->X1, c->G2, c->Wf, 1.0, 0.0));   // R0^-1 A R0^-1
+    LA(gemv_n_launch(c->G2, ld, n, n, c->lam1, 1.0, 0.0, c->v2, s));   // alpha0 = R0^-1 lambda_1
+    LA(gemv_n_launch(c->X1, ld, n, n, c->v2, 1.0, 0.0, c->v3, s));     // R0^-1 A alpha0
+    // dk/dr2 of Kuu into Wm (R^-1 is no longer needed; K itself goes to the scratch V)
+    LA(kuf_launch(c->kern_kind, c->kern_var, c->ZsT, n, c->z2, 0, M, n, c->Zs, c->z2, M, n, D, nullptr, c->V, n, nullptr, 0, 0, s, c->Wm));
+    LA(gamma_uu_white_launch(c->X2, c->Wf, c->G2, Ainv, c->v1, c->alpha, c->v2, c->v3, c->Wm, c->X1, c->V, ld, n, scale, s));   // X1 = Gamma, V = E_uu
+    LA(matdot_launch(c->X1, c->K, ld, n, c->scal + SC_G_K, c->red, s));
+    LA(xaug_launch(c->ZsT, n, 0, M, n, D, c->zaug, s, c->origin));
+    {   // F_uu = E_uu [zs | 1 | zs^2]
+        GemmP p;
+        p.A = c->V; p.lda = ld; p.a_kc = 1;
+        p.B = c->zaug; p.ldb = W; p.b_kc = 0;
+        p.C = c->fuu; p.ldc = W; p.m = n; p.n = W; p.k = n;
+        LA(mm_gemm(c, p, s));
+    }
+    Fuu.resize((size_t)n * W);
+    double tail[4], sc[N_SCAL];
+    int info_h[N_INFO];
+    CU(cudaMemcpyAsync(Fuu.data(), c->fuu, sizeof(double) * n * W, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(tail, c->stats[0] + mm + n, sizeof tail, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(sc, c->scal, sizeof sc, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(info_h, c->info, sizeof info_h, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    OK(check_info(c, info_h));
+    if (tail[1] != 0.0) FAIL(TSVGP_ERR_NONPOSITIVE_VARIANCE, "predict_f: non-positive predictive variance");
+    const double kl = 0.5 * (2.0 * (sc[SC_LOGDIAG_W] - sc[SC_PK0]) + sc[SC_TR_QK] - (double)n + sc[SC_M_ALPHA]);   // kl_white_from_scalars
+    *elbo = scale * tail[0] - kl;
+    *d_variance = (scale * (sc[SC_A_B] - 2.0 * (sc[SC_TR_QB] - sc[SC_TR_RB])) + sc[SC_G_K]) / c->kern_var + scale * tail[2];
+    *d_lik = scale * tail[3];
+    return TSVGP_OK;
+}
+
 // Lengthscale and Z gradients from F_uf = E_uf [xs | 1 | xs^2] (summed over the points) and F_uu (host, row stride waug):
 // d r2 / d lengthscale_d = -2 delta_d^2 / l_d, d r2 / d z_id = 2 delta_d / l_d with delta = zs - xs (scaled coordinates);
 // sums over points expanded through F:  sum_n E delta = zs S1 - EX ; sum E delta^2 = zs^2 S1 - 2 zs EX + C2
@@ -2456,7 +2560,8 @@ static int elbo_grad_one(tsvgp_ctx* c, int lat, double scale, const std::vector<
     select_latent(c, lat);
     std::vector<double> Fuf, Fuu;
     OK(read_fuf(c, Fuf));
-    OK(grad_epilogue(c, lat, scale, elbo, d_variance, d_lik, Fuu));
+    if (c->white) OK(grad_epilogue_white(c, lat, scale, elbo, d_variance, d_lik, Fuu));
+    else OK(grad_epilogue(c, lat, scale, elbo, d_variance, d_lik, Fuu));
     return f_to_grads(c, origin, Fuf, Fuu, dls, dZ);
 }
 
@@ -2483,7 +2588,6 @@ static int elbo_grad_coupled(tsvgp_ctx* c, double scale, const std::vector<doubl
 int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance, double* d_lengthscales, double* d_Z, double* d_lik) {
     if (!c || !elbo || !d_variance || !d_lengthscales || !d_Z || !d_lik) return TSVGP_ERR_INVALID;
     OK(require_model(c, true));
-    if (c->white) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not available for the whitened sibling model");
     if (c->lik.kind == LIK_HETEROSKEDASTIC) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for the heteroskedastic likelihood");
     if (c->sep) FAIL(TSVGP_ERR_INVALID, "elbo_grad is not built for separate kernels per latent");
     CU(cudaSetDevice(c->dev));
@@ -2494,6 +2598,7 @@ int tsvgp_elbo_grad(tsvgp_ctx* c, double scale, double* elbo, double* d_variance
     OK(ensure_xs(c));
     OK(ensure_posterior(c));
     OK(ensure_kl_terms(c));
+    if (c->white) OK(gram_lower_t(c, c->C6inv, c->P));   // A^-1 = LA^-T LA^-1, shared by every latent's epilogue (grad_epilogue_white)
     // common origin of the scaled coordinates: the centroid of the inducing inputs (see xaug_kernel)
     std::vector<double> origin(D, 0.0);
     {

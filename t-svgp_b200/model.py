@@ -578,8 +578,9 @@ class t_SVGP_white(t_SVGP):
     (`lambda_2 [1, M, M]`, default 1e-10 I), updated without any factorisation:
         lambda_1 <- (1-lr) lambda_1 + lr s K (G1 - 2 G2 mZ) ;  Lambda_2 <- (1-lr) Lambda_2 - 2 lr s K G2 K.
     Same constructor / natgrad_step / elbo / predict_f / prior_kl / get_mean_chol_cov_inducing_posterior surface
-    (+ `predict_f_extra_data`; any num_latent_gps with Gaussian / Bernoulli / StudentT; `elbo_and_grad` is not built for this
-    parameterisation)."""
+    (+ `predict_f_extra_data`; any num_latent_gps with Gaussian / Bernoulli / StudentT).  `elbo_and_grad` returns the M-step
+    objective and its hyperparameter gradients with lambda_1 and Lambda_2 held fixed, so `vem.fit` trains this model as it trains
+    `t_SVGP`."""
 
     def __init__(self, kernel, likelihood, inducing_variable, *, mean_function=None, num_latent_gps=1, lambda_1=None,
                  lambda_2=None, num_data=None, device=0):
@@ -605,9 +606,6 @@ class t_SVGP_white(t_SVGP):
     def assign_sites(self, lambda_1=None, lambda_2=None):
         """`lambda_1 [M, L]`, `lambda_2 [L, M, M]` (full symmetric matrices, tsvgp_white.py:79-89)."""
         super().assign_sites(lambda_1, lambda_2)
-
-    def elbo_and_grad(self, data=None, *, global_minibatch_size=None):
-        raise NotImplementedError("elbo_and_grad for t_SVGP_white")
 
     def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
         if full_cov:   # the reference's whitened conditional computes the diagonal only (tsvgp_white.py:122-132)
