@@ -64,7 +64,7 @@ TSVGP_API int tsvgp_set_option(tsvgp_ctx* ctx, const char* name, double value); 
 
 /* options: "chunk" (points per Kuf slab; 0 = automatic = 16384 points, i.e. Mp x 16384 x 8 B per slab stream — 268 MB at M = 2048,
  *          larger than the 126 MB L2: the slab is written once and re-read Mp/128 times through L2/HBM by compute-bound DMMA
- *          products, measured at ~4 % of the HBM roof), "streams" (1|2 ping-pong streams),
+ *          products, measured at ~4 % of the HBM roof), "streams" (1 to 4 ping-pong slab streams; default 2),
  * "cache_factors" (1 = keep chol(Kuu+jitter I) and the posterior factors while kernel, Z and sites are unchanged),
  * "invalidate" (any value: drop every cached factor now),
  * "route" (0 = automatic, 1 = fused: B = Kuf diag(h) Kfu then K9^-1 B K9^-1 — 2 M^2 flops per point, rounding ~ eps cond(Kuu)^2;
@@ -81,25 +81,18 @@ TSVGP_API int tsvgp_set_option(tsvgp_ctx* ctx, const char* name, double value); 
  *          pass (fused route forced or speculated) rank 0 builds the posterior factors, rank 1 the Kuu + jitter I chain, each
  *          broadcasts its result (ncclBroadcast) — every rank holds the same bits as without the split — and every rank but 0
  *          fills the wait with early slabs; pays off with row shares from tsvgp_b200.balance_weights, see DESIGN 5),
- * "streams" up to 4, "balance" / "fuse_b" (0 switches the balanced SYRK split / the fused b += Kuf g off, for A/B timing),
- * "spread_b" (1 = the fused b += Kuf g is shared by all tiles of a SYRK tile row, each adding into a private slot; 0 (default) =
- *          carried by the first tile column alone — measured equal or faster inside a step, see DESIGN 4),
  * "route_cond_max" (automatic: fused while the power-iteration estimate of cond(Kuu + jitter I) is below this; default 1e4),
  * "route_exact_min" (automatic: exact above this estimate, whitened in between; default 1e8),
- * "async_issue" (1 = at M <= 1024 a helper host thread enqueues the Kuu + jitter I factorisation chain on the side stream while
- *          the calling thread enqueues the posterior chain; 0 = one thread enqueues both),
  * "mc_seed" (Softmax: key of the Monte-Carlo generator; resets the draw counter),
  * "sample_seed" (tsvgp_predict_f_samples: key of its own generator; resets its own draw counter — never touches "mc_seed"'s),
  * "speculate" (1 = automatic route: when this context's last conditioning estimate chose the fused route, run the
  *          Kuu + jitter I chain UNDERNEATH the streaming pass instead of in front of it, read the probe after the pass and
  *          repeat the pass with the right route if the estimate crossed the threshold; 0 = always probe before the pass),
- * "k9_defer" (1 = from M = 2048 a Kuu + jitter I chain that is only needed after the pass starts behind the posterior chain
- *          instead of beside it; 0 = both chains start together, for A/B timing),
  * "early_slabs" (n = Gaussian likelihood, fused route: Kuf and the constant-weight SYRK of the first slab of up to n slab
  *          streams do not depend on the posterior and are enqueued before the posterior chain; 0 = off).
- * Environment (read once, A/B timing): TSVGP_PDL=0 plain stream order instead of programmatic dependent launch for the M x M
- * kernel chains; TSVGP_DIAG_VARIANT=0 the per-pivot diagonal-block Cholesky kernel, =2 the blocked kernel with look-ahead; TSVGP_GEMM_VARIANT=0 the CTA-barrier GEMM
- * pipeline; TSVGP_FUSED_SPLITK=1 the fused (last-CTA) split-K reduction; TSVGP_DEBUG_SYNC=1 synchronise after every launch. */
+ * Environment (read by tsvgp_create): TSVGP_PDL=0 plain stream order instead of programmatic dependent launch for
+ * the M x M kernel chains; TSVGP_DEBUG_SYNC=1 synchronise after every launch, so that a faulting kernel is reported at its call
+ * site. */
 
 /* ---- model objects read by the path (tsvgp.py:209,268-269; GPflow kernel / likelihood / inducing attributes) ------ */
 /* lengthscales: HOST pointer, n_ls = 1 (isotropic) or D (ARD).  One kernel shared by every latent (returns a context in

@@ -2,7 +2,6 @@
 #include "gemm.cuh"
 #include "kernels.cuh"
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace tsvgp {
 
@@ -71,9 +70,7 @@ __global__ void __launch_bounds__(256) strip_gemm_kernel(const double* __restric
         }
 }
 
-static int g_chol_strip = 1;   // TSVGP_CHOL_STRIP=0: the generic engine (split-K + reduction) for the panel / next-column products
 int dense_init() {
-    if (const char* v = getenv("TSVGP_CHOL_STRIP")) g_chol_strip = atoi(v);
     return (int)cudaFuncSetAttribute(strip_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SG_SMEM);
 }
 static int strip_gemm_launch(const double* A, long lda, const double* B, long ldb, double* C, long ldc, int rows, double alpha, double beta,
@@ -89,8 +86,7 @@ static int g_chol_outer = 512;   // outer panel width of the two-level blocking 
 //   diag(q) -> panel(q) = A[q+1:, q] L_qq^-T -> [wait: trailing(q-1) done] -> A[q+1:, q+1] -= panel(q) panel(q)[0]^T  -> diag(q+1) ...
 // and on aux->s2, once panel(q) exists:  A[q+2:, q+2:] -= panel(q)[1:] panel(q)[1:]^T  (lower tiles), hidden under diag(q+1).
 // The two streams always write disjoint block columns (q+1 on `s`, >= q+2 on s2); `s` joins s2 before it returns.
-static int chol_lower_lookahead(double* A, long ld, int n, double* dinv, int* info, cudaStream_t s, double* ws, size_t ws_doubles,
-                                const CholAux& aux) {
+static int chol_lower_lookahead(double* A, long ld, int n, double* dinv, int* info, cudaStream_t s, const CholAux& aux) {
 #define CUQ(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) return (int)e_; } while (0)
     bool f_pending = false;
     for (int q = 0; q < n; q += NB) {
@@ -100,16 +96,7 @@ static int chol_lower_lookahead(double* A, long ld, int n, double* dinv, int* in
         const int below = n - (q + NB);
         if (below <= 0) break;
         double* panel = A + (long)(q + NB) * ld + q;
-        if (g_chol_strip) {   // panel <- panel * L_qq^-T, 32-row strips
-            TRY(strip_gemm_launch(panel, ld, Dq, NB, panel, ld, below, 1.0, 0.0, 1, s));
-        } else {
-            GemmP p;
-            p.A = panel; p.lda = ld; p.a_kc = 1;
-            p.B = Dq; p.ldb = NB; p.b_kc = 1;
-            p.C = panel; p.ldc = ld;
-            p.m = below; p.n = NB; p.k = NB;
-            TRY(gemm_launch_auto(p, s, ws, ws_doubles));
-        }
+        TRY(strip_gemm_launch(panel, ld, Dq, NB, panel, ld, below, 1.0, 0.0, 1, s));   // panel <- panel * L_qq^-T, 32-row strips
         const int rest = below - NB;   // rows / columns from q + 2 blocks on
         if (rest > 0) {   // trailing update of the columns >= q+2 on the helper stream
             CUQ(cudaEventRecord(aux.e, s));
@@ -126,17 +113,7 @@ static int chol_lower_lookahead(double* A, long ld, int n, double* dinv, int* in
         }
         // block column q+1 on the critical stream; trailing(q-1), which also wrote this column, must be complete
         if (f_pending) CUQ(cudaStreamWaitEvent(s, aux.f, 0));
-        if (g_chol_strip) {
-            TRY(strip_gemm_launch(panel, ld, panel, ld, A + (long)(q + NB) * ld + (q + NB), ld, below, -1.0, 1.0, 0, s));
-        } else {
-            GemmP p;
-            p.A = panel; p.lda = ld; p.a_kc = 1;
-            p.B = panel; p.ldb = ld; p.b_kc = 1;
-            p.C = A + (long)(q + NB) * ld + (q + NB); p.ldc = ld;
-            p.m = below; p.n = NB; p.k = NB;
-            p.alpha = -1.0; p.beta = 1.0;
-            TRY(gemm_launch_auto(p, s, ws, ws_doubles));
-        }
+        TRY(strip_gemm_launch(panel, ld, panel, ld, A + (long)(q + NB) * ld + (q + NB), ld, below, -1.0, 1.0, 0, s));
         if (rest > 0) { CUQ(cudaEventRecord(aux.f, aux.s2)); f_pending = true; }
         else f_pending = false;
     }
@@ -146,10 +123,9 @@ static int chol_lower_lookahead(double* A, long ld, int n, double* dinv, int* in
 }
 
 int chol_lower(double* A, long ld, int n, double* dinv, int* info, cudaStream_t s, double* ws, size_t ws_doubles, const CholAux* aux) {
-    static const bool la_off = getenv("TSVGP_CHOL_LOOKAHEAD") && atoi(getenv("TSVGP_CHOL_LOOKAHEAD")) == 0;
     // measured (tools/diag_bench, profiles/diag_r02.txt): 1.12 -> 1.04 ms at n = 2048, 2.98 -> 2.90 ms at n = 4096; at n = 8192 the
     // single-level trailing updates (k = 128 per pass over the trailing matrix) lose to the two-level blocking below (12.4 vs 10.8 ms)
-    if (aux && aux->s2 && n >= 4 * NB && n <= 4096 && !la_off) return chol_lower_lookahead(A, ld, n, dinv, info, s, ws, ws_doubles, *aux);
+    if (aux && aux->s2 && n >= 4 * NB && n <= 4096) return chol_lower_lookahead(A, ld, n, dinv, info, s, *aux);
     const int OB = g_chol_outer;
     for (int P0 = 0; P0 < n; P0 += OB) {
         const int Pend = P0 + OB < n ? P0 + OB : n;

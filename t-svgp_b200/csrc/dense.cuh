@@ -19,8 +19,8 @@ struct CholAux { cudaStream_t s2 = nullptr; cudaEvent_t e = nullptr, f = nullptr
 int chol_lower(double* A, long ld, int n, double* dinv, int* info, cudaStream_t s, double* ws = nullptr, size_t ws_doubles = 0,
                const CholAux* aux = nullptr);
 
-// Linv = L^-1 for lower-triangular L.  dinv must hold the inverses of L's diagonal blocks (from chol_lower, or
-// diag_trtri_launch).  tmp: workspace [ceil(n/256)*128][ld].  Turns tf.linalg.triangular_solve / cholesky_solve
+// Linv = L^-1 for lower-triangular L.  dinv must hold the inverses of L's diagonal blocks (from chol_lower).
+// tmp: workspace [ceil(n/256)*128][ld].  Turns tf.linalg.triangular_solve / cholesky_solve
 // (reference tsvgp.py:271, util.py:386) into tensor-core products.
 int trtri_lower(const double* L, long ld, int n, const double* dinv, double* Linv, double* tmp, cudaStream_t s, double* ws = nullptr,
                 size_t ws_doubles = 0);

@@ -9,13 +9,12 @@
 #include <type_traits>
 #include <utility>
 #include <vector>
-#include <stdlib.h>
 
 namespace tsvgp {
 
 namespace {
 
-constexpr int BM = 128, BN = 128, BK = 16, STAGES = 4, NTHREADS = 256;
+constexpr int BM = 128, BN = 128, BK = 16, NTHREADS = 256;
 constexpr int KC_LD = BK + 4;    // [128][20] : rows 160 B apart -> the 4 rows of a half-warp fragment read hit distinct banks
 constexpr int MC_LD = BM + 4;    // [16][132]
 constexpr int KC_ELEMS = BM * KC_LD;
@@ -26,7 +25,6 @@ struct Smem {
     static constexpr int A_ELEMS = A_KC ? KC_ELEMS : MC_ELEMS;
     static constexpr int B_ELEMS = B_KC ? KC_ELEMS : MC_ELEMS;
     static constexpr int STAGE = A_ELEMS + B_ELEMS + (SCALE ? 2 * BK : 0);   // + per-k scale and mat-vec vectors
-    static constexpr int BYTES = STAGE * STAGES * 8;
 };
 
 template <bool KC>
@@ -52,7 +50,7 @@ __device__ __forceinline__ void load_tile(double* s, const double* __restrict__ 
 
 template <int EPI>
 __device__ __forceinline__ void gemm_epilogue(const GemmP& p, double (&acc)[8][4][2], double* smem, int ti, int tj, int bz, int ks,
-                                              int tid, int warp, int g, int t, int wm, int wn) {
+                                              int tid, int g, int t, int wm, int wn) {
     if (EPI == EPI_STORE || EPI == EPI_STORE_COLNORM) {
         const bool split = p.ksplit > 1;
         double* Cg = split ? p.part + (long)ks * p.part_stride + (long)bz * (p.part_sC ? p.part_sC : p.sC)
@@ -75,40 +73,6 @@ __device__ __forceinline__ void gemm_epilogue(const GemmP& p, double (&acc)[8][4
                     o.y += beta * old.y;
                 }
                 *ptr = o;
-            }
-        }
-        if (EPI == EPI_STORE && split && p.tile_ctr != nullptr) {
-            // Fused split-K reduction: the piece that arrives LAST at this tile's counter sums all partial tiles in the fixed order
-            // k = 0 .. ksplit-1 (deterministic) and writes C; no second kernel.  The counter resets itself for the next launch.
-            __shared__ int s_last;
-            __threadfence();
-            __syncthreads();
-            if (tid == 0) {
-                int* ctr = p.tile_ctr + ((long)bz * gridDim.y + ti) * gridDim.x + tj;
-                const int old = atomicAdd(ctr, 1);
-                s_last = old == p.ksplit - 1;
-                if (s_last) *ctr = 0;
-            }
-            __syncthreads();
-            if (s_last) {
-                __threadfence();
-                const double* part = p.part + (long)bz * (p.part_sC ? p.part_sC : p.sC);
-                double* C = p.C + (long)bz * p.sC;
-                for (int e = tid; e < BM * BN / 2; e += NTHREADS) {
-                    const int r = e / (BN / 2), c = (e % (BN / 2)) * 2;
-                    const long poff = (long)(ti * BM + r) * ldo + tj * BN + c;
-                    double2 sum = make_double2(0.0, 0.0);
-                    for (int k = 0; k < p.ksplit; ++k) {
-                        const double2 v = __ldcg(reinterpret_cast<const double2*>(part + (long)k * p.part_stride + poff));
-                        sum.x += v.x; sum.y += v.y;
-                    }
-                    double2* ptr = reinterpret_cast<double2*>(C + (long)(ti * BM + r) * p.ldc + tj * BN + c);
-                    if (p.beta != 0.0) {
-                        const double2 old = *ptr;
-                        sum.x += p.beta * old.x; sum.y += p.beta * old.y;
-                    }
-                    *ptr = sum;
-                }
             }
         }
     }
@@ -145,121 +109,15 @@ __device__ __forceinline__ void gemm_epilogue(const GemmP& p, double (&acc)[8][4
     }
 }
 
-template <bool A_KC, bool B_KC, bool SCALE, int EPI>
-__global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel(GemmP p) {
-    PDL_PROLOGUE();   // no-op unless launched with the programmatic-serialisation attribute (GemmP::pdl)
-    using S = Smem<A_KC, B_KC, SCALE>;
-    extern __shared__ __align__(16) double smem[];
-
-    const int tj = blockIdx.x, ti = blockIdx.y;
-    if (p.lower_out && tj > ti) return;
-    if (p.row_mod > 1 && ti % p.row_mod != p.row_rem) return;
-    const int zdiv = p.C2 != nullptr ? 2 : p.ksplit;
-    const int bz = blockIdx.z / zdiv, ks = blockIdx.z % zdiv;
-    const double* Ag = p.A + (long)bz * p.sA;
-    const double* Bg = p.B + (long)bz * p.sB;
-
-    int kb = 0, ke = p.k;
-    if (p.a_tri == 1) ke = min(ke, (ti + 1) * BM);
-    if (p.a_tri == 2) kb = max(kb, ti * BM);
-    if (p.b_tri == 1) ke = min(ke, (tj + 1) * BN);
-    if (p.b_tri == 2) kb = max(kb, tj * BN);
-    if (p.ksplit > 1) {
-        int nkt = max(ke - kb, 0) / BK;
-        int per = (nkt + p.ksplit - 1) / p.ksplit;
-        kb += ks * per * BK;
-        ke = min(ke, kb + per * BK);
-    }
-    const bool piece2 = p.C2 != nullptr && ks == 1;
-    if (p.C2 != nullptr) { if (piece2) kb = max(kb, p.ksp); else ke = min(ke, p.ksp); }
-    const int KT = max(ke - kb, 0) / BK;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    const int wm = (warp & 1) * 64, wn = (warp >> 1) * 32;
-
-    double acc[8][4][2];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
-    const bool matvec = SCALE && p.gvec != nullptr && tj == 0 && wn == 0;   // the two warps of the first tile column that cover all 128 rows
-    double bacc[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) bacc[i] = 0.0;
-
-    auto issue = [&](int kt) {
-        if (kt < KT) {
-            double* sa = smem + (kt % STAGES) * S::STAGE;
-            double* sb = sa + S::A_ELEMS;
-            const int k0 = kb + kt * BK;
-            load_tile<A_KC>(sa, Ag, p.lda, ti * BM, k0, tid);
-            load_tile<B_KC>(sb, Bg, p.ldb, tj * BN, k0, tid);
-            if (SCALE && tid < BK / 2) cp_async16(sb + S::B_ELEMS + tid * 2, p.kscale + k0 + tid * 2);
-            if (SCALE && tid >= 32 && tid < 32 + BK / 2 && p.gvec) cp_async16(sb + S::B_ELEMS + BK + (tid - 32) * 2, p.gvec + k0 + (tid - 32) * 2);
-        }
-        cp_async_commit();
-    };
-
-#pragma unroll
-    for (int s = 0; s < STAGES - 1; ++s) issue(s);
-
-    for (int kt = 0; kt < KT; ++kt) {
-        cp_async_wait<STAGES - 2>();
-        __syncthreads();
-        issue(kt + STAGES - 1);
-        const double* sa = smem + (kt % STAGES) * S::STAGE;
-        const double* sb = sa + S::A_ELEMS;
-        const double* ssc = sb + S::B_ELEMS;
-#pragma unroll
-        for (int kk = 0; kk < BK; kk += 4) {
-            double a[8], b[4];
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-                a[i] = A_KC ? sa[(wm + 8 * i + g) * KC_LD + kk + t] : sa[(kk + t) * MC_LD + wm + 8 * i + g];
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-                b[j] = B_KC ? sb[(wn + 8 * j + g) * KC_LD + kk + t] : sb[(kk + t) * MC_LD + wn + 8 * j + g];
-            if (SCALE) {
-                const double h = ssc[kk + t];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) b[j] *= h;
-                if (matvec) {
-                    const double gk = ssc[BK + kk + t];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) bacc[i] = fma(a[i], gk, bacc[i]);
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) dmma884(acc[i][j][0], acc[i][j][1], a[i], b[j]);
-        }
-    }
-    cp_async_wait<0>();
-    __syncthreads();   // every global read of this CTA is complete: C may alias A (in-place panel solves)
-
-    if (SCALE && matvec) {   // rows wm + 8 i + g : sum the 4 lanes that split k, then one lane adds into the (CTA-private) rows of b
-        double* bo = (p.C2 != nullptr && ks == 1) ? p.bout2 : p.bout;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            double v = bacc[i];
-            v += __shfl_xor_sync(0xffffffffu, v, 1);
-            v += __shfl_xor_sync(0xffffffffu, v, 2);
-            if (t == 0) bo[ti * BM + wm + 8 * i + g] += v;
-        }
-    }
-    gemm_epilogue<EPI>(p, acc, smem, ti, tj, bz, ks, tid, warp, g, t, wm, wn);
-}
-
-// ---- decoupled pipeline ---------------------------------------------------------------------------------------------
-// Same tiling, but stage hand-over goes through mbarriers instead of a CTA-wide barrier per k-tile: every thread's
-// cp.async group arrives on full[stage] when it lands; a warp that has consumed a stage arrives on empty[stage]; a stage is
-// refilled two tiles after it was consumed, so warps may drift up to two k-tiles apart and the DMMA pipe of an SM
-// sub-partition is not drained at every tile boundary (ncu r01: 84 % DMMA-pipe active with the barrier version).
+// ---- mainloop ---------------------------------------------------------------------------------------------------------
+// Stage hand-over goes through mbarriers instead of a CTA-wide barrier per k-tile: every thread's cp.async group arrives on
+// full[stage] when it lands; a warp that has consumed a stage arrives on empty[stage]; a stage is refilled two tiles after it was
+// consumed, so warps may drift up to two k-tiles apart and the DMMA pipe of an SM sub-partition is not drained at every tile
+// boundary (ncu r01: 84 % DMMA-pipe active with a CTA barrier per k-tile).
 constexpr int PSTAGES = 5;
 
 template <bool A_KC, bool B_KC, bool SCALE, int EPI>
-__global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
+__global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p, int order) {
     PDL_PROLOGUE();   // no-op unless launched with the programmatic-serialisation attribute (GemmP::pdl)
     using S = Smem<A_KC, B_KC, SCALE>;
     extern __shared__ __align__(16) double smem[];
@@ -268,10 +126,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
 
     // Launch order = longest tiles first.  CTAs are dispatched in linear block order (x fastest); with a triangular operand the
     // contraction length of a tile depends on its row or column, and the default order (tile rows ascending) can put the longest
-    // tiles LAST.  p.order: bit 0 = the tile COLUMN is the slow index, bit 1 = the slow index runs backwards (host: tile_order()).
+    // tiles LAST.  order: bit 0 = the tile COLUMN is the slow index, bit 1 = the slow index runs backwards (host: tile_order()).
     int tj = blockIdx.x, ti = blockIdx.y;
-    if (p.order & 1) { const int lin = blockIdx.y * gridDim.x + blockIdx.x; tj = lin / (int)gridDim.y; ti = lin % (int)gridDim.y; }
-    if (p.order & 2) { if (p.order & 1) tj = (int)gridDim.x - 1 - tj; else ti = (int)gridDim.y - 1 - ti; }
+    if (order & 1) { const int lin = blockIdx.y * gridDim.x + blockIdx.x; tj = lin / (int)gridDim.y; ti = lin % (int)gridDim.y; }
+    if (order & 2) { if (order & 1) tj = (int)gridDim.x - 1 - tj; else ti = (int)gridDim.y - 1 - ti; }
     if (p.lower_out && tj > ti) return;
     if (p.row_mod > 1 && ti % p.row_mod != p.row_rem) return;
     const int zdiv = p.C2 != nullptr ? 2 : p.ksplit;
@@ -322,13 +180,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
     for (int i = 0; i < 8; ++i)
 #pragma unroll
         for (int j = 0; j < 4; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
-    // Fused mat-vec b += A g: the two warps with wn == 0 cover all 128 rows of the tile.  With bstride == 0 only the first tile column
-    // carries it (round 1) — its 16 tiles then run 3 % longer than the rest and set the makespan of the launch.  With bstride > 0
-    // [r02] the tiles (ti, 0..ti) of a tile row share the work: tile (ti, tj) handles the k-tiles [KT tj/(ti+1), KT (tj+1)/(ti+1)) of
-    // its piece and adds into its PRIVATE slot bout[tj * bstride + row] (no atomics; the host sums the slots at the end of the pass).
-    const bool matvec = SCALE && p.gvec != nullptr && wn == 0 && (tj == 0 || p.bstride > 0);
-    int mv_lo = 0, mv_hi = KT;
-    if (matvec && p.bstride > 0) { mv_lo = (int)((long)KT * tj / (ti + 1)); mv_hi = (int)((long)KT * (tj + 1) / (ti + 1)); }
+    // Fused mat-vec b += A g, carried by the first tile column: its two warps with wn == 0 cover all 128 rows of the tile.
+    const bool matvec = SCALE && p.gvec != nullptr && wn == 0 && tj == 0;
     const bool use_scale = SCALE && p.kscale != nullptr;
     double bacc[8];
 #pragma unroll
@@ -404,7 +257,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
         using Yes = std::true_type;
         using No = std::false_type;
         if (SCALE) {   // statistics products: optional per-k weights (absent when the weights are one constant, Gaussian likelihood)
-            if (matvec && kt >= mv_lo && kt < mv_hi) {   // the two warps per row block that also carry b += A g, on their share of k
+            if (matvec) {   // the two warps of the first tile column that also carry b += A g
                 if (use_scale) { if (dj_pat == 1) k_tile(I8{}, J0{}, Yes{}, Yes{}); else k_tile(I8{}, FULLJ{}, Yes{}, Yes{}); }
                 else { if (dj_pat == 1) k_tile(I8{}, J0{}, Yes{}, No{}); else k_tile(I8{}, FULLJ{}, Yes{}, No{}); }
             } else if (use_scale) {
@@ -432,7 +285,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
     __syncthreads();   // every global read of this CTA has landed and every warp is out of the pipeline buffers
 
     if (SCALE && matvec) {   // rows wm + 8 i + g : sum the 4 lanes that split k, then one lane adds into the (CTA-private) rows of b
-        double* bo = ((p.C2 != nullptr && ks == 1) ? p.bout2 : p.bout) + (long)tj * p.bstride;
+        double* bo = (p.C2 != nullptr && ks == 1) ? p.bout2 : p.bout;
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             double v = bacc[i];
@@ -441,7 +294,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) gemm_kernel_mb(GemmP p) {
             if (t == 0) bo[ti * BM + wm + 8 * i + g] += v;
         }
     }
-    gemm_epilogue<EPI>(p, acc, smem, ti, tj, bz, ks, tid, warp, g, t, wm, wn);
+    gemm_epilogue<EPI>(p, acc, smem, ti, tj, bz, ks, tid, g, t, wm, wn);
 }
 
 constexpr int RED_SLICES = 8;   // row slices per 128 x 128 tile: the reduction is bandwidth work, spread it over 8x the CTAs
@@ -474,9 +327,8 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(GemmP p) {
     }
 }
 
-int g_variant = 1;   // 1 = mbarrier-decoupled pipeline (default), 0 = CTA-barrier pipeline (TSVGP_GEMM_VARIANT=0, for A/B timing)
-// warp -> (row half, column quarter) of the 128 x 128 CTA tile, one nibble per warp (warp 0 in the low nibble).
-// Default: wm = (w & 1) * 64, wn = (w >> 1) * 32.  TSVGP_WMAP / TSVGP_WMAP_DIAG (hex) override them for A/B timing (tools/gemm_bench).
+// warp -> (row half, column quarter) of the 128 x 128 CTA tile, one nibble per warp (warp 0 in the low nibble), used where
+// GemmP::wmap / wmap_diag are 0 (tools/gemm_bench sets them to compare maps).
 // Measured on B200 (tools/gemm_bench, profiles/gemm_bench_r02.txt):
 //  * general tiles: any map whose sub-partition partners (warps w, w + 4) sit in the SAME row half is fastest for the triangular
 //    variance product (1.056 ms per 8192-point slab at M = 2048); partners in different row halves cost 5 % (1.107 - 1.111 ms):
@@ -486,10 +338,8 @@ int g_variant = 1;   // 1 = mbarrier-decoupled pipeline (default), 0 = CTA-barri
 //    (64,64)+(0,32) — 32 / 32 / 36 / 36 per pipe — brings a diagonal tile to 0.78 x a full tile.
 unsigned g_wmap = 0x73625140u, g_wmap_diag = 0x17326054u;
 
-int g_tile_order = 1;   // TSVGP_TILE_ORDER=0: default launch order everywhere (A/B timing)
 // longest contraction first (see gemm_kernel_mb): which tile index bounds the k range, and in which direction it shrinks
 static int tile_order(const GemmP& p) {
-    if (p.tile_ctr) return 0;                               // the fused split-K reduction indexes its counters by grid position
     if (p.a_tri && p.b_tri) return 0;                       // k range depends on both indices: keep the default
     if (p.a_tri == 2) return 0;                             // k >= ti * 128: row 0 is longest and already first
     if (p.a_tri == 1) return 2;                             // k <  (ti + 1) * 128: last row longest -> rows backwards
@@ -504,35 +354,22 @@ constexpr int mb_bytes() { return Smem<A_KC, B_KC, SCALE>::STAGE * PSTAGES * 8 +
 template <bool A_KC, bool B_KC, bool SCALE, int EPI>
 int launch_inst(const GemmP& p, cudaStream_t stream) {
     dim3 grid(p.n / BN, p.m / BM, p.batch * (p.C2 ? 2 : p.ksplit));
-    if (g_variant != 1 && SCALE && !p.kscale) return -1;
-    if (g_variant == 1) {
-        GemmP q = p;
-        if (!q.wmap) q.wmap = g_wmap;
-        if (!q.wmap_diag) q.wmap_diag = g_wmap_diag;
-        if (q.order < 0) q.order = g_tile_order ? tile_order(q) : 0;
-        launch_k(p.pdl != 0, gemm_kernel_mb<A_KC, B_KC, SCALE, EPI>, grid, NTHREADS, mb_bytes<A_KC, B_KC, SCALE>(), stream, q);
-    }
-    else
-        launch_k(p.pdl != 0, gemm_kernel<A_KC, B_KC, SCALE, EPI>, grid, NTHREADS, Smem<A_KC, B_KC, SCALE>::BYTES, stream, p);
+    GemmP q = p;
+    if (!q.wmap) q.wmap = g_wmap;
+    if (!q.wmap_diag) q.wmap_diag = g_wmap_diag;
+    launch_k(p.pdl != 0, gemm_kernel_mb<A_KC, B_KC, SCALE, EPI>, grid, NTHREADS, mb_bytes<A_KC, B_KC, SCALE>(), stream, q, tile_order(q));
     return count_launch();
 }
 
 template <bool A_KC, bool B_KC, bool SCALE, int EPI>
 int init_inst() {
-    int e = (int)cudaFuncSetAttribute(gemm_kernel<A_KC, B_KC, SCALE, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      Smem<A_KC, B_KC, SCALE>::BYTES);
-    e |= (int)cudaFuncSetAttribute(gemm_kernel_mb<A_KC, B_KC, SCALE, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   mb_bytes<A_KC, B_KC, SCALE>());
-    return e;
+    return (int)cudaFuncSetAttribute(gemm_kernel_mb<A_KC, B_KC, SCALE, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     mb_bytes<A_KC, B_KC, SCALE>());
 }
 
 }  // namespace
 
 int gemm_init() {
-    if (const char* v = getenv("TSVGP_GEMM_VARIANT")) g_variant = atoi(v);
-    if (const char* v = getenv("TSVGP_TILE_ORDER")) g_tile_order = atoi(v);
-    if (const char* v = getenv("TSVGP_WMAP")) g_wmap = (unsigned)strtoul(v, nullptr, 16);
-    if (const char* v = getenv("TSVGP_WMAP_DIAG")) g_wmap_diag = (unsigned)strtoul(v, nullptr, 16);
     int e = 0;
     e |= init_inst<true, true, false, EPI_STORE>();
     e |= init_inst<true, true, true, EPI_STORE>();
@@ -658,20 +495,10 @@ int gemm_launch_auto(GemmP p, cudaStream_t stream, double* ws, size_t ws_doubles
         long ks = tiles > 0 ? sms / tiles : 1;
         if (ks > kt / 2) ks = kt / 2;                       // at least two k-tiles per piece
         const size_t slab = (size_t)p.batch * p.m * p.n;    // compact partial image of C
-        // the last GEMM_WS_COUNTER_DOUBLES doubles of the workspace are the self-resetting tile counters of the fused reduction
-        const size_t ws_part = ws_doubles > GEMM_WS_COUNTER_DOUBLES ? ws_doubles - GEMM_WS_COUNTER_DOUBLES : 0;
-        if (slab > 0 && ks > (long)(ws_part / slab)) ks = (long)(ws_part / slab);
+        if (slab > 0 && ks > (long)(ws_doubles / slab)) ks = (long)(ws_doubles / slab);
         if (ks > 16) ks = 16;
         if (ks >= 2) {
             p.ksplit = (int)ks; p.part = ws; p.part_stride = (long)slab; p.part_ld = p.n; p.part_sC = (long)p.m * p.n;
-            const long grid_tiles = (long)p.batch * nti * ntj;
-            // Measured slower than the separate 8x-parallel reduction kernel (one SM pulls ksplit x 128 KB of partials through its own
-            // L2 port: chol_lower(2048) 1.19 -> 1.69 ms, cfg2 1.39 -> 1.64 ms), so it is off unless TSVGP_FUSED_SPLITK=1 (A/B timing).
-            static const bool fused = getenv("TSVGP_FUSED_SPLITK") && atoi(getenv("TSVGP_FUSED_SPLITK")) != 0;
-            if (fused && grid_tiles <= (long)GEMM_WS_COUNTER_DOUBLES * 2) {   // one int counter per (batch, ti, tj)
-                p.tile_ctr = reinterpret_cast<int*>(ws + ws_part);
-                return gemm_launch(p, stream);
-            }
             int e = gemm_launch(p, stream);
             if (e) return e;
             return splitk_reduce_launch(p, stream);

@@ -1,4 +1,4 @@
-// FP64 DMMA GEMM engine: one tiled mainloop (128x128 CTA tile, 8 warps of 64x32, BK=16, 4-stage cp.async pipeline)
+// FP64 DMMA GEMM engine: one tiled mainloop (128x128 CTA tile, 8 warps of 64x32, BK=16, 5-stage cp.async pipeline)
 // reused by the streaming statistics pass (weighted SYRK, triangular variance product) and by every dense M x M
 // operation of the natural-gradient step (reference math: src/models/tsvgp.py:234-304, src/util.py:349-391).
 //
@@ -28,11 +28,9 @@ struct GemmP {
     // with kscale: optional fused mat-vec  bout[i] += sum_k A(i,k) gvec[k]  (b += Kuf g of the statistics pass), computed from the A
     // fragments the first tile column already holds in registers; the split-off k piece (C2) accumulates into bout2
     const double* gvec = nullptr; double* bout = nullptr; double* bout2 = nullptr;
-    long bstride = 0;   // > 0: the mat-vec is shared by the tiles of a tile row, tile column tj adds into bout[tj * bstride + row]
     int epilogue = EPI_STORE;
     double* norm_out = nullptr; long ldn = 0;   // EPI_COLNORM: norm_out[tile_i * ldn + j] = sum_{i in tile} C(i,j)^2
     int ksplit = 1; double* part = nullptr; long part_stride = 0;   // split-K partial slabs [ksplit][m*ldc]; caller reduces
-    int* tile_ctr = nullptr;          // split-K with a fused reduction: zero-initialised counters, one per (batch, tile_i, tile_j) of the grid
     long part_ld = 0, part_sC = 0;    // row / batch strides of the partial slabs when they are stored more compactly than C (0 = ldc / sC)
     int batch = 1; long sA = 0, sB = 0, sC = 0;
     // Two-piece k split for load balance (no atomics): CTAs with blockIdx.z == 0 contract k in [0, ksp) into C, CTAs with
@@ -45,7 +43,6 @@ struct GemmP {
     int pdl = 0;   // launch with the programmatic-serialisation attribute (the kernels always run the PDL prologue)
     // warp -> sub-tile maps (one nibble per warp; 0 = the library default, see gemm.cu): general tiles / diagonal tiles of a symmetric product
     unsigned wmap = 0, wmap_diag = 0;
-    int order = -1;   // tile launch order (see gemm.cu::tile_order); -1 = chosen by the library
 };
 
 // Launch on `stream`. Returns cudaError_t as int (0 = ok), -1 for an unsupported combination.
@@ -57,9 +54,8 @@ int splitk_reduce_launch(const GemmP& p, cudaStream_t stream);
 // gemm_launch that splits the contraction over otherwise idle SMs when the product has few output tiles (the latency-bound
 // M x M phases at small M, Cholesky panels, triangular-inverse nodes): partial tiles go to `ws` (ws_doubles doubles, owned by
 // the caller, one per stream) and are summed by splitk_reduce_launch.  Falls back to the plain launch when nothing is gained.
-// The last GEMM_WS_COUNTER_DOUBLES doubles of `ws` hold the tile counters of the fused reduction (the piece that finishes a tile
-// last sums the partials — no second kernel): the owner must zero them ONCE (cudaMemset) after allocating the workspace.
-constexpr size_t GEMM_WS_COUNTER_DOUBLES = 2048;
+// The piece count is capped by ws_doubles / (batch m n): the workspace size decides how some products are split, and with it
+// the order in which their partials are summed.
 int gemm_launch_auto(GemmP p, cudaStream_t stream, double* ws, size_t ws_doubles);
 
 // k split point for `tiles` equal output tiles of contraction length k on this device's SMs (multiple of 16; k = no split)

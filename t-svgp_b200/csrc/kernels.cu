@@ -2,7 +2,6 @@
 #include "kernels.cuh"
 #include "common.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace tsvgp {
 
@@ -773,270 +772,21 @@ int gemv_t_launch(const double* A, long lda, int m, int n, const double* x, doub
 // Diagonal 128x128 blocks: Cholesky (tf.linalg.cholesky at reference tsvgp.py:270,300 and util.py:377,382,388)
 // and triangular inverse (used to turn tf.linalg.triangular_solve / cholesky_solve into tensor-core products).
 // =====================================================================================================================
-constexpr int DB = 128, DB_LD = 129;
-
-// X = L^-1 for the lower-triangular 128x128 L in shared memory S (row-major, ld 129), written to Dinv (ld 128, dense, zeros
-// above the diagonal).  Same register tiling as the Cholesky below: thread (ti, tj) of a 16x16 grid owns X[16 ii + ti][16 jj + tj].
-// Right-looking elimination of L X = I: per pivot k the owners of row k scale it by 1 / L[k][k], publish it through a
-// double-buffered shared row (ONE barrier per pivot), and every thread updates its rows i > k with FMAs only
-// (X[i][c] -= L[i][k] X[k][c], c <= k).  The row-by-row dot-product form this replaces was latency-bound (160 us / block).
-__device__ void tri_inverse_regs(const double* S, double* Dinv) {
-    __shared__ double xrow[2][DB];
-    __shared__ double dinv[DB];
-    const int tid = threadIdx.x, ti = tid & 15, tj = tid >> 4;
-    if (tid < DB) dinv[tid] = 1.0 / S[tid * DB_LD + tid];
-    double x[8][8];
-#pragma unroll
-    for (int ii = 0; ii < 8; ++ii)
-#pragma unroll
-        for (int jj = 0; jj < 8; ++jj) x[ii][jj] = (16 * ii + ti == 16 * jj + tj) ? 1.0 : 0.0;
-    __syncthreads();
-    if (ti == 0) {   // publish row 0 : X[0][0] = 1 / L[0][0]
-        x[0][0] *= dinv[0];
-        if (tj == 0) xrow[0][0] = x[0][0];
-    }
-#pragma unroll
-    for (int kb = 0; kb < 8; ++kb) {
-        for (int kk = 0; kk < 16; ++kk) {
-            const int k = kb * 16 + kk, buf = k & 1;
-            __syncthreads();
-            double l[8];
-#pragma unroll
-            for (int ii = kb; ii < 8; ++ii) {
-                const int i = 16 * ii + ti;
-                l[ii] = i > k ? S[i * DB_LD + k] : 0.0;
-            }
-#pragma unroll
-            for (int jj = 0; jj <= kb; ++jj) {
-                const int c = 16 * jj + tj;
-                const double xk = c <= k ? xrow[buf][c] : 0.0;
-#pragma unroll
-                for (int ii = kb; ii < 8; ++ii) x[ii][jj] = fma(-l[ii], xk, x[ii][jj]);
-            }
-            // finish and publish row k + 1 (owners: row residue (kk + 1) % 16 in block kb, or residue 0 in block kb + 1)
-            if (k + 1 < DB) {
-                const int nb = buf ^ 1;
-                const double dk = dinv[k + 1];
-                if (kk < 15) {
-                    if (ti == kk + 1) {
-#pragma unroll
-                        for (int jj = 0; jj <= kb; ++jj) {
-                            x[kb][jj] *= dk;
-                            xrow[nb][16 * jj + tj] = x[kb][jj];
-                        }
-                    }
-                } else if (kb < 7) {
-                    constexpr int KN = 7;
-                    if (ti == 0) {
-#pragma unroll
-                        for (int jj = 0; jj <= (kb + 1 < 8 ? kb + 1 : KN); ++jj) {
-                            x[kb + 1 < 8 ? kb + 1 : KN][jj] *= dk;
-                            xrow[nb][16 * jj + tj] = x[kb + 1 < 8 ? kb + 1 : KN][jj];
-                        }
-                    }
-                }
-            }
-        }
-    }
-#pragma unroll
-    for (int ii = 0; ii < 8; ++ii)
-#pragma unroll
-        for (int jj = 0; jj < 8; ++jj) {
-            const int i = 16 * ii + ti, c = 16 * jj + tj;
-            Dinv[i * DB + c] = c <= i ? x[ii][jj] : 0.0;
-        }
-}
-
-// Cholesky A = L L^T of one 128x128 block AND X = L^-1, fused, with both matrices in REGISTERS: thread (ti, tj) of a 16x16
-// grid owns A[16 ii + ti][16 jj + tj] and X[16 ii + ti][16 jj + tj] for jj <= ii.  One barrier per pivot k:
-//   * the 16 owners of column k + 1 (one half-warp) take the pivot's 1/sqrt by shuffle and publish the SCALED column, so no
-//     other thread multiplies or masks anything: everyone just loads l_i, l_j and issues FMAs;
-//   * the right-looking elimination of L X = I rides on the same loads one pivot behind: X[i][:] -= L[i][k-1] X[k-1][:].
-// (r01: separate barrier-per-pivot Cholesky 55 us + inverse 47 us per block, both issue-bound on redundant scaling.)
-__global__ void __launch_bounds__(256) diag_potrf_inv_kernel(double* A, long lda, double* Dinv, int blk, int* info) {
-    extern __shared__ double S[];   // [128][129] : staging of L for the coalesced write-back
-    __shared__ double col[2][DB];   // scaled column k of L (zeros for rows <= k)
-    __shared__ double xrow[2][DB];  // finished row k of X
-    __shared__ double rsq[2];
-    __shared__ int sfail;
-    const int tid = threadIdx.x, ti = tid & 15, tj = tid >> 4, lane = tid & 31;
-    double a[8][8], x[8][8];
-#pragma unroll
-    for (int ii = 0; ii < 8; ++ii)
-#pragma unroll
-        for (int jj = 0; jj <= ii; ++jj) {
-            const int r = 16 * ii + ti, c = 16 * jj + tj;
-            a[ii][jj] = c <= r ? A[(long)r * lda + c] : 0.0;
-            x[ii][jj] = r == c ? 1.0 : 0.0;
-        }
-    for (int e = tid; e < DB * DB_LD; e += 256) S[e] = 0.0;
-    if (tid == 0) sfail = 0;
-    __syncthreads();
-    const double piv0 = __shfl_sync(0xffffffffu, a[0][0], lane & 16);
-    if (tj == 0) {   // publish the scaled column 0
-        const double piv = piv0;
-        const double rs = rsqrt(piv);
-        if (ti == 0) {
-            rsq[0] = rs;
-            if (!(piv > 0.0)) sfail = 1;
-            S[0] = piv * rs;
-        }
-#pragma unroll
-        for (int ii = 0; ii < 8; ++ii) {
-            const int r = 16 * ii + ti;
-            const double l = r > 0 ? a[ii][0] * rs : 0.0;
-            col[0][r] = l;
-            if (r > 0) S[r * DB_LD] = l;
-        }
-    }
-    double lprev[8];
-#pragma unroll
-    for (int ii = 0; ii < 8; ++ii) lprev[ii] = 0.0;
-    int failed = 0;
-#pragma unroll
-    for (int kb = 0; kb < 8; ++kb) {
-        for (int kk = 0; kk < 16; ++kk) {
-            const int k = kb * 16 + kk, buf = k & 1, nb = buf ^ 1;
-            __syncthreads();
-            if (sfail) { failed = sfail; goto finish; }   // uniform
-            double li[8];
-#pragma unroll
-            for (int ii = kb; ii < 8; ++ii) li[ii] = col[buf][16 * ii + ti];
-            // (1) inverse, one pivot behind: X[i][c] -= L[i][k-1] X[k-1][c]   (lprev is zero for rows <= k-1)
-            if (k > 0) {
-#pragma unroll
-                for (int jj = 0; jj <= kb; ++jj) {
-                    const int c = 16 * jj + tj;
-                    const double xr = c < k ? xrow[nb][c] : 0.0;
-#pragma unroll
-                    for (int ii = kb; ii < 8; ++ii) x[ii][jj] = fma(-lprev[ii], xr, x[ii][jj]);
-                }
-            }
-            // (2) row k of X is complete: scale by 1 / L[k][k] and publish
-            if (ti == kk) {
-                const double rs = rsq[buf];
-#pragma unroll
-                for (int jj = 0; jj <= kb; ++jj) {
-                    const int c = 16 * jj + tj;
-                    if (c <= k) {
-                        x[kb][jj] *= rs;
-                        xrow[buf][c] = x[kb][jj];
-                    }
-                }
-            }
-            // (3) Cholesky update with the scaled column k; the owners of column k + 1 go first and publish it
-            if (kk < 15) {
-                const bool own = tj == kk + 1;
-                if (own) {
-#pragma unroll
-                    for (int ii = kb; ii < 8; ++ii) a[ii][kb] = fma(-li[ii], col[buf][16 * kb + tj], a[ii][kb]);
-                }
-                // full-warp shuffle (a run-time half-warp mask costs a MATCH.ANY / BRA.DIV slow path per pivot): every
-                // half-warp reads its lane with ti == kk + 1; only the owners' half-warp uses the value
-                const double piv = __shfl_sync(0xffffffffu, a[kb][kb], (lane & 16) | (kk + 1));
-                if (own) {
-                    const double rs = rsqrt(piv);
-                    if (ti == tj) {
-                        rsq[nb] = rs;
-                        if (!(piv > 0.0)) sfail = k + 2;
-                        S[(k + 1) * DB_LD + k + 1] = piv * rs;
-                    }
-#pragma unroll
-                    for (int ii = kb; ii < 8; ++ii) {
-                        const int r = 16 * ii + ti;
-                        const double l = r > k + 1 ? a[ii][kb] * rs : 0.0;
-                        col[nb][r] = l;
-                        if (r > k + 1) S[r * DB_LD + k + 1] = l;
-                    }
-                }
-            } else if (kb < 7) {
-                constexpr int KN = 7;
-                const int jn = kb + 1 < 8 ? kb + 1 : KN;   // (static) block of column k + 1
-                const bool own = tj == 0;
-                if (own) {
-#pragma unroll
-                    for (int ii = jn; ii < 8; ++ii) a[ii][jn] = fma(-li[ii], col[buf][16 * jn], a[ii][jn]);
-                }
-                const double piv = __shfl_sync(0xffffffffu, a[jn][jn], lane & 16);         // the lane with ti == 0
-                if (own) {
-                    const double rs = rsqrt(piv);
-                    if (ti == 0) {
-                        rsq[nb] = rs;
-                        if (!(piv > 0.0)) sfail = k + 2;
-                        S[(k + 1) * DB_LD + k + 1] = piv * rs;
-                    }
-#pragma unroll
-                    for (int ii = jn; ii < 8; ++ii) {
-                        const int r = 16 * ii + ti;
-                        const double l = r > k + 1 ? a[ii][jn] * rs : 0.0;
-                        col[nb][r] = l;
-                        if (r > k + 1) S[r * DB_LD + k + 1] = l;
-                    }
-                }
-            }
-#pragma unroll
-            for (int jj = kb; jj < 8; ++jj) {
-                // the column published above was already updated by its owners: skip it there
-                const bool mine = kk < 15 ? (jj == kb && tj == kk + 1) : (jj == kb + 1 && tj == 0);
-                if (mine) continue;
-                const double lj = col[buf][16 * jj + tj];
-#pragma unroll
-                for (int ii = jj; ii < 8; ++ii) a[ii][jj] = fma(-li[ii], lj, a[ii][jj]);
-            }
-#pragma unroll
-            for (int ii = kb; ii < 8; ++ii) lprev[ii] = li[ii];
-        }
-    }
-finish:
-    __syncthreads();
-    if (failed) {
-        if (tid == 0) atomicCAS(info, 0, blk * DB + failed);
-        return;
-    }
-    for (int e = tid; e < DB * DB; e += 256) {
-        const int r = e >> 7, c = e & 127;
-        A[(long)r * lda + c] = c <= r ? S[r * DB_LD + c] : 0.0;
-    }
-#pragma unroll
-    for (int ii = 0; ii < 8; ++ii)
-#pragma unroll
-        for (int jj = 0; jj < 8; ++jj) {
-            const int i = 16 * ii + ti, c = 16 * jj + tj;
-            Dinv[i * DB + c] = (jj <= ii && c <= i) ? x[ii][jj < ii ? jj : ii] : 0.0;
-        }
-}
-
-__global__ void __launch_bounds__(256) diag_trtri_kernel(const double* L, long lda, double* Dinv) {
-    extern __shared__ double S[];
-    const double* A = L + (long)blockIdx.x * DB * lda + (long)blockIdx.x * DB;
-    for (int e = threadIdx.x; e < DB * DB; e += 256) {
-        const int r = e >> 7, c = e & 127;
-        S[r * DB_LD + c] = c <= r ? A[(long)r * lda + c] : 0.0;
-    }
-    __syncthreads();
-    tri_inverse_regs(S, Dinv + (long)blockIdx.x * DB * DB);
-}
-
+constexpr int DB = 128;
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Blocked variant of the same operation (Cholesky of one 128x128 block AND X = L^-1): 4 x 4 sub-blocks of 32 x 32 in shared
-// memory (row stride 36 doubles = 4 mod 16, so the DMMA fragment loads below are bank-conflict-free in both orientations).
+// Cholesky of one 128x128 block AND X = L^-1, blocked: 4 x 4 sub-blocks of 32 x 32 in shared memory (row stride 36 doubles
+// = 4 mod 16, so the DMMA fragment loads below are bank-conflict-free in both orientations).
 // Per block step j:
 //   (1) ONE warp factors the 32 x 32 diagonal sub-block with lane r owning row r in registers: per pivot one shuffle (the
 //       pivot), rsqrt, the scaled column published through a double-buffered shared column (one __syncwarp, no CTA barrier),
 //       FMAs only; the right-looking elimination of L X = I rides on the same pivot, so X_jj = L_jj^-1 comes out of the same loop;
 //   (2) all 8 warps, DMMA: panel L_ij = A_ij X_jj^T (i > j) and the finished block row of the inverse X_jc = X_jj Xcur_jc (c < j);
 //   (3) all 8 warps, DMMA: trailing A_ik -= L_ij L_kj^T (j < k <= i) and the inverse's elimination Xcur_ic -= L_ij X_jc (c <= j).
-// 11 CTA barriers instead of 128, and the O(n^3) part runs on the FP64 tensor pipe.  The per-pivot kernel above is latency-bound
-// on its barrier chain (77 us per block, 13 us of arithmetic: tools/diag_bench).
+// 11 CTA barriers instead of 128, and the O(n^3) part runs on the FP64 tensor pipe.  A per-pivot register kernel with one CTA
+// barrier per pivot was latency-bound on that barrier chain (77 us per block, 13 us of arithmetic: tools/diag_bench, r01).
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int QB = 32, QLD = 36, QBLK = QB * QLD, QNB = DB / QB;
-#ifdef TSVGP_DIAG_TIMING   // tools/diag_bench only: cycle stamps of the phases of one block (thread 0)
-__device__ long long g_diag_clk[32];
-#define DIAG_STAMP(i) do { if (threadIdx.x == 0) g_diag_clk[i] = clock64(); } while (0)
-#else
-#define DIAG_STAMP(i) do { } while (0)
-#endif
 __device__ __forceinline__ int qidx(int i, int j) { return (i * (i + 1) / 2 + j) * QBLK; }
 
 // One warp: the (8 TM) x (8 TN) region at (r0, n0) of the 32 x 32 block C from the 32 x 32 blocks A ([r][k]) and B
@@ -1110,55 +860,35 @@ __device__ __forceinline__ double rsqrt_pos(double m) {
     return y;
 }
 
-// PIPE = false: the round-1 loop.  PIPE = true [r02]: the next pivot's shuffle and reciprocal square root are issued BEFORE the
-// bulk of the current rank-1 update (a warp issues in order: behind 30 DFMAs the chain waited ~60 cycles per pivot for nothing),
-// and the reciprocal square root is the bare Newton form above.
-template <bool PIPE>
+// The next pivot's shuffle and reciprocal square root are issued BEFORE the bulk of the current rank-1 update (a warp issues in
+// order: behind 30 DFMAs the chain would wait ~60 cycles per pivot for nothing), and the reciprocal square root is the bare
+// Newton form above.
 __device__ __forceinline__ int warp_potrf_32(double* Ajj, double* colbuf, double* rsbuf, uint64_t* bars, int lane) {
     double a[QB];
 #pragma unroll
     for (int c = 0; c < QB; ++c) a[c] = c < lane ? Ajj[lane * QLD + c] : 0.0;
     double d = Ajj[lane * QLD + lane], dl = 0.0;
     int fail = 0;
-    if (!PIPE) {
+    double piv = __shfl_sync(0xffffffffu, d, 0);
+    if (!(piv > 0.0)) fail = 1;
+    double rs = rsqrt_pos(fail ? 1.0 : piv);
 #pragma unroll
-        for (int k = 0; k < QB; ++k) {
-            const double piv = __shfl_sync(0xffffffffu, d, k);
-            if (!(piv > 0.0) && fail == 0) fail = k + 1;   // uniform across the warp
-            const double rs = rsqrt(piv);
-            const double lk = lane > k ? a[k] * rs : 0.0;
-            d = fma(-lk, lk, d);
-            a[k] = lk;
-            if (lane == k) dl = piv * rs;
-            colbuf[k * QB + lane] = lk;
-            if (lane == 0) rsbuf[k] = rs;
-            mbar_arrive(bars + k);   // release: the column and rs are visible to whoever observes the completed phase
-            __syncwarp();
-#pragma unroll
-            for (int c = k + 1; c < QB; ++c) a[c] = fma(-lk, colbuf[k * QB + c], a[c]);
+    for (int k = 0; k < QB; ++k) {
+        const double lk = lane > k ? a[k] * rs : 0.0;
+        d = fma(-lk, lk, d);
+        a[k] = lk;
+        if (lane == k) dl = piv * rs;
+        colbuf[k * QB + lane] = lk;
+        if (lane == 0) rsbuf[k] = rs;
+        mbar_arrive(bars + k);   // release: the column and rs are visible to whoever observes the completed phase
+        __syncwarp();
+        if (k + 1 < QB) {   // the chain first: next pivot and its reciprocal square root
+            piv = __shfl_sync(0xffffffffu, d, k + 1);
+            if (!(piv > 0.0) && fail == 0) fail = k + 2;   // uniform across the warp
+            rs = rsqrt_pos(fail ? 1.0 : piv);
         }
-    } else {
-        double piv = __shfl_sync(0xffffffffu, d, 0);
-        if (!(piv > 0.0)) fail = 1;
-        double rs = rsqrt_pos(fail ? 1.0 : piv);
 #pragma unroll
-        for (int k = 0; k < QB; ++k) {
-            const double lk = lane > k ? a[k] * rs : 0.0;
-            d = fma(-lk, lk, d);
-            a[k] = lk;
-            if (lane == k) dl = piv * rs;
-            colbuf[k * QB + lane] = lk;
-            if (lane == 0) rsbuf[k] = rs;
-            mbar_arrive(bars + k);   // release: the column and rs are visible to whoever observes the completed phase
-            __syncwarp();
-            if (k + 1 < QB) {   // the chain first: next pivot and its reciprocal square root
-                piv = __shfl_sync(0xffffffffu, d, k + 1);
-                if (!(piv > 0.0) && fail == 0) fail = k + 2;   // uniform across the warp
-                rs = rsqrt_pos(fail ? 1.0 : piv);
-            }
-#pragma unroll
-            for (int c = k + 1; c < QB; ++c) a[c] = fma(-lk, colbuf[k * QB + c], a[c]);
-        }
+        for (int c = k + 1; c < QB; ++c) a[c] = fma(-lk, colbuf[k * QB + c], a[c]);
     }
 #pragma unroll
     for (int c = 0; c < QB; ++c) Ajj[lane * QLD + c] = c < lane ? a[c] : (c == lane ? dl : 0.0);
@@ -1181,111 +911,10 @@ __device__ __forceinline__ void warp_trtri_32(double* Xjj, const double* colbuf,
     for (int c = 0; c < QB; ++c) Xjj[c * QLD + lane] = x[c];   // zero above the diagonal by construction
 }
 
-__global__ void __launch_bounds__(256) diag_potrf_inv_blocked_kernel(double* A, long lda, double* Dinv, int blk, int* info, int fast) {
-    PDL_PROLOGUE();
-    extern __shared__ __align__(16) double S[];
-    double* As = S;                                       // 10 lower sub-blocks of A -> L
-    double* Xs = S + (QNB * (QNB + 1) / 2) * QBLK;        // 10 lower sub-blocks of X = L^-1
-    __shared__ __align__(16) double colbuf[QB * QB];   // scaled columns of the diagonal sub-block being factored
-    __shared__ __align__(16) double rsbuf[QB];
-    __shared__ __align__(8) uint64_t bars[QB];          // one per pivot: warp 0 -> warp 1 hand-over (phase = block step)
-    __shared__ int sfail;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) sfail = 0;
-    if (tid < QB) mbar_init(bars + tid, 32);
-    DIAG_STAMP(0);
-    const bool vec_ok = ((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(Dinv) | (uintptr_t)(lda * 8)) & 15) == 0;
-    if (vec_ok) {   // all 16-byte pieces of the lower sub-blocks in flight at once
-        for (int u = tid; u < DB * (DB / 2); u += 256) {
-            const int r = u >> 6, c = (u & 63) * 2;
-            if ((c >> 5) <= (r >> 5)) cp_async16(As + qidx(r >> 5, c >> 5) + (r & 31) * QLD + (c & 31), A + (long)r * lda + c);
-        }
-        cp_async_commit();
-        cp_async_wait<0>();
-    } else {
-        for (int e = tid; e < DB * DB; e += 256) {
-            const int r = e >> 7, c = e & 127;
-            if ((c >> 5) <= (r >> 5)) As[qidx(r >> 5, c >> 5) + (r & 31) * QLD + (c & 31)] = A[(long)r * lda + c];
-        }
-    }
-    __syncthreads();
-    DIAG_STAMP(1);
-#pragma unroll 1
-    for (int j = 0; j < QNB; ++j) {
-        if (warp == 0) {
-            const int f = fast ? warp_potrf_32<true>(As + qidx(j, j), colbuf, rsbuf, bars, lane)
-                               : warp_potrf_32<false>(As + qidx(j, j), colbuf, rsbuf, bars, lane);
-            if (f && lane == 0) sfail = j * QB + f;
-        } else if (warp == 1) {
-            warp_trtri_32(Xs + qidx(j, j), colbuf, rsbuf, bars, (uint32_t)(j & 1), lane);
-        }
-        __syncthreads();
-        DIAG_STAMP(2 + 3 * j);
-        if (sfail) break;   // uniform
-        {   // (2) panel rows below (row halves: the product is in place on A_ij) and the finished block row j of X (column halves)
-            int tsk = 0;
-            for (int i = j + 1; i < QNB; ++i)
-                for (int h = 0; h < 2; ++h)
-                    if ((tsk++ & 7) == warp)
-                        qblk_mma<2, 4, true, 1>(As + qidx(i, j), As + qidx(i, j), Xs + qidx(j, j), 16 * h, 0, 0, 0, lane);
-            for (int c = 0; c < j; ++c)
-                for (int h = 0; h < 2; ++h)
-                    if ((tsk++ & 7) == warp)
-                        qblk_mma<4, 2, false, 2>(Xs + qidx(j, c), Xs + qidx(j, j), Xs + qidx(j, c), 0, 16 * h, 0, 0, lane);
-        }
-        __syncthreads();
-        DIAG_STAMP(3 + 3 * j);
-        if (j + 1 < QNB) {   // (3) trailing update of A and the elimination step of L X = I, in 16 x 16 quarters
-            int tsk = 0;
-            for (int i = j + 1; i < QNB; ++i) {
-                for (int k = j + 1; k <= i; ++k)
-                    for (int qd = 0; qd < 4; ++qd) {
-                        if (i == k && qd == 1) continue;   // strictly upper quarter of a diagonal block
-                        if ((tsk++ & 7) == warp)
-                            qblk_mma<2, 2, true, 0>(As + qidx(i, k), As + qidx(i, j), As + qidx(k, j), 16 * (qd >> 1), 16 * (qd & 1), 1, 0, lane);
-                    }
-                for (int c = 0; c <= j; ++c)
-                    for (int qd = 0; qd < 4; ++qd)
-                        if ((tsk++ & 7) == warp)   // c == j: X_jj is lower triangular, rows k < n0 contribute nothing
-                            qblk_mma<2, 2, false, 0>(Xs + qidx(i, c), As + qidx(i, j), Xs + qidx(j, c), 16 * (qd >> 1), 16 * (qd & 1),
-                                                     c == j ? 2 : 1, c == j ? 16 * (qd & 1) : 0, lane);
-            }
-            __syncthreads();
-            DIAG_STAMP(4 + 3 * j);
-        }
-    }
-    if (sfail) {
-        if (tid == 0) atomicCAS(info, 0, blk * DB + sfail);
-        return;
-    }
-    if (vec_ok) {
-#pragma unroll 4
-        for (int u = tid; u < DB * (DB / 2); u += 256) {
-            const int r = u >> 6, c = (u & 63) * 2;
-            if ((c >> 5) > (r >> 5)) continue;   // strictly upper sub-blocks: A's are zeroed by the caller (chol_lower), Dinv's stay zero
-            const int o = qidx(r >> 5, c >> 5) + (r & 31) * QLD + (c & 31);
-            double2 l = *reinterpret_cast<const double2*>(As + o);
-            double2 x = *reinterpret_cast<const double2*>(Xs + o);
-            if (c > r) l.x = x.x = 0.0;
-            if (c + 1 > r) l.y = x.y = 0.0;
-            *reinterpret_cast<double2*>(A + (long)r * lda + c) = l;
-            *reinterpret_cast<double2*>(Dinv + r * DB + c) = x;
-        }
-    } else {
-        for (int e = tid; e < DB * DB; e += 256) {
-            const int r = e >> 7, c = e & 127;
-            if ((c >> 5) > (r >> 5)) continue;
-            const int o = qidx(r >> 5, c >> 5) + (r & 31) * QLD + (c & 31);
-            A[(long)r * lda + c] = c <= r ? As[o] : 0.0;
-            Dinv[e] = c <= r ? Xs[o] : 0.0;
-        }
-    }
-    DIAG_STAMP(14);
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// Look-ahead variant of the blocked kernel.  The pivot chain of warps 0 / 1 (8 k cycles per 32 x 32 sub-block) is the critical
-// path; everything else is arranged around it:
+// Look-ahead schedule of the blocked factorisation (36.9 us per block, 38.9 us with steps (1)-(3) in plain order: tools/diag_bench,
+// r02).  The pivot chain of warps 0 / 1 (8 k cycles per 32 x 32 sub-block) is the critical path; everything else is arranged
+// around it:
 //   * the trailing update of step j is split: T_j^A = the blocks step j + 1 needs (block column j + 1 of A, block row j + 1 of the
 //     inverse's work matrix) runs on all warps right after the panel; T_j^B = the rest is DEFERRED and runs on warps 2..7 while
 //     warps 0 / 1 factor sub-block j + 1;
@@ -1336,7 +965,7 @@ __device__ __forceinline__ void qwriteback(const double* As, const double* Xs, d
             if ((tsk++ % nw) + w0 == warp) qstore_rows(Xs + qidx(j, c), Dinv, DB, j, c, 16 * h, 16, lane);
 }
 
-__global__ void __launch_bounds__(256) diag_potrf_inv_lookahead_kernel(double* A, long lda, double* Dinv, int blk, int* info, int fast) {
+__global__ void __launch_bounds__(256) diag_potrf_inv_lookahead_kernel(double* A, long lda, double* Dinv, int blk, int* info) {
     PDL_PROLOGUE();
     extern __shared__ __align__(16) double S[];
     double* As = S;
@@ -1366,8 +995,7 @@ __global__ void __launch_bounds__(256) diag_potrf_inv_lookahead_kernel(double* A
 #pragma unroll 1
     for (int j = 0; j < QNB; ++j) {
         if (warp == 0) {
-            const int f = fast ? warp_potrf_32<true>(As + qidx(j, j), colbuf, rsbuf, bars, lane)
-                               : warp_potrf_32<false>(As + qidx(j, j), colbuf, rsbuf, bars, lane);
+            const int f = warp_potrf_32(As + qidx(j, j), colbuf, rsbuf, bars, lane);
             if (f && lane == 0) sfail = j * QB + f;
         } else if (warp == 1) {
             warp_trtri_32(Xs + qidx(j, j), colbuf, rsbuf, bars, (uint32_t)(j & 1), lane);
@@ -1401,34 +1029,15 @@ __global__ void __launch_bounds__(256) diag_potrf_inv_lookahead_kernel(double* A
     qwriteback(As, Xs, A, lda, Dinv, QNB - 1, 0, 8, warp, lane);
 }
 
-#ifdef TSVGP_DIAG_TIMING
-int diag_read_stamps(long long* out32) { return (int)cudaMemcpyFromSymbol(out32, g_diag_clk, sizeof(long long) * 32); }
-#endif
-static int g_diag_fast = 1;      // 1 = pipelined pivot chain with the bare Newton rsqrt (TSVGP_DIAG_FAST=0: the round-1 loop, A/B timing)
-static int g_diag_variant = 2;   // 2 = blocked (DMMA) kernel with look-ahead (36.9 us per block), 1 = without (38.9 us), 0 = per-pivot register kernel (A/B timing: tools/diag_bench, TSVGP_DIAG_VARIANT)
-void diag_set_variant(int v) { g_diag_variant = v; }
-void diag_set_fast(int f) { g_diag_fast = f; }
 constexpr int DIAG_BLOCKED_SMEM = 2 * (QNB * (QNB + 1) / 2) * QBLK * 8;
 
-// opt in to the large dynamic shared memory of the diagonal-block kernels on the CURRENT device (call once per context)
+// opt in to the large dynamic shared memory of the diagonal-block kernel on the CURRENT device (call once per context)
 int diag_init() {
-    int e = (int)cudaFuncSetAttribute(diag_potrf_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DB * DB_LD * 8);
-    e |= (int)cudaFuncSetAttribute(diag_trtri_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DB * DB_LD * 8);
-    e |= (int)cudaFuncSetAttribute(diag_potrf_inv_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_BLOCKED_SMEM);
-    e |= (int)cudaFuncSetAttribute(diag_potrf_inv_lookahead_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_BLOCKED_SMEM);
-    if (const char* v = getenv("TSVGP_DIAG_VARIANT")) g_diag_variant = atoi(v);
-    if (const char* v = getenv("TSVGP_DIAG_FAST")) g_diag_fast = atoi(v);
-    return e;
+    return (int)cudaFuncSetAttribute(diag_potrf_inv_lookahead_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_BLOCKED_SMEM);
 }
 
 int diag_potrf_inv_launch(double* A, long lda, double* Dinv, int blk_index, int* info, cudaStream_t s) {
-    if (g_diag_variant == 2) launch_k(true, diag_potrf_inv_lookahead_kernel, 1, 256, DIAG_BLOCKED_SMEM, s, A, lda, Dinv, blk_index, info, g_diag_fast);
-    else if (g_diag_variant == 1) launch_k(true, diag_potrf_inv_blocked_kernel, 1, 256, DIAG_BLOCKED_SMEM, s, A, lda, Dinv, blk_index, info, g_diag_fast);
-    else diag_potrf_inv_kernel<<<1, 256, DB * DB_LD * 8, s>>>(A, lda, Dinv, blk_index, info);
-    return count_launch();
-}
-int diag_trtri_launch(const double* L, long lda, double* Dinv, int nblk, cudaStream_t s) {
-    diag_trtri_kernel<<<nblk, 256, DB * DB_LD * 8, s>>>(L, lda, Dinv);
+    launch_k(true, diag_potrf_inv_lookahead_kernel, 1, 256, DIAG_BLOCKED_SMEM, s, A, lda, Dinv, blk_index, info);
     return count_launch();
 }
 
@@ -1513,10 +1122,6 @@ int finalize_sites_launch(const double* P, double* L2, long ld, int M, int Mp, c
     launch_k(true, finalize_sites_kernel, EW_GRID(n), 0, s, P, L2, ld, M, Mp, bad, info);
     return count_launch();
 }
-__global__ void place_block_kernel(const double* src, long lds, double* dst, long ldd, int rows, int cols) {
-    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
-    if (i < rows && j < cols) dst[(long)i * ldd + j] = src[(long)i * lds + j];
-}
 // Linv = blockdiag(dinv[0], dinv[1], ...) with zeros elsewhere: the seed of the bottom-up triangular inverse, one launch
 __global__ void trtri_seed_kernel(const double* dinv, double* Linv, long ld, int n) {
     PDL_PROLOGUE();
@@ -1526,19 +1131,6 @@ __global__ void trtri_seed_kernel(const double* dinv, double* Linv, long ld, int
 }
 int trtri_seed_launch(const double* dinv, double* Linv, long ld, int n, cudaStream_t s) {
     launch_k(true, trtri_seed_kernel, EW_GRID(n), 0, s, dinv, Linv, ld, n);
-    return count_launch();
-}
-int place_block_launch(const double* src, long lds, double* dst, long ldd, int rows, int cols, cudaStream_t s) {
-    place_block_kernel<<<dim3((cols + 31) / 32, (rows + 7) / 8), dim3(32, 8), 0, s>>>(src, lds, dst, ldd, rows, cols);
-    return count_launch();
-}
-__global__ void copy_lower_kernel(const double* src, long lds, int M, double* dst, long ldd, int n) {
-    EW_IJ;
-    dst[(long)i * ldd + j] = (i < M && j <= i) ? src[(long)i * lds + j] : 0.0;
-}
-int copy_lower_launch(const double* src, long lds, int M, double* dst, long ldd, int Mp, cudaStream_t s) {
-    const int n = Mp;
-    copy_lower_kernel<<<EW_GRID(n), 0, s>>>(src, lds, M, dst, ldd, Mp);
     return count_launch();
 }
 
@@ -1554,34 +1146,6 @@ __device__ __forceinline__ double block_sum_256(double v, double* sred) {
     __syncthreads();
     return s;   // valid on thread 0
 }
-__global__ void __launch_bounds__(256) frob_part_kernel(const double* A, long lda, int n, double* part) {
-    __shared__ double sred[8];
-    double s = 0.0;
-    const long total = (long)n * n;
-    for (long e = (long)blockIdx.x * 256 + threadIdx.x; e < total; e += (long)RED_BLOCKS * 256) {
-        const double v = A[(e / n) * lda + (e % n)];
-        s = fma(v, v, s);
-    }
-    s = block_sum_256(s, sred);
-    if (threadIdx.x == 0) part[blockIdx.x] = s;
-}
-__global__ void __launch_bounds__(256) frob_logdiag_finish_kernel(const double* A, long lda, int n, const double* part, double* out) {
-    __shared__ double sred[8];
-    double s = threadIdx.x < RED_BLOCKS ? part[threadIdx.x] : 0.0;
-    s = block_sum_256(s, sred);
-    if (threadIdx.x == 0) out[0] = s;
-    double l = 0.0;
-    for (int i = threadIdx.x; i < n; i += 256) l += log(A[(long)i * lda + i]);
-    l = block_sum_256(l, sred);
-    if (threadIdx.x == 0) out[1] = l;
-}
-int frob_logdiag_launch(const double* A, long lda, int n, double* out, double* part, cudaStream_t s) {
-    if (!part) return -1;
-    frob_part_kernel<<<RED_BLOCKS, 256, 0, s>>>(A, lda, n, part);
-    frob_logdiag_finish_kernel<<<1, 256, 0, s>>>(A, lda, n, part, out);
-    ++g_launches;
-    return count_launch();
-}
 __global__ void __launch_bounds__(256) dot_kernel(const double* x, const double* y, int n, double* out) {
     PDL_PROLOGUE();
     __shared__ double sred[8];
@@ -1592,17 +1156,6 @@ __global__ void __launch_bounds__(256) dot_kernel(const double* x, const double*
 }
 int dot_launch(const double* x, const double* y, int n, double* out, cudaStream_t s) {
     launch_k(true, dot_kernel, 1, 256, 0, s, x, y, n, out);
-    return count_launch();
-}
-__global__ void __launch_bounds__(256) sum_kernel(const double* x, long n, double* out) {
-    __shared__ double sred[8];
-    double s = 0.0;
-    for (long i = threadIdx.x; i < n; i += 256) s += x[i];
-    s = block_sum_256(s, sred);
-    if (threadIdx.x == 0) out[0] = s;
-}
-int sum_launch(const double* x, long n, double* out, cudaStream_t s) {
-    sum_kernel<<<1, 256, 0, s>>>(x, n, out);
     return count_launch();
 }
 __global__ void update_lambda1_kernel(double* l1, const double* G1, const double* G2mZ, int n, double lr, double scale,
@@ -1725,17 +1278,6 @@ __global__ void vadd_inplace_kernel(double* dst, const double* src, long n) {
     PDL_PROLOGUE();
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) dst[i] += src[i];
-}
-__global__ void sum_rows_into_kernel(const double* __restrict__ src, int rows, int n, double* __restrict__ dst) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
-    double s = 0.0;
-    for (int r = 0; r < rows; ++r) s += src[(long)r * n + j];
-    dst[j] += s;
-}
-int sum_rows_into_launch(const double* src, int rows, int n, double* dst, cudaStream_t s) {
-    sum_rows_into_kernel<<<(n + 255) / 256, 256, 0, s>>>(src, rows, n, dst);
-    return count_launch();
 }
 int vadd_inplace_launch(double* dst, const double* src, long n, cudaStream_t s) {
     launch_k(true, vadd_inplace_kernel, (unsigned)((n + 255) / 256), 256, 0, s, dst, src, n);

@@ -110,17 +110,13 @@ int gemv_t_part_launch(const double* A, long lda, int m, int n, const double* x,
 // Zs[i][d] = ZsT[d][i]  (row-major copy of the scaled inducing inputs, [Mp][D])
 int unpack_rows_launch(const double* ZsT, long ldz, int Mp, int D, double* Zs, cudaStream_t s);
 
-int diag_init();   // once per device/context: opt in to the dynamic shared memory of the diagonal-block kernels
-void diag_set_fast(int f);      // 1 = pipelined pivot chain + bare Newton rsqrt (default), 0 = the round-1 loop (env TSVGP_DIAG_FAST)
-void diag_set_variant(int v);   // 1 = blocked DMMA kernel (default), 0 = per-pivot register kernel (A/B timing; env TSVGP_DIAG_VARIANT)
+int diag_init();   // once per device/context: opt in to the dynamic shared memory of the diagonal-block kernel
 // --- diagonal blocks --------------------------------------------------------------------------------------------
 // In-place lower Cholesky of the 128x128 block at A (lda) and its inverse into Dinv (ld 128, dense lower).
 // info[0] = first failing global pivot index + 1 (blk_index*128 + k + 1), left untouched on success.
-// Dinv must have been zero-filled once (cudaMemset) by its owner: the blocked kernel never writes the strictly upper 32 x 32
+// Dinv must have been zero-filled once (cudaMemset) by its owner: the kernel never writes the strictly upper 32 x 32
 // sub-blocks of Dinv, and leaves those of A to the caller (chol_lower zeroes the upper triangle at the end).
 int diag_potrf_inv_launch(double* A, long lda, double* Dinv, int blk_index, int* info, cudaStream_t s);
-// Dinv[b] = inverse of the lower-triangular 128x128 diagonal block b of L, b < nblk (batched)
-int diag_trtri_launch(const double* L, long lda, double* Dinv, int nblk, cudaStream_t s);
 
 // --- elementwise M x M utilities ---------------------------------------------------------------------------------
 int add_diag_launch(double* A, long lda, int n, double v, cudaStream_t s);
@@ -132,12 +128,7 @@ int zero_upper_launch(double* A, long lda, int n, cudaStream_t s);
 // L2 = -tril(P) on [0,M)^2, 0 elsewhere — skipped on the device when *bad != 0 or any of info[0..3] != 0 (failed step keeps old sites)
 int finalize_sites_launch(const double* P, double* L2, long ld, int M, int Mp, const double* bad, const int* info, cudaStream_t s);
 int trtri_seed_launch(const double* dinv, double* Linv, long ld, int n, cudaStream_t s);   // Linv = blockdiag(dinv[b]) (128 x 128 blocks), zero elsewhere
-int place_block_launch(const double* src, long lds, double* dst, long ldd, int rows, int cols, cudaStream_t s);  // dst[0:rows,0:cols] = src
-int copy_lower_launch(const double* src, long lds, int M, double* dst, long ldd, int Mp, cudaStream_t s);  // dst = [[tril(src),0],[0,0]]
-// scalars: out[0] = sum_ij A^2 ; out[1] = sum_i log(diag A) ; single block, deterministic
-int frob_logdiag_launch(const double* A, long lda, int n, double* out, double* part /* [128] caller-owned scratch */, cudaStream_t s);
 int dot_launch(const double* x, const double* y, int n, double* out, cudaStream_t s);
-int sum_launch(const double* x, long n, double* out, cudaStream_t s);
 // lambda_1 <- (1-lr) lambda_1 + lr*scale*(G1 - 2 G2mZ)
 int update_lambda1_launch(double* l1, const double* G1, const double* G2mZ, int n, double lr, double scale, const double* bad,
                           const int* info, cudaStream_t s);
@@ -157,7 +148,6 @@ int probe_vector_launch(double* v, int M, int Mp, cudaStream_t s);
 // P = a P + b X on [0,M)^2 unless *bad != 0 or any info slot != 0 (guarded commit of the whitened sibling's Lambda_2)
 int axpby_guarded_launch(double* P, const double* X, long ld, int M, double a, double b, const double* bad, const int* info, cudaStream_t s);
 int vadd_inplace_launch(double* dst, const double* src, long n, cudaStream_t s);
-int sum_rows_into_launch(const double* src, int rows, int n, double* dst, cudaStream_t s);   // dst[j] += sum_r src[r][j]  (fixed order)
 int stats_tail_launch(const double* ve_blocks, long nblocks, const int* flags, const double* aux, double* out, cudaStream_t s);
 // Gaussian natgrad_step, whose pass took var = k(x,x): with tr[0] = tr(P^T B P) and q = tr[0] * inv_c = sum_n |T^T k_n|^2,
 // out[0] (sum ve) += half_inv_s2 * q, and out[1] (the variance flag) = 1 unless sum_n v_n = sum_kdiag - q is finite and positive

@@ -87,12 +87,6 @@ struct tsvgp_ctx {
     int shard_min_m = 2048;    // from this (padded) M upwards the statistics are reduce-SCATTERED by tile rows and the two products of
     int split_chains = 0;      // 1: rank 0 builds the posterior factors, rank 1 the K9 chain, both broadcast their results (see chain_split_active)
                                // G2 = K9^-1 B K9^-1 run on each rank's rows only, assembled by two all-gathers (sharded_update)
-    int async_issue = 1;       // small M: enqueue the K9 chain from a helper host thread while this thread enqueues the posterior chain
-    int fuse_b = 1;            // accumulate b += Kuf g inside the SYRK kernel instead of a separate mat-vec pass over the slab
-    int spread_b = 0;          // 1: ... shared by all tiles of a tile row (private slots) instead of carried by the first tile column alone.
-                               // Measured (M = 2048, 262 144 rows): the SYRK launch alone 1.087 -> 1.076 ms, but the step 74.55 -> 74.63 ms
-                               // (two slab streams already hide the longer first-column tiles; the extra zeroing and summing are not free)
-    int balance = 1;           // split the SYRK's contraction in two pieces so that every SM gets equal work
     int cache_factors = 1;     // keep chol(K9) and the posterior factors between calls while their inputs are unchanged
     int route_opt = ROUTE_AUTO;     // statistics route: fused (B = Kuf H Kfu, then K9^-1 B K9^-1) or whitened (C9^-1 Kuf first)
     double route_cond_max = 1e4;    // auto: fused while the estimated cond(Kuu + jitter I) is below this (measured fused error
@@ -109,7 +103,6 @@ struct tsvgp_ctx {
     double cond_hint = 0.0;
     bool cond_hint_valid = false;
     int speculate = 1;
-    int k9_defer = 0;   // measured slower (M = 2048, 131072 rows: 41.1 vs 39.9 ms): under the pass every chain kernel waits for an SM slot
     // Gaussian likelihood, fused route: h_n is a constant, so Kuf and the SYRK of a slab do not depend on the posterior.  The first
     // slab of every slab stream is enqueued BEFORE the posterior chain (latency-bound, SMs mostly idle) and fills the idle SMs.
     int early_slabs = 1;
@@ -219,7 +212,6 @@ struct tsvgp_ctx {
     Pool pc;
     long chunk = 0;
     int chunk_Mp = 0;
-    int chunk_route = 0;
     int slab_streams = 0;
     double *wslab[MAXS] = {};
     double *slab_all[MAXS] = {};   // [slab_lat][Mp][nc]: one Kuf slab per latent in separate mode
@@ -235,7 +227,6 @@ struct tsvgp_ctx {
     int grad_lat = 0;     // U slabs per slab stream in the gradient workspace: L for a coupled likelihood (one pass), else 1
     int waug = 128;       // columns of the augmented blocks [xs | 1 | xs^2 | 0] (xaug, zaug, facc, fuu, fpart): aug_width(D)
     double* kpart[MAXS] = {};     // split-K partial tiles of the SYRK when M is so small that its tiles cannot fill the SMs
-    double* bacc[MAXS] = {};      // fused b += Kuf g shared by the tiles of a tile row: [L][2 pieces][Mp/128 tile columns][Mp] private slots
     int ksplit = 1;
     // Gaussian step, fused route: the constant-weight SYRK as an exact int8 Gram product (int8_gram.cuh) — per slab stream the
     // 16 residue planes of the slab and the residues of the lower tiles; allocated for a Gaussian model (i8_alloc)
@@ -361,11 +352,10 @@ int alloc_m_state(tsvgp_ctx* c, int M, int D) {
     NEED(c->alpha_all = p.get(nl * mp)); NEED(c->mZ_all = p.get(nl * mp)); NEED(c->mq_all = p.get(nl * mp)); NEED(c->v1 = p.get(mp)); NEED(c->v2 = p.get(mp));
     NEED(c->v3 = p.get(mp)); NEED(c->gwork = p.get((size_t)(c->Mp / 64 + 1) * mp)); NEED(c->scal_all = p.get(nl * N_SCAL)); NEED(c->red = p.get(128));
     NEED(c->info = (int*)p.get(N_INFO)); NEED(c->flags = (int*)p.get(2));
-    c->gws_doubles = (size_t)4 << 20;   // 32 MB per stream: up to 16 partial images of a 512 x 512 product, 4 of a 1024 x 1024 one
+    // 32 MB per stream, less 2048 doubles: up to 15 partial images of a 512 x 512 product, 3 of a 1024 x 1024 one.  The size caps
+    // the split-K piece count of the M x M products, and with it the order in which their partials are summed.
+    c->gws_doubles = ((size_t)4 << 20) - 2048;
     NEED(c->gws = p.get(c->gws_doubles)); NEED(c->gws2 = p.get(c->gws_doubles));
-    // (on the context's own stream: it is non-blocking, a legacy-stream memset would not be ordered with it)
-    CU(cudaMemsetAsync(c->gws + c->gws_doubles - GEMM_WS_COUNTER_DOUBLES, 0, sizeof(double) * GEMM_WS_COUNTER_DOUBLES, c->s_main));    // tile counters
-    CU(cudaMemsetAsync(c->gws2 + c->gws_doubles - GEMM_WS_COUNTER_DOUBLES, 0, sizeof(double) * GEMM_WS_COUNTER_DOUBLES, c->s_main));
     c->waug = aug_width(D);
     NEED(c->zaug = p.get(mp * c->waug)); NEED(c->fuu = p.get(mp * c->waug)); NEED(c->origin = p.get(D));
     NEED(c->C6 = p.get(mm)); NEED(c->C6inv = p.get(mm));
@@ -754,30 +744,33 @@ long used_chunk(const tsvgp_ctx* c, long n_points, long nc, int nstr) {
     return ncu < nc ? ncu : nc;
 }
 
+// slab streams of a pass: option "streams", one in profile mode
+int slab_stream_count(const tsvgp_ctx* c) {
+    return c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
+}
+
 // the likelihood couples the latents (one point kernel over all of them, Y [N, 1]): Softmax, heteroskedastic Normal
 inline bool coupled(const tsvgp_ctx* c) { return c->lik.kind == LIK_SOFTMAX || c->lik.kind == LIK_HETEROSKEDASTIC; }
 
 int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
     const long nc = pick_chunk(c);
     const int u_lat = need_grad && coupled(c) ? c->L : 1;   // the gradient pass of a coupled likelihood keeps every latent's U
-    const int nstr_used = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
-    const long ncu = used_chunk(c, n_points, nc, nstr_used);
+    const int ns = slab_stream_count(c);
+    const long ncu = used_chunk(c, n_points, nc, ns);
     const long nchunks = (n_points + ncu - 1) / ncu;
     const long ve_need = (nchunks + 1) * ((nc + 255) / 256);
     const bool need_w = c->route == ROUTE_WHITENED || c->route == ROUTE_EXACT;
-    const int want_streams = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     const int slab_lat = c->sep ? c->L : 1;
     const bool want_i8 = c->lik.kind == LIK_GAUSSIAN && !c->white && nc <= I8_MAX_COLS;
     const bool need_a = need_grad && c->white;   // the whitened gradient pass keeps LA^-1 K beside LR^-1 K
     if (c->chunk == nc && c->chunk_Mp == c->Mp && c->ve_cap >= ve_need && (!need_w || c->wslab[0]) && (!need_grad || (c->grad_ws && c->grad_lat >= u_lat)) &&
         (!need_a || c->aslab[0]) &&
-        c->slab_streams >= want_streams && c->slab_lat == slab_lat && c->i8_alloc == want_i8)
+        c->slab_streams >= ns && c->slab_lat == slab_lat && c->i8_alloc == want_i8)
         return TSVGP_OK;
     CU(cudaStreamSynchronize(c->s_main));
     c->pc.release();
     for (int s = 0; s < MAXS; ++s) c->wslab[s] = c->aslab[s] = nullptr;
     Pool& p = c->pc;
-    const int ns = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
     c->slab_streams = ns;
     for (int s = 0; s < ns; ++s) {
         NEED(c->slab_all[s] = c->slab[s] = p.get((size_t)slab_lat * c->Mp * nc));
@@ -812,7 +805,6 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
         LA(i8_planes_init(c->i8_planes[s], c->Mp, nc, c->s_main));
     }
     NEED(c->ve_all = p.get((size_t)c->L * ve_need));
-    for (int s = 0; s < ns; ++s) NEED(c->bacc[s] = p.get((size_t)c->L * 2 * (c->Mp / 128) * c->Mp));
     c->grad_ws = false;
     c->grad_lat = 0;
     if (need_grad) {
@@ -860,7 +852,6 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
 // phase 1 has been enqueued: the early slabs only run their posterior-dependent part (means, variance product, point statistics,
 // b += Kuf g).
 enum { PASS_WHOLE = 0, PASS_EARLY = 1, PASS_REST = 2 };
-inline bool grad_spread_skip(const tsvgp_ctx*) { return false; }
 // y / mean_out / var_out of latent l live at + l * y_stride / + l * out_stride (Y transposed to [L][n_pad]; outputs [L][n_pad_out]).
 // lat_only >= 0 restricts the per-latent work to that latent (the M-step gradient pass runs latent by latent).
 // Separate kernels: latent l's scaled coordinates are at XsT + l * xs_lat, x2 + l * x2_lat, and every latent builds its own slab.
@@ -872,7 +863,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
     if (phase != PASS_REST) OK(ensure_slabs(c, N, grad));
     const long nc = c->chunk;
     const int Mp = c->Mp;
-    const int nstr = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
+    const int nstr = slab_stream_count(c);
     const bool prof = c->profile && mode == MODE_STATS && c->L == 1;
     const int l_lo = lat_only >= 0 ? lat_only : 0, l_hi = lat_only >= 0 ? lat_only + 1 : c->L;
     const bool multi = c->L > 1;
@@ -904,7 +895,6 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             if (stats) {   // every slab stream zeroes its own accumulators (off the main stream, which runs the posterior chain)
                 CU(cudaMemsetAsync(c->stats_all[s], 0, sizeof(double) * c->L * (mm + Mp + 4), c->s_pp[s]));
                 CU(cudaMemsetAsync(c->stats2_all[s], 0, sizeof(double) * c->L * (mm + Mp), c->s_pp[s]));
-                if (c->spread_b) CU(cudaMemsetAsync(c->bacc[s], 0, sizeof(double) * c->L * 2 * (Mp / 128) * Mp, c->s_pp[s]));
                 if (grad) CU(cudaMemsetAsync(c->facc[s], 0, sizeof(double) * (size_t)Mp * c->waug, c->s_pp[s]));
             }
         }
@@ -935,14 +925,10 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             LA(gemm_launch(p, s));
             LA(splitk_reduce_launch(p, s));
         } else {
-            const int ksp = c->balance ? balanced_ksplit(nt * (nt + 1) / 2, ncols) : ncols;
+            const int ksp = balanced_ksplit(nt * (nt + 1) / 2, ncols);
             if (ksp < ncols) { p.ksp = ksp; p.C2 = c->stats2[b]; }
-            if (c->fuse_b && with_b) {   // b += K g rides on the A fragments the SYRK already holds
+            if (with_b) {   // b += K g rides on the A fragments the SYRK already holds
                 p.gvec = c->gbuf[b]; p.bout = c->stats[b] + (size_t)Mp * Mp; p.bout2 = c->stats2[b] + (size_t)Mp * Mp;
-                if (c->spread_b) {   // shared by the tiles of a tile row, one private slot per tile column (summed at the end of the pass)
-                    double* base = c->bacc[b] + (size_t)c->cur * 2 * nt * Mp;
-                    p.bout = base; p.bout2 = base + (size_t)nt * Mp; p.bstride = Mp;
-                }
                 fused_b = true;
             }
             LA(gemm_launch(p, s));
@@ -1168,24 +1154,15 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         CU(cudaEventRecord(c->ev_join[s], c->s_pp[s]));
         CU(cudaStreamWaitEvent(sm, c->ev_join[s], 0));
     }
-    if (stats && c->spread_b && c->fuse_b && !grad_spread_skip(c)) {   // b_l += sum over streams, pieces and tile columns of the private mat-vec slots
-        const int nt = Mp / 128;
-        for (int l = l_lo; l < l_hi; ++l) {
-            select_latent(c, l);
-            for (int s = 0; s < nstr; ++s)
-                LA(sum_rows_into_launch(c->bacc[s] + (size_t)l * 2 * nt * Mp, 2 * nt, Mp, c->stats[0] + mm, sm));
-        }
-    }
     if (stats) {   // the latents' accumulators are contiguous: one launch per pair of buffers sums all of them
-        const long cnt = (long)((l_hi - l_lo) * (mm + Mp + 4)), cnt2 = (long)((l_hi - l_lo) * (mm + Mp));
+        const long cnt = (long)((l_hi - l_lo) * (mm + Mp + 4));
         select_latent(c, l_lo);
         for (int s = 1; s < nstr; ++s) LA(vadd_inplace_launch(c->stats[0], c->stats[s], cnt, sm));
         for (int s = 1; s < nstr && grad; ++s) LA(vadd_inplace_launch(c->facc[0], c->facc[s], (long)Mp * c->waug, sm));
-        for (int l = l_lo; l < l_hi && c->balance; ++l) {
+        for (int l = l_lo; l < l_hi; ++l) {
             select_latent(c, l);
             for (int s = 0; s < nstr; ++s) LA(vadd_inplace_launch(c->stats[0], c->stats2[s], (long)(mm + Mp), sm));
         }
-        (void)cnt2;
         for (int l = l_lo + 1; l < l_hi && one_syrk; ++l)
             CU(cudaMemcpyAsync(c->stats_all[0] + l * (mm + Mp + 4), c->stats_all[0] + l_lo * (mm + Mp + 4), sizeof(double) * mm,
                                cudaMemcpyDeviceToDevice, sm));
@@ -1257,8 +1234,8 @@ int start_k9(tsvgp_ctx* c, double jitter) {
 }
 
 // Both chains of the prepare phase are ~40 dependent small kernels; at small M their GPU time is comparable to the time the host
-// needs to enqueue them, so enqueueing them one after the other delays the second chain by the first one's issue time.  With
-// `async_issue` a helper thread enqueues the K9 chain on the side stream while the calling thread enqueues the posterior chain.
+// needs to enqueue them, so enqueueing them one after the other delays the second chain by the first one's issue time.  Up to
+// M = 1024 a helper thread therefore enqueues the K9 chain on the side stream while the calling thread enqueues the posterior chain.
 struct SideIssue {
     std::thread th;
     int rc = TSVGP_OK;
@@ -1275,7 +1252,7 @@ struct SideIssue {
 int start_k9_async(tsvgp_ctx* c, double jitter, SideIssue& side) {
     if (k9_cached(c, jitter)) return TSVGP_OK;
     OK(k9_fork(c));
-    if (!c->async_issue || c->Mp > 1024) return k9_chain(c, jitter);
+    if (c->Mp > 1024) return k9_chain(c, jitter);
     try {
         side.th = std::thread([c, jitter, &side]() {
             const long l0 = g_launches;
@@ -1853,7 +1830,6 @@ int tsvgp_set_option(tsvgp_ctx* c, const char* name, double value) {
     if (!strcmp(name, "mc_seed")) { c->mc_seed = (unsigned long long)value; c->mc_draw = 0; return TSVGP_OK; }
     if (!strcmp(name, "sample_seed")) { c->sample_seed = (unsigned long long)value; c->sample_draw = 0; return TSVGP_OK; }
     if (!strcmp(name, "speculate")) { c->speculate = value != 0.0; return TSVGP_OK; }
-    if (!strcmp(name, "k9_defer")) { c->k9_defer = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "early_slabs")) { c->early_slabs = value < 0 ? 0 : (int)value; return TSVGP_OK; }
     if (!strcmp(name, "route_cond_max")) { c->route_cond_max = value; return TSVGP_OK; }
     if (!strcmp(name, "route_exact_min")) { c->route_exact_min = value; return TSVGP_OK; }
@@ -1866,10 +1842,6 @@ int tsvgp_set_option(tsvgp_ctx* c, const char* name, double value) {
     if (!strcmp(name, "dist_min_m")) { c->dist_min_m = (int)value; return TSVGP_OK; }
     if (!strcmp(name, "shard_min_m")) { c->shard_min_m = (int)value; return TSVGP_OK; }
     if (!strcmp(name, "split_chains")) { c->split_chains = value != 0.0; return TSVGP_OK; }
-    if (!strcmp(name, "async_issue")) { c->async_issue = value != 0.0; return TSVGP_OK; }
-    if (!strcmp(name, "fuse_b")) { c->fuse_b = value != 0.0; return TSVGP_OK; }
-    if (!strcmp(name, "spread_b")) { c->spread_b = value != 0.0; return TSVGP_OK; }
-    if (!strcmp(name, "balance")) { c->balance = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "profile")) { c->profile = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "cache_factors")) { c->cache_factors = value != 0.0; return TSVGP_OK; }
     if (!strcmp(name, "invalidate")) { c->kuu_valid = c->post_valid = c->kl_valid = c->k9_valid = c->c6_valid = c->wpost_valid = c->wkl_valid = false; return TSVGP_OK; }
@@ -2237,16 +2209,16 @@ int tsvgp_natgrad_step(tsvgp_ctx* c, double lr, double jitter, double scale, dou
             c->route = ROUTE_FUSED;
             join_before = false;
         }
-        // ... and when does it start?  Side by side with the posterior chain the two latency-bound chains slow each other down
-        // (measured at M = 2048: posterior chain 2.6 ms alone, 3.4 ms beside the K9 chain, programmatic launch suspended).  When the
-        // chain is only needed after the pass it therefore starts once the posterior chain is complete and runs under the pass.
+        // ... and when does it start?  At once, on the side stream beside the posterior chain.  The two latency-bound chains slow
+        // each other down (measured at M = 2048: posterior chain 2.6 ms alone, 3.4 ms beside the K9 chain, programmatic launch
+        // suspended), but starting the K9 chain behind the posterior chain, under the pass, was slower still: there every chain
+        // kernel waits for an SM slot (M = 2048, 131 072 rows: 41.1 against 39.9 ms per step).
         // several ranks: the two chains are split over the ranks of a pair and exchanged (chain_split_active)
         const bool split = k9_runs && !join_before && c->sites_set && chain_split_active(c);
         chain_role = split ? chain_role_of(c) : ROLE_BOTH;
         const bool k9_here = chain_role == ROLE_BOTH || chain_role == ROLE_K9, post_here = chain_role == ROLE_BOTH || chain_role == ROLE_POSTERIOR;
-        const bool defer_k9 = k9_runs && !join_before && c->k9_defer && c->Mp >= 2048 && !split;
-        if (c->Mp >= 2048 && k9_runs && !defer_k9 && !split) g_pdl_suspended = 1;   // two concurrent chains of large kernels: see common.cuh
-        if (!defer_k9 && k9_here) rc = start_k9_async(c, jitter, side);
+        if (c->Mp >= 2048 && k9_runs && !split) g_pdl_suspended = 1;   // two concurrent chains of large kernels: see common.cuh
+        if (k9_here) rc = start_k9_async(c, jitter, side);
         if (rc == TSVGP_OK && !k9_runs) rc = choose_route(c, jitter);   // cached factors: the route is known at once
         c->n_early = 0;
         // split chains: no early slabs on the rank that builds the posterior factors — every rank waits for that chain
@@ -2260,7 +2232,6 @@ int tsvgp_natgrad_step(tsvgp_ctx* c, double lr, double jitter, double scale, dou
             if (!post_here && c->n_early > 0) CU(cudaStreamWaitEvent(s, c->ev_early0, 0));
             rc = exchange_posterior(c, elbo_before != nullptr);   // rank 0: behind its chain; the others receive
         }
-        if (rc == TSVGP_OK && defer_k9) rc = start_k9(c, jitter);   // forks from the main stream HERE: behind the posterior chain
         side.join_into(g_launches);
         if (rc != TSVGP_OK) return rc;
         if (side.rc != TSVGP_OK) return side.rc;
@@ -2306,8 +2277,7 @@ int tsvgp_natgrad_step(tsvgp_ctx* c, double lr, double jitter, double scale, dou
     cudaEventElapsedTime(&ms, c->ev[EV_T0], c->ev[EV_DENSE]);
     c->timings[0] = ms;
     {
-        const int nstr_t = c->profile ? 1 : (c->n_streams < 1 ? 1 : (c->n_streams > MAXS ? MAXS : c->n_streams));
-        const long ncu_t = used_chunk(c, c->N, c->chunk, nstr_t);
+        const long ncu_t = used_chunk(c, c->N, c->chunk, slab_stream_count(c));
         c->timings[5] = (double)((c->N + ncu_t - 1) / ncu_t);
     }
     c->timings[6] = (double)(g_launches - launches0);

@@ -143,18 +143,39 @@ def test_header_is_plain_c_and_the_c_example_links():
             assert run.returncode != 0 and "no CUDA device" in run.stderr
 
 
+def _header_option_comment():
+    # the comment block of include/tsvgp.h that documents tsvgp_set_option: (the options, its Environment paragraph)
+    header = open(HEADER).read()
+    start = header.index("/* options:")
+    block = header[start:header.index("*/", start)]
+    return block[:block.index("Environment")], block[block.index("Environment"):]
+
+
 def test_every_library_option_is_documented_in_the_header():
-    # tsvgp_set_option(name, value): the names the library accepts (csrc/tsvgp.cu) and the names include/tsvgp.h documents
-    import re
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    src = open(os.path.join(root, "t-svgp_b200", "csrc", "tsvgp.cu")).read()
+    # tsvgp_set_option(name, value): the names the library accepts (csrc/tsvgp.cu) and the names the header's option comment
+    # documents, in both directions
+    src = open(os.path.join(ROOT, "t-svgp_b200", "csrc", "tsvgp.cu")).read()
     body = src[src.index("int tsvgp_set_option("):src.index("int tsvgp_set_kernel(")]
     accepted = set(re.findall(r'strcmp\(name, "([a-z_0-9]+)"\)', body))
-    header = open(os.path.join(root, "include", "tsvgp.h")).read()
-    documented = set(re.findall(r'"([a-z_0-9]+)"', header))
+    documented = set(re.findall(r'"([a-z_0-9]+)"', _header_option_comment()[0]))
     assert accepted, "no options found in tsvgp_set_option"
+    assert documented, "no options found in the header's option comment"
     internal = {"profile"}   # measurement switch behind tsvgp_get_kernel_profile, described there
     assert accepted - internal <= documented, sorted(accepted - internal - documented)
+    assert documented <= accepted, sorted(documented - accepted)
+
+
+def test_every_environment_variable_is_documented_in_the_header():
+    # every getenv("TSVGP_...") of the library is named in the Environment paragraph of the header's option comment, and
+    # every name there is read
+    csrc = os.path.join(ROOT, "t-svgp_b200", "csrc")
+    read = set()
+    for fn in os.listdir(csrc):
+        if fn.endswith(".cu"):
+            read |= set(re.findall(r'getenv\("(TSVGP_[A-Z0-9_]+)"\)', open(os.path.join(csrc, fn)).read()))
+    documented = set(re.findall(r"\b(TSVGP_[A-Z0-9_]+)", _header_option_comment()[1]))
+    assert read, "no getenv(\"TSVGP_...\") found in t-svgp_b200/csrc"
+    assert read == documented, (sorted(read - documented), sorted(documented - read))
 
 
 def test_weighted_shards_and_balance_weights():

@@ -1,4 +1,4 @@
-// Tooling: times the 128x128 diagonal-block kernels (Cholesky + inverse, inverse alone) and the blocked chol_lower / trtri_lower.
+// Tooling: times the 128x128 diagonal-block kernel (Cholesky + inverse) and the blocked chol_lower / trtri_lower.
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
@@ -8,7 +8,7 @@
 #include "../t-svgp_b200/csrc/dense.cuh"
 #include "../t-svgp_b200/csrc/gemm.cuh"
 #include "../t-svgp_b200/csrc/common.cuh"
-namespace tsvgp { thread_local long g_launches = 0; int g_debug_sync = 0; int g_pdl = 1; thread_local int g_pdl_suspended = 0; int diag_read_stamps(long long* out32); }
+namespace tsvgp { thread_local long g_launches = 0; int g_debug_sync = 0; int g_pdl = 1; thread_local int g_pdl_suspended = 0; }
 using namespace tsvgp;
 #define CK(x) do { cudaError_t e = (x); if (e != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e), __FILE__, __LINE__); exit(1);} } while (0)
 int main(int argc, char** argv) {
@@ -20,19 +20,14 @@ int main(int argc, char** argv) {
     CK(cudaMalloc(&dA, sizeof(double) * n * n)); CK(cudaMalloc(&dW, sizeof(double) * n * n)); CK(cudaMalloc(&dLinv, sizeof(double) * n * n));
     CK(cudaMalloc(&tmp, sizeof(double) * n * n)); CK(cudaMalloc(&dinv, sizeof(double) * (n / 128) * 128 * 128)); CK(cudaMalloc(&info, 16)); CK(cudaMemset(info, 0, 16)); CK(cudaMemset(dinv, 0, sizeof(double) * (n / 128) * 128 * 128));
     CK(cudaMemcpy(dA, A.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
-    double* ws; const size_t ws_doubles = (size_t)4 << 20; CK(cudaMalloc(&ws, sizeof(double) * ws_doubles)); CK(cudaMemset(ws, 0, sizeof(double) * ws_doubles));   // split-K workspace (gemm_launch_auto)
+    double* ws; const size_t ws_doubles = ((size_t)4 << 20) - 2048; CK(cudaMalloc(&ws, sizeof(double) * ws_doubles));   // split-K workspace (gemm_launch_auto), the library's size
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1); float ms;
-    for (int vv = 0; vv < 5; ++vv) {   // 0: per-pivot; 1, 2: blocked / blocked + look-ahead with the round-1 pivot loop; 3, 4: the same with the pipelined pivot chain
-        const int variant = vv < 3 ? vv : vv - 2;
-        diag_set_variant(variant);
-        diag_set_fast(vv >= 3);
-        printf("-- pivot chain: %s\n", vv >= 3 ? "pipelined + Newton rsqrt [r02]" : "round-1 loop");
-        for (int rep = 0; rep < 3; ++rep) {
-            CK(cudaMemcpy(dW, dA, sizeof(double) * n * n, cudaMemcpyDeviceToDevice));
-            cudaEventRecord(e0); diag_potrf_inv_launch(dW, n, dinv, 0, info, 0); cudaEventRecord(e1); CK(cudaEventSynchronize(e1));
-            cudaEventElapsedTime(&ms, e0, e1); printf("diag_potrf_inv variant %d (%s, 1 block): %.1f us\n", variant, variant == 2 ? "blocked DMMA + look-ahead" : (variant ? "blocked DMMA" : "per-pivot"), ms * 1e3);
-        }
-        // the block against a host Cholesky + inverse
+    for (int rep = 0; rep < 3; ++rep) {
+        CK(cudaMemcpy(dW, dA, sizeof(double) * n * n, cudaMemcpyDeviceToDevice));
+        cudaEventRecord(e0); diag_potrf_inv_launch(dW, n, dinv, 0, info, 0); cudaEventRecord(e1); CK(cudaEventSynchronize(e1));
+        cudaEventElapsedTime(&ms, e0, e1); printf("diag_potrf_inv (1 block): %.1f us\n", ms * 1e3);
+    }
+    {   // the block against a host Cholesky + inverse
         std::vector<double> Lb(128 * 128), Xb(128 * 128), Lh(128 * 128, 0.0);
         CK(cudaMemcpy2D(Lb.data(), 128 * 8, dW, (size_t)n * 8, 128 * 8, 128, cudaMemcpyDeviceToHost));
         CK(cudaMemcpy(Xb.data(), dinv, sizeof(double) * 128 * 128, cudaMemcpyDeviceToHost));
@@ -55,36 +50,17 @@ int main(int argc, char** argv) {
                 eX = fmax(eX, fabs(u - (i == j ? 1.0 : 0.0)));
                 if (j > i) eU = fmax(eU, fabs(Xb[i * 128 + j]));
             }
-        printf("  variant %d: max |L - L_host| %.2e   max |X L_host - I| %.2e   max |upper of X| %.2e\n", variant, eL, eX, eU);
+        printf("  max |L - L_host| %.2e   max |X L_host - I| %.2e   max |upper of X| %.2e\n", eL, eX, eU);
     }
-    {   // phase stamps of the blocked kernel (cycles of thread 0): load | per step j: factor, panel, trailing | store
-        long long clk[32];
-        CK((cudaError_t)tsvgp::diag_read_stamps(clk));
-        printf("  blocked kernel cycles: load %lld", clk[1] - clk[0]);
-        long long prev = clk[1];
-        for (int j = 0; j < 4; ++j) {
-            printf(" | j=%d factor %lld panel %lld", j, clk[2 + 3 * j] - prev, clk[3 + 3 * j] - clk[2 + 3 * j]);
-            prev = clk[3 + 3 * j];
-            if (j < 3) { printf(" trailing %lld", clk[4 + 3 * j] - clk[3 + 3 * j]); prev = clk[4 + 3 * j]; }
-        }
-        printf(" | store %lld | total %lld\n", clk[14] - prev, clk[14] - clk[0]);
-    }
-    for (int variant = 0; variant < 3; ++variant) {   // failure reporting: a non-positive pivot at row 70 of block 3
-        diag_set_variant(variant);
+    {   // failure reporting: a non-positive pivot at row 70 of block 3
         std::vector<double> Bad(128 * 128, 0.0);
         for (int i = 0; i < 128; ++i) Bad[i * 128 + i] = i == 70 ? -1.0 : 2.0;
         CK(cudaMemcpy2D(dW, (size_t)n * 8, Bad.data(), 128 * 8, 128 * 8, 128, cudaMemcpyHostToDevice));
         CK(cudaMemset(info, 0, 16));
         diag_potrf_inv_launch(dW, n, dinv, 3, info, 0);
         int h; CK(cudaMemcpy(&h, info, 4, cudaMemcpyDeviceToHost));
-        printf("  variant %d: failing pivot reported %d (expected %d)\n", variant, h, 3 * 128 + 71);
+        printf("  failing pivot reported %d (expected %d)\n", h, 3 * 128 + 71);
         CK(cudaMemset(info, 0, 16));
-    }
-    diag_set_variant(argc > 2 ? atoi(argv[2]) : 1);
-    diag_set_fast(argc > 3 ? atoi(argv[3]) : 1);
-    for (int rep = 0; rep < 2; ++rep) {
-        cudaEventRecord(e0); diag_trtri_launch(dW, n, dinv, 1, 0); cudaEventRecord(e1); CK(cudaEventSynchronize(e1));
-        cudaEventElapsedTime(&ms, e0, e1); printf("diag_trtri (1 block): %.1f us\n", ms * 1e3);
     }
     for (int rep = 0; rep < 3; ++rep) {
         CK(cudaMemcpy(dW, dA, sizeof(double) * n * n, cudaMemcpyDeviceToDevice));
