@@ -120,7 +120,7 @@ TSVGP_API int tsvgp_set_inducing(tsvgp_ctx* ctx, const double* Z, int M, int D, 
  * product, the weighted SYRK and the site update run per latent.  Layouts follow the reference: lambda_1 [M, L], lambda_2_sqrt
  * [L, M, M], Y [N, L] (independent likelihood terms, summed over the latent axis) or [N, 1] class labels (Softmax), predictive
  * moments [N, L].  Resets the sites and drops the resident data.  The whitened sibling (option "white") takes any L too — Lambda_2
- * [L, M, M], tsvgp_white.py:79-89 — except with the Softmax likelihood.                                                          */
+ * [L, M, M], tsvgp_white.py:79-89 — the Softmax likelihood included (variance gradient unclipped, as tsvgp_white.py:183-212).   */
 TSVGP_API int tsvgp_set_num_latent(tsvgp_ctx* ctx, int L);
 TSVGP_API int tsvgp_num_latent(const tsvgp_ctx* ctx);
 /* TSVGP_LIK_SOFTMAX (gpflow.likelihoods.Softmax, docs/notebooks/mnist.py:117-122): set_likelihood with p0 = number of classes
@@ -167,8 +167,8 @@ TSVGP_API int tsvgp_prior_kl(tsvgp_ctx* ctx, double* out);
  * Gradients are w.r.t. the constrained (natural) parameter values; Zero mean function; any D; one kernel shared by the
  * latents.  Softmax: the derivatives of the Monte-Carlo sum for the call's draws (one per call, see tsvgp_set_mc_epsilon),
  * with h = d ve / d var unclipped; one pass over the data for all latents.  The whitened sibling (option "white") holds its
- * own sites fixed, lambda_1 and the full Lambda_2, and runs one pass per latent like the plain model (DESIGN 10).  Collective
- * with several ranks.  Not built for the heteroskedastic likelihood or separate kernels per latent (TSVGP_ERR_INVALID).    */
+ * own sites fixed, lambda_1 and the full Lambda_2, and runs one pass per latent like the plain model, or with Softmax one pass
+ * over all latents (DESIGN 10).  Collective with several ranks.  Not built for the heteroskedastic likelihood or separate kernels per latent (TSVGP_ERR_INVALID).    */
 TSVGP_API int tsvgp_elbo_grad(tsvgp_ctx* ctx, double scale, double* elbo, double* d_variance, double* d_lengthscales,
                               double* d_Z, double* d_lik);
 /* base_SVGP.predict_f, full_cov = False (tsvgp.py:97-114): mean_out, var_out [N, L]                                     */
@@ -187,7 +187,8 @@ TSVGP_API int tsvgp_predict_f_samples(tsvgp_ctx* ctx, const double* Xnew, int64_
                                       int full_cov, const double* eps, double* samples_out);
 /* t_SVGP_white.predict_f_extra_data (tsvgp_white.py:134-158; whitened sibling only): predictions at Xnew after conditioning the
  * current sites on the RESIDENT minibatch (the "extra data") without changing them; jitter is the reference's argument
- * (default gpflow default_jitter = 1e-6; its test passes 0).  mean_out, var_out [N, L].                                   */
+ * (default gpflow default_jitter = 1e-6; its test passes 0).  mean_out, var_out [N, L].  Softmax: the conditioning evaluates
+ * the likelihood once, with one Monte-Carlo draw (see tsvgp_set_mc_epsilon).                                              */
 TSVGP_API int tsvgp_predict_f_extra_data(tsvgp_ctx* ctx, const double* Xnew, int64_t N, int D, const double* mean_X, double jitter,
                                          double* mean_out, double* var_out);
 /* t_SVGP.get_mean_chol_cov_inducing_posterior (tsvgp.py:202-212): m [M, L], chol_S [L, M, M]                           */

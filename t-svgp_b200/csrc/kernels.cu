@@ -400,13 +400,18 @@ __global__ void __launch_bounds__(128) softmax_stats_kernel(SoftmaxArgs a) {
         double mu[MAX_SOFTMAX_CLASSES], sd[MAX_SOFTMAX_CLASSES], gm[MAX_SOFTMAX_CLASSES], gs[MAX_SOFTMAX_CLASSES];
         bool bad = false;
         const double off = a.mean_off ? a.mean_off[c] : 0.0;
+        double qs = 0.0;
+        if (a.q_shared)
+            for (int p = 0; p < a.n_q_part; ++p) qs += a.q_shared[(long)p * a.ldq + c];
+        if (a.x2) bad = !isfinite(a.x2[c]);
         for (int l = 0; l < a.L; ++l) {
             double m = 0.0, q = 0.0;
             for (int p = 0; p < a.n_mu_part; ++p) m += a.mu_part[l * a.mu_lat + (long)p * a.ldmu + c];
             for (int p = 0; p < a.n_q_part; ++p) q += a.q_part[l * a.q_lat + (long)p * a.ldq + c];
-            const double var = a.kdiag[l] - q;
+            // (the whitened sibling rounds as point_stats_kernel does: k(x,x) - (|LA^-1 k|^2 - |LR_l^-1 k|^2), util.py:83-85)
+            const double var = a.q_shared ? a.kdiag[l] - (qs - q) : a.kdiag[l] - q;
             mu[l] = m + off;
-            bad = bad || !(var > 0.0);
+            bad = bad || !(var > 0.0) || (a.x2 && !isfinite(mu[l]));
             sd[l] = sqrt(var);
             gm[l] = 0.0; gs[l] = 0.0;
             if (valid && a.mean_out) { a.mean_out[l * a.out_lat + c] = mu[l]; a.var_out[l * a.out_lat + c] = var; }

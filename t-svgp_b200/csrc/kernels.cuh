@@ -71,6 +71,12 @@ struct SoftmaxArgs {
     unsigned long long seed, draw;
     int clip = 1;                   // clip h_l at -1e-8 (natgrad_step); the ELBO gradient does not (heteroskedastic: always clipped)
     double* aux_blocks = nullptr;   // out (Softmax M-step): per 256 points [sum h over points and latents, 0], as PointArgs
+    // whitened sibling (Softmax only): partial |LA^-1 k|^2 [n_q_part][ldq], one set shared by the latents and SUBTRACTED, while
+    // the per-latent q_part (|LR_l^-1 k|^2) are ADDED: var_l = k(x,x) - (|LA^-1 k|^2 - |LR_l^-1 k|^2).  Null: var_l = k(x,x) - q_l
+    const double* q_shared = nullptr;
+    // [ncols] squared norms of the scaled points (chunk-local), or null.  Given, a point whose norm or any mean is not finite raises
+    // the flag: the covariance clamps a NaN distance to a finite k, so such a point can leave every var_l finite and positive
+    const double* x2 = nullptr;
 };
 int softmax_stats_launch(const SoftmaxArgs& a, cudaStream_t s);
 // Heteroskedastic Normal likelihood over L = 2 latents (GPflow HeteroskedasticTFPConditional(Normal, scale_transform) with its

@@ -815,15 +815,16 @@ int ensure_slabs(tsvgp_ctx* c, long n_points, bool need_grad = false) {
         if (c->fsplit < 1) c->fsplit = 1;
         const size_t W = (size_t)c->waug;
         // U of every latent survives until the joint point kernel has run: L Mp nc doubles per slab stream; the whitened sibling
-        // keeps one more Mp x nc slab per stream (LA^-1 K)
+        // keeps one more Mp x nc slab per stream (LA^-1 K), with Softmax (2 + L + 1) Mp x nc slabs per stream in all
         if (u_lat > 1 || need_a) {
             const size_t need = ((size_t)(2 + u_lat + (need_a ? 1 : 0)) * c->Mp * nc + nc * W + (size_t)(c->fsplit + 1) * c->Mp * W) * ns + 2 * ve_need;
             size_t free_b = 0, total_b = 0;
             CU(cudaMemGetInfo(&free_b, &total_b));
             if (need * sizeof(double) > free_b) {
                 if (need_a)
-                    FAIL(TSVGP_ERR_INVALID, "elbo_grad of the whitened sibling at M = %d needs %zu bytes of device memory for its slab "
-                         "workspace, %zu are free (option \"chunk\" narrows the slabs)", c->M, need * sizeof(double), free_b);
+                    FAIL(TSVGP_ERR_INVALID, "elbo_grad of the whitened sibling%s at M = %d needs %zu bytes of device memory for its slab "
+                         "workspace, %zu are free (option \"chunk\" narrows the slabs)", u_lat > 1 ? " with coupled latents" : "", c->M,
+                         need * sizeof(double), free_b);
                 FAIL(TSVGP_ERR_INVALID, "elbo_grad with %d coupled latents at M = %d needs %zu bytes of device memory for its slab workspace, "
                      "%zu are free (option \"chunk\" narrows the slabs)", c->L, c->M, need * sizeof(double), free_b);
             }
@@ -1016,6 +1017,27 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
                     if (grad) { p.C = which == 0 ? c->aslab[b] : c->vslab[b]; p.ldc = nc; }
                     LA(gemm_launch(p, s));
                 }
+                if (grad && joint) {   // U_l = LA^-T (LA^-1 K) - LR_l^-T (LR_l^-1 K) now, into latent l's own U slab: V is
+                    // overwritten by the next latent.  W0 = LA^-T (LA^-1 K) does not depend on the latent: it is formed once, into
+                    // U_0, and copied to the other latents' slabs before U_0 is updated; each U_l then takes the bits the
+                    // independent pass below gives it (the same two products, the second with alpha = -1, beta = 1)
+                    const size_t us = (size_t)Mp * nc;
+                    if (l == l_lo) {
+                        GemmP w;
+                        w.A = c->C6inv; w.lda = Mp; w.a_kc = 0; w.a_tri = 2;
+                        w.B = c->aslab[b]; w.ldb = nc; w.b_kc = 0;
+                        w.C = c->uslab[b]; w.ldc = nc; w.m = Mp; w.n = ncols; w.k = Mp;
+                        LA(gemm_launch(w, s));
+                        for (int k = l_lo + 1; k < l_hi; ++k)
+                            CU(cudaMemcpy2DAsync(c->uslab[b] + k * us, sizeof(double) * nc, c->uslab[b], sizeof(double) * nc,
+                                                 sizeof(double) * ncols, Mp, cudaMemcpyDeviceToDevice, s));
+                    }
+                    GemmP u;
+                    u.A = c->T; u.lda = Mp; u.a_kc = 0; u.a_tri = 2;
+                    u.B = c->vslab[b]; u.ldb = nc; u.b_kc = 0;
+                    u.C = c->uslab[b] + l * us; u.ldc = nc; u.m = Mp; u.n = ncols; u.k = Mp; u.alpha = -1.0; u.beta = 1.0;
+                    LA(gemm_launch(u, s));
+                }
             }
             mark(s);
             if (!joint) {   // (c) marginals -> likelihood expectations and gradients, latent by latent (independent likelihood terms)
@@ -1043,6 +1065,10 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             SoftmaxArgs a;
             a.mu_part = c->mu_part[b]; a.n_mu_part = Mp / 64; a.ldmu = nc; a.mu_lat = (long)(Mp / 64) * nc;
             a.q_part = c->q_part[b]; a.n_q_part = Mp / 128; a.ldq = nc; a.q_lat = (long)(Mp / 128) * nc;
+            // whitened sibling: - |LA^-1 k|^2 + |LR_l^-1 k|^2, and a non-finite point raises the flag as the reference's
+            // predict_f raises on its NaN variance (the plain model's Softmax pass keeps its behaviour)
+            a.q_shared = c->white ? c->q2_part[b] : nullptr;
+            a.x2 = c->white ? x2 + n0 : nullptr;
             a.L = c->L; a.S = c->lik.n_gh;
             a.y = y ? y + n0 : nullptr;
             a.mean_off = mean_off ? mean_off + n0 : nullptr;
@@ -1054,7 +1080,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
             a.flags = c->flags;
             a.eps = (c->mc_eps && c->mc_eps_n == N) ? c->mc_eps : nullptr;
             a.seed = c->mc_seed; a.draw = c->mc_draw;
-            a.clip = grad ? 0 : 1;   // the ELBO gradient takes h unclipped
+            a.clip = (grad || c->white) ? 0 : 1;   // the ELBO gradient takes h unclipped, and so does tsvgp_white.py:183-212
             a.aux_blocks = grad ? c->aux_blocks + 2 * ci * vstride : nullptr;
             if (c->lik.kind == LIK_HETEROSKEDASTIC) LA(heteroskedastic_stats_launch(c->lik, a, c->gh, s));
             else LA(softmax_stats_launch(a, s));
@@ -1097,7 +1123,7 @@ int stream_pass(tsvgp_ctx* c, const double* XsT, long ldx, const double* x2, lon
         }
         if (grad) {
             select_latent(c, l_lo);
-            if (c->white) {   // U = Q K = LA^-T (LA^-1 K) - LR^-T (LR^-1 K)  (two upper-triangular products over the stored slabs)
+            if (c->white && !joint) {   // U = Q K = LA^-T (LA^-1 K) - LR^-T (LR^-1 K)  (two upper-triangular products over the stored slabs)
                 for (int which = 0; which < 2; ++which) {
                     GemmP p;
                     p.A = which == 0 ? c->C6inv : c->T; p.lda = Mp; p.a_kc = 0; p.a_tri = 2;
@@ -2171,7 +2197,6 @@ static int require_model(tsvgp_ctx* c, bool need_data) {
     if (need_data && !c->X) FAIL(TSVGP_ERR_STATE, "no data resident (tsvgp_set_data)");
     if (c->lik.kind == LIK_SOFTMAX && (int)c->lik.p0 != c->L)
         FAIL(TSVGP_ERR_INVALID, "Softmax with %d classes needs num_latent_gps = %d (tsvgp_set_num_latent), not %d", (int)c->lik.p0, (int)c->lik.p0, c->L);
-    if (c->white && c->lik.kind == LIK_SOFTMAX) FAIL(TSVGP_ERR_INVALID, "the whitened sibling model is not built for the Softmax likelihood");
     if (c->lik.kind == LIK_HETEROSKEDASTIC && c->L != 2)
         FAIL(TSVGP_ERR_INVALID, "the heteroskedastic likelihood needs num_latent_gps = 2 (loc, scale), not %d", c->L);
     if (c->white && c->lik.kind == LIK_HETEROSKEDASTIC)
@@ -2546,7 +2571,8 @@ static int elbo_grad_coupled(tsvgp_ctx* c, double scale, const std::vector<doubl
     double e_sum = 0.0, dv_sum = 0.0, dl_sum = 0.0;
     for (int l = 0; l < c->L; ++l) {
         double e = 0.0, dv = 0.0, dl = 0.0;
-        OK(grad_epilogue(c, l, scale, &e, &dv, &dl, Fuu));
+        if (c->white) OK(grad_epilogue_white(c, l, scale, &e, &dv, &dl, Fuu));
+        else OK(grad_epilogue(c, l, scale, &e, &dv, &dl, Fuu));
         if (l == 0) Fuu_sum = Fuu;
         else for (size_t i = 0; i < Fuu.size(); ++i) Fuu_sum[i] += Fuu[i];
         e_sum += e; dv_sum += dv; dl_sum += dl;
@@ -2864,6 +2890,7 @@ int tsvgp_predict_f_extra_data(tsvgp_ctx* c, const double* Xnew, int64_t N, int 
         double tail[4];
         int info_h[N_INFO];
         OK(read_tails(c, tail, nullptr, info_h));
+        ++c->mc_draw;   // Softmax: the pass above evaluated the likelihood once, with one Monte-Carlo draw
         OK(check_info(c, info_h));
         if (tail[1] != 0.0) FAIL(TSVGP_ERR_NONPOSITIVE_VARIANCE, "predict_f_extra_data: non-positive predictive variance at the extra data");
     }

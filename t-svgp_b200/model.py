@@ -578,7 +578,8 @@ class t_SVGP_white(t_SVGP):
     (`lambda_2 [1, M, M]`, default 1e-10 I), updated without any factorisation:
         lambda_1 <- (1-lr) lambda_1 + lr s K (G1 - 2 G2 mZ) ;  Lambda_2 <- (1-lr) Lambda_2 - 2 lr s K G2 K.
     Same constructor / natgrad_step / elbo / predict_f / prior_kl / get_mean_chol_cov_inducing_posterior surface
-    (+ `predict_f_extra_data`; any num_latent_gps with Gaussian / Bernoulli / StudentT).  `elbo_and_grad` returns the M-step
+    (+ `predict_f_extra_data`; any num_latent_gps with Gaussian / Bernoulli / StudentT, and Softmax(C) with num_latent_gps = C and
+    Y [N, 1] class labels, one Monte-Carlo draw per call that evaluates the likelihood).  `elbo_and_grad` returns the M-step
     objective and its hyperparameter gradients with lambda_1 and Lambda_2 held fixed, so `vem.fit` trains this model as it trains
     `t_SVGP`."""
 
@@ -588,8 +589,8 @@ class t_SVGP_white(t_SVGP):
             lambda_2 = np.asarray(lambda_2, dtype=np.float64)
             assert lambda_2.ndim == 3  # tsvgp_white.py:87
             num_latent_gps = lambda_2.shape[0]
-        if _coupled(likelihood):
-            raise NotImplementedError(f"t_SVGP_white with the {type(likelihood).__name__} likelihood")
+        if type(likelihood).__name__ == "HeteroskedasticTFPConditional":
+            raise NotImplementedError("t_SVGP_white with the HeteroskedasticTFPConditional likelihood")
         if _separate(kernel):
             raise NotImplementedError("t_SVGP_white with SeparateIndependent kernels")
         super().__init__(kernel, likelihood, inducing_variable, mean_function=mean_function, num_latent_gps=num_latent_gps,
